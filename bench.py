@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- audio-seconds synthesised per wall-second on the VISinger inference hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--precision bf16|fp32] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--precision bf16|fp32] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (models/visinger.py:107-111 of the reference: prior sampling ->
 ResidualCouplingBlock reverse -> HiFi-GAN Generator) over one batch of synthetic input: B=16 utterances
@@ -71,7 +71,30 @@ def parse():
     ap.add_argument("--no-full-model", action="store_true", help="skip the 64-utterance full-model leg (configs[3])")
     ap.add_argument("--no-chain-streams", action="store_true", help="run the resblock chains of a stage one after the other")
     ap.add_argument("--two-streams", action="store_true", help="store raw and activated copies of the resblock stream")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of `arrays` as out_dir/<name>.npy in float32.  Should they hold more than DUMP_BYTES in all,
+    each is cut to the same fraction of its elements: a fixed sample (seed 0) of its flat indices, in index order, 1-D."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BYTES - 4096 * len(arrays)           # room for the .npy headers
+    for name, a in arrays.items():
+        if total > budget:
+            idx = np.random.default_rng(0).choice(a.size, a.size * budget // total, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -201,8 +224,10 @@ def run_reference(args, rank):
     hp, inputs = bench_weights_and_inputs(args.batch, Ts)
     cpu = CpuHotPath(hp.state_dict())
     one = [t[:1].contiguous() for t in inputs]
-    times, _ = cpu_hot_path_time(cpu, one, args.warmup + args.steps, cores)
+    times, (wav, z_q) = cpu_hot_path_time(cpu, one, args.warmup + args.steps, cores)
     times = times[args.warmup:]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"wav": wav, "z_q": z_q})
     audio = Ts * FRAME_SEC
     tot = sum(times)
     val = audio * len(times) / tot
@@ -431,11 +456,13 @@ def main():
         for dst, src in zip((graph.mu_p, graph.logs_p, graph.noise, graph.mask, graph.g), devin):
             dst.copy_(src)
 
+    last = {}                  # (wav, z_q) of the latest resident step, for --dump-outputs
+
     def step_resident():
         if graph is not None:
-            graph.replay()
+            last["out"] = graph.replay()
         else:
-            hp.infer(*devin)
+            last["out"] = hp.infer(*devin)
 
     # e2e: the public serving loop (HotPath.pipeline): every step uploads its inputs from pinned host memory and
     # downloads its waveform into pinned host memory; copies of neighbouring steps overlap the kernels (3 streams)
@@ -470,6 +497,8 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     ms = timed(step_resident, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("wav", "z_q"), last["out"])))
     for _ in range(3):
         step_e2e()
     ms_e2e = timed(step_e2e, args.steps, after=pipe.flush if pipe is not None else None)

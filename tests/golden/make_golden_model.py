@@ -32,6 +32,7 @@ from models.visinger import VISinger  # noqa: E402  (reference)
 from modules.visinger import encoder as ref_encoder  # noqa: E402
 
 from model_inputs import SMALL_HPARAMS, synth_utterances  # noqa: E402
+from helpers import save_npz_parts  # noqa: E402
 
 torch.set_grad_enabled(False)
 
@@ -75,9 +76,10 @@ def main():
     # training-only modules (posterior encoder, CTC phoneme head) are not needed to reproduce forward(infer=True)
     sd = {k: v.numpy() for k, v in model.state_dict().items()
           if not k.startswith(("posterior_encoder.", "phoneme_predictor."))}
-    np.savez_compressed(os.path.join(HERE, "small_model.npz"), noise=noise.numpy(), wav_out=out["wav_out"].numpy(),
-                        f0_pred=out["f0_pred"].numpy(), mu_p=mu_p.numpy(), logs_p=logs_p.numpy(),
-                        **{"in/" + k: v.numpy() for k, v in batch.items()}, **{"w/" + k: v for k, v in sd.items()})
+    save_npz_parts("small_model", dict(noise=noise.numpy(), wav_out=out["wav_out"].numpy(), f0_pred=out["f0_pred"].numpy(),
+                                       mu_p=mu_p.numpy(), logs_p=logs_p.numpy(),
+                                       **{"in/" + k: v.numpy() for k, v in batch.items()},
+                                       **{"w/" + k: v for k, v in sd.items()}))
     print("wav_out", tuple(out["wav_out"].shape), "|wav|max", float(out["wav_out"].abs().max()),
           "mu_p", tuple(mu_p.shape), "params", sum(v.size for v in sd.values()))
 

@@ -7,7 +7,7 @@ longest), from the unmodified reference model.  Run in the build container only:
 The 60.9 M weights are not stored: they are the seeded state dict of tests/model_inputs.py::full_model_mirror, loaded
 into the reference through its own load_state_dict (strict).  The fixture keeps outputs only: the waveform at a stride,
 the last 20 frames of every utterance and the PADDED region after it in full (the decoder is unmasked,
-models/visinger.py:111, so the reference's waveform is non-zero there and must be matched), f0_pred, mu_p / logs_p strided.
+models/visinger.py:111, so the reference's waveform is non-zero there and must be matched) and f0_pred.
 Oracle patches as in make_golden_model.py (SURVEY.md 8c)."""
 import os
 import sys
@@ -31,8 +31,7 @@ sys.modules["utils.audio"] = pkg
 from models.visinger import VISinger  # noqa: E402  (reference)
 from modules.visinger import encoder as ref_encoder  # noqa: E402
 
-from model_inputs import (full_hparams, full_model_mirror, full_model_batch, FULL_GOLDEN_WAV_STRIDE,  # noqa: E402
-                          FULL_GOLDEN_T_STRIDE)
+from model_inputs import full_hparams, full_model_mirror, full_model_batch, FULL_GOLDEN_WAV_STRIDE  # noqa: E402
 
 torch.set_grad_enabled(False)
 HOP = 300
@@ -59,13 +58,6 @@ def main():
                     spk_id=batch["spk_ids"], infer=True)
     finally:
         torch.randn_like = real
-    mask = (batch["mel2ph"] > 0).float().unsqueeze(1)
-    prior_inp = model.text_encoder(batch["text_tokens"], batch["note_pitch"], batch["note_dur"], batch["mel2ph"]) * mask
-    pos = model.embed_positions(prior_inp.shape[0], prior_inp.shape[2], prior_inp.transpose(1, 2)[..., 0])
-    prior_inp = prior_inp + pos.transpose(1, 2)
-    spk = model.speaker_embedding(None, batch["spk_ids"]).transpose(1, 2)
-    cond = model.forward_pitch(prior_inp, None, None, spk, mask, {})
-    mu_p, logs_p = model.frame_prior(prior_inp, mask, cond)
     wav = out["wav_out"]
     T = batch["mel2ph"].shape[1]
     tails, pads = [], []
@@ -75,8 +67,7 @@ def main():
         pads.append(np.pad(seg, (0, 10 * HOP - len(seg))))
     np.savez_compressed(os.path.join(HERE, "full_model.npz"), lengths=lengths, T=T,
                         wav_strided=wav[:, ::FULL_GOLDEN_WAV_STRIDE].numpy(), wav_tails=np.stack(tails),
-                        wav_pads=np.stack(pads), f0_pred=out["f0_pred"].numpy(),
-                        mu_p=mu_p[:, :, ::FULL_GOLDEN_T_STRIDE].numpy(), logs_p=logs_p[:, :, ::FULL_GOLDEN_T_STRIDE].numpy())
+                        wav_pads=np.stack(pads), f0_pred=out["f0_pred"].numpy())
     print("lengths", lengths.tolist(), "T", T, "wav", tuple(wav.shape), "|wav|max", float(wav.abs().max()),
           "|pad region|max", float(np.abs(np.stack(pads)).max()))
 

@@ -16,6 +16,41 @@ def load_npz(name):
     return np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
 
 
+PART_BYTES = 800_000        # array bytes per fixture file: random float32 weights barely compress, and files stay < 1 MB
+
+
+def _part_path(name, i):
+    return os.path.join(GOLDEN, name + (f"_part{i}" if i else "") + ".npz")
+
+
+def save_npz_parts(name, arrays):
+    """np.savez_compressed of `arrays` into GOLDEN/<name>.npz, continued in <name>_part1.npz, <name>_part2.npz, ...
+    whenever a file would hold more than PART_BYTES of array data."""
+    parts, size = [{}], 0
+    for k, v in arrays.items():
+        if parts[-1] and size + v.nbytes > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += v.nbytes
+    for i, p in enumerate(parts):
+        np.savez_compressed(_part_path(name, i), **p)
+    i = len(parts)
+    while os.path.exists(_part_path(name, i)):          # parts left over from a larger earlier fixture
+        os.remove(_part_path(name, i))
+        i += 1
+
+
+def load_npz_parts(name):
+    """The arrays of <name>.npz and of its continuation files (save_npz_parts) as one dict."""
+    out, i = {}, 0
+    while os.path.exists(_part_path(name, i)):
+        with np.load(_part_path(name, i), allow_pickle=False) as z:
+            out.update({k: z[k] for k in z.files})
+        i += 1
+    return out
+
+
 def flow_cfg_of(z):
     return {k: int(v) for k, v in zip(z["cfg_keys"].tolist(), z["cfg_vals"].tolist())}
 

@@ -94,7 +94,6 @@ def full_model_mirror(seed=4321, precision="fp32"):
 
 FULL_GOLDEN_B = 8
 FULL_GOLDEN_WAV_STRIDE = 53
-FULL_GOLDEN_T_STRIDE = 7
 
 
 def full_model_batch():

@@ -1,5 +1,5 @@
 """The whole-model mirror `visinger_b200.models.visinger.VISinger` against the reference-generated golden
-(tests/golden/small_model.npz, made by tests/golden/make_golden_model.py from the unmodified reference model).
+(tests/golden/small_model*.npz, made by tests/golden/make_golden_model.py from the unmodified reference model).
 
 CPU: constructor / state-dict contract and the PyTorch prior network (everything upstream of z_p).
 GPU: the full forward(infer=True) waveform in fp32 mode (<= 1e-4) and bf16 / bf16x3 modes."""
@@ -7,19 +7,19 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import load_npz, maxabs
+from helpers import load_npz, load_npz_parts, maxabs
 from model_inputs import SMALL_HPARAMS, full_hparams, synth_utterances
 
 
 def _build(precision="fp32"):
     from visinger_b200.models.visinger import VISinger
-    z = load_npz("small_model")
+    z = load_npz_parts("small_model")
     m = VISinger(73, 117, 132, dict(SMALL_HPARAMS), precision=precision).eval()
-    sd = {k[2:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("w/")}
+    sd = {k[2:]: torch.from_numpy(z[k]) for k in z if k.startswith("w/")}
     missing, unexpected = m.load_state_dict(sd, strict=False)
     assert not unexpected
     assert all(k.startswith(("posterior_encoder.", "phoneme_predictor.")) for k in missing)   # training-only modules
-    batch = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("in/")}
+    batch = {k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith("in/")}
     return m, z, batch
 
 
@@ -114,8 +114,7 @@ def test_config4_full_hparams_mixed_length_batch_vs_reference_golden(cuda_device
     IDENTICAL padded batch, weights and noise (tests/golden/make_golden_model_full.py) -- strided over the whole waveform,
     the last 20 frames of every utterance in full, and the padded region after each utterance in full (the decoder is
     unmasked, models/visinger.py:111: the reference's output is NOT zero there)."""
-    from model_inputs import (full_model_mirror, full_model_batch, FULL_GOLDEN_WAV_STRIDE as WS,
-                              FULL_GOLDEN_T_STRIDE as TS)
+    from model_inputs import full_model_mirror, full_model_batch, FULL_GOLDEN_WAV_STRIDE as WS
     z = load_npz("full_model")
     batch, noise, lengths = full_model_batch()
     assert lengths.tolist() == z["lengths"].tolist() and batch["mel2ph"].shape[1] == int(z["T"])
