@@ -236,6 +236,8 @@ size_t vsg_relenc_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int
  * [B, gin, 1] (g_per_frame == 0, e.g. the speaker embedding of the PitchPredictor) or [B, gin, T] (g_per_frame != 0,
  * e.g. the frame-level f0 of the FramePriorNetwork).  Attention: full T x T softmax per head with +-window relative-
  * position key / value embeddings, masked scores filled with -1e4 (:167), channel LayerNorm eps 1e-4.
+ * VSG_PRECISION_BF16 takes head widths hidden / n_heads of 16, 32, 48, 64 and 96, windows <= 7 and T <= 2048, and
+ * returns VSG_EUNSUPPORTED otherwise; the fp32 mode also takes head width 128.
  */
 int vsg_relenc_forward(const VsgPack* pack, const float* x, const float* mask, const float* g, int32_t g_per_frame,
                        float* y, int32_t B, int32_t T, int32_t precision, void* workspace, size_t workspace_bytes,
@@ -320,6 +322,32 @@ int vsg_debug_resblock_bf16(const void* xa_bf16, const float* w, const float* b,
                             const int32_t* dilations, const void* add1_bf16, float scale, float* out_f32,
                             void* out_raw_bf16, void* out_act_bf16, int32_t B, int32_t L, int32_t C, int32_t k,
                             int32_t max_mb, int32_t sets, int32_t device);
+
+/*
+ * Per-kernel parity hooks of the relative-position encoder's attention (tests only; they synchronise):
+ * MultiHeadAttention.attention (modules/rel_transformer.py:137-177, self-attention, heads_share = True) for n_heads heads
+ * of width dk and relative-position window w:
+ *   s_ij = (q_i . k_j + [|j-i| <= w] q_i . Ek[j-i+w]) / sqrt(dk);  s_ij = -1e4 where mask_i * mask_j == 0
+ *   o_i = sum_j softmax_j(s)_ij (v_j + [|j-i| <= w] Ev[j-i+w])
+ * mask: device fp32 [B, T]; ek, ev: device fp32 [2w+1][dk].
+ *   _bf16: the tcgen05 kernel of the bf16 encoder.  qkv: device bf16 [B, T, 3 * n_heads * dk] channels-last (q | k | v,
+ *   head h at channels h*dk ..); o: device bf16 [B, T, n_heads * dk].  dk in {16, 32, 48, 64, 96}, w <= 7, T <= 2048;
+ *   VSG_EUNSUPPORTED otherwise (dk = 128 exceeds a B200 block's shared memory).  VSG_ECUDA if the kernel's error flag is set.
+ *   _f32: the fp32 kernel of the parity mode.  qkv: device fp32 [B, 3 * n_heads * dk, T]; o: device fp32 [B, n_heads * dk, T].
+ */
+int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev, void* o_bf16,
+                             int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device);
+int vsg_debug_attention_f32(const float* qkv, const float* mask, const float* ek, const float* ev, float* o, int32_t B,
+                            int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device);
+
+/*
+ * Per-kernel parity hook of the bf16 encoder's fused step after each residual add (tests only; synchronises), in place on
+ * x (device bf16 [B, T, C] channels-last, C even and <= 256):
+ *   x = (LayerNorm_C(x; gamma, beta, eps) [+ g]) * mask      (rel_transformer.py:24-42, :293-295)
+ * gamma, beta: device fp32 [C]; g: device fp32 [B, C] (g_t = 0) or [B, C, T] (g_t = 1), or NULL; mask: device fp32 [B, T].
+ */
+int vsg_debug_layernorm_bf16(void* x_bf16, const float* gamma, const float* beta, const float* g, int32_t g_t,
+                             const float* mask, float eps, int32_t B, int32_t T, int32_t C, int32_t device);
 
 /* Tuning aids for tools/tune_plans.py: force the tile plan (0 / -1 = automatic) and the number of timed repetitions of
  * the following vsg_debug_conv1d_bf16 calls; average kernel milliseconds of the last such call. */

@@ -156,3 +156,27 @@ def test_relenc_bf16_full_config_vs_oracle(cuda_device):
     rel = float((y.cpu() - yo).norm() / yo.norm())
     print(f"relenc bf16 full: rel-L2 {rel:.3e} max-abs {maxabs(y.cpu(), yo):.3e}")
     assert rel <= 8.5e-3 and maxabs(y.cpu(), yo) <= 0.09       # 1.5x the measured 5.6e-3 / 5.8e-2
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("hidden,n_heads", [(64, 2), (128, 2)])
+@pytest.mark.parametrize("window", [1, 7])
+@pytest.mark.parametrize("T", [129, 1000, 2048])
+def test_relenc_bf16_head_widths_and_windows_vs_oracle(cuda_device, hidden, n_heads, window, T):
+    """bf16 encoder at head widths 32 and 64, windows 1 and 7, up to the 16 key tiles of T = 2048, one ragged utterance;
+    the full-config gates (measured at most 4.6e-3 / 4.7e-2 on a B200)."""
+    cfg = dict(hidden=hidden, filter=4 * hidden, n_heads=n_heads, n_layers=2, kernel_size=9, window=window, gin=16)
+    sd = O.synth_rel_encoder_state_dict(O.rel_encoder_param_shapes(hidden, 4 * hidden, n_heads, 2, 9, window, 16), hidden + window)
+    gen = torch.Generator().manual_seed(T + window)
+    x, g = torch.randn(2, hidden, T, generator=gen), torch.randn(2, 16, 1, generator=gen)
+    mask = torch.ones(2, 1, T)
+    mask[1, :, T * 2 // 3:] = 0
+    with torch.no_grad():
+        yo = O.rel_encoder(sd, x, mask, g, **_okw(cfg))
+    m = _build(cfg, sd, cuda_device)
+    m.precision = "bf16"
+    y = m(x.to(cuda_device), mask.to(cuda_device), g.to(cuda_device)).cpu()
+    rel = float((y - yo).norm() / yo.norm())
+    print(f"relenc bf16 hidden={hidden} heads={n_heads} w={window} T={T}: rel-L2 {rel:.3e} max-abs {maxabs(y, yo):.3e}")
+    assert rel <= 8.5e-3 and maxabs(y, yo) <= 0.09
+    assert float((y * (1 - mask)).abs().max()) == 0.0

@@ -217,6 +217,11 @@ def lib() -> ctypes.CDLL:
         L.vsg_debug_set_plan.restype = ctypes.c_int
         L.vsg_debug_set_plan.argtypes = [i32, i32, i32, i32, i32]
         L.vsg_debug_last_ms.restype = ctypes.c_float
+        for fn in (L.vsg_debug_attention_bf16, L.vsg_debug_attention_f32):
+            fn.restype = ctypes.c_int
+            fn.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32]
+        L.vsg_debug_layernorm_bf16.restype = ctypes.c_int
+        L.vsg_debug_layernorm_bf16.argtypes = [vp, vp, vp, vp, i32, vp, ctypes.c_float, i32, i32, i32, i32]
         if L.vsg_abi_version() != 1:
             raise RuntimeError("visinger_b200: ABI version mismatch between _lib.py and the shared library")
         _lib = L
@@ -514,6 +519,60 @@ def debug_resblock_bf16(xa_bld: torch.Tensor, ws, bs, dilations, add1=None, scal
     if x3 and raw is not None:
         raw = torch.cat([raw[0], raw[1]], dim=-1)
     return (out, raw, act, ms) if reps > 1 else (out, raw, act)
+
+
+def _debug_attention(name, qkv, mask, ek, ev, n_heads: int, channels_last: bool):
+    require_cuda(qkv, "qkv")
+    assert qkv.is_contiguous()
+    B, T = (qkv.shape[0], qkv.shape[1]) if channels_last else (qkv.shape[0], qkv.shape[2])
+    H = (qkv.shape[2] if channels_last else qkv.shape[1]) // 3
+    nrel, dk = ek.shape
+    dev = qkv.device
+    mask, ek, ev = (as_f32c(t.to(dev)).reshape(-1) for t in (mask, ek, ev))
+    assert mask.numel() == B * T and ev.numel() == nrel * dk and nrel % 2 == 1 and H == n_heads * dk
+    o = torch.zeros((B, T, H) if channels_last else (B, H, T), dtype=qkv.dtype, device=dev)
+    torch.cuda.synchronize(dev)
+    rc = getattr(lib(), name)(qkv.data_ptr(), mask.data_ptr(), ek.data_ptr(), ev.data_ptr(), o.data_ptr(), B, T, n_heads, dk,
+                              (nrel - 1) // 2, dev.index or 0)
+    check(rc, name)
+    return o
+
+
+def debug_attention_bf16(qkv_btc: torch.Tensor, mask, ek, ev, n_heads: int) -> torch.Tensor:
+    """Per-kernel parity hook of the tcgen05 attention kernel (csrc/attn_tc.cuh).  qkv_btc: CUDA bf16 [B, T, 3H]
+    (q | k | v, channels-last, as the fused QKV projection writes it); mask [B, T] (or [B, 1, T]); ek / ev: [2w+1, dk]
+    fp32.  Returns o: bf16 [B, T, H]."""
+    assert qkv_btc.dtype == torch.bfloat16
+    return _debug_attention("vsg_debug_attention_bf16", qkv_btc, mask, ek, ev, n_heads, True)
+
+
+def debug_attention_f32(qkv_bct: torch.Tensor, mask, ek, ev, n_heads: int) -> torch.Tensor:
+    """Per-kernel parity hook of the fp32 attention kernel (csrc/relenc_f32.cuh).  qkv_bct: CUDA fp32 [B, 3H, T];
+    returns o: fp32 [B, H, T]."""
+    assert qkv_bct.dtype == torch.float32
+    return _debug_attention("vsg_debug_attention_f32", qkv_bct, mask, ek, ev, n_heads, False)
+
+
+def debug_layernorm_bf16(x_btc: torch.Tensor, gamma, beta, mask, g=None, eps: float = 1e-4) -> torch.Tensor:
+    """Per-kernel parity hook of the bf16 encoder's LayerNorm -> + g -> * mask step (csrc/relenc_tc.cuh), on a copy of
+    x_btc (CUDA bf16 [B, T, C]); g: None, [B, C] per utterance or [B, C, T] per frame.  Returns the bf16 result."""
+    require_cuda(x_btc, "x")
+    assert x_btc.dtype == torch.bfloat16
+    B, T, C = x_btc.shape
+    dev = x_btc.device
+    y = x_btc.contiguous().clone()
+    gamma, beta, mask = (as_f32c(t.to(dev)) for t in (gamma, beta, mask))
+    assert mask.numel() == B * T
+    g_t = 0
+    if g is not None:
+        g = as_f32c(g.to(dev))
+        g_t = 1 if g.dim() == 3 else 0
+        assert g.shape == ((B, C, T) if g_t else (B, C))
+    torch.cuda.synchronize(dev)
+    rc = lib().vsg_debug_layernorm_bf16(y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), g.data_ptr() if g is not None else None,
+                                        g_t, mask.data_ptr(), float(eps), B, T, C, dev.index or 0)
+    check(rc, "vsg_debug_layernorm_bf16")
+    return y
 
 
 def split_bf16(x: torch.Tensor) -> torch.Tensor:

@@ -221,6 +221,19 @@ int launch_attention_f32(const float* qkv, const float* mask, const float* ek, c
   VSG_LAUNCH_CHECK("relenc_attention_f32_kernel");
   return VSG_OK;
 }
+
+int attention_f32(int dk, const float* qkv, const float* mask, const float* ek, const float* ev, float* o, int B, int n_heads,
+                  int T, int w, cudaStream_t st) {
+  switch (dk) {
+    case 16: return launch_attention_f32<16>(qkv, mask, ek, ev, o, B, n_heads, T, w, st);
+    case 32: return launch_attention_f32<32>(qkv, mask, ek, ev, o, B, n_heads, T, w, st);
+    case 48: return launch_attention_f32<48>(qkv, mask, ek, ev, o, B, n_heads, T, w, st);
+    case 64: return launch_attention_f32<64>(qkv, mask, ek, ev, o, B, n_heads, T, w, st);
+    case 96: return launch_attention_f32<96>(qkv, mask, ek, ev, o, B, n_heads, T, w, st);
+    case 128: return launch_attention_f32<128>(qkv, mask, ek, ev, o, B, n_heads, T, w, st);
+    default: return fail(VSG_EUNSUPPORTED, "attention head width %d (supported: 16, 32, 48, 64, 96, 128)", dk);
+  }
+}
 }  // namespace
 
 // RelativeEncoder.forward, modules/rel_transformer.py:286-320 (post-LN; dropout is the identity in eval mode).
@@ -258,15 +271,7 @@ int relenc_forward_f32(const VsgPack* P, const float* x, const float* mask, cons
       p.y = qkv; p.y_bs = 3 * HT; p.y_cs = T;
       VSG_TRY(launch_conv_f32(p, B, st));
     }
-    switch (dk) {                                                   // attention :137-177
-      case 16: VSG_TRY(launch_attention_f32<16>(qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st)); break;
-      case 32: VSG_TRY(launch_attention_f32<32>(qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st)); break;
-      case 48: VSG_TRY(launch_attention_f32<48>(qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st)); break;
-      case 64: VSG_TRY(launch_attention_f32<64>(qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st)); break;
-      case 96: VSG_TRY(launch_attention_f32<96>(qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st)); break;
-      case 128: VSG_TRY(launch_attention_f32<128>(qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st)); break;
-      default: return fail(VSG_EUNSUPPORTED, "attention head width %d (supported: 16, 32, 48, 64, 96, 128)", dk);
-    }
+    VSG_TRY(attention_f32(dk, qkv, mask, L.ek, L.ev, o, B, e.n_heads, T, e.window, st));   // attention :137-177
     {  // x = x + conv_o(attn)                                        :130, :301
       ConvF32 p = base_conv(L.o, o, HT, T, T, 0, 1);
       p.res = y; p.res_bs = HT; p.res_cs = T;
@@ -432,3 +437,17 @@ int mask_mul(const float* x, const float* mask, float* y, int B, int C, int T, c
 }
 
 }  // namespace vsg
+
+// Per-kernel parity hook of the fp32 attention kernel (tests only; synchronises).  See include/visinger_b200.h.
+extern "C" int vsg_debug_attention_f32(const float* qkv, const float* mask, const float* ek, const float* ev, float* o,
+                                       int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device) {
+  using namespace vsg;
+  g_launches = 0;
+  if (!qkv || !mask || !ek || !ev || !o) return fail(VSG_EINVAL, "null pointer");
+  if (B < 1 || T < 1 || n_heads < 1 || w < 0) return fail(VSG_EINVAL, "bad argument");
+  VSG_CUDA_TRY(cudaSetDevice(device));
+  VSG_TRY(attention_f32(dk, qkv, mask, ek, ev, o, B, n_heads, T, w, 0));
+  const cudaError_t ce = cudaDeviceSynchronize();
+  if (ce != cudaSuccess) return fail(VSG_ECUDA, "relenc_attention_f32_kernel execution failed: %s", cudaGetErrorString(ce));
+  return VSG_OK;
+}

@@ -1230,6 +1230,12 @@ int launch_attention_bf16(const __nv_bfloat16* qkv, const float* mask, const flo
   int dev = 0;
   VSG_CUDA_TRY(cudaGetDevice(&dev));
   if (!attr_set[dev & 63]) {
+    // dk = 128 needs 261 536 bytes (Q, two K, two V and two P tiles), more than the 232 448 a B200 block may opt in to
+    int optin = 0;
+    VSG_CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    if (sm > (size_t)optin)
+      return fail(VSG_EUNSUPPORTED, "attention head width %d needs %zu bytes of shared memory per block, above this device's "
+                  "limit of %d (supported head widths: 16, 32, 48, 64, 96)", DK, sm, optin);
     VSG_CUDA_TRY(cudaFuncSetAttribute(relenc_attention_tc_kernel<DK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     attr_set[dev & 63] = true;
   }
@@ -1237,6 +1243,19 @@ int launch_attention_bf16(const __nv_bfloat16* qkv, const float* mask, const flo
   relenc_attention_tc_kernel<DK><<<grid, tc::kAtThreads, sm, st>>>(tm, p);
   VSG_LAUNCH_CHECK("relenc_attention_tc_kernel");
   return VSG_OK;
+}
+
+int attention_bf16(int dk, const __nv_bfloat16* qkv, const float* mask, const float* ek, const float* ev, __nv_bfloat16* o,
+                   int B, int n_heads, int T, int w, int* err, cudaStream_t st) {
+  switch (dk) {
+    case 16: return launch_attention_bf16<16>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
+    case 32: return launch_attention_bf16<32>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
+    case 48: return launch_attention_bf16<48>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
+    case 64: return launch_attention_bf16<64>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
+    case 96: return launch_attention_bf16<96>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
+    case 128: return launch_attention_bf16<128>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);   // refused by the shared-memory check on a B200
+    default: return fail(VSG_EUNSUPPORTED, "attention head width %d (supported: 16, 32, 48, 64, 96)", dk);
+  }
 }
 }  // namespace
 
@@ -1281,15 +1300,7 @@ static int relenc_core_tc(const VsgPack* P, const float* x, const float* mask, c
       ep.bias = L.qkv_tc.bias; ep.out_raw = qkv;
       VSG_TRY(launch_conv_tc(P, L.qkv_tc, xb, B, T, 0, 1, T, 1, 0, T, ep, opt, err, st));
     }
-    switch (dk) {
-      case 16: VSG_TRY(launch_attention_bf16<16>(qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st)); break;
-      case 32: VSG_TRY(launch_attention_bf16<32>(qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st)); break;
-      case 48: VSG_TRY(launch_attention_bf16<48>(qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st)); break;
-      case 64: VSG_TRY(launch_attention_bf16<64>(qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st)); break;
-      case 96: VSG_TRY(launch_attention_bf16<96>(qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st)); break;
-      case 128: VSG_TRY(launch_attention_bf16<128>(qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st)); break;
-      default: return fail(VSG_EUNSUPPORTED, "attention head width %d (supported: 16, 32, 48, 64, 96, 128)", dk);
-    }
+    VSG_TRY(attention_bf16(dk, qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st));
     {  // x = x + conv_o(attn)
       EpiTC ep;
       ep.bias = L.o_tc.bias; ep.add0 = xb; ep.out_raw = xb;
@@ -1970,6 +1981,46 @@ extern "C" int vsg_debug_resblock_bf16(const void* xa_bf16, const float* w, cons
   if (err) cudaFree(err);
   for (void* q : tmp.allocs) cudaFree(q);
   return rc;
+}
+
+// Per-kernel parity hook of the bf16 attention kernel (tests only; allocates and synchronises).  See include/visinger_b200.h.
+extern "C" int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev, void* o_bf16,
+                                        int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device) {
+  g_launches = 0;
+  if (!qkv_bf16 || !mask || !ek || !ev || !o_bf16) return fail(VSG_EINVAL, "null pointer");
+  if (B < 1 || T < 1 || n_heads < 1 || w < 0) return fail(VSG_EINVAL, "bad argument");
+  VSG_CUDA_TRY(cudaSetDevice(device));
+  int* err = nullptr;
+  VSG_CUDA_TRY(cudaMalloc(&err, sizeof(int)));
+  int rc = cudaMemset(err, 0, sizeof(int)) == cudaSuccess ? VSG_OK : fail(VSG_ECUDA, "cudaMemset failed");
+  if (rc == VSG_OK)
+    rc = attention_bf16(dk, (const __nv_bfloat16*)qkv_bf16, mask, ek, ev, (__nv_bfloat16*)o_bf16, B, n_heads, T, w, err, 0);
+  if (rc == VSG_OK) {
+    int flag = 0;
+    cudaError_t ce = cudaDeviceSynchronize();
+    if (ce == cudaSuccess) ce = cudaMemcpy(&flag, err, sizeof(int), cudaMemcpyDeviceToHost);
+    if (ce != cudaSuccess) rc = fail(VSG_ECUDA, "relenc_attention_tc_kernel execution failed: %s", cudaGetErrorString(ce));
+    else if (flag) rc = fail(VSG_ECUDA, "relenc_attention_tc_kernel set its error flag (%d)", flag);
+  }
+  cudaFree(err);
+  return rc;
+}
+
+// Per-kernel parity hook of the bf16 encoder's fused LayerNorm -> condition -> mask step (tests only; synchronises).
+extern "C" int vsg_debug_layernorm_bf16(void* x_bf16, const float* gamma, const float* beta, const float* g, int32_t g_t,
+                                        const float* mask, float eps, int32_t B, int32_t T, int32_t C, int32_t device) {
+  g_launches = 0;
+  if (!x_bf16 || !gamma || !beta || !mask) return fail(VSG_EINVAL, "null pointer");
+  if (B < 1 || T < 1) return fail(VSG_EINVAL, "bad argument");
+  if (C < 2 || C > 256 || (C & 1)) return fail(VSG_EUNSUPPORTED, "LayerNorm over %d channels (supported: even, <= 256)", C);
+  VSG_CUDA_TRY(cudaSetDevice(device));
+  const long long rows = (long long)B * T;
+  relenc_layernorm_bf16_kernel<256><<<(unsigned)((rows + 7) / 8), 256>>>((__nv_bfloat16*)x_bf16, gamma, beta, g, g_t, mask, eps,
+                                                                         C, T, rows);
+  VSG_LAUNCH_CHECK("relenc_layernorm_bf16_kernel");
+  const cudaError_t ce = cudaDeviceSynchronize();
+  if (ce != cudaSuccess) return fail(VSG_ECUDA, "relenc_layernorm_bf16_kernel execution failed: %s", cudaGetErrorString(ce));
+  return VSG_OK;
 }
 
 // Host-only: print the tile plan the launcher would choose for one convolution (tuning aid; no GPU needed).
