@@ -236,8 +236,10 @@ size_t vsg_relenc_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int
  * [B, gin, 1] (g_per_frame == 0, e.g. the speaker embedding of the PitchPredictor) or [B, gin, T] (g_per_frame != 0,
  * e.g. the frame-level f0 of the FramePriorNetwork).  Attention: full T x T softmax per head with +-window relative-
  * position key / value embeddings, masked scores filled with -1e4 (:167), channel LayerNorm eps 1e-4.
- * VSG_PRECISION_BF16 takes head widths hidden / n_heads of 16, 32, 48, 64 and 96, windows <= 7 and T <= 2048, and
- * returns VSG_EUNSUPPORTED otherwise; the fp32 mode also takes head width 128.
+ * VSG_PRECISION_BF16 takes head widths hidden / n_heads of 16, 32, 48, 64 and 96 and windows <= 7, and returns
+ * VSG_EUNSUPPORTED otherwise; the fp32 mode also takes head width 128.  Both take any T.  Beyond T = 2048 the bf16
+ * attention runs over key chunks of 2048 frames plus a combine, and the workspace grows by about
+ * ceil(T / 2048) * B * T * hidden * 4 bytes (vsg_relenc_workspace_bytes includes it).
  */
 int vsg_relenc_forward(const VsgPack* pack, const float* x, const float* mask, const float* g, int32_t g_per_frame,
                        float* y, int32_t B, int32_t T, int32_t precision, void* workspace, size_t workspace_bytes,
@@ -333,10 +335,16 @@ int vsg_debug_resblock_bf16(const void* xa_bf16, const float* w, const float* b,
  *   _bf16: the tcgen05 kernel of the bf16 encoder.  qkv: device bf16 [B, T, 3 * n_heads * dk] channels-last (q | k | v,
  *   head h at channels h*dk ..); o: device bf16 [B, T, n_heads * dk].  dk in {16, 32, 48, 64, 96}, w <= 7, T <= 2048;
  *   VSG_EUNSUPPORTED otherwise (dk = 128 exceeds a B200 block's shared memory).  VSG_ECUDA if the kernel's error flag is set.
+ *   _split_bf16: the split-key path of the bf16 encoder at any T: the same kernel over key chunks of key_chunk frames (a
+ *   multiple of 128 up to 2048; 0 = 2048, what the encoder uses beyond T = 2048), then the combine of the chunks.  Same
+ *   layouts, head widths and windows as _bf16; VSG_EINVAL for any other key_chunk.
  *   _f32: the fp32 kernel of the parity mode.  qkv: device fp32 [B, 3 * n_heads * dk, T]; o: device fp32 [B, n_heads * dk, T].
  */
 int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev, void* o_bf16,
                              int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device);
+int vsg_debug_attention_split_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev, void* o_bf16,
+                                   int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t key_chunk,
+                                   int32_t device);
 int vsg_debug_attention_f32(const float* qkv, const float* mask, const float* ek, const float* ev, float* o, int32_t B,
                             int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device);
 

@@ -220,6 +220,8 @@ def lib() -> ctypes.CDLL:
         for fn in (L.vsg_debug_attention_bf16, L.vsg_debug_attention_f32):
             fn.restype = ctypes.c_int
             fn.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32]
+        L.vsg_debug_attention_split_bf16.restype = ctypes.c_int
+        L.vsg_debug_attention_split_bf16.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32]
         L.vsg_debug_layernorm_bf16.restype = ctypes.c_int
         L.vsg_debug_layernorm_bf16.argtypes = [vp, vp, vp, vp, i32, vp, ctypes.c_float, i32, i32, i32, i32]
         if L.vsg_abi_version() != 1:
@@ -521,7 +523,7 @@ def debug_resblock_bf16(xa_bld: torch.Tensor, ws, bs, dilations, add1=None, scal
     return (out, raw, act, ms) if reps > 1 else (out, raw, act)
 
 
-def _debug_attention(name, qkv, mask, ek, ev, n_heads: int, channels_last: bool):
+def _debug_attention(name, qkv, mask, ek, ev, n_heads: int, channels_last: bool, *extra):
     require_cuda(qkv, "qkv")
     assert qkv.is_contiguous()
     B, T = (qkv.shape[0], qkv.shape[1]) if channels_last else (qkv.shape[0], qkv.shape[2])
@@ -533,7 +535,7 @@ def _debug_attention(name, qkv, mask, ek, ev, n_heads: int, channels_last: bool)
     o = torch.zeros((B, T, H) if channels_last else (B, H, T), dtype=qkv.dtype, device=dev)
     torch.cuda.synchronize(dev)
     rc = getattr(lib(), name)(qkv.data_ptr(), mask.data_ptr(), ek.data_ptr(), ev.data_ptr(), o.data_ptr(), B, T, n_heads, dk,
-                              (nrel - 1) // 2, dev.index or 0)
+                              (nrel - 1) // 2, *extra, dev.index or 0)
     check(rc, name)
     return o
 
@@ -544,6 +546,14 @@ def debug_attention_bf16(qkv_btc: torch.Tensor, mask, ek, ev, n_heads: int) -> t
     fp32.  Returns o: bf16 [B, T, H]."""
     assert qkv_btc.dtype == torch.bfloat16
     return _debug_attention("vsg_debug_attention_bf16", qkv_btc, mask, ek, ev, n_heads, True)
+
+
+def debug_attention_split_bf16(qkv_btc: torch.Tensor, mask, ek, ev, n_heads: int, key_chunk: int = 0) -> torch.Tensor:
+    """Per-kernel parity hook of the split-key attention path (csrc/attn_tc.cuh split mode + combine) at any T: keys in
+    chunks of key_chunk frames (a multiple of 128 up to 2048; 0 = 2048, the encoder's choice beyond T = 2048).  Same
+    arguments and result as debug_attention_bf16."""
+    assert qkv_btc.dtype == torch.bfloat16
+    return _debug_attention("vsg_debug_attention_split_bf16", qkv_btc, mask, ek, ev, n_heads, True, int(key_chunk))
 
 
 def debug_attention_f32(qkv_bct: torch.Tensor, mask, ek, ev, n_heads: int) -> torch.Tensor:

@@ -18,6 +18,12 @@
 // a thread owns one query row (its TMEM lane): row reductions need no shuffles.
 // Warp roles (320 threads): 0 TMA producer, 1 TMEM allocator + MMA issuer, 2..9 softmax sets 0 / 1 (warp % 4 = TMEM lane
 // quarter).  Every barrier wait is bounded (trap + error flag).
+// Split-key mode (T > 2048, or any T through the debug hook): the keys are cut into chunks of chunk_tiles tiles at fixed
+// multiples of the chunk size from key 0, and one CTA runs the two passes above over one (query tile, head, utterance,
+// key chunk).  Key indices, the >= T test and the diagonal offset stay absolute, so a relative-position window that
+// straddles a chunk border contributes to each chunk the weights of that chunk's keys.  Instead of normalising, set 0
+// writes the chunk's unnormalised output (including the relative-value term), row maximum (exp2 domain) and row sum;
+// attention_combine_kernel merges the chunks.
 #pragma once
 #include "conv_tc.cuh"
 #include "rb_tc.cuh"
@@ -27,10 +33,14 @@ namespace vsg {
 struct AttnTC {
   int B, T, n_heads, w;
   int n_tiles;                    // ceil(T / 128): key tiles (= query tiles)
+  int chunk_tiles;                // key tiles per CTA (<= kAtMaxTiles); blockIdx.x = query tile + n_tiles * key chunk
   const float* mask;              // [B, T]
   const float* Ek;                // fp32 [2w+1][DK]
   const float* Ev;
   __nv_bfloat16* o;               // [B, T, n_heads * DK]
+  float* o_part;                  // split-key mode (else null): fp32 [chunks][B][T][n_heads * DK] unnormalised output,
+  float* m_part;                  //   [chunks][B][n_heads][T] row maxima (exp2 domain)
+  float* l_part;                  //   [chunks][B][n_heads][T] row sums
   int* error_flag;
 };
 
@@ -38,7 +48,7 @@ namespace tc {
 constexpr int kAtQFull = 0, kAtKFull = 1, kAtKEmpty = 3, kAtVFull = 5, kAtVEmpty = 7, kAtSFull = 9, kAtSEmpty = 11,
               kAtPFull = 13, kAtPEmpty = 15, kAtOFull = 17, kAtNumBars = 18;
 constexpr int kAtThreads = 320;
-constexpr int kAtMaxTiles = 16;   // T <= 2048
+constexpr int kAtMaxTiles = 16;   // key tiles of one CTA: T <= 2048 in one launch, the key-chunk size of the split mode
 }  // namespace tc
 
 template <int DK>
@@ -80,8 +90,9 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
   float* const ls_s = reinterpret_cast<float*>(sgen + SM::ls_off);
   uint32_t* const km_s = reinterpret_cast<uint32_t*>(sgen + SM::km_off);
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
-  const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * 128;
-  const int T = p.T, H = p.n_heads * DK, nt = p.n_tiles, w = p.w, nrel = 2 * w + 1;
+  const int b = blockIdx.z, h = blockIdx.y, kc = blockIdx.x / p.n_tiles, q0 = (blockIdx.x - kc * p.n_tiles) * 128;
+  const int kt0 = kc * p.chunk_tiles;                           // first key tile of this CTA's chunk
+  const int T = p.T, H = p.n_heads * DK, nt = min(p.chunk_tiles, p.n_tiles - kt0), w = p.w, nrel = 2 * w + 1;
   int* const error_flag = p.error_flag;
 
   if (warp == 0 && lane == 0) {
@@ -106,7 +117,7 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
   }
   for (int i = threadIdx.x; i < 2 * 128 * 16; i += blockDim.x) pw_s[i] = 0.f;
   for (int i = warp; i < nt * 4; i += (int)(blockDim.x >> 5)) {
-    const int t = i * 32 + lane;
+    const int t = (kt0 * 4 + i) * 32 + lane;
     const uint32_t bits = __ballot_sync(0xffffffffu, t < T && p.mask[(long long)b * T + t] != 0.f);
     if (lane == 0) km_s[i] = bits;
   }
@@ -125,7 +136,7 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
       for (int c = 0; c < NCH; ++c) tma_load_3d(sbase + SM::q_off + c * CHB, &tmQKV, bar(kAtQFull), h * DK + c * CW, q0, b);
     }
     for (int v = 0; v < n_visits; ++v) {
-      const int s = v & 1, k0 = (v % nt) * 128;
+      const int s = v & 1, k0 = (kt0 + v % nt) * 128;
       mbar_wait(bar(kAtKEmpty + s), (((uint32_t)v >> 1) & 1u) ^ 1u, error_flag);
       if (elect_one()) {
         mbar_expect_tx(bar(kAtKFull + s), TILEB);
@@ -216,7 +227,7 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
     bool have_rel = false;
     // One visit = one key tile in one pass.  PASS2 = false: row maximum only; true: P, row sum, diagonal weights.
     auto visit = [&](int v, bool pass2) {
-      const int k0 = (v % nt) * 128;
+      const int k0 = (kt0 + v % nt) * 128;
       mbar_wait(bar(kAtSFull + g), n_s & 1u, error_flag);
       ++n_s;
       fence_after_sync();
@@ -302,7 +313,13 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
     ls_s[g * 128 + row] = l_run;
     epi_bar_sync(2, 256);
     if (g == 0) {
-      const float inv = 1.0f / (ls_s[row] + ls_s[128 + row]);
+      const float lsum = ls_s[row] + ls_s[128 + row];
+      const float inv = 1.0f / lsum;
+      if (p.o_part && qi < T) {
+        const long long r = (((long long)kc * p.B + b) * p.n_heads + h) * T + qi;
+        p.m_part[r] = m_run;
+        p.l_part[r] = lsum;
+      }
       mbar_wait(bar(kAtOFull), 0u, error_flag);
       fence_after_sync();
       __nv_bfloat16* orow = p.o + ((long long)b * T + qi) * H + h * DK;
@@ -319,7 +336,12 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
 #pragma unroll
           for (int i = 0; i < 16; ++i) v[i] = fmaf(pm, __ldg(p.Ev + m * DK + c0 + i), v[i]);
         }
-        if (qi < T) {
+        if (p.o_part) {
+          float* orow32 = p.o_part + (((long long)kc * p.B + b) * T + qi) * H + h * DK + c0;
+          if (qi < T)
+#pragma unroll
+            for (int i = 0; i < 16; i += 4) *reinterpret_cast<float4*>(orow32 + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
+        } else if (qi < T) {
           uint32_t hh[8];
 #pragma unroll
           for (int i = 0; i < 8; ++i) hh[i] = pack_bf16x2(v[2 * i] * inv, v[2 * i + 1] * inv);
@@ -335,6 +357,48 @@ relenc_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Attn
     fence_after_sync();
     tmem_dealloc(tmem_base, 512);
   }
+}
+
+// Merge of the split-key mode's chunks, one thread per 8 channels of one (utterance, frame):
+//   M = max_c m_c;  w_c = exp2(m_c - M);  o = sum_c w_c o_c;  l = sum_c w_c l_c  (fmaf in chunk order from 0);  bf16(o / l)
+// The chunk holding the maximum gets weight exactly 1 (one chunk reproduces the single-launch epilogue bit for bit); a
+// chunk whose keys are all masked for a valid row has m_c = -1e4 log2(e) and weight exactly 0, and its finite o_c adds
+// exactly 0, so masked padding leaves the result unchanged bit for bit.  A masked query row has m_c = -1e4 log2(e) in
+// every chunk: weights 1, a uniform softmax over all T keys as in the reference.
+__global__ void attention_combine_kernel(const float* __restrict__ o_part, const float* __restrict__ m_part,
+                                         const float* __restrict__ l_part, __nv_bfloat16* __restrict__ o, int B, int T,
+                                         int n_heads, int dk, int n_chunks) {
+  using namespace tc;
+  const int H = n_heads * dk, H8 = H / 8;
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)B * T * H8) return;
+  const long long bt = i / H8;                                  // b * T + t
+  const int c = (int)(i - bt * H8) * 8, b = (int)(bt / T), t = (int)(bt - (long long)b * T), h = c / dk;
+  const long long mrow = ((long long)b * n_heads + h) * T + t, mstride = (long long)B * n_heads * T;
+  const long long orow = bt * H + c, ostride = (long long)B * T * H;
+  float M = -INFINITY;
+  for (int k = 0; k < n_chunks; ++k) M = fmaxf(M, m_part[k * mstride + mrow]);
+  float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, l = 0.f;
+  for (int k = 0; k < n_chunks; ++k) {
+    const float wk = exp2f(m_part[k * mstride + mrow] - M);
+    l = fmaf(wk, l_part[k * mstride + mrow], l);
+    const float4 a = *reinterpret_cast<const float4*>(o_part + k * ostride + orow);
+    const float4 d = *reinterpret_cast<const float4*>(o_part + k * ostride + orow + 4);
+    const float x[8] = {a.x, a.y, a.z, a.w, d.x, d.y, d.z, d.w};
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = fmaf(wk, x[j], acc[j]);
+  }
+  const float inv = 1.0f / l;
+  uint32_t hh[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) hh[j] = pack_bf16x2(acc[2 * j] * inv, acc[2 * j + 1] * inv);
+  stg128(o + orow, make_uint4(hh[0], hh[1], hh[2], hh[3]));
+}
+
+// fp32 workspace of the split-key mode: o_part, then m_part, then l_part (see AttnTC)
+inline size_t attention_split_floats(int B, int T, int n_heads, int dk, int chunk_tiles) {
+  const size_t n_chunks = (size_t)((T + 127) / 128 + chunk_tiles - 1) / chunk_tiles;
+  return n_chunks * B * T * ((size_t)n_heads * dk + 2 * n_heads);
 }
 
 }  // namespace vsg

@@ -217,48 +217,55 @@ __global__ void __launch_bounds__(256) relenc_attention_f32_kernel(const float* 
 //   y[b, :, t] += table[pos_t, :]                                           models/visinger.py:79-82 (table row 0 is zero)
 // -- the position of a frame is the running count of frames whose channel 0 is non-zero, the reference's data-dependent
 // definition.  enc: [B, H, T_ph]; mel2ph: int64 [B, T]; table: [rows, H] (SinusoidalPositionalEmbedding.weights) or null.
-__global__ void length_regulate_pos_kernel(const float* __restrict__ enc, const long long* __restrict__ mel2ph,
-                                           const float* __restrict__ table, int table_rows, float* __restrict__ y, int H,
-                                           int T_ph, int T) {
-  extern __shared__ int lr_sm[];                 // [T] token index (-1 = padding), then [T] position
-  int* tok = lr_sm;
-  int* pos = lr_sm + T;
-  __shared__ int warp_tot[32];
-  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+// The utterance is processed in chunks of kLrChunk frames (token indices, scan with the carry of the chunks before, then
+// the chunk's y), so shared memory does not depend on T.  Launch with kLrThreads threads.
+constexpr int kLrThreads = 512, kLrChunk = 2048;
+__global__ void __launch_bounds__(kLrThreads) length_regulate_pos_kernel(const float* __restrict__ enc,
+                                                                         const long long* __restrict__ mel2ph,
+                                                                         const float* __restrict__ table, int table_rows,
+                                                                         float* __restrict__ y, int H, int T_ph, int T) {
+  __shared__ int tok[kLrChunk];                  // token index of each frame of the chunk (-1 = padding)
+  __shared__ int pos[kLrChunk];                  // its position
+  __shared__ int warp_tot[kLrThreads / 32];
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = kLrThreads / 32;
   const float* eb = enc + (long long)b * H * T_ph;
   float* yb = y + (long long)b * H * T;
-  for (int t = tid; t < T; t += blockDim.x) {
-    const long long m = mel2ph[(long long)b * T + t];
-    tok[t] = (m > 0 && m <= T_ph) ? (int)(m - 1) : -1;
-  }
-  __syncthreads();
-  // inclusive scan of keep_t over the utterance, a chunk of blockDim.x frames at a time
-  int carry = 0;
-  for (int t0 = 0; t0 < T; t0 += blockDim.x) {
-    const int t = t0 + tid;
-    int keep = 0;
-    if (t < T && tok[t] >= 0) keep = (eb[tok[t]] != 0.f) ? 1 : 0;             // channel 0 of the gathered row
-    int v = keep;
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      const int n = __shfl_up_sync(0xffffffffu, v, off);
-      if (lane >= off) v += n;
+  int carry = 0;                                 // frames kept before this chunk
+  for (int c0 = 0; c0 < T; c0 += kLrChunk) {
+    const int n = min(kLrChunk, T - c0);
+    for (int t = tid; t < n; t += kLrThreads) {
+      const long long m = mel2ph[(long long)b * T + c0 + t];
+      tok[t] = (m > 0 && m <= T_ph) ? (int)(m - 1) : -1;
     }
-    if (lane == 31) warp_tot[warp] = v;
     __syncthreads();
-    int before = carry;
-    for (int wv = 0; wv < warp; ++wv) before += warp_tot[wv];
-    if (t < T) pos[t] = keep ? before + v : 0;
-    int chunk = 0;
-    for (int wv = 0; wv < nw; ++wv) chunk += warp_tot[wv];
-    carry += chunk;
-    __syncthreads();
-  }
-  for (int i = tid; i < H * T; i += blockDim.x) {
-    const int c = i / T, t = i - c * T;
-    float v = tok[t] >= 0 ? eb[(long long)c * T_ph + tok[t]] : 0.f;
-    if (table && pos[t] < table_rows) v += table[(long long)pos[t] * H + c];
-    yb[i] = v;
+    // inclusive scan of keep_t, kLrThreads frames at a time
+    for (int t0 = 0; t0 < n; t0 += kLrThreads) {
+      const int t = t0 + tid;
+      int keep = 0;
+      if (t < n && tok[t] >= 0) keep = (eb[tok[t]] != 0.f) ? 1 : 0;           // channel 0 of the gathered row
+      int v = keep;
+#pragma unroll
+      for (int off = 1; off < 32; off <<= 1) {
+        const int x = __shfl_up_sync(0xffffffffu, v, off);
+        if (lane >= off) v += x;
+      }
+      if (lane == 31) warp_tot[warp] = v;
+      __syncthreads();
+      int before = carry;
+      for (int wv = 0; wv < warp; ++wv) before += warp_tot[wv];
+      if (t < n) pos[t] = keep ? before + v : 0;
+      int part = 0;
+      for (int wv = 0; wv < nw; ++wv) part += warp_tot[wv];
+      carry += part;
+      __syncthreads();
+    }
+    for (int i = tid; i < H * n; i += kLrThreads) {
+      const int c = i / n, t = i - c * n;
+      float v = tok[t] >= 0 ? eb[(long long)c * T_ph + tok[t]] : 0.f;
+      if (table && pos[t] < table_rows) v += table[(long long)pos[t] * H + c];
+      yb[(long long)c * T + c0 + t] = v;
+    }
+    __syncthreads();                             // tok / pos are rewritten by the next chunk
   }
 }
 

@@ -316,11 +316,7 @@ int frame_prior_forward_f32(const VsgPack* P, const float* x, const float* mask,
 
 int length_regulate(const float* enc, const long long* mel2ph, const float* table, int table_rows, float* y, int B, int H,
                     int T_ph, int T, cudaStream_t st) {
-  const size_t sm = (size_t)2 * T * sizeof(int);
-  if (sm > 96 * 1024) return fail(VSG_EUNSUPPORTED, "sequence too long for the length regulator (%d frames)", T);
-  if (sm > 48 * 1024)
-    VSG_CUDA_TRY(cudaFuncSetAttribute(length_regulate_pos_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-  length_regulate_pos_kernel<<<B, 512, sm, st>>>(enc, mel2ph, table, table_rows, y, H, T_ph, T);
+  length_regulate_pos_kernel<<<B, kLrThreads, 0, st>>>(enc, mel2ph, table, table_rows, y, H, T_ph, T);
   VSG_LAUNCH_CHECK("length_regulate_pos_kernel");
   return VSG_OK;
 }

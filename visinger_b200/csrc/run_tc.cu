@@ -1209,22 +1209,37 @@ size_t relenc_ws_bytes_tc(const VsgPack* P, int B, int T, int g_t) {
   n += align256((size_t)B * T * 3 * e.hidden * 2);            // q | k | v
   n += align256((size_t)B * T * e.filter * 2);                // FFN hidden
   n += align256((size_t)B * e.hidden * (g_t ? T : 1) * sizeof(float));
+  if (T > 128 * tc::kAtMaxTiles)                              // split-key attention: per-chunk partial outputs
+    n += align256(attention_split_floats(B, T, e.n_heads, e.hidden / e.n_heads, tc::kAtMaxTiles) * sizeof(float));
   return n + 512;
 }
 
 namespace {
+// chunk_tiles = 0: one launch over all key tiles (T <= 2048), normalised output.  chunk_tiles > 0: the split-key launch
+// over key chunks of that many tiles, its partials in `part` (attention_split_floats), then the combine.
 template <int DK>
 int launch_attention_bf16(const __nv_bfloat16* qkv, const float* mask, const float* ek, const float* ev, __nv_bfloat16* o, int B,
-                          int n_heads, int T, int w, int* err, cudaStream_t st) {
-  if (T > 128 * tc::kAtMaxTiles) return fail(VSG_EUNSUPPORTED, "attention: sequence of %d frames (supported: <= %d)", T, 128 * tc::kAtMaxTiles);
+                          int n_heads, int T, int w, int chunk_tiles, float* part, int* err, cudaStream_t st) {
+  const int n_tiles = (T + 127) / 128;
+  if (chunk_tiles == 0 && n_tiles > tc::kAtMaxTiles)
+    return fail(VSG_EUNSUPPORTED, "attention: sequence of %d frames (supported: <= %d)", T, 128 * tc::kAtMaxTiles);
+  if (chunk_tiles < 0 || chunk_tiles > tc::kAtMaxTiles || (chunk_tiles > 0 && !part))
+    return fail(VSG_EINVAL, "attention: key chunk of %d tiles (supported: 1 .. %d, with a partials buffer)", chunk_tiles, tc::kAtMaxTiles);
   if (w > 7) return fail(VSG_EUNSUPPORTED, "attention: relative-position window %d (supported: <= 7)", w);
   const int H = n_heads * DK;
   constexpr int CW = AttnSmem<DK>::CW;
   CUtensorMap tm;   // the fused projection's output [B, T, 3H] as (channels, frames, utterances)
   VSG_TRY(encode_3d(&tm, qkv, (uint64_t)3 * H, (uint64_t)T, (uint64_t)B, (uint64_t)3 * H, (uint64_t)T * 3 * H, (uint32_t)CW, 128, CW));
   AttnTC p;
-  p.B = B; p.T = T; p.n_heads = n_heads; p.w = w; p.n_tiles = (T + 127) / 128;
+  p.B = B; p.T = T; p.n_heads = n_heads; p.w = w; p.n_tiles = n_tiles; p.chunk_tiles = chunk_tiles ? chunk_tiles : n_tiles;
   p.mask = mask; p.Ek = ek; p.Ev = ev; p.o = o; p.error_flag = err;
+  const int n_chunks = (n_tiles + p.chunk_tiles - 1) / p.chunk_tiles;
+  p.o_part = p.m_part = p.l_part = nullptr;
+  if (chunk_tiles) {
+    p.o_part = part;
+    p.m_part = part + (size_t)n_chunks * B * T * H;
+    p.l_part = p.m_part + (size_t)n_chunks * B * n_heads * T;
+  }
   const size_t sm = AttnSmem<DK>::bytes;
   static bool attr_set[64] = {false};
   int dev = 0;
@@ -1239,21 +1254,28 @@ int launch_attention_bf16(const __nv_bfloat16* qkv, const float* mask, const flo
     VSG_CUDA_TRY(cudaFuncSetAttribute(relenc_attention_tc_kernel<DK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     attr_set[dev & 63] = true;
   }
-  dim3 grid(p.n_tiles, n_heads, B);
+  dim3 grid(n_tiles * n_chunks, n_heads, B);
   relenc_attention_tc_kernel<DK><<<grid, tc::kAtThreads, sm, st>>>(tm, p);
   VSG_LAUNCH_CHECK("relenc_attention_tc_kernel");
+  if (chunk_tiles) {
+    const long long n = (long long)B * T * H / 8;
+    attention_combine_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p.o_part, p.m_part, p.l_part, o, B, T, n_heads, DK,
+                                                                           n_chunks);
+    VSG_LAUNCH_CHECK("attention_combine_kernel");
+  }
   return VSG_OK;
 }
 
 int attention_bf16(int dk, const __nv_bfloat16* qkv, const float* mask, const float* ek, const float* ev, __nv_bfloat16* o,
-                   int B, int n_heads, int T, int w, int* err, cudaStream_t st) {
+                   int B, int n_heads, int T, int w, int chunk_tiles, float* part, int* err, cudaStream_t st) {
   switch (dk) {
-    case 16: return launch_attention_bf16<16>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
-    case 32: return launch_attention_bf16<32>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
-    case 48: return launch_attention_bf16<48>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
-    case 64: return launch_attention_bf16<64>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
-    case 96: return launch_attention_bf16<96>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);
-    case 128: return launch_attention_bf16<128>(qkv, mask, ek, ev, o, B, n_heads, T, w, err, st);   // refused by the shared-memory check on a B200
+    case 16: return launch_attention_bf16<16>(qkv, mask, ek, ev, o, B, n_heads, T, w, chunk_tiles, part, err, st);
+    case 32: return launch_attention_bf16<32>(qkv, mask, ek, ev, o, B, n_heads, T, w, chunk_tiles, part, err, st);
+    case 48: return launch_attention_bf16<48>(qkv, mask, ek, ev, o, B, n_heads, T, w, chunk_tiles, part, err, st);
+    case 64: return launch_attention_bf16<64>(qkv, mask, ek, ev, o, B, n_heads, T, w, chunk_tiles, part, err, st);
+    case 96: return launch_attention_bf16<96>(qkv, mask, ek, ev, o, B, n_heads, T, w, chunk_tiles, part, err, st);
+    case 128:   // refused by the shared-memory check on a B200
+      return launch_attention_bf16<128>(qkv, mask, ek, ev, o, B, n_heads, T, w, chunk_tiles, part, err, st);
     default: return fail(VSG_EUNSUPPORTED, "attention head width %d (supported: 16, 32, 48, 64, 96)", dk);
   }
 }
@@ -1261,7 +1283,8 @@ int attention_bf16(int dk, const __nv_bfloat16* qkv, const float* mask, const fl
 
 // RelativeEncoder.forward (modules/rel_transformer.py:286-320) in the throughput mode: channels-last bf16 activations, the
 // projections and the FFN on the tcgen05 convolution kernel (residual adds, ReLU and masks in its epilogue), attention on
-// the warp-mma flash kernel, LayerNorm + condition + mask fused in one pass.
+// the tcgen05 kernel of attn_tc.cuh (split into key chunks of 2048 plus a combine beyond T = 2048), LayerNorm + condition
+// + mask fused in one pass.
 static int relenc_core_tc(const VsgPack* P, const float* x, const float* mask, const float* g, int g_t, int B, int T,
                           Workspace& ws, cudaStream_t st, __nv_bfloat16** xb_out, int** err_out) {
   const RelEncPack& e = P->relenc;
@@ -1275,6 +1298,8 @@ static int relenc_core_tc(const VsgPack* P, const float* x, const float* mask, c
   bf* qkv = ws.take<bf>((size_t)B * T * 3 * H);
   bf* fb = ws.take<bf>((size_t)B * T * F);
   float* gp = ws.take<float>((size_t)B * H * (g_t ? T : 1));
+  const int chunk_tiles = T > 128 * tc::kAtMaxTiles ? tc::kAtMaxTiles : 0;
+  float* part = chunk_tiles ? ws.take<float>(attention_split_floats(B, T, e.n_heads, dk, chunk_tiles)) : nullptr;
   int* err = ws.take<int>(1);
   if (ws.overflow) return fail(VSG_ENOMEM, "encoder workspace too small: need %zu bytes", ws.off);
   VSG_CUDA_TRY(cudaMemsetAsync(err, 0, sizeof(int), st));
@@ -1300,7 +1325,7 @@ static int relenc_core_tc(const VsgPack* P, const float* x, const float* mask, c
       ep.bias = L.qkv_tc.bias; ep.out_raw = qkv;
       VSG_TRY(launch_conv_tc(P, L.qkv_tc, xb, B, T, 0, 1, T, 1, 0, T, ep, opt, err, st));
     }
-    VSG_TRY(attention_bf16(dk, qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, err, st));
+    VSG_TRY(attention_bf16(dk, qkv, mask, L.ek, L.ev, ob, B, e.n_heads, T, e.window, chunk_tiles, part, err, st));
     {  // x = x + conv_o(attn)
       EpiTC ep;
       ep.bias = L.o_tc.bias; ep.add0 = xb; ep.out_raw = xb;
@@ -1994,7 +2019,8 @@ extern "C" int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask,
   VSG_CUDA_TRY(cudaMalloc(&err, sizeof(int)));
   int rc = cudaMemset(err, 0, sizeof(int)) == cudaSuccess ? VSG_OK : fail(VSG_ECUDA, "cudaMemset failed");
   if (rc == VSG_OK)
-    rc = attention_bf16(dk, (const __nv_bfloat16*)qkv_bf16, mask, ek, ev, (__nv_bfloat16*)o_bf16, B, n_heads, T, w, err, 0);
+    rc = attention_bf16(dk, (const __nv_bfloat16*)qkv_bf16, mask, ek, ev, (__nv_bfloat16*)o_bf16, B, n_heads, T, w, 0, nullptr,
+                        err, 0);
   if (rc == VSG_OK) {
     int flag = 0;
     cudaError_t ce = cudaDeviceSynchronize();
@@ -2002,6 +2028,40 @@ extern "C" int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask,
     if (ce != cudaSuccess) rc = fail(VSG_ECUDA, "relenc_attention_tc_kernel execution failed: %s", cudaGetErrorString(ce));
     else if (flag) rc = fail(VSG_ECUDA, "relenc_attention_tc_kernel set its error flag (%d)", flag);
   }
+  cudaFree(err);
+  return rc;
+}
+
+// Per-kernel parity hook of the split-key attention path: the split launch plus the combine, at any T and a key chunk of
+// key_chunk frames (a multiple of 128 up to 2048; 0 = 2048).  Tests only; allocates and synchronises.
+extern "C" int vsg_debug_attention_split_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev,
+                                              void* o_bf16, int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w,
+                                              int32_t key_chunk, int32_t device) {
+  g_launches = 0;
+  if (!qkv_bf16 || !mask || !ek || !ev || !o_bf16) return fail(VSG_EINVAL, "null pointer");
+  if (B < 1 || T < 1 || n_heads < 1 || w < 0 || dk < 1) return fail(VSG_EINVAL, "bad argument");
+  if (key_chunk == 0) key_chunk = 128 * tc::kAtMaxTiles;
+  if (key_chunk < 0 || key_chunk % 128 || key_chunk > 128 * tc::kAtMaxTiles)
+    return fail(VSG_EINVAL, "key chunk of %d frames (supported: a multiple of 128 up to %d, or 0)", key_chunk, 128 * tc::kAtMaxTiles);
+  VSG_CUDA_TRY(cudaSetDevice(device));
+  const int chunk_tiles = key_chunk / 128;
+  int* err = nullptr;
+  float* part = nullptr;
+  VSG_CUDA_TRY(cudaMalloc(&err, sizeof(int)));
+  int rc = cudaMalloc(&part, attention_split_floats(B, T, n_heads, dk, chunk_tiles) * sizeof(float)) == cudaSuccess
+               ? VSG_OK : fail(VSG_ENOMEM, "cudaMalloc of the split-key partials failed");
+  if (rc == VSG_OK && cudaMemset(err, 0, sizeof(int)) != cudaSuccess) rc = fail(VSG_ECUDA, "cudaMemset failed");
+  if (rc == VSG_OK)
+    rc = attention_bf16(dk, (const __nv_bfloat16*)qkv_bf16, mask, ek, ev, (__nv_bfloat16*)o_bf16, B, n_heads, T, w, chunk_tiles,
+                        part, err, 0);
+  if (rc == VSG_OK) {
+    int flag = 0;
+    cudaError_t ce = cudaDeviceSynchronize();
+    if (ce == cudaSuccess) ce = cudaMemcpy(&flag, err, sizeof(int), cudaMemcpyDeviceToHost);
+    if (ce != cudaSuccess) rc = fail(VSG_ECUDA, "split-key attention execution failed: %s", cudaGetErrorString(ce));
+    else if (flag) rc = fail(VSG_ECUDA, "relenc_attention_tc_kernel set its error flag (%d)", flag);
+  }
+  if (part) cudaFree(part);
   cudaFree(err);
   return rc;
 }

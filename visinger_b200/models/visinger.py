@@ -346,6 +346,11 @@ class VISinger(nn.Module):
     Extra keyword arguments (not in the reference): `noise` injects the prior noise instead of
     `torch.randn_like(mu_p)` (CPU and CUDA generators differ, so parity tests need it); `precision` selects
     "fp32" | "bf16" | "bf16x3" for the native path.
+
+    Supported lengths: utterances of any number of latent frames T up to T * hop <= 2^29 samples, in all three modes.
+    The prior network has no frame cap of its own: the length regulator works in fixed chunks of frames, and the bf16
+    attention splits the keys into chunks of 2048 frames beyond T = 2048 (a workspace of about
+    ceil(T / 2048) * B * T * hidden * 4 bytes per encoder).
     """
 
     def __init__(self, ph_dict_size, pitch_size, dur_size, hparams, out_dims=None, precision="fp32"):

@@ -2,11 +2,13 @@
 `modules/rel_transformer.py` (RelativeEncoder :257-320, MultiHeadAttention :103-254, FFN :323-345,
 LayerNorm :24-42, SinusoidalPositionalEmbedding :45-100).
 
-This is NOT on the B200 hot path: it is the prior network that runs before `z_p` (SURVEY.md 8f rows f1/f2),
-kept in PyTorch so that `visinger_b200.models.visinger.VISinger` is a complete drop-in for
-`VISinger.forward(infer=True)`.  It is written from the reference's behaviour, with the reference's parameter
-names and shapes (so checkpoints load), but in its own formulation: the relative-position logits/values are
-moved between "relative" and "absolute" indexing with diagonal views instead of the pad-and-reshape trick.
+These modules are the prior network that runs before `z_p` (SURVEY.md 8f rows f1/f2).  On a CUDA device
+`RelativeEncoder.forward` is one call into the native library (fp32 kernels, or tcgen05 kernels in bf16 mode, for
+utterances of any length), so the prior network runs on the GPU with the hot path.  The PyTorch formulation here is
+the readable statement of that arithmetic and the CPU path.  It is written from the reference's behaviour, with the
+reference's parameter names and shapes (so checkpoints load), but in its own formulation: the relative-position
+logits/values are moved between "relative" and "absolute" indexing with diagonal views instead of the pad-and-reshape
+trick.
 """
 from __future__ import annotations
 
