@@ -276,8 +276,83 @@ int vsg_length_regulate(const float* enc, const int64_t* mel2ph, const float* po
 int vsg_infer_zp(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav, float* z_q_out,
                  int32_t B, int32_t T, int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
 
+/*
+ * The whole model: VISinger.forward(infer=True) from note tokens to waveform in one call
+ * (VISinger(ph_dict_size, pitch_size, dur_size, hparams), the fields below; window_size is RelativeEncoder's 4,
+ * spk_embed_dim the 256 inputs of spk_embed_proj).  The speaker condition has hot.flow_gin (= hot.dec_gin) channels.
+ * use_pos_embed adds the sinusoidal frame positions to the prior input (models/visinger.py:79-82); the text encoder's own
+ * positional term (modules/visinger/encoder.py:50-53) is always on, as VISinger builds its TextEncoder with it.
+ */
+typedef struct VsgModelConfig {
+  int32_t ph_dict_size, pitch_size, dur_size;
+  int32_t hidden, filter, n_heads, ffn_kernel_size, window_size;   /* hidden_size, ffn_filter_channels, num_heads */
+  int32_t enc_layers, pitch_predictor_layers, frame_prior_layers;
+  int32_t use_pos_embed, use_pitch_embed, use_spk_id, use_spk_embed, num_spk, spk_embed_dim;
+  VsgConfig hot;   /* flow + decoder, as vsg_pack_create takes it */
+} VsgModelConfig;
+
+/*
+ * Pre-pack of a whole VISinger state dict: `weights` are the checkpoint's entries under `prefix` ("" or "model.").
+ * Builds the existing pack types inside (text_encoder.text_encoder.*, pitch_predictor.pitch_predictor.*, frame_prior.*,
+ * flow.* + decoder.*) and uploads the token-rate weights: the three embedding tables, text_encoder.linear,
+ * spk_id_proj / spk_embed_proj, pitch_predictor.linear.  posterior_encoder.*, phoneme_predictor.* and *._float_tensor are
+ * ignored.  A missing required entry returns VSG_EINVAL naming it.
+ *   Optional entry `prefix` + "embed_positions.freq" ([hidden / 2] fp32): the frequencies of the sinusoidal position
+ * table, exp(k * -(ln 10000 / (hidden/2 - 1))), as the framework that made the reference's table computed them
+ * (SinusoidalPositionalEmbedding.get_embedding evaluates that exp in fp32 with torch's CPU exp, which is not correctly
+ * rounded).  Without it they are the correctly rounded fp32 values; at hidden = 192 one of the 96 differs from torch's by
+ * one ulp, which moves the table by up to 7.6e-6 at position 30 000 (1.2e-4 at hidden = 256).
+ * The result is freed by vsg_pack_destroy and accepted only by vsg_model_*.
+ */
+int vsg_model_pack_create(const VsgModelConfig* cfg, const VsgTensor* weights, int32_t n_weights, const char* prefix,
+                          int32_t device, VsgPack** out);
+/* Bytes of workspace vsg_model_forward needs for (B, T_ph, T) in `precision`; 0 on invalid arguments. */
+size_t vsg_model_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T_ph, int32_t T, int32_t precision);
+
+/*
+ * VISinger.forward(text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed, spk_id, f0, uv, infer=True)
+ * -> wav [B, T * hop] (and f0_pred, z_q).  Device pointers unless noted:
+ *   text_tokens, pitch_tokens, dur_tokens: int64 [B, T_ph], 0 = padding; mel2ph: int64 [B, T], 1-based, 0 = padding;
+ *   spk_id: HOST int64 [B] iff use_spk_id (else NULL), each in [0, num_spk) -- it is checked before anything is launched,
+ *     so it is read at call time: a CUDA graph captured from this call replays the ids of the capture;
+ *   spk_embed: fp32 [B, spk_embed_dim] iff use_spk_embed (else NULL);
+ *   f0, uv: fp32 [B, T] each, or both NULL = the pitch predictor's own (f0 = pred[..., 0], voiced = pred[..., 1] <= 0;
+ *     given: voiced = uv == 0); both must be NULL without use_pitch_embed;
+ *   noise: fp32 [B, hidden, T] prior noise, or NULL: drawn as vsg_normal_noise(seeds) -- seeds: uint64 [B], used iff
+ *     noise is NULL;
+ *   wav: fp32 [B, T * hop]; f0_pred: fp32 [B, T, 2] or NULL (NULL without use_pitch_embed); z_q_out: fp32 [B, hidden, T]
+ *     or NULL.
+ * Precision: the RelativeEncoder stacks and the frame-prior head run bf16 in VSG_PRECISION_BF16 and fp32 otherwise; the
+ * flow and decoder run as in vsg_infer_zp.  The token-rate glue (embeddings, Linear(3H -> H), speaker condition, pitch
+ * head) is fp32 on CUDA cores in every mode.  Token and mel2ph values are device data and are not checked: an id outside
+ * its table reads a zero row, a mel2ph entry above T_ph a padding frame.  Argument errors return VSG_EINVAL, a workspace
+ * smaller than vsg_model_workspace_bytes VSG_ENOMEM, both before any launch.  Any T and T_ph the stacks take are accepted.
+ */
+int vsg_model_forward(const VsgPack* pack, const int64_t* text_tokens, const int64_t* pitch_tokens,
+                      const int64_t* dur_tokens, const int64_t* mel2ph, const int64_t* spk_id, const float* spk_embed,
+                      const float* f0, const float* uv, const float* noise, const uint64_t* seeds, float* wav,
+                      float* f0_pred, float* z_q_out, int32_t B, int32_t T_ph, int32_t T, int32_t precision,
+                      void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Seeded standard-normal noise, out: fp32 [B, C, T].  Element (b, c, t) is Box-Muller on one Philox4x32-10 draw with
+ * key (lo32(seeds[b]), hi32(seeds[b])) and counter (t, c, 0, 0): with x0, x1 its first two words,
+ *   u1 = (x0 + 1) / 2^32,  u2 = x1 / 2^32,  out = fp32( sqrt(-2 ln u1) * cos(2 pi u2) )   (evaluated in double)
+ * -- so an utterance's noise depends on its seed only, not on B, its batch neighbours or the padded length.
+ * seeds: device uint64 [B].  Asynchronous, no allocation, capturable.
+ */
+int vsg_normal_noise(const uint64_t* seeds, float* out, int32_t B, int32_t C, int32_t T, void* stream);
+
+/*
+ * The sinusoidal position table vsg_model_forward builds in its workspace (SinusoidalPositionalEmbedding.get_embedding,
+ * padding_idx 0): out[p, k] = sin(a), out[p, half + k] = cos(a) with a = fp32(p) * freq[k] rounded to fp32 and sin / cos
+ * evaluated in double, rounded to fp32; row 0 and an odd dim's last column are 0.  freq: device fp32 [dim / 2], or NULL
+ * for the correctly rounded values (see vsg_model_pack_create).  out: device fp32 [rows, dim].  Asynchronous.
+ */
+int vsg_debug_position_table(const float* freq, int32_t rows, int32_t dim, float* out, void* stream);
+
 /* Samples produced per latent frame (prod(upsample_rates)); 0 if the pack has no decoder. */
-int32_t vsg_hop_size(const VsgPack* pack);
+int32_t vsg_hop_size(const VsgPack* pack);   /* (a model pack: its decoder's) */
 
 /* Number of kernels launched by the most recent run call on this thread (bench bookkeeping). */
 int32_t vsg_last_launch_count(void);

@@ -10,6 +10,7 @@ from __future__ import annotations
 
 import ctypes
 import hashlib
+import math
 import os
 import shutil
 import subprocess
@@ -23,7 +24,7 @@ _CSRC = os.path.join(_HERE, "csrc")
 _LIBDIR = os.path.join(_HERE, "lib")
 _LIBPATH = os.path.join(_LIBDIR, "libvisinger_b200.so")
 _HEADER = os.path.join(os.path.dirname(_HERE), "include", "visinger_b200.h")
-_SOURCES = ["api.cu", "pack.cu", "run_f32.cu", "run_tc.cu", "output.cu"]
+_SOURCES = ["api.cu", "pack.cu", "run_f32.cu", "run_tc.cu", "output.cu", "model.cu"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC", "-diag-suppress", "550"]
@@ -74,6 +75,13 @@ class VsgRelEncConfig(ctypes.Structure):
     _fields_ = [("hidden_channels", ctypes.c_int32), ("filter_channels", ctypes.c_int32), ("n_heads", ctypes.c_int32),
                 ("n_layers", ctypes.c_int32), ("kernel_size", ctypes.c_int32), ("window_size", ctypes.c_int32),
                 ("gin_channels", ctypes.c_int32)]
+
+
+class VsgModelConfig(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in (
+        "ph_dict_size", "pitch_size", "dur_size", "hidden", "filter", "n_heads", "ffn_kernel_size", "window_size",
+        "enc_layers", "pitch_predictor_layers", "frame_prior_layers", "use_pos_embed", "use_pitch_embed", "use_spk_id",
+        "use_spk_embed", "num_spk", "spk_embed_dim")] + [("hot", VsgConfig)]
 
 
 class VsgTensor(ctypes.Structure):
@@ -224,6 +232,17 @@ def lib() -> ctypes.CDLL:
         L.vsg_debug_attention_split_bf16.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32]
         L.vsg_debug_layernorm_bf16.restype = ctypes.c_int
         L.vsg_debug_layernorm_bf16.argtypes = [vp, vp, vp, vp, i32, vp, ctypes.c_float, i32, i32, i32, i32]
+        L.vsg_model_pack_create.restype = ctypes.c_int
+        L.vsg_model_pack_create.argtypes = [ctypes.POINTER(VsgModelConfig), ctypes.POINTER(VsgTensor), i32, ctypes.c_char_p,
+                                            i32, ctypes.POINTER(ctypes.c_void_p)]
+        L.vsg_model_workspace_bytes.restype = sz
+        L.vsg_model_workspace_bytes.argtypes = [vp, i32, i32, i32, i32]
+        L.vsg_model_forward.restype = ctypes.c_int
+        L.vsg_model_forward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, sz, vp]
+        L.vsg_normal_noise.restype = ctypes.c_int
+        L.vsg_normal_noise.argtypes = [vp, vp, i32, i32, i32, vp]
+        L.vsg_debug_position_table.restype = ctypes.c_int
+        L.vsg_debug_position_table.argtypes = [vp, i32, i32, vp, vp]
         if L.vsg_abi_version() != 1:
             raise RuntimeError("visinger_b200: ABI version mismatch between _lib.py and the shared library")
         _lib = L
@@ -379,6 +398,72 @@ class RelEncPack:
                 self._h = ctypes.c_void_p()
         except Exception:
             pass
+
+
+def position_freq(dim: int) -> torch.Tensor:
+    """The frequencies of SinusoidalPositionalEmbedding.get_embedding, from the same torch expression (CPU fp32), so that
+    the native table is that table: torch's fp32 exp is not correctly rounded."""
+    half = dim // 2
+    return torch.exp(torch.arange(half, dtype=torch.float) * -(math.log(10000) / (half - 1)))
+
+
+class ModelPack:
+    """Owner of the VsgPack* of a whole VISinger (vsg_model_pack_create): `state_dict` is the model's (reference
+    checkpoint keys under `prefix`); the entry `prefix + "embed_positions.freq"` is added from `position_freq`."""
+
+    def __init__(self, cfg: VsgModelConfig, state_dict: Dict[str, torch.Tensor], prefix: str, device: torch.device):
+        self._h = ctypes.c_void_p()
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("visinger_b200: weights must live on a CUDA device; there is no CPU fallback")
+        host = {k: v.detach().to("cpu", torch.float32).contiguous() for k, v in state_dict.items() if k.startswith(prefix)}
+        host[prefix + "embed_positions.freq"] = position_freq(cfg.hidden)
+        arr, keep = _weight_table(host)
+        idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        rc = lib().vsg_model_pack_create(ctypes.byref(cfg), arr, len(host), prefix.encode(), idx, ctypes.byref(self._h))
+        check(rc, "vsg_model_pack_create")
+        self.cfg = cfg
+        self.index = idx
+        self.hop = int(lib().vsg_hop_size(self._h))
+
+    @property
+    def handle(self):
+        return self._h
+
+    def workspace_bytes(self, B: int, T_ph: int, T: int, precision: int) -> int:
+        return int(lib().vsg_model_workspace_bytes(self._h, B, T_ph, T, precision))
+
+    def __del__(self):
+        try:
+            if self._h and _lib is not None:
+                _lib.vsg_pack_destroy(self._h)
+                self._h = ctypes.c_void_p()
+        except Exception:
+            pass
+
+
+def normal_noise(seeds: torch.Tensor, C: int, T: int) -> torch.Tensor:
+    """vsg_normal_noise: seeds CUDA int64 [B] (read as uint64) -> fp32 [B, C, T], element (b, c, t) a function of
+    (seeds[b], c, t) only."""
+    require_cuda(seeds, "seeds")
+    s = seeds.to(torch.int64).contiguous()
+    out = torch.empty(s.numel(), C, T, dtype=torch.float32, device=s.device)
+    with torch.cuda.device(s.device):
+        rc = lib().vsg_normal_noise(s.data_ptr(), out.data_ptr(), s.numel(), C, T, stream_ptr(s.device))
+    check(rc, "vsg_normal_noise")
+    return out
+
+
+def debug_position_table(rows: int, dim: int, freq: Optional[torch.Tensor], device) -> torch.Tensor:
+    """vsg_debug_position_table: the sinusoidal table [rows, dim] the model call builds (freq None = correctly rounded)."""
+    device = torch.device(device)
+    fq = as_f32c(freq.to(device)) if freq is not None else None
+    out = torch.empty(rows, dim, dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        rc = lib().vsg_debug_position_table(fq.data_ptr() if fq is not None else None, rows, dim, out.data_ptr(),
+                                            stream_ptr(device))
+    check(rc, "vsg_debug_position_table")
+    return out
 
 
 def length_regulate(enc: torch.Tensor, mel2ph: torch.Tensor, pos_table: Optional[torch.Tensor]) -> torch.Tensor:

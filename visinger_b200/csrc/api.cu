@@ -15,16 +15,6 @@ int check_common(const VsgPack* pack, int B, int T, int precision) {
   return VSG_OK;
 }
 
-struct DeviceGuard {
-  int prev = -1;
-  bool ok = true;
-  explicit DeviceGuard(int dev) {
-    if (cudaGetDevice(&prev) != cudaSuccess) { ok = false; return; }
-    if (prev != dev && cudaSetDevice(dev) != cudaSuccess) ok = false;
-  }
-  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-
 size_t flow_ws(const VsgPack* p, int B, int T, int prec) {
   if (!p->has_flow) return 0;
   if (prec == VSG_PRECISION_BF16) return flow_ws_bytes_tc(p, B, T, 1);
@@ -247,9 +237,15 @@ extern "C" int vsg_infer_zp(const VsgPack* pack, const float* z_p, const float* 
   if (!workspace) return fail(VSG_ENOMEM, "workspace is NULL");
   DeviceGuard dg(pack->device);
   if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
-  cudaStream_t st = (cudaStream_t)stream;
-  const int C = pack->cfg.flow_channels;
   Workspace ws(workspace, workspace_bytes);
+  return infer_zp_run(pack, z_p, mask, g, wav, z_q_out, B, T, precision, ws, (cudaStream_t)stream);
+}
+
+namespace vsg {
+
+int infer_zp_run(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav, float* z_q_out,
+                 int B, int T, int precision, Workspace& ws, cudaStream_t st) {
+  const int C = pack->cfg.flow_channels;
   float* z = ws.take<float>((size_t)B * C * T);
   if (ws.overflow) return fail(VSG_ENOMEM, "workspace too small");
   const size_t mark = ws.off;
@@ -265,3 +261,5 @@ extern "C" int vsg_infer_zp(const VsgPack* pack, const float* z_p, const float* 
   else VSG_TRY(generator_forward_tc(pack, zq, g, wav, B, T, ws, st, precision == VSG_PRECISION_BF16X3));
   return VSG_OK;
 }
+
+}  // namespace vsg

@@ -543,7 +543,10 @@ using namespace vsg;
 extern "C" int vsg_abi_version(void) { return VSG_ABI_VERSION; }
 extern "C" const char* vsg_last_error(void) { return vsg::g_err; }
 extern "C" int32_t vsg_last_launch_count(void) { return vsg::g_launches; }
-extern "C" int32_t vsg_hop_size(const VsgPack* p) { return (p && p->has_dec) ? p->hop : 0; }
+extern "C" int32_t vsg_hop_size(const VsgPack* p) {
+  if (p && p->model) p = p->model->hot;
+  return (p && p->has_dec) ? p->hop : 0;
+}
 
 extern "C" int vsg_pack_create(const VsgConfig* cfg, const VsgTensor* weights, int32_t n_weights,
                                const char* flow_prefix, const char* dec_prefix, int32_t device, VsgPack** out) {
@@ -691,6 +694,7 @@ static int relenc_pack_create(const VsgRelEncConfig* cfg, const VsgTensor* weigh
 
 extern "C" void vsg_pack_destroy(VsgPack* pack) {
   if (!pack) return;
+  if (pack->model) vsg::model_pack_free(pack->model);
   int prev = 0;
   cudaGetDevice(&prev);
   cudaSetDevice(pack->device);

@@ -62,4 +62,8 @@ int frame_prior_forward_tc(const VsgPack* P, const float* x, const float* mask, 
 int length_regulate(const float* enc, const long long* mel2ph, const float* table, int table_rows, float* y, int B, int H,
                     int T_ph, int T, cudaStream_t st);
 
+// vsg_infer_zp after validation (api.cu): flow reverse from z_p, mask, decoder; shared with vsg_model_forward
+int infer_zp_run(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav, float* z_q_out,
+                 int B, int T, int precision, Workspace& ws, cudaStream_t st);
+
 }  // namespace vsg

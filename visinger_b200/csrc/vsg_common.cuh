@@ -146,9 +146,26 @@ struct UpStage {
   std::vector<ResBlockPack> blocks;
 };
 
+// The whole model (vsg_model_pack_create): the four sub-packs of the existing pack types plus the token-rate weights that
+// no stack owns.  Device arrays live in the owning VsgPack's `allocs`; the sub-packs are destroyed with it.
+struct ModelPack {
+  VsgModelConfig cfg;
+  VsgPack *text = nullptr, *pitch = nullptr, *prior = nullptr, *hot = nullptr;
+  const float *ph_emb = nullptr, *pitch_emb = nullptr, *dur_emb = nullptr;   // [n][H]
+  const float* lin_wt = nullptr;       // text_encoder.linear.weight transposed: [3H][H]
+  const float* lin_b = nullptr;        // [H]
+  const float* spk_id_w = nullptr;     // spk_id_proj.weight [num_spk][gin]
+  const float *spk_embed_w = nullptr, *spk_embed_b = nullptr;   // spk_embed_proj: [gin][spk_embed_dim], [gin]
+  const float *pitch_w = nullptr, *pitch_b = nullptr;           // pitch_predictor.linear: [2][H], [2]
+  const float* freq = nullptr;         // embed_positions.freq [H/2], or null: computed on the device
+  int gin = 0;
+};
+void model_pack_free(ModelPack* m);
+
 }  // namespace vsg
 
 struct VsgPack {
+  vsg::ModelPack* model = nullptr;
   VsgConfig cfg;
   int device = 0;
   int hop = 0;
@@ -192,5 +209,16 @@ struct Workspace {
 };
 
 inline size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
+
+// Makes `dev` current for the scope of a run call and restores the caller's device.
+struct DeviceGuard {
+  int prev = -1;
+  bool ok = true;
+  explicit DeviceGuard(int dev) {
+    if (cudaGetDevice(&prev) != cudaSuccess) { ok = false; return; }
+    if (prev != dev && cudaSetDevice(dev) != cudaSuccess) ok = false;
+  }
+  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+};
 
 }  // namespace vsg

@@ -340,8 +340,9 @@ class VISinger(nn.Module):
     and frame prior (`vsg_relenc_forward`), the length regulator with its data-dependent frame positions
     (`vsg_length_regulate`) and the fused frame-prior head (`vsg_frame_prior_forward`: encoder -> proj -> prior sampling);
     from `z_p` on -- flow reverse, HiFi-GAN decoder (models/visinger.py:107-111) -- one `vsg_infer_zp` call.  What stays in
-    PyTorch is token-rate glue: three embedding lookups, one Linear(576 -> 192), the speaker embedding and the 1x1 head of
-    the pitch predictor.  `infer=False` (training) is out of scope and raises.
+    PyTorch in `forward` is token-rate glue: three embedding lookups, one Linear(576 -> 192), the speaker embedding and the
+    1x1 head of the pitch predictor.  `forward_native` runs the same model, glue included, as one `vsg_model_forward`
+    call.  `infer=False` (training) is out of scope and raises.
 
     Extra keyword arguments (not in the reference): `noise` injects the prior noise instead of
     `torch.randn_like(mu_p)` (CPU and CUDA generators differ, so parity tests need it); `precision` selects
@@ -451,6 +452,93 @@ class VISinger(nn.Module):
             static[k].copy_(v, non_blocking=True)
         graph.replay()
         return out
+
+    def _model_pack(self, device) -> "_lib.ModelPack":
+        """The whole-model pack (vsg_model_pack_create), rebuilt when a parameter's storage or version changes."""
+        wkey = (str(device),) + tuple((p.data_ptr(), p._version) for p in self.parameters())
+        cached = self.__dict__.get("_native_pack")
+        if cached is None or cached[0] != wkey:
+            hp = self.hparams
+            te = self.text_encoder
+            cfg = _lib.VsgModelConfig(
+                te.ph_emb.num_embeddings, te.pitch_emb.num_embeddings, te.dur_emb.num_embeddings, self.hidden_size,
+                hp["ffn_filter_channels"], hp["num_heads"], hp["ffn_kernel_size"], te.text_encoder.window_size,
+                self.enc_layers, hp["pitch_predictor_layers"] if hp["use_pitch_embed"] else 0, hp["frame_prior_layers"],
+                int(bool(self.use_pos_embed)), int(bool(hp["use_pitch_embed"])), int(bool(hp["use_spk_id"])),
+                int(bool(hp["use_spk_embed"])), hp["num_spk"] if hp["use_spk_id"] else 0,
+                self.spk_embed_proj.in_features if hp["use_spk_embed"] else 0, self._hot._vsg_config())
+            pack = _lib.ModelPack(cfg, dict(self.state_dict()), "", device)
+            self.__dict__["_native_pack"] = cached = (wkey, pack)
+        return cached[1]
+
+    @torch.no_grad()
+    def forward_native(self, text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed=None, spk_id=None, f0=None, uv=None,
+                       noise=None, seeds=None):
+        """`forward(..., infer=True)` as ONE library call (vsg_model_forward): token front end, the three RelativeEncoder
+        stacks, length regulator, speaker condition, pitch head, frame prior, flow and decoder, with no PyTorch op in
+        between.  Same inputs and result keys (`wav_out` [B, T*hop], `f0_pred` [B, T, 2] with the pitch predictor, `z_q`
+        [B, H, T]).  The prior noise is `noise` [B, H, T] if given, else drawn on the device from `seeds` (int64 [B], one
+        Philox stream per utterance: vsg_normal_noise), else from seeds taken from torch's default CPU generator.
+        `spk_id` is read on the host (the library range-checks it before it launches anything)."""
+        hp = self.hparams
+        ins = {"text_tokens": text_tokens, "pitch_tokens": pitch_tokens, "dur_tokens": dur_tokens, "mel2ph": mel2ph}
+        if hp["use_spk_embed"]:
+            ins["spk_embed"] = spk_embed
+        if hp["use_pitch_embed"] and (f0 is not None or uv is not None):
+            ins["f0"], ins["uv"] = f0, uv
+        if noise is not None:
+            ins["noise"] = noise
+        elif seeds is not None:
+            ins["seeds"] = seeds
+        for k, v in ins.items():
+            if v is None:
+                raise RuntimeError(f"{k} is required by this model's configuration")
+            _lib.require_cuda(v, k)
+        if text_tokens.dim() != 2 or mel2ph.dim() != 2 or mel2ph.shape[0] != text_tokens.shape[0]:
+            raise RuntimeError("expected tokens [B, T_ph] and mel2ph [B, T]")
+        B, T_ph = text_tokens.shape
+        T, H = mel2ph.shape[1], self.hidden_size
+        shapes = {"pitch_tokens": (B, T_ph), "dur_tokens": (B, T_ph), "f0": (B, T), "uv": (B, T), "noise": (B, H, T),
+                  "seeds": (B,)}
+        if hp["use_spk_embed"]:
+            shapes["spk_embed"] = (B, self.spk_embed_proj.in_features)
+        for k, shape in shapes.items():
+            if k in ins and tuple(ins[k].shape) != shape:
+                raise RuntimeError(f"expected {k} of shape {shape}, got {tuple(ins[k].shape)}")
+        dev = mel2ph.device
+        for k, v in ins.items():
+            if v.device != dev:
+                raise RuntimeError(f"{k} is on {v.device}, mel2ph on {dev}")
+        spk_host = None
+        if hp["use_spk_id"]:
+            if spk_id is None:
+                raise RuntimeError("spk_id is required by this model's configuration")
+            spk_host = torch.as_tensor(spk_id).to("cpu", torch.int64).contiguous().reshape(-1)
+            if spk_host.numel() != B:
+                raise RuntimeError(f"expected spk_id of shape ({B},), got {tuple(torch.as_tensor(spk_id).shape)}")
+        if "noise" not in ins and "seeds" not in ins:
+            ins["seeds"] = torch.randint(0, 2 ** 62, (B,), dtype=torch.int64).to(dev)
+        a = {k: v.to(torch.int64).contiguous() if k in ("text_tokens", "pitch_tokens", "dur_tokens", "mel2ph", "seeds")
+             else _lib.as_f32c(v) for k, v in ins.items()}
+        pack = self._model_pack(dev)
+        prec = _lib.precision_code(self.precision)
+        wav = torch.empty(B, T * pack.hop, dtype=torch.float32, device=dev)
+        f0_pred = torch.empty(B, T, 2, dtype=torch.float32, device=dev) if hp["use_pitch_embed"] else None
+        z_q = torch.empty(B, H, T, dtype=torch.float32, device=dev)
+        ptr = lambda k: a[k].data_ptr() if k in a else None   # noqa: E731
+        with torch.cuda.device(dev):
+            ws = _lib.workspace(dev, pack.workspace_bytes(B, T_ph, T, prec))
+            rc = _lib.lib().vsg_model_forward(
+                pack.handle, ptr("text_tokens"), ptr("pitch_tokens"), ptr("dur_tokens"), ptr("mel2ph"),
+                spk_host.data_ptr() if spk_host is not None else None, ptr("spk_embed"), ptr("f0"), ptr("uv"), ptr("noise"),
+                ptr("seeds"), wav.data_ptr(), f0_pred.data_ptr() if f0_pred is not None else None, z_q.data_ptr(), B, T_ph,
+                T, prec, ws.data_ptr(), ws.numel(), _lib.stream_ptr(dev))
+        _lib.check(rc, "vsg_model_forward")
+        self.last_launches = _lib.last_launch_count()
+        ret = {"wav_out": wav, "z_q": z_q}
+        if f0_pred is not None:
+            ret["f0_pred"] = f0_pred
+        return ret
 
     def prior(self, text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed=None, spk_id=None, f0=None, uv=None,
               ret=None, noise=None, sample=False):
