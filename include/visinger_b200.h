@@ -335,6 +335,62 @@ int vsg_model_forward(const VsgPack* pack, const int64_t* text_tokens, const int
                       void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * Voice conversion (VITS SynthesizerTrn.voice_conversion on VISinger's modules), from a waveform or a linear spectrogram:
+ *   spec  = linear_spectrogram(wav)                          [B, bins, T], bins = n_fft / 2 + 1
+ *   z     = posterior_encoder(spec, mask, g_src, noise)      (modules/visinger/encoder.py:92-98)
+ *   z_hat = flow(flow(z, mask, g_src), mask, g_tgt, reverse) * mask
+ *   wav'  = decoder(z_hat * mask, g_tgt)                     g_* = speaker_embedding of the source / target speaker
+ *
+ * vsg_convert_pack_create builds what vsg_model_pack_create builds (vsg_model_forward accepts the result and computes the
+ * same bits on it) plus the `prefix` + "posterior_encoder.*" pack -- PosteriorEncoder(bins, hidden, hidden, kernel, 1,
+ * n_layers, gin), bins, kernel and n_layers read from the weights -- and the spectrogram's DFT basis.  n_fft =
+ * 2 * (bins - 1); the hop is the decoder's, prod(upsample_rates), so spectrogram frames are latent frames; win_length
+ * (1 .. n_fft) is the periodic Hann window's length, zero-padded centrally to n_fft as torch.stft pads it.  VSG_EINVAL on
+ * a missing entry (named in the message), on win_length outside [1, n_fft] and on n_fft < hop.
+ *
+ * The linear spectrogram (VITS spectrogram_torch, per utterance): frame f covers samples [f*hop - p, f*hop - p + n_fft),
+ * p = (n_fft - hop) / 2 (rounded down); samples outside utterance b's own [0, lengths[b] * hop) are reflected about its
+ * ends as torch's 'reflect' padding does (no edge repeat, folded again while outside);
+ * spec = sqrt(re^2 + im^2 + 1e-6) * mask.  When n_fft - hop is even this is spectrogram_torch of the utterance alone,
+ * frame for frame.  It runs as Conv1d(hop -> 2 * bins, ceil(win_length / hop)) over the signal cut into rows of hop
+ * samples, with the window-folded DFT basis (evaluated in double, rounded once to fp32) as weights: on tcgen05 in bf16
+ * (operands rounded to bf16, fp32 accumulation) in VSG_PRECISION_BF16, on the FFMA kernel in fp32 otherwise.
+ *
+ * Common arguments (device pointers unless noted):
+ *   wav: fp32 [B, T * hop]; utterance b is its first lengths[b] * hop samples;
+ *   lengths: int32 [B], valid latent frames per utterance; device data, clamped to [0, T] and not checked otherwise;
+ *     mask [b, t] = t < lengths[b].
+ * vsg_convert_workspace_bytes covers vsg_spectrogram and vsg_model_convert (0 on invalid arguments).
+ */
+int vsg_convert_pack_create(const VsgModelConfig* cfg, const VsgTensor* weights, int32_t n_weights, const char* prefix,
+                            int32_t win_length, int32_t device, VsgPack** out);
+size_t vsg_convert_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t precision);
+
+/* spec: fp32 [B, bins, T].  In VSG_PRECISION_BF16 it holds the bf16 values the posterior consumes, widened. */
+int vsg_spectrogram(const VsgPack* pack, const float* wav, const int32_t* lengths, float* spec, int32_t B, int32_t T,
+                    int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Exactly one of wav (fp32 [B, T * hop]) and spec (fp32 [B, bins, T], e.g. the reference's forward(..., mel=...) input).
+ *   src_spk_id, tgt_spk_id: HOST int64 [B] iff use_spk_id (else NULL), range-checked before any launch (a CUDA graph
+ *     captured from this call replays the ids of the capture); src_spk_embed, tgt_spk_embed: fp32 [B, spk_embed_dim] iff
+ *     use_spk_embed;
+ *   noise: fp32 [B, hidden, T] posterior noise, or NULL: vsg_normal_noise(seeds) (uint64 [B], used iff noise is NULL);
+ *   wav_out: fp32 [B, T * hop]; spec_out: fp32 [B, bins, T] or NULL, the spectrogram of wav (NULL when spec is given);
+ *   z_out: fp32 [B, hidden, T] or NULL, receives z_hat.
+ * Precision: the spectrogram and the posterior run bf16 in VSG_PRECISION_BF16 and fp32 otherwise (as
+ * vsg_posterior_forward); the flow runs in both directions and the decoder runs as in vsg_infer_zp.  The result equals
+ * vsg_spectrogram -> vsg_posterior_forward -> vsg_flow_forward(reverse = 0) -> vsg_infer_zp bit for bit.  Argument errors
+ * return VSG_EINVAL, a workspace smaller than vsg_convert_workspace_bytes VSG_ENOMEM, both before any launch.  No
+ * allocation, no synchronisation: capturable.
+ */
+int vsg_model_convert(const VsgPack* pack, const float* wav, const float* spec, const int32_t* lengths,
+                      const int64_t* src_spk_id, const float* src_spk_embed, const int64_t* tgt_spk_id,
+                      const float* tgt_spk_embed, const float* noise, const uint64_t* seeds, float* wav_out,
+                      float* spec_out, float* z_out, int32_t B, int32_t T, int32_t precision, void* workspace,
+                      size_t workspace_bytes, void* stream);
+
+/*
  * Seeded standard-normal noise, out: fp32 [B, C, T].  Element (b, c, t) is Box-Muller on one Philox4x32-10 draw with
  * key (lo32(seeds[b]), hi32(seeds[b])) and counter (t, c, 0, 0): with x0, x1 its first two words,
  *   u1 = (x0 + 1) / 2^32,  u2 = x1 / 2^32,  out = fp32( sqrt(-2 ln u1) * cos(2 pi u2) )   (evaluated in double)

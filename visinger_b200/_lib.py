@@ -239,6 +239,15 @@ def lib() -> ctypes.CDLL:
         L.vsg_model_workspace_bytes.argtypes = [vp, i32, i32, i32, i32]
         L.vsg_model_forward.restype = ctypes.c_int
         L.vsg_model_forward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, sz, vp]
+        L.vsg_convert_pack_create.restype = ctypes.c_int
+        L.vsg_convert_pack_create.argtypes = [ctypes.POINTER(VsgModelConfig), ctypes.POINTER(VsgTensor), i32,
+                                              ctypes.c_char_p, i32, i32, ctypes.POINTER(ctypes.c_void_p)]
+        L.vsg_convert_workspace_bytes.restype = sz
+        L.vsg_convert_workspace_bytes.argtypes = [vp, i32, i32, i32]
+        L.vsg_spectrogram.restype = ctypes.c_int
+        L.vsg_spectrogram.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, sz, vp]
+        L.vsg_model_convert.restype = ctypes.c_int
+        L.vsg_model_convert.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, sz, vp]
         L.vsg_normal_noise.restype = ctypes.c_int
         L.vsg_normal_noise.argtypes = [vp, vp, i32, i32, i32, vp]
         L.vsg_debug_position_table.restype = ctypes.c_int
@@ -440,6 +449,53 @@ class ModelPack:
                 self._h = ctypes.c_void_p()
         except Exception:
             pass
+
+
+class ConvertPack(ModelPack):
+    """Owner of the VsgPack* of a whole VISinger with its posterior encoder and linear spectrogram
+    (vsg_convert_pack_create): everything a ModelPack holds, plus `prefix + "posterior_encoder.*"` and the DFT basis of
+    a periodic Hann window of `win_length` samples."""
+
+    def __init__(self, cfg: VsgModelConfig, state_dict: Dict[str, torch.Tensor], prefix: str, win_length: int,
+                 device: torch.device):
+        self._h = ctypes.c_void_p()
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("visinger_b200: weights must live on a CUDA device; there is no CPU fallback")
+        host = {k: v.detach().to("cpu", torch.float32).contiguous() for k, v in state_dict.items() if k.startswith(prefix)}
+        host[prefix + "embed_positions.freq"] = position_freq(cfg.hidden)
+        arr, keep = _weight_table(host)
+        idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        rc = lib().vsg_convert_pack_create(ctypes.byref(cfg), arr, len(host), prefix.encode(), int(win_length), idx,
+                                           ctypes.byref(self._h))
+        check(rc, "vsg_convert_pack_create")
+        self.cfg = cfg
+        self.index = idx
+        self.hop = int(lib().vsg_hop_size(self._h))
+        self.bins = int(host[prefix + "posterior_encoder.pre.weight"].shape[1])
+        self.win_length = int(win_length)
+
+    def convert_workspace_bytes(self, B: int, T: int, precision: int) -> int:
+        return int(lib().vsg_convert_workspace_bytes(self._h, B, T, precision))
+
+    def spectrogram(self, wav: torch.Tensor, lengths: torch.Tensor, precision: int) -> torch.Tensor:
+        """vsg_spectrogram: wav CUDA fp32 [B, T * hop], lengths CUDA int32 [B] (latent frames) -> fp32 [B, bins, T]."""
+        require_cuda(wav, "wav")
+        require_cuda(lengths, "lengths")
+        B, L = wav.shape
+        if L % self.hop or lengths.numel() != B:
+            raise RuntimeError(f"expected wav [B, T * {self.hop}] and lengths [B]")
+        T = L // self.hop
+        w, ln = as_f32c(wav), lengths.to(torch.int32).contiguous()
+        spec = torch.empty(B, self.bins, T, dtype=torch.float32, device=wav.device)
+        if B == 0 or T == 0:
+            return spec
+        with torch.cuda.device(wav.device):
+            ws = workspace(wav.device, self.convert_workspace_bytes(B, T, precision))
+            rc = lib().vsg_spectrogram(self._h, w.data_ptr(), ln.data_ptr(), spec.data_ptr(), B, T, precision,
+                                       ws.data_ptr(), ws.numel(), stream_ptr(wav.device))
+        check(rc, "vsg_spectrogram")
+        return spec
 
 
 def normal_noise(seeds: torch.Tensor, C: int, T: int) -> torch.Tensor:

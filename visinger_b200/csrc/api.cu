@@ -21,13 +21,22 @@ size_t flow_ws(const VsgPack* p, int B, int T, int prec) {
   if (prec == VSG_PRECISION_BF16X3) return std::max(flow_ws_bytes_tc(p, B, T, 3), flow_ws_bytes_f32(p, B, T));
   return flow_ws_bytes_f32(p, B, T);
 }
+size_t dec_ws(const VsgPack* p, int B, int T, int prec) {
+  if (!p->has_dec) return 0;
+  return prec == VSG_PRECISION_FP32 ? dec_ws_bytes_f32(p, B, T) : dec_ws_bytes_tc(p, B, T, prec == VSG_PRECISION_BF16X3);
+}
+
+}  // namespace
+
+namespace vsg {
+
 // fp32: CUDA-core FFMA kernels.  bf16: tcgen05, one bf16 plane.  bf16x3: tcgen05 on three bf16 planes per value (the
 // flow's z <= 1e-5 needs all 24 mantissa bits of its state; the decoder's 1e-4 is met by two planes).
 // *masked (optional): in = the caller wants y * mask; out = true if the flow's last kernel applied it (tensor-core modes:
 // the mask rides on the final layout change), false if the caller still has to
 int run_flow(const VsgPack* pack, const float* x, const float* mask, const float* g, float* y, int B, int T, int reverse,
-             int precision, Workspace& ws, cudaStream_t st, bool* masked = nullptr, const float* ps_logs = nullptr,
-             const float* ps_noise = nullptr, bool* sampled = nullptr) {
+             int precision, Workspace& ws, cudaStream_t st, bool* masked, const float* ps_logs, const float* ps_noise,
+             bool* sampled) {
   // ps_logs / ps_noise (with `sampled`): x is mu_p; *sampled = true if the flow's first kernel drew the prior sample itself
   if (sampled) *sampled = false;
   const bool want = masked && *masked;
@@ -43,12 +52,8 @@ int run_flow(const VsgPack* pack, const float* x, const float* mask, const float
   }
   return flow_forward_f32(pack, x, mask, g, y, B, T, reverse, ws, st);
 }
-size_t dec_ws(const VsgPack* p, int B, int T, int prec) {
-  if (!p->has_dec) return 0;
-  return prec == VSG_PRECISION_FP32 ? dec_ws_bytes_f32(p, B, T) : dec_ws_bytes_tc(p, B, T, prec == VSG_PRECISION_BF16X3);
-}
 
-}  // namespace
+}  // namespace vsg
 
 extern "C" size_t vsg_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t precision) {
   if (check_common(pack, B, T, precision) != VSG_OK) return 0;

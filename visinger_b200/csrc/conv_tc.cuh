@@ -95,10 +95,11 @@ struct ConvTC {
   uint32_t e_out_swz_mask;      // swizzle of the output staging rows (GATE halves the row width)
   float* out_f32;               // optional fp32 copy of the raw value [B, Lout, Cout] (debug / parity hook); EPI_TC_TANH: the output
   int tanh_cols;                // EPI_TC_TANH: out_f32[(b * Lq + q) * tanh_cols + i] = tanh(acc[i]), i < tanh_cols (<= 4)
+  int mag_ch;                   // EPI_TC_MAG: output channels >= mag_ch are written as 0 (the consumer's zero pad channels)
   int* error_flag;              // set to 1 if a barrier wait times out
 };
 
-enum : int { EPI_TC_LINEAR = 0, EPI_TC_GATE = 1, EPI_TC_COUPLE = 2, EPI_TC_TANH = 3 };
+enum : int { EPI_TC_LINEAR = 0, EPI_TC_GATE = 1, EPI_TC_COUPLE = 2, EPI_TC_TANH = 3, EPI_TC_MAG = 4 };
 
 // Epilogue signatures: the decoder's two dominant epilogues get their own kernel instantiations in which every feature
 // flag is a compile-time constant.  The generic kernel carries 12 epilogue variants (3 chunk widths x 4 modes; ~15 k SASS
@@ -121,7 +122,8 @@ enum : int { EPI_SIG_GENERIC = 0, EPI_SIG_ACT = 1, EPI_SIG_RES_ACT = 2, EPI_SIG_
              EPI_SIG_POST = 8,     // conv_post on the row-packed stage output: tanh of <= 4 accumulator columns -> fp32 waveform
              EPI_SIG_ACT_X3 = 9, EPI_SIG_RES_ACT_X3 = 10,   // ACT / RES_ACT on two bf16 planes per tensor (the bf16x3 decoder)
              EPI_SIG_SUM0_X3 = 11, EPI_SIG_SUM1_X3 = 12, EPI_SIG_FINAL_X3 = 13,
-             EPI_SIG_COUNT = 14 };
+             EPI_SIG_MAG = 14,     // the linear spectrogram: |(re, im)| of interleaved channel pairs, masked, one bf16 output
+             EPI_SIG_COUNT = 15 };
 
 namespace tc {
 
@@ -391,6 +393,8 @@ __device__ __forceinline__ void stage_out(const float* v, uint32_t base, uint32_
 //                      the output tensor has Cout / 2 channels
 //       EPI_TC_COUPLE  m = (acc + bias) * mask; out = (add0 - m) * mask | m + add0 * mask  (flow.py:78,83)
 //       EPI_TC_TANH    wav = tanh(acc) of the first tanh_cols columns, fp32, straight to global memory (decoder.py:56-57)
+//       EPI_TC_MAG     channel pairs (2c, 2c+1) hold (re, im) of one frequency bin (the window-folded DFT basis):
+//                      out[c] = sqrt(re^2 + im^2 + 1e-6) * mask, 0 for c >= mag_ch; the output has Cout / 2 channels
 template <int CW, int MODE, int NP, int SIG = EPI_SIG_GENERIC>
 __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, const CUtensorMap& tmAdd1,
                                                  const CUtensorMap& tmRaw, const CUtensorMap& tmAct, const ConvTC& p,
@@ -399,7 +403,8 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
   using namespace tc;
   bar_base += 8u * (uint32_t)p.bar_slot0;
   tmem_base += (uint32_t)p.tmem_col0;
-  constexpr int OW = (MODE == EPI_TC_GATE) ? CW / 2 : CW;   // output channels per chunk
+  constexpr bool kPairs = MODE == EPI_TC_GATE || MODE == EPI_TC_MAG;   // two accumulator columns per output channel
+  constexpr int OW = kPairs ? CW / 2 : CW;   // output channels per chunk
   const int tile_stride = p.tile_stride;
   const bool lead = (warp == lead_warp);   // this (converged) warp issues every epilogue TMA operation of the CTA
   const int n_sets = p.epi_sets > 1 ? 2 : 1;
@@ -415,7 +420,9 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
   constexpr bool kGen = SIG == EPI_SIG_GENERIC || SIG == EPI_SIG_X6;
   constexpr bool kX3Sig = SIG == EPI_SIG_ACT_X3 || SIG == EPI_SIG_RES_ACT_X3 || SIG == EPI_SIG_SUM0_X3 || SIG == EPI_SIG_SUM1_X3 ||
                           SIG == EPI_SIG_FINAL_X3;
-  static_assert(kGen || ((MODE == EPI_TC_LINEAR || (MODE == EPI_TC_TANH && SIG == EPI_SIG_POST)) && NP == (kX3Sig ? 2 : 1)),
+  constexpr bool kMag = SIG == EPI_SIG_MAG;
+  static_assert(kGen || ((MODE == EPI_TC_LINEAR || (MODE == EPI_TC_TANH && SIG == EPI_SIG_POST) || (MODE == EPI_TC_MAG && kMag)) &&
+                         NP == (kX3Sig ? 2 : 1)),
                 "specialised signatures are linear epilogues on one bf16 plane (two for the _X3 images)");
   constexpr bool kRt = kGen || SIG == EPI_SIG_LINEAR;      // adds / outputs / scale decided at run time
   constexpr bool kSum0 = SIG == EPI_SIG_SUM0 || SIG == EPI_SIG_SUM0_X3, kSum1 = SIG == EPI_SIG_SUM1 || SIG == EPI_SIG_SUM1_X3,
@@ -423,14 +430,14 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
   constexpr bool kSum = kSum0 || kSum1 || kFinal;
   const bool has_add0 = kRt ? (p.has_add0 != 0) : (SIG == EPI_SIG_RES_ACT || SIG == EPI_SIG_RES_ACT_X3 || kSum);
   const bool has_add1 = kRt ? (p.has_add1 && MODE == EPI_TC_LINEAR) : (kSum1 || kFinal);
-  const bool has_raw = kRt ? (p.has_raw != 0) : (kSum0 || kSum1);
-  const bool has_act = kRt ? (p.has_act && MODE == EPI_TC_LINEAR) : !(kSum0 || kSum1 || SIG == EPI_SIG_POST);
+  const bool has_raw = kRt ? (p.has_raw != 0) : (kSum0 || kSum1 || kMag);
+  const bool has_act = kRt ? (p.has_act && MODE == EPI_TC_LINEAR) : !(kSum0 || kSum1 || SIG == EPI_SIG_POST || kMag);
   const float scale = (kRt || kFinal) ? p.scale : 1.0f, slope = p.slope;
   const bool add0_is_act = kRt ? (p.add0_is_act != 0) : true;
   const float inv_slope = 1.0f / p.slope;
   const float* const bias = p.bias;
   const float* const bcond = kGen ? p.bcond : nullptr;
-  const float* const maskp = kGen ? p.mask : nullptr;
+  const float* const maskp = (kGen || kMag) ? p.mask : nullptr;
   float* const out_f32 = kGen ? p.out_f32 : nullptr;
   int* const error_flag = p.error_flag;
   // staging carve-up: [add0 x n_add_bufs][add1 x n_add_bufs][raw x 2][act x 2], each e_buf_bytes
@@ -498,7 +505,7 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
     for (int cc = 0; cc < n_echunks; ++cc) {
       if (has_add && lead) issue_next_add();     // refills the buffer drained by the previous unit (barrier B below)
       const int ch = nt * n_tile + cc * CW;
-      const int och = (MODE == EPI_TC_GATE) ? ch / 2 : ch;
+      const int och = kPairs ? ch / 2 : ch;
       if (has_add) {
         mbar_wait(add_bar0 + 8u * add_buf, (add_phase >> add_buf) & 1u, error_flag);
         add_phase ^= 1u << add_buf;
@@ -626,6 +633,11 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
               v[c] = tanhf(v[2 * c]) * (1.0f / (1.0f + expf(-v[2 * c + 1])));
             }
           }
+        }
+        if (MODE == EPI_TC_MAG) {
+#pragma unroll
+          for (int c = 0; c < CW / 2; ++c)
+            v[c] = och + c < p.mag_ch ? sqrtf(fmaf(v[2 * c], v[2 * c], fmaf(v[2 * c + 1], v[2 * c + 1], 1e-6f))) * mk : 0.f;
         }
         if (MODE == EPI_TC_TANH) {   // one 16-byte store per row; the lanes of a warp cover 512 contiguous bytes
           if (srow < tile_stride && q < p.Lq) {
@@ -932,6 +944,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         conv_tc_epilogue<32, EPI_TC_LINEAR, 2, SIG>(tmAdd0, tmAdd1, tmRaw, tmAct, p, smem_base, bar_base, tmem_base, warp, lane, set, lead_warp);
       else
         conv_tc_epilogue<16, EPI_TC_LINEAR, 2, SIG>(tmAdd0, tmAdd1, tmRaw, tmAct, p, smem_base, bar_base, tmem_base, warp, lane, set, lead_warp);
+    } else if constexpr (SIG == EPI_SIG_MAG) {
+      if (!SMALL && p.cw == 64)
+        conv_tc_epilogue<64, EPI_TC_MAG, 1, SIG>(tmAdd0, tmAdd1, tmRaw, tmAct, p, smem_base, bar_base, tmem_base, warp, lane, set, lead_warp);
+      else if (p.cw == 32)
+        conv_tc_epilogue<32, EPI_TC_MAG, 1, SIG>(tmAdd0, tmAdd1, tmRaw, tmAct, p, smem_base, bar_base, tmem_base, warp, lane, set, lead_warp);
+      else
+        conv_tc_epilogue<16, EPI_TC_MAG, 1, SIG>(tmAdd0, tmAdd1, tmRaw, tmAct, p, smem_base, bar_base, tmem_base, warp, lane, set, lead_warp);
     } else if constexpr (SIG == EPI_SIG_POST) {
       conv_tc_epilogue<16, EPI_TC_TANH, 1, SIG>(tmAdd0, tmAdd1, tmRaw, tmAct, p, smem_base, bar_base, tmem_base, warp, lane, set, lead_warp);
     } else {   // specialised signature: plain-bf16 linear epilogue with compile-time feature flags

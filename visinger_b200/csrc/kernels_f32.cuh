@@ -10,7 +10,8 @@
 //     (decoder.py:45,55,93,97,126);
 //   * epi = the op the reference runs right after the conv: gate (encoder.py:206-213), residual/skip
 //     routing (encoder.py:188-194), coupling (flow.py:78,83), residual add / resblock mean (decoder.py:
-//     48-54,102), tanh (decoder.py:57).
+//     48-54,102), tanh (decoder.py:57);
+//   * MAG (template flag): channel pairs (re, im) -> sqrt(re^2 + im^2 + 1e-6) * mask, the linear spectrogram (spec.cuh).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -51,7 +52,7 @@ constexpr int F32_CI_CHUNK = 8;
 __device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.f ? v : v * slope; }
 __device__ __forceinline__ float sigmoid_accurate(float v) { return 1.0f / (1.0f + expf(-v)); }
 
-template <int WARPS_CO, int WARPS_Q>
+template <int WARPS_CO, int WARPS_Q, bool MAG = false>
 __global__ void __launch_bounds__(256) conv_f32_kernel(const ConvF32 p) {
   constexpr int CO_TILE = 8 * WARPS_CO;
   constexpr int Q_TILE = 256 * WARPS_Q;
@@ -128,7 +129,15 @@ __global__ void __launch_bounds__(256) conv_f32_kernel(const ConvF32 p) {
     const int n = q * p.out_stride + p.out_phase;
     if (q >= p.Lq || n >= p.Lout) continue;
     const float mk = mrow ? mrow[n] : 1.0f;
-    if (p.epi == EPI_GATE) {
+    if constexpr (MAG) {   // y[b, c, n] = |(acc[2c], acc[2c + 1])| * mask (no bias)
+#pragma unroll
+      for (int c = 0; c < 8; c += 2) {
+        const int co = cbase + c;
+        if (co >= p.Cout) continue;
+        const float a = acc[c][i], s = acc[c + 1][i];
+        p.y[(long long)b * p.y_bs + (long long)(co >> 1) * p.y_cs + n] = sqrtf(fmaf(a, a, fmaf(s, s, 1e-6f))) * mk;
+      }
+    } else if (p.epi == EPI_GATE) {
 #pragma unroll
       for (int c = 0; c < 8; c += 2) {
         const int co = cbase + c;

@@ -1,8 +1,11 @@
 // The whole model in one call (vsg_model_pack_create / vsg_model_forward): the token-rate glue of VISinger.forward as
 // fp32 CUDA-core kernels, chained with the existing stacks (RelativeEncoder, length regulator, frame-prior head, flow and
-// decoder).  Also the seeded prior noise (vsg_normal_noise) and the sinusoidal position table.
+// decoder).  Also the seeded prior noise (vsg_normal_noise) and the sinusoidal position table.  Voice conversion
+// (vsg_convert_pack_create / vsg_spectrogram / vsg_model_convert): waveform -> linear spectrogram -> posterior encoder ->
+// flow forward -> flow reverse -> decoder, with the DFT basis of the spectrogram packed here.
 #include "vsg_common.cuh"
 #include "run.cuh"
+#include "pack_tc.cuh"
 
 #include <math.h>
 
@@ -255,6 +258,23 @@ size_t model_ws_bytes(const VsgPack* P, int B, int T_ph, int T, int precision) {
   return persist + std::max(p1 + sub, hot) + 4096;
 }
 
+// g [B, gin] = VISinger.speaker_embedding for host ids spk_id (range-checked by the caller) and device spk_embed
+int speaker_cond(const ModelPack& m, const int64_t* spk_id, const float* spk_embed, float* g, int B, cudaStream_t st) {
+  const VsgModelConfig& c = m.cfg;
+  const int gin = m.gin;
+  for (int b0 = 0; b0 < B; b0 += kSpkChunk) {
+    const int nb = std::min(kSpkChunk, B - b0);
+    SpkIds ids;
+    for (int i = 0; i < kSpkChunk; ++i) ids.id[i] = (spk_id && i < nb) ? (int32_t)spk_id[b0 + i] : 0;
+    const long long threads = (long long)nb * gin * 32;
+    speaker_cond_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(
+        c.use_spk_embed ? m.spk_embed_w : nullptr, m.spk_embed_b, spk_embed, c.spk_embed_dim,
+        c.use_spk_id ? m.spk_id_w : nullptr, ids, b0, nb, g, gin);
+    VSG_LAUNCH_CHECK("speaker_cond_kernel");
+  }
+  return VSG_OK;
+}
+
 // VISinger.forward(infer=True), after validation.
 int model_forward(const VsgPack* P, const long long* text, const long long* pitch, const long long* dur,
                   const long long* mel2ph, const int64_t* spk_id, const float* spk_embed, const float* f0, const float* uv,
@@ -299,16 +319,7 @@ int model_forward(const VsgPack* P, const long long* text, const long long* pitc
   // length regulator + frame positions
   VSG_TRY(length_regulate(tok, mel2ph, c.use_pos_embed ? table : nullptr, c.use_pos_embed ? rows : 0, x, B, H, T_ph, T, st));
   // speaker condition [B, gin, 1]
-  for (int b0 = 0; b0 < B; b0 += kSpkChunk) {
-    const int nb = std::min(kSpkChunk, B - b0);
-    SpkIds ids;
-    for (int i = 0; i < kSpkChunk; ++i) ids.id[i] = (spk_id && i < nb) ? (int32_t)spk_id[b0 + i] : 0;
-    const long long threads = (long long)nb * gin * 32;
-    speaker_cond_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(
-        c.use_spk_embed ? m.spk_embed_w : nullptr, m.spk_embed_b, spk_embed, c.spk_embed_dim,
-        c.use_spk_id ? m.spk_id_w : nullptr, ids, b0, nb, g, gin);
-    VSG_LAUNCH_CHECK("speaker_cond_kernel");
-  }
+  VSG_TRY(speaker_cond(m, spk_id, spk_embed, g, B, st));
   if (c.use_pitch_embed) {   // VISinger.forward_pitch
     VSG_TRY(relenc_run(m.pitch, x, mask, g, hp, B, T, precision, ws, st));
     pitch_head_kernel<<<(unsigned)((BT + 255) / 256), 256, 0, st>>>(hp, m.pitch_w, m.pitch_b, f0, uv, mask, pred, cond, H, T,
@@ -329,6 +340,86 @@ int model_forward(const VsgPack* P, const long long* text, const long long* pitc
   // flow reverse + decoder (models/visinger.py:109-111)
   ws.off = mark0;
   return infer_zp_run(m.hot, z_p, mask, g, wav, z_q_out, B, T, precision, ws, st);
+}
+
+// ---- voice conversion -----------------------------------------------------------------------------------------------
+
+bool convert_bf16(int precision) { return precision == VSG_PRECISION_BF16; }   // spectrogram + posterior on tcgen05
+
+// what vsg_spectrogram takes: mask, the bf16 spectrogram (tcgen05 path) and the framed rows
+size_t spectrogram_ws_bytes(const VsgPack* P, int B, int T, int precision) {
+  const ModelPack& m = *P->model;
+  const size_t BT = (size_t)B * T;
+  const bool bf = convert_bf16(precision);
+  return align256(BT * 4) + (bf ? align256(BT * m.post->enc.in_pad * 2) : 0) + spec_frames_bytes(m.spec, B, T, bf) + 256;
+}
+
+size_t convert_ws_bytes(const VsgPack* P, int B, int T, int precision) {
+  const ModelPack& m = *P->model;
+  const EncPack& en = m.post->enc;
+  const size_t BT = (size_t)B * T, H = m.cfg.hidden;
+  const bool bf = convert_bf16(precision);
+  const size_t persist = align256(BT * 4) + 2 * align256((size_t)B * m.gin * 4) + 2 * align256(BT * H * 4);
+  const size_t keep = (bf ? align256(BT * en.in_pad * 2) : align256(BT * m.spec.bins * 4)) + align256(BT * H * 4) +
+                      align256(BT * 2 * en.out_channels * 4);
+  const size_t post = bf ? posterior_ws_bytes_tc(m.post, B, T) : posterior_ws_bytes_f32(m.post, B, T);
+  const size_t stage1 = keep + std::max(spec_frames_bytes(m.spec, B, T, bf) + 256, post);
+  return persist + std::max(stage1, vsg_workspace_bytes(m.hot, B, T, precision)) + 4096;
+}
+
+// vsg_model_convert after validation: exactly one of wav / spec.
+int model_convert(const VsgPack* P, const float* wav, const float* spec, const int32_t* lengths, const int64_t* src_id,
+                  const float* src_embed, const int64_t* tgt_id, const float* tgt_embed, const float* noise,
+                  const uint64_t* seeds, float* wav_out, float* spec_out, float* z_out, int B, int T, int precision,
+                  Workspace& ws, cudaStream_t st) {
+  const ModelPack& m = *P->model;
+  const SpecPack& S = m.spec;
+  const EncPack& en = m.post->enc;
+  const int H = m.cfg.hidden, gin = m.gin;
+  const size_t BT = (size_t)B * T;
+  const bool bf = convert_bf16(precision);
+  // live for the whole call
+  float* mask = ws.take<float>(BT);
+  float* g_src = ws.take<float>((size_t)B * gin);
+  float* g_tgt = ws.take<float>((size_t)B * gin);
+  float* z = ws.take<float>(BT * H);         // posterior sample
+  float* z_p = ws.take<float>(BT * H);       // flow(z, g_src)
+  const size_t mark0 = ws.off;
+  // live until the posterior has run
+  __nv_bfloat16* u = (bf && wav) ? ws.take<__nv_bfloat16>(BT * en.in_pad) : nullptr;
+  float* x = (!bf && wav) ? (spec_out ? spec_out : ws.take<float>(BT * S.bins)) : nullptr;
+  float* nz = noise ? nullptr : ws.take<float>(BT * H);
+  float* stats = ws.take<float>(BT * 2 * en.out_channels);
+  if (ws.overflow) return fail(VSG_ENOMEM, "convert workspace too small: need %zu bytes", ws.off);
+
+  VSG_TRY(lengths_mask(lengths, mask, B, T, st));
+  VSG_TRY(speaker_cond(m, src_id, src_embed, g_src, B, st));
+  VSG_TRY(speaker_cond(m, tgt_id, tgt_embed, g_tgt, B, st));
+  if (!noise) {
+    VSG_TRY(launch_noise(seeds, nz, B, H, T, st));
+    noise = nz;
+  }
+  // z = posterior_encoder(spec, mask, g_src)                       (modules/visinger/encoder.py:92-98)
+  if (bf && wav) {
+    VSG_TRY(spectrogram_tc(P, S, en.in_pad, wav, lengths, mask, u, B, T, ws, st));
+    if (spec_out) VSG_TRY(widen_bf16(u, spec_out, B, S.bins, en.in_pad, T, st));
+    VSG_TRY(posterior_core_tc(m.post, u, mask, g_src, noise, z, stats, B, T, ws, st));
+  } else if (bf) {
+    VSG_TRY(posterior_forward_tc(m.post, spec, mask, g_src, noise, z, stats, B, T, ws, st));
+  } else {
+    if (wav) {
+      const size_t mark = ws.off;
+      VSG_TRY(spectrogram_f32(S, wav, lengths, mask, x, B, T, ws, st));
+      ws.off = mark;
+      spec = x;
+    }
+    VSG_TRY(posterior_forward_f32(m.post, spec, mask, g_src, noise, z, stats, B, T, ws, st));
+  }
+  // z_p = flow(z, mask, g_src); then flow(z_p, mask, g_tgt, reverse) * mask and the decoder under g_tgt
+  ws.off = mark0;
+  VSG_TRY(run_flow(m.hot, z, mask, g_src, z_p, B, T, 0, precision, ws, st));
+  ws.off = mark0;
+  return infer_zp_run(m.hot, z_p, mask, g_tgt, wav_out, z_out, B, T, precision, ws, st);
 }
 
 // ---- pack creation --------------------------------------------------------------------------------------------------
@@ -368,9 +459,44 @@ int check_config(const VsgModelConfig& c) {
   return VSG_OK;
 }
 
+// The window-folded DFT basis (spec.cuh, SpecPack), evaluated in double with the phase k * n reduced mod n_fft exactly,
+// rounded once to fp32: the FFMA pack [hop][taps][CoutP]; the tcgen05 pack rounds those values to bf16, like every
+// other weight, into Cout = 2 * in_pad rows (zero pad pairs) of hopP channels.  A periodic Hann window of win samples,
+// zero-padded centrally to n_fft as torch.stft does.
+int pack_spec(VsgPack* P, SpecPack& S, int in_pad) {
+  const int N = S.n_fft, W = S.win, h = S.hop, K = S.taps, bins = S.bins, lead = (N - W) / 2;
+  const int Cout = 2 * bins, CoutP = (Cout + 63) / 64 * 64, CoutT = 2 * in_pad;
+  std::vector<float> wf((size_t)h * K * CoutP, 0.f), wt((size_t)CoutT * S.hopP * K, 0.f), bt(CoutT, 0.f);
+  const double two_pi = 6.283185307179586476925286766559;
+  for (int t = 0; t < K; ++t)
+    for (int j = 0; j < h; ++j) {
+      const int nr = t * h + j;               // sample inside the window
+      if (nr >= W) continue;
+      const long long n = lead + nr;          // sample inside the n_fft frame
+      const double w = 0.5 - 0.5 * cos(two_pi * nr / W);
+      for (int k = 0; k < bins; ++k) {
+        const double a = two_pi * (double)((k * n) % N) / N;
+        const float re = (float)(w * cos(a)), im = (float)(-w * sin(a));
+        wf[((size_t)j * K + t) * CoutP + 2 * k] = re;
+        wf[((size_t)j * K + t) * CoutP + 2 * k + 1] = im;
+        wt[((size_t)(2 * k) * S.hopP + j) * K + t] = re;
+        wt[((size_t)(2 * k + 1) * S.hopP + j) * K + t] = im;
+      }
+    }
+  void* q = nullptr;
+  VSG_CUDA_TRY(cudaMalloc(&q, wf.size() * sizeof(float)));
+  P->allocs.push_back(q);
+  VSG_CUDA_TRY(cudaMemcpy(q, wf.data(), wf.size() * sizeof(float), cudaMemcpyHostToDevice));
+  S.f32.w = (float*)q;
+  S.f32.bias = nullptr;
+  S.f32.Cin = h; S.f32.Cout = Cout; S.f32.CoutP = CoutP; S.f32.ktaps = K;
+  return pack_conv_tc(P, wt, bt, CoutT, S.hopP, K, &S.tc);
+}
+
 }  // namespace
 
 void model_pack_free(ModelPack* m) {
+  vsg_pack_destroy(m->post);
   vsg_pack_destroy(m->text);
   vsg_pack_destroy(m->pitch);
   vsg_pack_destroy(m->prior);
@@ -537,4 +663,151 @@ extern "C" int vsg_debug_position_table(const float* freq, int32_t rows, int32_t
   if (rows == 0) return VSG_OK;
   if (!out) return fail(VSG_EINVAL, "null pointer");
   return launch_prep(nullptr, nullptr, 0, freq, out, rows, dim, (cudaStream_t)stream);
+}
+
+extern "C" int vsg_convert_pack_create(const VsgModelConfig* cfg, const VsgTensor* weights, int32_t n_weights,
+                                       const char* prefix, int32_t win_length, int32_t device, VsgPack** out) {
+  if (!cfg || !out || (!weights && n_weights > 0) || n_weights < 0) return fail(VSG_EINVAL, "null argument");
+  *out = nullptr;
+  VSG_TRY(check_config(*cfg));
+  const VsgModelConfig& c = *cfg;
+  const std::string p = prefix ? prefix : "";
+  const std::string pe = p + "posterior_encoder.";
+  // PosteriorEncoder(num_linear_bins, hidden, hidden, kernel_size, 1, n_layers, gin) (models/visinger.py:59-60): the bins,
+  // kernel and layer count come from the weights, the dilation rate is VISinger's 1
+  const VsgTensor* pre = find_weight(weights, n_weights, pe + "pre.weight");
+  if (!pre) return fail(VSG_EINVAL, "missing weight %spre.weight", pe.c_str());
+  if (!pre->data || pre->ndim < 2 || pre->ndim > 3 || pre->shape[0] != c.hidden || pre->shape[1] < 2 ||
+      (pre->ndim == 3 && pre->shape[2] != 1))
+    return fail(VSG_EINVAL, "weight %spre.weight must be [hidden = %d, bins >= 2, 1]", pe.c_str(), c.hidden);
+  const VsgTensor* proj = find_weight(weights, n_weights, pe + "proj.weight");
+  if (!proj) return fail(VSG_EINVAL, "missing weight %sproj.weight", pe.c_str());
+  if (proj->ndim < 2 || proj->shape[0] != 2 * c.hidden)
+    return fail(VSG_EINVAL, "weight %sproj.weight must have 2 * hidden = %d output channels (the flow's)", pe.c_str(),
+                2 * c.hidden);
+  auto in_layer = [&](int i) {
+    const std::string k = pe + "enc.in_layers." + std::to_string(i);
+    const VsgTensor* t = find_weight(weights, n_weights, k + ".weight");
+    return t ? t : find_weight(weights, n_weights, k + ".weight_v");
+  };
+  int n_layers = 0;
+  while (in_layer(n_layers)) ++n_layers;
+  if (n_layers == 0) return fail(VSG_EINVAL, "missing weight %senc.in_layers.0.weight (or .weight_v)", pe.c_str());
+  const VsgTensor* l0 = in_layer(0);
+  if (l0->ndim != 3) return fail(VSG_EINVAL, "weight %senc.in_layers.0 must be [2 * hidden, hidden, kernel]", pe.c_str());
+  const int bins = (int)pre->shape[1], n_fft = 2 * (bins - 1);
+  int hop = 1;
+  for (int i = 0; i < c.hot.dec_n_ups && i < VSG_MAX_UPS; ++i) hop *= c.hot.dec_upsample_rates[i];
+  if (win_length <= 0 || win_length > n_fft)
+    return fail(VSG_EINVAL, "win_length %d is outside [1, n_fft = %d] (n_fft = 2 * (bins - 1), bins = %d)", win_length, n_fft,
+                bins);
+  if (n_fft < hop) return fail(VSG_EINVAL, "n_fft %d is below the decoder's hop %d: frames would skip samples", n_fft, hop);
+
+  VsgPack* P = nullptr;
+  VSG_TRY(vsg_model_pack_create(cfg, weights, n_weights, prefix, device, &P));
+  struct Restore { int prev = -1; ~Restore() { if (prev >= 0) cudaSetDevice(prev); } } restore;
+  auto build = [&]() -> int {
+    ModelPack& m = *P->model;
+    const VsgEncConfig ec = {bins, c.hidden, c.hidden, (int32_t)l0->shape[2], 1, n_layers, m.gin};
+    VSG_TRY(vsg_enc_pack_create(&ec, weights, n_weights, pe.c_str(), device, &m.post));
+    SpecPack& S = m.spec;
+    S.n_fft = n_fft; S.win = win_length; S.hop = hop; S.bins = bins;
+    S.taps = (win_length + hop - 1) / hop;
+    S.off = (n_fft - win_length) / 2 - (n_fft - hop) / 2;
+    S.hopP = (hop + 63) / 64 * 64;
+    VSG_CUDA_TRY(cudaGetDevice(&restore.prev));
+    VSG_CUDA_TRY(cudaSetDevice(device));
+    return pack_spec(P, S, m.post->enc.in_pad);
+  };
+  const int rc = build();
+  if (rc != VSG_OK) {
+    vsg_pack_destroy(P);
+    return rc;
+  }
+  *out = P;
+  return VSG_OK;
+}
+
+extern "C" size_t vsg_convert_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t precision) {
+  if (!pack || !pack->model || !pack->model->post || B < 0 || T < 0 || B > 65535) return 0;
+  if (precision != VSG_PRECISION_FP32 && precision != VSG_PRECISION_BF16 && precision != VSG_PRECISION_BF16X3) return 0;
+  return convert_ws_bytes(pack, B, T, precision);
+}
+
+namespace {
+
+int check_convert(const VsgPack* pack, int B, int T, int precision) {
+  if (!pack || !pack->model || !pack->model->post)
+    return fail(VSG_EINVAL, "pack has no posterior encoder or spectrogram (create it with vsg_convert_pack_create)");
+  if (B < 0 || T < 0) return fail(VSG_EINVAL, "negative batch (%d) or length (%d)", B, T);
+  if (B > 65535) return fail(VSG_EUNSUPPORTED, "batch %d exceeds 65535", B);
+  if (precision != VSG_PRECISION_FP32 && precision != VSG_PRECISION_BF16 && precision != VSG_PRECISION_BF16X3)
+    return fail(VSG_EINVAL, "unknown precision %d", precision);
+  if ((long long)T * pack->model->spec.hop > 0x7fffffffLL / 4) return fail(VSG_EUNSUPPORTED, "sequence too long (%d frames)", T);
+  return VSG_OK;
+}
+
+}  // namespace
+
+extern "C" int vsg_spectrogram(const VsgPack* pack, const float* wav, const int32_t* lengths, float* spec, int32_t B,
+                               int32_t T, int32_t precision, void* workspace, size_t workspace_bytes, void* stream) {
+  g_launches = 0;
+  VSG_TRY(check_convert(pack, B, T, precision));
+  if (B == 0 || T == 0) return VSG_OK;
+  if (!wav || !lengths || !spec) return fail(VSG_EINVAL, "null pointer: wav, lengths and spec are required");
+  const size_t need = spectrogram_ws_bytes(pack, B, T, precision);
+  if (!workspace || workspace_bytes < need)
+    return fail(VSG_ENOMEM, "workspace of %zu bytes is too small: need %zu", workspace ? workspace_bytes : (size_t)0, need);
+  DeviceGuard dg(pack->device);
+  if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
+  const ModelPack& m = *pack->model;
+  cudaStream_t st = (cudaStream_t)stream;
+  Workspace ws(workspace, workspace_bytes);
+  float* mask = ws.take<float>((size_t)B * T);
+  if (!convert_bf16(precision)) {
+    if (ws.overflow) return fail(VSG_ENOMEM, "spectrogram workspace too small");
+    VSG_TRY(lengths_mask(lengths, mask, B, T, st));
+    return spectrogram_f32(m.spec, wav, lengths, mask, spec, B, T, ws, st);
+  }
+  const int in_pad = m.post->enc.in_pad;
+  __nv_bfloat16* u = ws.take<__nv_bfloat16>((size_t)B * T * in_pad);
+  if (ws.overflow) return fail(VSG_ENOMEM, "spectrogram workspace too small");
+  VSG_TRY(lengths_mask(lengths, mask, B, T, st));
+  VSG_TRY(spectrogram_tc(pack, m.spec, in_pad, wav, lengths, mask, u, B, T, ws, st));
+  return widen_bf16(u, spec, B, m.spec.bins, in_pad, T, st);
+}
+
+extern "C" int vsg_model_convert(const VsgPack* pack, const float* wav, const float* spec, const int32_t* lengths,
+                                 const int64_t* src_spk_id, const float* src_spk_embed, const int64_t* tgt_spk_id,
+                                 const float* tgt_spk_embed, const float* noise, const uint64_t* seeds, float* wav_out,
+                                 float* spec_out, float* z_out, int32_t B, int32_t T, int32_t precision, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  g_launches = 0;
+  VSG_TRY(check_convert(pack, B, T, precision));
+  const VsgModelConfig& c = pack->model->cfg;
+  if (B == 0 || T == 0) return VSG_OK;
+  if ((wav == nullptr) == (spec == nullptr)) return fail(VSG_EINVAL, "give exactly one of wav and spec");
+  if (spec && spec_out) return fail(VSG_EINVAL, "spec_out receives the spectrogram of wav: it must be NULL when spec is given");
+  if (!lengths || !wav_out) return fail(VSG_EINVAL, "null pointer: lengths and wav_out are required");
+  if (c.use_spk_id != (src_spk_id != nullptr) || c.use_spk_id != (tgt_spk_id != nullptr))
+    return fail(VSG_EINVAL, c.use_spk_id ? "src_spk_id and tgt_spk_id are required (use_spk_id)"
+                                         : "speaker ids given but the model has no use_spk_id");
+  if (c.use_spk_embed != (src_spk_embed != nullptr) || c.use_spk_embed != (tgt_spk_embed != nullptr))
+    return fail(VSG_EINVAL, c.use_spk_embed ? "src_spk_embed and tgt_spk_embed are required (use_spk_embed)"
+                                            : "speaker embeddings given but the model has no use_spk_embed");
+  if (!noise && !seeds) return fail(VSG_EINVAL, "noise and seeds are both NULL: one of them is required");
+  for (const int64_t* ids : {src_spk_id, tgt_spk_id})
+    if (ids)
+      for (int b = 0; b < B; ++b)
+        if (ids[b] < 0 || ids[b] >= c.num_spk)
+          return fail(VSG_EINVAL, "%s_spk_id[%d] = %lld is outside [0, %d)", ids == src_spk_id ? "src" : "tgt", b,
+                      (long long)ids[b], c.num_spk);
+  const size_t need = convert_ws_bytes(pack, B, T, precision);
+  if (!workspace || workspace_bytes < need)
+    return fail(VSG_ENOMEM, "workspace of %zu bytes is too small: need %zu", workspace ? workspace_bytes : (size_t)0, need);
+  DeviceGuard dg(pack->device);
+  if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
+  Workspace ws(workspace, workspace_bytes);
+  return model_convert(pack, wav, spec, lengths, src_spk_id, src_spk_embed, tgt_spk_id, tgt_spk_embed, noise, seeds,
+                       wav_out, spec_out, z_out, B, T, precision, ws, (cudaStream_t)stream);
 }

@@ -62,6 +62,26 @@ int frame_prior_forward_tc(const VsgPack* P, const float* x, const float* mask, 
 int length_regulate(const float* enc, const long long* mel2ph, const float* table, int table_rows, float* y, int B, int H,
                     int T_ph, int T, cudaStream_t st);
 
+// vsg_flow_forward after validation (api.cu): the precision's flow kernels; see api.cu for masked / ps_* / sampled
+int run_flow(const VsgPack* pack, const float* x, const float* mask, const float* g, float* y, int B, int T, int reverse,
+             int precision, Workspace& ws, cudaStream_t st, bool* masked = nullptr, const float* ps_logs = nullptr,
+             const float* ps_noise = nullptr, bool* sampled = nullptr);
+
+// The linear spectrogram (spec.cuh).  mask [B, T] = t < lengths[b] (lengths clamped to [0, T]).
+int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st);
+size_t spec_frames_bytes(const SpecPack& S, int B, int T, bool tc);
+// fp32: spec [B, bins, T] on the FFMA kernel (run_f32.cu)
+int spectrogram_f32(const SpecPack& S, const float* wav, const int32_t* lengths, const float* mask, float* spec, int B,
+                    int T, Workspace& ws, cudaStream_t st);
+// bf16: u [B, T, in_pad] channels-last bf16 (the posterior's `pre` input, pad channels 0) on tcgen05 (run_tc.cu)
+int spectrogram_tc(const VsgPack* P, const SpecPack& S, int in_pad, const float* wav, const int32_t* lengths,
+                   const float* mask, __nv_bfloat16* u, int B, int T, Workspace& ws, cudaStream_t st);
+// [B, T, ld] bf16 -> [B, C, T] fp32
+int widen_bf16(const __nv_bfloat16* x, float* y, int B, int C, int ld, int T, cudaStream_t st);
+// the bf16 posterior from its channels-last input u [B, T, in_pad] (posterior_forward_tc after its transpose)
+int posterior_core_tc(const VsgPack* P, const __nv_bfloat16* u, const float* mask, const float* g, const float* noise,
+                      float* z, float* stats, int B, int T, Workspace& ws, cudaStream_t st);
+
 // vsg_infer_zp after validation (api.cu): flow reverse from z_p, mask, decoder; shared with vsg_model_forward
 int infer_zp_run(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav, float* z_q_out,
                  int B, int T, int precision, Workspace& ws, cudaStream_t st);

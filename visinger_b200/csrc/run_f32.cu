@@ -3,11 +3,13 @@
 #include "kernels_f32.cuh"
 #include "relenc_f32.cuh"
 #include "run.cuh"
+#include "spec.cuh"
 
 namespace vsg {
 
 namespace {
 
+template <bool MAG = false>
 int launch_conv_f32(const ConvF32& p, int B, cudaStream_t st) {
   if (p.ktaps < 1) return fail(VSG_EUNSUPPORTED, "convolution with no taps");
   const int halo = (p.ktaps - 1) * p.dil;
@@ -19,9 +21,9 @@ int launch_conv_f32(const ConvF32& p, int B, cudaStream_t st) {
     const size_t sm = smem_for(8 * WC, 256 * WQ);                                                           \
     if (sm > 200 * 1024) return fail(VSG_EUNSUPPORTED, "conv window too large for shared memory (%zu B)", sm); \
     if (sm > 48 * 1024)                                                                                     \
-      VSG_CUDA_TRY(cudaFuncSetAttribute(conv_f32_kernel<WC, WQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)); \
+      VSG_CUDA_TRY(cudaFuncSetAttribute(conv_f32_kernel<WC, WQ, MAG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)); \
     dim3 grid((p.Lq + 256 * WQ - 1) / (256 * WQ), (p.Cout + 8 * WC - 1) / (8 * WC), B);                     \
-    conv_f32_kernel<WC, WQ><<<grid, 256, sm, st>>>(p);                                                      \
+    conv_f32_kernel<WC, WQ, MAG><<<grid, 256, sm, st>>>(p);                                                 \
     VSG_LAUNCH_CHECK("conv_f32_kernel");                                                                    \
   } while (0)
   if (p.Lq <= 0) return VSG_OK;
@@ -193,6 +195,35 @@ int posterior_forward_f32(const VsgPack* P, const float* x, const float* mask, c
   posterior_sample_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(stats, noise, mask, z, Co, T, n);
   VSG_LAUNCH_CHECK("posterior_sample_kernel");
   return VSG_OK;
+}
+
+int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st) {
+  const long long n = (long long)B * T;
+  lengths_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(lengths, mask, T, n);
+  VSG_LAUNCH_CHECK("lengths_mask_kernel");
+  return VSG_OK;
+}
+
+// framed rows of the spectrogram: [B, R, hopP] bf16 (tcgen05) or [B, hop, R] fp32 (FFMA), R = T + taps - 1
+size_t spec_frames_bytes(const SpecPack& S, int B, int T, bool tc) {
+  const size_t R = (size_t)T + S.taps - 1;
+  return align256((size_t)B * R * (tc ? S.hopP * 2 : S.hop * 4));
+}
+
+// spec [B, bins, T] = |STFT| * mask: the framed rows, then Conv1d(hop -> 2 bins, taps) with the magnitude epilogue.
+int spectrogram_f32(const SpecPack& S, const float* wav, const int32_t* lengths, const float* mask, float* spec, int B,
+                    int T, Workspace& ws, cudaStream_t st) {
+  const int R = T + S.taps - 1;
+  float* rows = ws.take<float>((size_t)B * S.hop * R);
+  if (ws.overflow) return fail(VSG_ENOMEM, "spectrogram workspace too small: need %zu bytes", ws.off);
+  const long long n = (long long)B * S.hop * R;
+  spec_frames_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(wav, lengths, rows, T, R, S.hop, S.hop, S.off,
+                                                                           S.taps, n);
+  VSG_LAUNCH_CHECK("spec_frames_kernel");
+  ConvF32 p = base_conv(S.f32, rows, (long long)S.hop * R, R, R, 0, 1);
+  p.Lq = T; p.Lout = T;
+  p.y = spec; p.y_bs = (long long)S.bins * T; p.y_cs = T; p.mask = mask; p.mask_bs = T;
+  return launch_conv_f32<true>(p, B, st);
 }
 
 int conv_f32_plain(const ConvW32& w, const float* x, int B, int T, float* y, cudaStream_t st) {

@@ -8,6 +8,7 @@
 #include "rp_tc.cuh"
 #include "relenc_tc.cuh"
 #include "attn_tc.cuh"
+#include "spec.cuh"
 
 #include <algorithm>
 #include <map>
@@ -107,6 +108,7 @@ struct EpiTC {
   __nv_bfloat16* out_act = nullptr;
   float* out_f32 = nullptr;
   int tanh_cols = 0;                // EPI_TC_TANH: samples per row written to out_f32
+  int mag_ch = 0;                   // EPI_TC_MAG: output channels below this are magnitudes, the rest are written as 0
 };
 
 // HALO mode verified on B200 (tools/tc_probe.py): the UMMA unit applies the swizzle XOR to absolute
@@ -171,7 +173,8 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
   bool small = NT <= 64 && (NT <= 32 || NT % 32 == 0);
   int cw_max = small ? std::min(NT, 32) : pick_cw(NT);
   if (w.planes == 3) cw_max = std::min(cw_max, 32);       // the three-plane epilogue is instantiated for 32 / 16 channels
-  const int cout_eff = e.mode == EPI_TC_GATE ? w.Cout / 2 : w.Cout;  // channels of the add / out tensors
+  const bool pairs = e.mode == EPI_TC_GATE || e.mode == EPI_TC_MAG;   // two accumulator columns per output channel
+  const int cout_eff = pairs ? w.Cout / 2 : w.Cout;  // channels of the add / out tensors
   const int n_parts = a_planes;
   const int part_stride = e.part_stride ? e.part_stride : cout_eff;
   const int ld = e.ld ? e.ld : n_parts * cout_eff;
@@ -347,7 +350,7 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
   }
   if (!planned) return fail(VSG_EUNSUPPORTED, "conv tile does not fit in shared memory");
   const int cw = p.cw;
-  const int ow = e.mode == EPI_TC_GATE ? cw / 2 : cw;                // output channels per chunk
+  const int ow = pairs ? cw / 2 : cw;                                // output channels per chunk
   p.B = B; p.Lq = Lq; p.Lout = Lout;
   p.out_stride = out_stride; p.out_phase = out_phase;
   p.tile_stride = 128 * p.mb;
@@ -369,6 +372,7 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
   p.scale = e.scale; p.slope = e.slope;
   p.out_f32 = e.out_f32;
   p.tanh_cols = e.tanh_cols;
+  p.mag_ch = e.mag_ch;
   p.error_flag = error_flag;
 
   static const bool debug_plan = getenv("VSG_DEBUG_PLAN") != nullptr;
@@ -404,12 +408,12 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
        conv_tc_kernel<false, EPI_SIG_LINEAR>, conv_tc_kernel<false, EPI_SIG_X6>, conv_tc_kernel<false, EPI_SIG_SUM0>,
        conv_tc_kernel<false, EPI_SIG_SUM1>, conv_tc_kernel<false, EPI_SIG_FINAL>, conv_tc_kernel<false, EPI_SIG_POST>,
        conv_tc_kernel<false, EPI_SIG_ACT_X3>, conv_tc_kernel<false, EPI_SIG_RES_ACT_X3>, conv_tc_kernel<false, EPI_SIG_SUM0_X3>,
-       conv_tc_kernel<false, EPI_SIG_SUM1_X3>, conv_tc_kernel<false, EPI_SIG_FINAL_X3>},
+       conv_tc_kernel<false, EPI_SIG_SUM1_X3>, conv_tc_kernel<false, EPI_SIG_FINAL_X3>, conv_tc_kernel<false, EPI_SIG_MAG>},
       {conv_tc_kernel<true, EPI_SIG_GENERIC>, conv_tc_kernel<true, EPI_SIG_ACT>, conv_tc_kernel<true, EPI_SIG_RES_ACT>,
        conv_tc_kernel<true, EPI_SIG_LINEAR>, conv_tc_kernel<true, EPI_SIG_X6>, conv_tc_kernel<true, EPI_SIG_SUM0>,
        conv_tc_kernel<true, EPI_SIG_SUM1>, conv_tc_kernel<true, EPI_SIG_FINAL>, conv_tc_kernel<true, EPI_SIG_POST>,
        conv_tc_kernel<true, EPI_SIG_ACT_X3>, conv_tc_kernel<true, EPI_SIG_RES_ACT_X3>, conv_tc_kernel<true, EPI_SIG_SUM0_X3>,
-       conv_tc_kernel<true, EPI_SIG_SUM1_X3>, conv_tc_kernel<true, EPI_SIG_FINAL_X3>}};
+       conv_tc_kernel<true, EPI_SIG_SUM1_X3>, conv_tc_kernel<true, EPI_SIG_FINAL_X3>, conv_tc_kernel<true, EPI_SIG_MAG>}};
   // the opt-in to > 48 KB of dynamic shared memory is a per-device function attribute
   static bool attr_set_dev[64] = {false};
   bool& attr_set = attr_set_dev[P->device & 63];
@@ -425,6 +429,11 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
     if (a_planes != 1 || p.cw != 16 || e.tanh_cols < 1 || e.tanh_cols > 4 || !e.out_f32 || out_stride != 1 || Lq != Lout)
       return fail(VSG_EINVAL, "tanh epilogue: needs a plain-bf16 N = 16 convolution and an fp32 output");
     sig = EPI_SIG_POST;
+  }
+  if (e.mode == EPI_TC_MAG) {
+    if (a_planes != 1 || !e.out_raw || e.out_act || e.add0 || e.add1 || e.bias || e.bcond || e.out_f32)
+      return fail(VSG_EINVAL, "magnitude epilogue: needs a plain-bf16 convolution with one raw output and no bias or adds");
+    sig = EPI_SIG_MAG;
   }
   if (opt.epi_sigs >= 2 && e.mode == EPI_TC_LINEAR && a_planes == 2 && e.bias && !e.bcond && !e.mask && !e.out_f32) {
     // the bf16x3 decoder's epilogues (single activated stream), as for one plane below
@@ -1131,14 +1140,26 @@ size_t posterior_ws_bytes_tc(const VsgPack* P, int B, int T) {
 int posterior_forward_tc(const VsgPack* P, const float* x, const float* mask, const float* g, const float* noise,
                          float* z, float* stats, int B, int T, Workspace& ws, cudaStream_t st) {
   const EncPack& en = P->enc;
-  const int H = en.hidden, NL = en.n_layers, K = en.kernel, Cin = en.in_channels, CinP = en.in_pad, Co = en.out_channels;
+  __nv_bfloat16* u = ws.take<__nv_bfloat16>((size_t)B * T * en.in_pad);
+  if (ws.overflow) return fail(VSG_ENOMEM, "posterior workspace too small: need %zu bytes", ws.off);
+  {
+    dim3 grid((T + 31) / 32, (en.in_pad + 31) / 32, B), block(32, 8);
+    transpose_pad_to_bf16_kernel<<<grid, block, 0, st>>>(x, u, en.in_channels, en.in_pad, T);
+    VSG_LAUNCH_CHECK("transpose_pad_to_bf16_kernel");
+  }
+  return posterior_core_tc(P, u, mask, g, noise, z, stats, B, T, ws, st);
+}
+
+int posterior_core_tc(const VsgPack* P, const __nv_bfloat16* u, const float* mask, const float* g, const float* noise,
+                      float* z, float* stats, int B, int T, Workspace& ws, cudaStream_t st) {
+  const EncPack& en = P->enc;
+  const int H = en.hidden, NL = en.n_layers, K = en.kernel, CinP = en.in_pad, Co = en.out_channels;
   if (en.pre_tc.empty() || !en.pre_tc[0].has_tmap || !en.proj_tc.has_tmap || (int)en.wn.in_tc.size() != NL ||
       !en.wn.in_tc[0].has_tmap)
     return fail(VSG_EUNSUPPORTED, "bf16 posterior encoder needs hidden and 2 * out channels to be multiples of 16");
   const int condO = 2 * H * NL;
   typedef __nv_bfloat16 bf;
   float* cond = ws.take<float>((size_t)B * condO);
-  bf* u = ws.take<bf>((size_t)B * T * CinP);
   bf* h = ws.take<bf>((size_t)B * T * H);
   bf* acts = ws.take<bf>((size_t)B * T * H);
   bf* out = ws.take<bf>((size_t)B * T * H);
@@ -1150,11 +1171,6 @@ int posterior_forward_tc(const VsgPack* P, const float* x, const float* mask, co
   if (en.gin > 0) {
     if (!g) return fail(VSG_EINVAL, "posterior encoder was built with gin_channels=%d but g is NULL", en.gin);
     VSG_TRY(launch_cond(en.wn.cond_w, en.wn.cond_b, g, cond, condO, en.gin, B, st));
-  }
-  {
-    dim3 grid((T + 31) / 32, (CinP + 31) / 32, B), block(32, 8);
-    transpose_pad_to_bf16_kernel<<<grid, block, 0, st>>>(x, u, Cin, CinP, T);
-    VSG_LAUNCH_CHECK("transpose_pad_to_bf16_kernel");
   }
   for (size_t s = 0; s < en.pre_tc.size(); ++s) {   // h = pre(x) * mask, one launch per input-channel slab
     const bool last = (s + 1 == en.pre_tc.size());
@@ -1199,6 +1215,35 @@ int posterior_forward_tc(const VsgPack* P, const float* x, const float* mask, co
   const long long n = (long long)B * Co * T;
   posterior_sample_from_stats_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(stats, noise, mask, z, Co, T, n);
   VSG_LAUNCH_CHECK("posterior_sample_from_stats_kernel");
+  return VSG_OK;
+}
+
+// u [B, T, in_pad] = |STFT| * mask in bf16: the framed rows, then Conv1d(hopP -> 2 in_pad, taps) on tcgen05 with the
+// magnitude epilogue (conv_tc.cuh, EPI_TC_MAG), which also zeroes the pad channels.
+int spectrogram_tc(const VsgPack* P, const SpecPack& S, int in_pad, const float* wav, const int32_t* lengths,
+                   const float* mask, __nv_bfloat16* u, int B, int T, Workspace& ws, cudaStream_t st) {
+  if (!S.tc.has_tmap || S.tc.Cout != 2 * in_pad) return fail(VSG_EUNSUPPORTED, "no tensor-core spectrogram pack");
+  const int R = T + S.taps - 1;
+  const size_t mark = ws.off;
+  __nv_bfloat16* rows = ws.take<__nv_bfloat16>((size_t)B * R * S.hopP);
+  int* err = ws.take<int>(1);
+  if (ws.overflow) return fail(VSG_ENOMEM, "spectrogram workspace too small: need %zu bytes", ws.off);
+  VSG_CUDA_TRY(cudaMemsetAsync(err, 0, sizeof(int), st));
+  const long long n = (long long)B * R * S.hopP;
+  spec_frames_kernel<true><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(wav, lengths, rows, T, R, S.hop, S.hopP, S.off,
+                                                                          S.taps, n);
+  VSG_LAUNCH_CHECK("spec_frames_kernel");
+  EpiTC e;
+  e.mode = EPI_TC_MAG; e.mask = mask; e.out_raw = u; e.mag_ch = S.bins;
+  VSG_TRY(launch_conv_tc(P, S.tc, rows, B, R, 0, 1, T, 1, 0, T, e, g_default_opts, err, st));
+  ws.off = mark;   // stream-ordered: the next user of the rows runs after the convolution
+  return VSG_OK;
+}
+
+int widen_bf16(const __nv_bfloat16* x, float* y, int B, int C, int ld, int T, cudaStream_t st) {
+  dim3 grid((T + 31) / 32, (C + 31) / 32, B), block(32, 8);
+  widen_bf16_kernel<<<grid, block, 0, st>>>(x, y, C, ld, T);
+  VSG_LAUNCH_CHECK("widen_bf16_kernel");
   return VSG_OK;
 }
 

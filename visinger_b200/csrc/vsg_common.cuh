@@ -146,6 +146,17 @@ struct UpStage {
   std::vector<ResBlockPack> blocks;
 };
 
+// The linear spectrogram of vsg_model_convert (spec.cuh): Conv1d(hop -> 2 * bins, taps) over rows of hop samples with
+// the window-folded DFT basis as weights -- output channels (2k, 2k + 1) = (w[n] cos(2 pi k n / n_fft),
+// -w[n] sin(2 pi k n / n_fft)) at n = lead + tap * hop + j, lead = (n_fft - win) / 2, zero beyond the window.
+struct SpecPack {
+  int n_fft = 0, win = 0, hop = 0, bins = 0, taps = 0;
+  int off = 0;                         // first sample of frame 0's window: (n_fft - win) / 2 - (n_fft - hop) / 2
+  int hopP = 0;                        // hop rounded up to 64: channels of a bf16 row
+  ConvW32 f32;                         // Cin = hop, Cout = 2 * bins
+  ConvWTC tc;                          // Cin = hopP, Cout = 2 * in_pad of the posterior (pad pairs zero)
+};
+
 // The whole model (vsg_model_pack_create): the four sub-packs of the existing pack types plus the token-rate weights that
 // no stack owns.  Device arrays live in the owning VsgPack's `allocs`; the sub-packs are destroyed with it.
 struct ModelPack {
@@ -159,6 +170,9 @@ struct ModelPack {
   const float *pitch_w = nullptr, *pitch_b = nullptr;           // pitch_predictor.linear: [2][H], [2]
   const float* freq = nullptr;         // embed_positions.freq [H/2], or null: computed on the device
   int gin = 0;
+  // voice conversion (vsg_convert_pack_create): the posterior_encoder.* pack and the spectrogram; post is null otherwise
+  VsgPack* post = nullptr;
+  SpecPack spec;
 };
 void model_pack_free(ModelPack* m);
 

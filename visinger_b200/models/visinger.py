@@ -342,7 +342,9 @@ class VISinger(nn.Module):
     from `z_p` on -- flow reverse, HiFi-GAN decoder (models/visinger.py:107-111) -- one `vsg_infer_zp` call.  What stays in
     PyTorch in `forward` is token-rate glue: three embedding lookups, one Linear(576 -> 192), the speaker embedding and the
     1x1 head of the pitch predictor.  `forward_native` runs the same model, glue included, as one `vsg_model_forward`
-    call.  `infer=False` (training) is out of scope and raises.
+    call.  `voice_conversion` takes audio (or a linear spectrogram) through the posterior encoder and the flow to another
+    speaker's voice as one `vsg_model_convert` call; `spectrogram` is its linear spectrogram alone.  `infer=False`
+    (training) is out of scope and raises.
 
     Extra keyword arguments (not in the reference): `noise` injects the prior noise instead of
     `torch.randn_like(mu_p)` (CPU and CUDA generators differ, so parity tests need it); `precision` selects
@@ -453,23 +455,123 @@ class VISinger(nn.Module):
         graph.replay()
         return out
 
+    def _model_config(self) -> "_lib.VsgModelConfig":
+        hp = self.hparams
+        te = self.text_encoder
+        return _lib.VsgModelConfig(
+            te.ph_emb.num_embeddings, te.pitch_emb.num_embeddings, te.dur_emb.num_embeddings, self.hidden_size,
+            hp["ffn_filter_channels"], hp["num_heads"], hp["ffn_kernel_size"], te.text_encoder.window_size,
+            self.enc_layers, hp["pitch_predictor_layers"] if hp["use_pitch_embed"] else 0, hp["frame_prior_layers"],
+            int(bool(self.use_pos_embed)), int(bool(hp["use_pitch_embed"])), int(bool(hp["use_spk_id"])),
+            int(bool(hp["use_spk_embed"])), hp["num_spk"] if hp["use_spk_id"] else 0,
+            self.spk_embed_proj.in_features if hp["use_spk_embed"] else 0, self._hot._vsg_config())
+
     def _model_pack(self, device) -> "_lib.ModelPack":
         """The whole-model pack (vsg_model_pack_create), rebuilt when a parameter's storage or version changes."""
         wkey = (str(device),) + tuple((p.data_ptr(), p._version) for p in self.parameters())
         cached = self.__dict__.get("_native_pack")
         if cached is None or cached[0] != wkey:
-            hp = self.hparams
-            te = self.text_encoder
-            cfg = _lib.VsgModelConfig(
-                te.ph_emb.num_embeddings, te.pitch_emb.num_embeddings, te.dur_emb.num_embeddings, self.hidden_size,
-                hp["ffn_filter_channels"], hp["num_heads"], hp["ffn_kernel_size"], te.text_encoder.window_size,
-                self.enc_layers, hp["pitch_predictor_layers"] if hp["use_pitch_embed"] else 0, hp["frame_prior_layers"],
-                int(bool(self.use_pos_embed)), int(bool(hp["use_pitch_embed"])), int(bool(hp["use_spk_id"])),
-                int(bool(hp["use_spk_embed"])), hp["num_spk"] if hp["use_spk_id"] else 0,
-                self.spk_embed_proj.in_features if hp["use_spk_embed"] else 0, self._hot._vsg_config())
-            pack = _lib.ModelPack(cfg, dict(self.state_dict()), "", device)
+            pack = _lib.ModelPack(self._model_config(), dict(self.state_dict()), "", device)
             self.__dict__["_native_pack"] = cached = (wkey, pack)
         return cached[1]
+
+    @property
+    def win_length(self) -> int:
+        """Hann window length of the linear spectrogram: hparams["win_size"], else n_fft = 2 * (num_linear_bins - 1)."""
+        return int(self.hparams.get("win_size", 2 * (self.posterior_encoder.in_channels - 1)))
+
+    def _convert_pack(self, device) -> "_lib.ConvertPack":
+        """The voice-conversion pack (vsg_convert_pack_create), rebuilt like `_model_pack`."""
+        wkey = (str(device), self.win_length) + tuple((p.data_ptr(), p._version) for p in self.parameters())
+        cached = self.__dict__.get("_native_convert_pack")
+        if cached is None or cached[0] != wkey:
+            pack = _lib.ConvertPack(self._model_config(), dict(self.state_dict()), "", self.win_length, device)
+            self.__dict__["_native_convert_pack"] = cached = (wkey, pack)
+        return cached[1]
+
+    @torch.no_grad()
+    def spectrogram(self, wav, lengths):
+        """The linear spectrogram the posterior encoder reads (vsg_spectrogram): wav CUDA [B, T * hop], lengths CUDA int
+        [B] latent frames per utterance -> fp32 [B, num_linear_bins, T].  VITS's spectrogram_torch of each utterance on
+        its own (reflect padding about the utterance's ends, periodic Hann window of `win_length`, sqrt(|X|^2 + 1e-6)),
+        masked beyond lengths.  bf16 precision: the bf16 values the posterior consumes."""
+        _lib.require_cuda(lengths, "lengths")
+        pack = self._convert_pack(wav.device)
+        return pack.spectrogram(wav, lengths, _lib.precision_code(self.precision))
+
+    @torch.no_grad()
+    def voice_conversion(self, wav=None, lengths=None, spk_id=None, spk_embed=None, tgt_spk_id=None, tgt_spk_embed=None,
+                         spec=None, noise=None, seeds=None):
+        """Audio to audio in one library call (vsg_model_convert), VITS's voice_conversion on this model's modules:
+        spectrogram -> posterior encoder under the source speaker -> flow -> flow reverse and decoder under the target
+        speaker.  Give `wav` [B, T * hop] or a precomputed `spec` [B, num_linear_bins, T], and `lengths` (int [B], valid
+        latent frames).  spk_id / spk_embed describe the source speaker, tgt_spk_id / tgt_spk_embed the target, as the
+        model's configuration requires (ids are read on the host).  The posterior noise is `noise` [B, H, T], else drawn
+        on the device from `seeds` (int64 [B]), else from seeds taken from torch's default CPU generator.
+        Returns {"wav_out": [B, T * hop], "z": z_hat [B, H, T], "spec": the spectrogram the posterior read}."""
+        hp = self.hparams
+        if (wav is None) == (spec is None):
+            raise RuntimeError("give exactly one of wav and spec")
+        src = wav if wav is not None else spec
+        ins = {"wav" if wav is not None else "spec": src, "lengths": lengths}
+        if hp["use_spk_embed"]:
+            ins["spk_embed"], ins["tgt_spk_embed"] = spk_embed, tgt_spk_embed
+        if noise is not None:
+            ins["noise"] = noise
+        elif seeds is not None:
+            ins["seeds"] = seeds
+        for k, v in ins.items():
+            if v is None:
+                raise RuntimeError(f"{k} is required by this model's configuration")
+            _lib.require_cuda(v, k)
+        dev = src.device
+        pack = self._convert_pack(dev)
+        B, H = src.shape[0], self.hidden_size
+        if wav is not None:
+            if wav.dim() != 2 or wav.shape[1] % pack.hop:
+                raise RuntimeError(f"expected wav [B, T * {pack.hop}], got {tuple(wav.shape)}")
+            T = wav.shape[1] // pack.hop
+        else:
+            if spec.dim() != 3 or spec.shape[1] != pack.bins:
+                raise RuntimeError(f"expected spec [B, {pack.bins}, T], got {tuple(spec.shape)}")
+            T = spec.shape[2]
+        shapes = {"lengths": (B,), "noise": (B, H, T), "seeds": (B,)}
+        if hp["use_spk_embed"]:
+            shapes["spk_embed"] = shapes["tgt_spk_embed"] = (B, self.spk_embed_proj.in_features)
+        for k, shape in shapes.items():
+            if k in ins and tuple(ins[k].shape) != shape:
+                raise RuntimeError(f"expected {k} of shape {shape}, got {tuple(ins[k].shape)}")
+        for k, v in ins.items():
+            if v.device != dev:
+                raise RuntimeError(f"{k} is on {v.device}, {'wav' if wav is not None else 'spec'} on {dev}")
+        hosts = {}
+        if hp["use_spk_id"]:
+            for k, v in (("spk_id", spk_id), ("tgt_spk_id", tgt_spk_id)):
+                if v is None:
+                    raise RuntimeError(f"{k} is required by this model's configuration")
+                hosts[k] = torch.as_tensor(v).to("cpu", torch.int64).contiguous().reshape(-1)
+                if hosts[k].numel() != B:
+                    raise RuntimeError(f"expected {k} of shape ({B},), got {tuple(torch.as_tensor(v).shape)}")
+        if "noise" not in ins and "seeds" not in ins:
+            ins["seeds"] = torch.randint(0, 2 ** 62, (B,), dtype=torch.int64).to(dev)
+        a = {k: v.to(torch.int32).contiguous() if k == "lengths" else v.to(torch.int64).contiguous() if k == "seeds"
+             else _lib.as_f32c(v) for k, v in ins.items()}
+        prec = _lib.precision_code(self.precision)
+        wav_out = torch.empty(B, T * pack.hop, dtype=torch.float32, device=dev)
+        z = torch.empty(B, H, T, dtype=torch.float32, device=dev)
+        spec_out = torch.empty(B, pack.bins, T, dtype=torch.float32, device=dev) if wav is not None else None
+        ptr = lambda k: a[k].data_ptr() if k in a else None   # noqa: E731
+        hptr = lambda k: hosts[k].data_ptr() if k in hosts else None   # noqa: E731
+        with torch.cuda.device(dev):
+            ws = _lib.workspace(dev, pack.convert_workspace_bytes(B, T, prec))
+            rc = _lib.lib().vsg_model_convert(
+                pack.handle, ptr("wav"), ptr("spec"), ptr("lengths"), hptr("spk_id"), ptr("spk_embed"), hptr("tgt_spk_id"),
+                ptr("tgt_spk_embed"), ptr("noise"), ptr("seeds"), wav_out.data_ptr(),
+                spec_out.data_ptr() if spec_out is not None else None, z.data_ptr(), B, T, prec, ws.data_ptr(), ws.numel(),
+                _lib.stream_ptr(dev))
+        _lib.check(rc, "vsg_model_convert")
+        self.last_launches = _lib.last_launch_count()
+        return {"wav_out": wav_out, "z": z, "spec": spec_out if spec_out is not None else spec}
 
     @torch.no_grad()
     def forward_native(self, text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed=None, spk_id=None, f0=None, uv=None,
