@@ -412,6 +412,9 @@ int32_t vsg_hop_size(const VsgPack* pack);   /* (a model pack: its decoder's) */
 
 /* Number of kernels launched by the most recent run call on this thread (bench bookkeeping). */
 int32_t vsg_last_launch_count(void);
+/* Launches of the convolution kernel per epilogue image in that call: out[i] = launches of image i (EPI_SIG_* numbering,
+ * see vsg_debug_conv_tc), 0 beyond the library's images.  VSG_EINVAL if out is NULL or n < 0. */
+int vsg_last_launch_images(int32_t* out, int32_t n);
 
 /*
  * Per-layer parity hook (tests and tuning only; it allocates and synchronises, unlike the run calls):
@@ -430,6 +433,58 @@ int vsg_debug_conv1d_bf16(const void* x_bf16, const float* w, const float* bias,
                           const void* add1_bf16, float scale, float* out_f32, void* out_raw_bf16, void* out_act_bf16,
                           int32_t B, int32_t L, int32_t Cin, int32_t Cout, int32_t k, int32_t dilation, int32_t flags,
                           int32_t device);
+
+/*
+ * Per-launch hook of the convolution kernel (tests only; allocates and synchronises): one launch with every epilogue
+ * field and output geometry the library's own calls use.  B utterances, Cin -> Cout channels, k taps at dilation dil;
+ * row q < Lq of the output (time step n = q * out_stride + out_phase < Lout) reads input rows q + in_off0 + j * dil
+ * (zero outside 0 .. Lin - 1):
+ *   linear (mode 0):  v = ((acc + bias + bcond) + add0 + add1) * scale [* mask]
+ *   gate (mode 1):    output channel c of Cout / 2 = tanh(v[2c]) * sigmoid(v[2c + 1]), v = acc + bias + bcond
+ *   couple (mode 2):  m = (acc + bias) * mask; out = (add0 - m) * mask (couple_sign < 0) | m + add0 * mask (> 0)
+ * planes: bf16 planes per weight and activation value -- 1 plain bf16; 2 split-bf16 (hi, lo; linear mode only); 3 (hi,
+ * mid, lo).  A tensor with several planes holds them part_stride (x: x_part_stride) channels apart in rows of ld (x: x_ld)
+ * channels; 0 = the tensor's own width (rows [hi | lo]).  Planar layouts put whole planes apart: ld = C, part_stride =
+ * B * L * C.  add0_is_act: add0 holds leaky_relu(r, slope) of the residual r, inverted in the epilogue.  out_raw = v,
+ * out_act = leaky_relu(v, slope), each split into planes; out_f32 = v in fp32 [B, Lout, Cout (gate: Cout / 2)].
+ * epi_sigs as in the library's defaults (2): 0 runs the generic image only, 1 adds ACT / RES_ACT / LINEAR, 2 the
+ * running-sum images.  *image_out = the EPI_SIG_* image launched (GENERIC 0, ACT 1, RES_ACT 2, LINEAR 3, X6 4, SUM0 5,
+ * SUM1 6, FINAL 7, ACT_X3 9, RES_ACT_X3 10, SUM0_X3 11, SUM1_X3 12, FINAL_X3 13).
+ * x, add0, add1, out_raw, out_act, mask ([B][Lout]) and bcond ([B][bcond_bs] from output channel 0) are device pointers;
+ * w (fp32 [Cout][Cin][k]) and bias (fp32 [Cout]) live on the host.  Optional pointers may be NULL.
+ */
+typedef struct VsgDebugConv {
+  const void* x;
+  const float* w;
+  const float* bias;
+  const float* bcond;
+  const float* mask;
+  const void* add0;
+  const void* add1;
+  void* out_raw;
+  void* out_act;
+  float* out_f32;
+  int32_t planes, mode, couple_sign, add0_is_act, bcond_bs;
+  float scale, slope;
+  int32_t B, Lin, Cin, Cout, k, dil, in_off0, Lq, out_stride, out_phase, Lout;
+  int32_t x_ld, x_part_stride, ld, part_stride;
+  int32_t epi_sigs;
+} VsgDebugConv;
+int vsg_debug_conv_tc(const VsgDebugConv* d, int32_t* image_out, int32_t device);
+
+/*
+ * The decoder's upsampler as the generator launches it (tests only; allocates and synchronises):
+ *   y = conv_transpose1d(x, w, bias, stride = rate, padding = (k - rate) / 2)   (modules/visinger/decoder.py:46)
+ * w: HOST fp32 [Cin][Cout][k]; bias: HOST fp32 [Cout].  x: device bf16 [B, Lin, Cin]; out_act = leaky_relu(y, 0.1) and
+ * out_raw = y (or NULL): device bf16 [B, Lin * rate, Cout]; out_f32: device fp32 [B, Lin * rate, Cout] or NULL (the fp32
+ * copy runs the generic image; without it the production image runs).  flags bit 0: merged form (one convolution
+ * Cin -> rate * Cout) instead of one launch per polyphase; bit 1: two bf16 planes per value; bit 2: planar input (planes
+ * B * Lin * Cin apart; otherwise rows [hi | lo]); bit 3: planar outputs (planes B * Lin * rate * Cout apart).  The merged
+ * two-plane form needs planar outputs.  *image_out = the EPI_SIG_* image of the last launch.
+ */
+int vsg_debug_upsample_tc(const void* x_bf16, const float* w, const float* bias, int32_t Cin, int32_t Cout, int32_t rate,
+                          int32_t k, int32_t B, int32_t Lin, void* out_act_bf16, void* out_raw_bf16, float* out_f32,
+                          int32_t flags, int32_t* image_out, int32_t device);
 
 /*
  * Per-layer parity hook for the fused ResBlock1 pair kernel (tests and tuning only; allocates and synchronises):

@@ -89,6 +89,24 @@ class VsgTensor(ctypes.Structure):
                 ("shape", ctypes.c_int64 * 4)]
 
 
+class VsgDebugConv(ctypes.Structure):
+    """Descriptor of vsg_debug_conv_tc (include/visinger_b200.h)."""
+    _fields_ = ([(n, ctypes.c_void_p) for n in ("x", "w", "bias", "bcond", "mask", "add0", "add1", "out_raw", "out_act",
+                                                "out_f32")] +
+                [(n, ctypes.c_int32) for n in ("planes", "mode", "couple_sign", "add0_is_act", "bcond_bs")] +
+                [("scale", ctypes.c_float), ("slope", ctypes.c_float)] +
+                [(n, ctypes.c_int32) for n in ("B", "Lin", "Cin", "Cout", "k", "dil", "in_off0", "Lq", "out_stride",
+                                               "out_phase", "Lout", "x_ld", "x_part_stride", "ld", "part_stride",
+                                               "epi_sigs")])
+
+
+# epilogue images of the convolution kernel (csrc/conv_tc.cuh, EPI_SIG_*), as vsg_debug_conv_tc and vsg_last_launch_images
+# number them
+EPI_SIG = dict(GENERIC=0, ACT=1, RES_ACT=2, LINEAR=3, X6=4, SUM0=5, SUM1=6, FINAL=7, POST=8, ACT_X3=9, RES_ACT_X3=10,
+               SUM0_X3=11, SUM1_X3=12, FINAL_X3=13, MAG=14)
+EPI_TC_LINEAR, EPI_TC_GATE, EPI_TC_COUPLE = 0, 1, 2
+
+
 def _source_files():
     files = [os.path.join(_CSRC, f) for f in sorted(os.listdir(_CSRC)) if f.endswith((".cu", ".cuh", ".h", ".inc"))]
     return files + [_HEADER]
@@ -192,6 +210,13 @@ def lib() -> ctypes.CDLL:
         L.vsg_debug_conv1d_bf16.restype = ctypes.c_int
         L.vsg_debug_conv1d_bf16.argtypes = [vp, vp, vp, vp, vp, ctypes.c_float, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32,
                                             i32]
+        L.vsg_last_launch_images.restype = ctypes.c_int
+        L.vsg_last_launch_images.argtypes = [vp, i32]
+        L.vsg_debug_conv_tc.restype = ctypes.c_int
+        L.vsg_debug_conv_tc.argtypes = [ctypes.POINTER(VsgDebugConv), ctypes.POINTER(ctypes.c_int32), i32]
+        L.vsg_debug_upsample_tc.restype = ctypes.c_int
+        L.vsg_debug_upsample_tc.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, i32,
+                                            ctypes.POINTER(ctypes.c_int32), i32]
         L.vsg_set_tc_options.restype = ctypes.c_int
         L.vsg_set_tc_options.argtypes = [i32, i32, i32, i32]
         L.vsg_debug_pair_bf16.restype = ctypes.c_int
@@ -266,6 +291,13 @@ def check(rc: int, what: str) -> None:
 
 def last_launch_count() -> int:
     return int(lib().vsg_last_launch_count())
+
+
+def last_launch_images() -> Dict[str, int]:
+    """Launches of the convolution kernel per epilogue image (EPI_SIG names) in the most recent call on this thread."""
+    out = (ctypes.c_int32 * len(EPI_SIG))()
+    check(lib().vsg_last_launch_images(out, len(EPI_SIG)), "vsg_last_launch_images")
+    return {name: int(out[i]) for name, i in EPI_SIG.items()}
 
 
 def require_cuda(t: torch.Tensor, name: str) -> None:
@@ -591,6 +623,51 @@ def debug_conv1d_bf16(x_bld: torch.Tensor, w: torch.Tensor, bias, dilation: int,
                                      B, Lx, Cin, Cout, k, dilation, flags, dev.index or 0)
     check(rc, "vsg_debug_conv1d_bf16")
     return (out, raw, act) if want_bf16 else out
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def debug_conv_tc(x, w, bias=None, *, B, Lin, Lq, Lout=None, dil=1, in_off0=None, out_stride=1, out_phase=0, planes=1,
+                  mode=EPI_TC_LINEAR, couple_sign=-1, add0_is_act=0, bcond=None, bcond_bs=0, mask=None, add0=None, add1=None,
+                  out_raw=None, out_act=None, out_f32=None, scale=1.0, slope=0.1, x_ld=0, x_part_stride=0, ld=0,
+                  part_stride=0, epi_sigs=2) -> int:
+    """One launch of the convolution kernel through vsg_debug_conv_tc (include/visinger_b200.h).  x, bcond, mask, adds and
+    outputs are caller-allocated CUDA tensors (outputs written in place); w [Cout, Cin, k] and bias [Cout] may live anywhere.
+    in_off0 defaults to the centred -(k - 1) * dil / 2.  Returns the EPI_SIG_* image the launch ran."""
+    require_cuda(x, "x")
+    for t in (x, bcond, mask, add0, add1, out_raw, out_act, out_f32):
+        assert t is None or (t.is_cuda and t.is_contiguous())
+    Cout, Cin, k = w.shape
+    wh = w.detach().to("cpu", torch.float32).contiguous()
+    bh = bias.detach().to("cpu", torch.float32).contiguous() if bias is not None else None
+    d = VsgDebugConv(_ptr(x), wh.data_ptr(), _ptr(bh), _ptr(bcond), _ptr(mask), _ptr(add0), _ptr(add1), _ptr(out_raw),
+                     _ptr(out_act), _ptr(out_f32), planes, mode, couple_sign, add0_is_act, bcond_bs, scale, slope, B, Lin,
+                     Cin, Cout, k, dil, -((k - 1) * dil // 2) if in_off0 is None else in_off0, Lq, out_stride, out_phase,
+                     Lq if Lout is None else Lout, x_ld, x_part_stride, ld, part_stride, epi_sigs)
+    img = ctypes.c_int32(-1)
+    torch.cuda.synchronize(x.device)
+    check(lib().vsg_debug_conv_tc(ctypes.byref(d), ctypes.byref(img), x.device.index or 0), "vsg_debug_conv_tc")
+    return int(img.value)
+
+
+def debug_upsample_tc(x, w, bias, rate: int, flags: int, out_act, out_raw=None, out_f32=None) -> int:
+    """The decoder's upsampler through vsg_debug_upsample_tc: x CUDA bf16 (layout per flags), w [Cin, Cout, k] (the
+    ConvTranspose1d weight), bias [Cout]; caller-allocated outputs.  Returns the EPI_SIG_* image of the last launch."""
+    require_cuda(x, "x")
+    for t in (x, out_act, out_raw, out_f32):
+        assert t is None or (t.is_cuda and t.is_contiguous())
+    Cin, Cout, k = w.shape
+    B, Lin = x.shape[-3], x.shape[-2]
+    wh = w.detach().to("cpu", torch.float32).contiguous()
+    bh = bias.detach().to("cpu", torch.float32).contiguous()
+    img = ctypes.c_int32(-1)
+    torch.cuda.synchronize(x.device)
+    check(lib().vsg_debug_upsample_tc(x.data_ptr(), wh.data_ptr(), bh.data_ptr(), Cin, Cout, rate, k, B, Lin, out_act.data_ptr(),
+                                      _ptr(out_raw), _ptr(out_f32), flags, ctypes.byref(img), x.device.index or 0),
+          "vsg_debug_upsample_tc")
+    return int(img.value)
 
 
 def debug_pair_bf16(xa_bld: torch.Tensor, w1, b1, w2, b2, d1: int, add0=None, add1=None, scale: float = 1.0,

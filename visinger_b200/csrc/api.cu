@@ -64,7 +64,7 @@ extern "C" size_t vsg_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T,
 
 extern "C" int vsg_prior_sample(const float* mu_p, const float* logs_p, const float* noise, const float* mask,
                                 float* z_p, int32_t B, int32_t C, int32_t T, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   if (B < 0 || C < 0 || T < 0) return fail(VSG_EINVAL, "negative dimension");
   if ((long long)B * C * T == 0) return VSG_OK;
   if (!mu_p || !logs_p || !noise || !mask || !z_p) return fail(VSG_EINVAL, "null pointer");
@@ -74,7 +74,7 @@ extern "C" int vsg_prior_sample(const float* mu_p, const float* logs_p, const fl
 extern "C" int vsg_flow_forward(const VsgPack* pack, const float* x, const float* mask, const float* g, float* y,
                                 int32_t B, int32_t T, int32_t reverse, int32_t precision, void* workspace,
                                 size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_flow) return fail(VSG_EINVAL, "pack has no flow");
   if (B == 0 || T == 0) return VSG_OK;
@@ -89,7 +89,7 @@ extern "C" int vsg_flow_forward(const VsgPack* pack, const float* x, const float
 extern "C" int vsg_generator_forward(const VsgPack* pack, const float* z, const float* g, float* wav, int32_t B,
                                      int32_t T, int32_t precision, void* workspace, size_t workspace_bytes,
                                      void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_dec) return fail(VSG_EINVAL, "pack has no decoder");
   if (B == 0 || T == 0) return VSG_OK;
@@ -107,7 +107,7 @@ extern "C" int vsg_generator_forward(const VsgPack* pack, const float* z, const 
 extern "C" int vsg_infer(const VsgPack* pack, const float* mu_p, const float* logs_p, const float* noise,
                          const float* mask, const float* g, float* wav, float* z_q_out, int32_t B, int32_t T,
                          int32_t precision, void* workspace, size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_flow || !pack->has_dec) return fail(VSG_EINVAL, "vsg_infer needs a pack with both flow and decoder");
   if (pack->cfg.flow_channels != pack->cfg.dec_initial_channel)
@@ -160,7 +160,7 @@ extern "C" size_t vsg_posterior_workspace_bytes(const VsgPack* pack, int32_t B, 
 extern "C" int vsg_posterior_forward(const VsgPack* pack, const float* x, const float* mask, const float* g,
                                      const float* noise, float* z_q, float* stats, int32_t B, int32_t T, int32_t precision,
                                      void* workspace, size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_enc) return fail(VSG_EINVAL, "pack has no posterior encoder (create it with vsg_enc_pack_create)");
   if (B == 0 || T == 0) return VSG_OK;
@@ -182,7 +182,7 @@ extern "C" size_t vsg_relenc_workspace_bytes(const VsgPack* pack, int32_t B, int
 extern "C" int vsg_relenc_forward(const VsgPack* pack, const float* x, const float* mask, const float* g, int32_t g_per_frame,
                                   float* y, int32_t B, int32_t T, int32_t precision, void* workspace, size_t workspace_bytes,
                                   void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_relenc) return fail(VSG_EINVAL, "pack has no relative-position encoder (create it with vsg_relenc_pack_create)");
   if (B == 0 || T == 0) return VSG_OK;
@@ -204,7 +204,7 @@ extern "C" size_t vsg_frame_prior_workspace_bytes(const VsgPack* pack, int32_t B
 extern "C" int vsg_frame_prior_forward(const VsgPack* pack, const float* x, const float* mask, const float* g,
                                        const float* noise, float* stats, float* z_p, int32_t B, int32_t T, int32_t precision,
                                        void* workspace, size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_relenc || !pack->relenc.proj_w)
     return fail(VSG_EINVAL, "pack has no frame prior network (create it with vsg_frame_prior_pack_create)");
@@ -221,7 +221,7 @@ extern "C" int vsg_frame_prior_forward(const VsgPack* pack, const float* x, cons
 
 extern "C" int vsg_length_regulate(const float* enc, const int64_t* mel2ph, const float* pos_table, int32_t pos_rows,
                                    float* y, int32_t B, int32_t H, int32_t T_ph, int32_t T, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   if (B < 0 || H <= 0 || T_ph < 0 || T < 0) return fail(VSG_EINVAL, "bad dimension");
   if (B == 0 || T == 0) return VSG_OK;
   if (!enc || !mel2ph || !y || (pos_table && pos_rows <= 0)) return fail(VSG_EINVAL, "null pointer");
@@ -231,7 +231,7 @@ extern "C" int vsg_length_regulate(const float* enc, const int64_t* mel2ph, cons
 extern "C" int vsg_infer_zp(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav,
                             float* z_q_out, int32_t B, int32_t T, int32_t precision, void* workspace, size_t workspace_bytes,
                             void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_common(pack, B, T, precision));
   if (!pack->has_flow || !pack->has_dec) return fail(VSG_EINVAL, "vsg_infer_zp needs a pack with both flow and decoder");
   if (pack->cfg.flow_channels != pack->cfg.dec_initial_channel)

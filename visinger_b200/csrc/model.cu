@@ -612,7 +612,7 @@ extern "C" int vsg_model_forward(const VsgPack* pack, const int64_t* text_tokens
                                  const float* spk_embed, const float* f0, const float* uv, const float* noise,
                                  const uint64_t* seeds, float* wav, float* f0_pred, float* z_q_out, int32_t B, int32_t T_ph,
                                  int32_t T, int32_t precision, void* workspace, size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!pack || !pack->model) return fail(VSG_EINVAL, "pack is not a model pack (create it with vsg_model_pack_create)");
   const ModelPack& m = *pack->model;
   const VsgModelConfig& c = m.cfg;
@@ -650,7 +650,7 @@ extern "C" int vsg_model_forward(const VsgPack* pack, const int64_t* text_tokens
 }
 
 extern "C" int vsg_normal_noise(const uint64_t* seeds, float* out, int32_t B, int32_t C, int32_t T, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   if (B < 0 || C < 0 || T < 0) return fail(VSG_EINVAL, "negative dimension");
   if ((long long)B * C * T == 0) return VSG_OK;
   if (!seeds || !out) return fail(VSG_EINVAL, "null pointer");
@@ -658,7 +658,7 @@ extern "C" int vsg_normal_noise(const uint64_t* seeds, float* out, int32_t B, in
 }
 
 extern "C" int vsg_debug_position_table(const float* freq, int32_t rows, int32_t dim, float* out, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   if (rows < 0 || dim < 4) return fail(VSG_EINVAL, "bad table shape (%d rows, dim %d; dim >= 4)", rows, dim);
   if (rows == 0) return VSG_OK;
   if (!out) return fail(VSG_EINVAL, "null pointer");
@@ -751,7 +751,7 @@ int check_convert(const VsgPack* pack, int B, int T, int precision) {
 
 extern "C" int vsg_spectrogram(const VsgPack* pack, const float* wav, const int32_t* lengths, float* spec, int32_t B,
                                int32_t T, int32_t precision, void* workspace, size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_convert(pack, B, T, precision));
   if (B == 0 || T == 0) return VSG_OK;
   if (!wav || !lengths || !spec) return fail(VSG_EINVAL, "null pointer: wav, lengths and spec are required");
@@ -782,7 +782,7 @@ extern "C" int vsg_model_convert(const VsgPack* pack, const float* wav, const fl
                                  const float* tgt_spk_embed, const float* noise, const uint64_t* seeds, float* wav_out,
                                  float* spec_out, float* z_out, int32_t B, int32_t T, int32_t precision, void* workspace,
                                  size_t workspace_bytes, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   VSG_TRY(check_convert(pack, B, T, precision));
   const VsgModelConfig& c = pack->model->cfg;
   if (B == 0 || T == 0) return VSG_OK;

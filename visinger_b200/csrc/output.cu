@@ -104,7 +104,7 @@ using namespace vsg;
 
 extern "C" int vsg_wav_to_int16(const float* wav, const int32_t* lengths, int16_t* pcm, float* peak, int32_t B, int32_t L,
                                 int32_t norm, void* stream) {
-  g_launches = 0;
+  reset_launch_counts();
   if (B < 0 || L < 0) return fail(VSG_EINVAL, "negative batch (%d) or length (%d)", B, L);
   if (B > 65535) return fail(VSG_EUNSUPPORTED, "batch %d exceeds 65535", B);
   if ((long long)B * L == 0) return VSG_OK;

@@ -18,6 +18,7 @@ namespace vsg {
 
 thread_local char g_err[1024] = {0};
 thread_local int g_launches = 0;
+thread_local int g_image_launches[kImageSlots] = {0};
 
 namespace {
 
@@ -410,49 +411,11 @@ int pack_decoder(const Loader& L, const std::string& pre, VsgPack* P) {
     const std::string pu = pre + "ups." + std::to_string(i);
     VSG_TRY(L.eff_weight(pu, st.Cin, st.Cout, st.kernel, W));
     VSG_TRY(L.bias(pu, st.Cout, b, true));
-    // polyphase split: y[q*s + r] = sum_{jj} sum_ci x[ci, q + in_off0 + jj] * W[ci][co][j0 + s*(n_r-1-jj)]
-    st.phases.resize(st.rate);
-    for (int r = 0; r < st.rate; ++r) {
-      const int s = st.rate, k = st.kernel, p = st.pad;
-      const int j0 = (r + p) % s;
-      const int nr = (k - 1 - j0) / s + 1;
-      const int cr = (r + p - j0) / s;
-      UpsPhase& ph = st.phases[r];
-      ph.in_off0 = cr - nr + 1;
-      std::vector<float> Wc((size_t)st.Cout * st.Cin * nr);   // as a Conv1d weight [co][ci][jj]
-      for (int co = 0; co < st.Cout; ++co)
-        for (int ci = 0; ci < st.Cin; ++ci)
-          for (int jj = 0; jj < nr; ++jj)
-            Wc[((size_t)co * st.Cin + ci) * nr + jj] = W[((size_t)ci * st.Cout + co) * k + j0 + s * (nr - 1 - jj)];
-      VSG_TRY(pack_conv_f32(L, Wc, b, st.Cout, st.Cin, nr, Identity{}, &ph.f32));
-      VSG_TRY(pack_conv_tc(P, Wc, b, st.Cout, st.Cin, nr, &ph.tc));
-      VSG_TRY(pack_conv_tc(P, Wc, b, st.Cout, st.Cin, nr, &ph.x3, 2));
-    }
-    {   // merged polyphase convolution for the tensor-core path (one launch, contiguous stores)
-      int off_min = 1 << 30, off_max = -(1 << 30);
-      for (int r = 0; r < st.rate; ++r) {
-        const int nr = st.phases[r].f32.ktaps;
-        off_min = std::min(off_min, st.phases[r].in_off0);
-        off_max = std::max(off_max, st.phases[r].in_off0 + nr - 1);
-      }
-      const int kt = off_max - off_min + 1, s = st.rate, k = st.kernel, p = st.pad;
-      std::vector<float> Wm((size_t)s * st.Cout * st.Cin * kt, 0.f), bm((size_t)s * st.Cout);
-      for (int r = 0; r < s; ++r) {
-        const int j0 = (r + p) % s, nr = (k - 1 - j0) / s + 1, off_r = st.phases[r].in_off0;
-        for (int co = 0; co < st.Cout; ++co) {
-          bm[(size_t)r * st.Cout + co] = b[co];
-          for (int ci = 0; ci < st.Cin; ++ci)
-            for (int t = 0; t < kt; ++t) {
-              const int tp = off_min + t - off_r;            // tap index inside phase r
-              if (tp < 0 || tp >= nr) continue;
-              Wm[(((size_t)r * st.Cout + co) * st.Cin + ci) * kt + t] = W[((size_t)ci * st.Cout + co) * k + j0 + s * (nr - 1 - tp)];
-            }
-        }
-      }
-      st.merged_in_off0 = off_min;
-      VSG_TRY(pack_conv_tc(P, Wm, bm, s * st.Cout, st.Cin, kt, &st.merged_tc));
-      VSG_TRY(pack_conv_tc(P, Wm, bm, s * st.Cout, st.Cin, kt, &st.merged_x3, 2));   // (bf16x3: used where the output is planar)
-    }
+    std::vector<std::vector<float>> phase_w;
+    VSG_TRY(pack_upsampler(P, W, b, st.Cin, st.Cout, st.rate, st.kernel, &st, &phase_w));
+    for (int r = 0; r < st.rate; ++r)
+      VSG_TRY(pack_conv_f32(L, phase_w[r], b, st.Cout, st.Cin, (int)(phase_w[r].size() / ((size_t)st.Cout * st.Cin)), Identity{},
+                            &st.phases[r].f32));
     // resblocks                                                            decoder.py:28-32
     st.blocks.resize(c.dec_n_kernels);
     for (int j = 0; j < c.dec_n_kernels; ++j) {
@@ -543,6 +506,11 @@ using namespace vsg;
 extern "C" int vsg_abi_version(void) { return VSG_ABI_VERSION; }
 extern "C" const char* vsg_last_error(void) { return vsg::g_err; }
 extern "C" int32_t vsg_last_launch_count(void) { return vsg::g_launches; }
+extern "C" int vsg_last_launch_images(int32_t* out, int32_t n) {
+  if (!out || n < 0) return vsg::fail(VSG_EINVAL, "vsg_last_launch_images: null output or negative count");
+  for (int32_t i = 0; i < n; ++i) out[i] = i < vsg::kImageSlots ? vsg::g_image_launches[i] : 0;
+  return VSG_OK;
+}
 extern "C" int32_t vsg_hop_size(const VsgPack* p) {
   if (p && p->model) p = p->model->hot;
   return (p && p->has_dec) ? p->hop : 0;

@@ -469,7 +469,7 @@ int mask_mul(const float* x, const float* mask, float* y, int B, int C, int T, c
 extern "C" int vsg_debug_attention_f32(const float* qkv, const float* mask, const float* ek, const float* ev, float* o,
                                        int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device) {
   using namespace vsg;
-  g_launches = 0;
+  reset_launch_counts();
   if (!qkv || !mask || !ek || !ev || !o) return fail(VSG_EINVAL, "null pointer");
   if (B < 1 || T < 1 || n_heads < 1 || w < 0) return fail(VSG_EINVAL, "bad argument");
   VSG_CUDA_TRY(cudaSetDevice(device));

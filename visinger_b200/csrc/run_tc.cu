@@ -154,7 +154,7 @@ static const TunedPlan kTunedPlans[] = {
 // One convolution launch.  x: [B, Lin, Cin] bf16 channels-last; add/out tensors: [B, Lout, Cout].
 int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, int B, int Lin, int in_off0, int dil,
                    int Lq, int out_stride, int out_phase, int Lout, const EpiTC& e, const TCOptions& opt, int* error_flag,
-                   cudaStream_t st, int x_ld = 0, int x_part_stride = 0) {
+                   cudaStream_t st, int x_ld = 0, int x_part_stride = 0, int* image_out = nullptr) {
   const int a_planes = w.wsplit ? 1 : w.planes;           // bf16 planes of the activations and of every epilogue tensor
   if (x_ld == 0) x_ld = a_planes * w.Cin;
   if (x_part_stride == 0) x_part_stride = w.Cin;          // channels between the bf16 planes of an input row
@@ -479,6 +479,9 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
   }
   if (le != cudaSuccess) return fail(VSG_ECUDA, "launch of conv_tc_kernel failed: %s", cudaGetErrorString(le));
   VSG_LAUNCH_CHECK("conv_tc_kernel");
+  static_assert(EPI_SIG_COUNT <= kImageSlots, "one launch counter per epilogue image");
+  ++g_image_launches[sig];
+  if (image_out) *image_out = sig;
   return VSG_OK;
 }
 
@@ -958,6 +961,60 @@ int pack_conv_tc(VsgPack* P, const std::vector<float>& W, const std::vector<floa
   out->bias = (float*)db;
   VSG_TRY(encode_2d(&out->tmap, dw, (uint64_t)CinT, (uint64_t)k * Cout, (uint32_t)KC, (uint32_t)NT, KC));
   out->has_tmap = true;
+  return VSG_OK;
+}
+
+// ConvTranspose1d(Cin -> Cout, k, stride = rate, padding = (k - rate) / 2) with weight W[ci][co][j] as convolutions over
+// the input rate.  Polyphase split: y[q*s + r] = sum_{jj} sum_ci x[ci, q + in_off0 + jj] * W[ci][co][j0 + s*(n_r-1-jj)].
+int pack_upsampler(VsgPack* P, const std::vector<float>& W, const std::vector<float>& b, int Cin, int Cout, int rate, int k,
+                   UpStage* out, std::vector<std::vector<float>>* phase_w) {
+  UpStage& st = *out;
+  st.rate = rate; st.kernel = k; st.Cin = Cin; st.Cout = Cout; st.pad = (k - rate) / 2;
+  if (rate < 1 || k < rate || (k - rate) % 2)
+    return fail(VSG_EUNSUPPORTED, "upsampler: kernel %d / stride %d needs kernel >= stride and (kernel - stride) even", k, rate);
+  st.phases.resize(st.rate);
+  if (phase_w) phase_w->assign(st.rate, std::vector<float>());
+  for (int r = 0; r < st.rate; ++r) {
+    const int s = st.rate, p = st.pad;
+    const int j0 = (r + p) % s;
+    const int nr = (k - 1 - j0) / s + 1;
+    const int cr = (r + p - j0) / s;
+    UpsPhase& ph = st.phases[r];
+    ph.in_off0 = cr - nr + 1;
+    std::vector<float> Wc((size_t)st.Cout * st.Cin * nr);   // as a Conv1d weight [co][ci][jj]
+    for (int co = 0; co < st.Cout; ++co)
+      for (int ci = 0; ci < st.Cin; ++ci)
+        for (int jj = 0; jj < nr; ++jj)
+          Wc[((size_t)co * st.Cin + ci) * nr + jj] = W[((size_t)ci * st.Cout + co) * k + j0 + s * (nr - 1 - jj)];
+    VSG_TRY(pack_conv_tc(P, Wc, b, st.Cout, st.Cin, nr, &ph.tc));
+    VSG_TRY(pack_conv_tc(P, Wc, b, st.Cout, st.Cin, nr, &ph.x3, 2));
+    if (phase_w) (*phase_w)[r] = std::move(Wc);
+  }
+  {   // merged polyphase convolution for the tensor-core path (one launch, contiguous stores)
+    int off_min = 1 << 30, off_max = -(1 << 30);
+    for (int r = 0; r < st.rate; ++r) {
+      const int nr = (k - 1 - (r + st.pad) % st.rate) / st.rate + 1;
+      off_min = std::min(off_min, st.phases[r].in_off0);
+      off_max = std::max(off_max, st.phases[r].in_off0 + nr - 1);
+    }
+    const int kt = off_max - off_min + 1, s = st.rate, p = st.pad;
+    std::vector<float> Wm((size_t)s * st.Cout * st.Cin * kt, 0.f), bm((size_t)s * st.Cout);
+    for (int r = 0; r < s; ++r) {
+      const int j0 = (r + p) % s, nr = (k - 1 - j0) / s + 1, off_r = st.phases[r].in_off0;
+      for (int co = 0; co < st.Cout; ++co) {
+        bm[(size_t)r * st.Cout + co] = b[co];
+        for (int ci = 0; ci < st.Cin; ++ci)
+          for (int t = 0; t < kt; ++t) {
+            const int tp = off_min + t - off_r;            // tap index inside phase r
+            if (tp < 0 || tp >= nr) continue;
+            Wm[(((size_t)r * st.Cout + co) * st.Cin + ci) * kt + t] = W[((size_t)ci * st.Cout + co) * k + j0 + s * (nr - 1 - tp)];
+          }
+      }
+    }
+    st.merged_in_off0 = off_min;
+    VSG_TRY(pack_conv_tc(P, Wm, bm, s * st.Cout, st.Cin, kt, &st.merged_tc));
+    VSG_TRY(pack_conv_tc(P, Wm, bm, s * st.Cout, st.Cin, kt, &st.merged_x3, 2));   // (bf16x3: used where the output is planar)
+  }
   return VSG_OK;
 }
 
@@ -1445,6 +1502,36 @@ int frame_prior_forward_tc(const VsgPack* P, const float* x, const float* mask, 
   return VSG_OK;
 }
 
+// ConvTranspose1d of decoder stage `us` (decoder.py:46) + its bias over nb utterances: out_act = leaky_relu(y) and, if
+// given, out_raw = y and out_f32 = y, [nb, Lin * rate, Cout] channels-last.  merged: ONE Conv1d(Cin -> rate * Cout) over the
+// input rate, whose [nb, Lin, rate * Cout] output is, byte for byte, the upsampled tensor; else one strided launch per
+// polyphase.  x3: two bf16 planes per tensor.  out_part > 0: the output planes are planar, out_part elements apart (rows of
+// Cout channels); 0: rows [hi | lo] (the merged form needs planar planes in x3).  in_ld / in_part: the input's layout as
+// launch_conv_tc takes it (0 = rows [hi | lo]).
+int launch_upsample_tc(const VsgPack* P, const UpStage& us, bool x3, bool merged, const __nv_bfloat16* xin, int nb, int Lin,
+                       __nv_bfloat16* out_act, __nv_bfloat16* out_raw, float* out_f32, int out_part, int in_ld, int in_part,
+                       const TCOptions& opt, int* err, cudaStream_t st, int* image_out = nullptr) {
+  const int Lout = Lin * us.rate, ch = us.Cout;
+  if (merged) {
+    EpiTC e;
+    e.bias = us.merged_tc.bias;
+    e.out_act = out_act; e.out_raw = out_raw; e.out_f32 = out_f32;
+    if (out_part) { e.ld = us.rate * ch; e.part_stride = out_part; }
+    return launch_conv_tc(P, x3 ? us.merged_x3 : us.merged_tc, xin, nb, Lin, us.merged_in_off0, 1, Lin, 1, 0, Lin, e, opt, err,
+                          st, in_ld, in_part, image_out);
+  }
+  for (int r = 0; r < us.rate; ++r) {   // one strided launch per polyphase
+    EpiTC e;
+    e.bias = us.phases[r].tc.bias;
+    e.out_act = out_act; e.out_raw = out_raw; e.out_f32 = out_f32;
+    if (out_part) { e.ld = ch; e.part_stride = out_part; }
+    const int Lq = (Lout - r + us.rate - 1) / us.rate;
+    VSG_TRY(launch_conv_tc(P, x3 ? us.phases[r].x3 : us.phases[r].tc, xin, nb, Lin, us.phases[r].in_off0, 1, Lq, us.rate, r,
+                           Lout, e, opt, err, st, in_ld, in_part, image_out));
+  }
+  return VSG_OK;
+}
+
 // ---- L2-resident batch tiling --------------------------------------------------------------------------------
 // Un-fused, one stage of the decoder streams 54 tensor passes through memory (SURVEY.md 7.2-3).  The stage tensors of
 // ONE utterance are small (<= 9.6 MB in bf16), so each upsampling stage is run over sub-batches whose intermediates
@@ -1619,7 +1706,7 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
     bool stage_planar_out = false;
     for (int b0 = 0; b0 < B; b0 += pl.sub[i]) {
       const int nb = std::min(pl.sub[i], B - b0);
-      const bf* xin = stage_in + (size_t)b0 * Lin * Cin * np;
+      const bf* xin = stage_in + (size_t)b0 * Lin * Cin * (prev_planar ? 1 : np);   // (planar: plane 0 of utterance b0)
       bf* xout = stage_out + (size_t)b0 * L * ch * np;
       // C <= 64 stages: every ResBlock1 is ONE kernel (rb_tc.cuh); the three launches of a stage are chained through the
       // running sum, so they stay on the caller's stream (their CTAs own all of tensor memory and cannot co-reside anyway)
@@ -1650,34 +1737,16 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
       const bool planar_any = planar || stage_planar;
       stage_planar_out = stage_planar;
       const int up_ld = planar_any ? ch : 0, up_part = planar_any ? (int)((size_t)nb * L * ch) : 0;
-      // the stage input is planar if the previous stage wrote it so
-      const int in_ld = prev_planar ? Cin : 0, in_part = prev_planar ? (int)((size_t)nb * Lin * Cin) : 0;
+      // the stage input is planar if the previous stage wrote it so: that stage ran whole (nb == B), so its planes are
+      // B * Lin * Cin elements apart whatever this stage's sub-batches are
+      const int in_ld = prev_planar ? Cin : 0, in_part = prev_planar ? (int)((size_t)B * Lin * Cin) : 0;
       // (split-bf16 planes interleaved per row would come out wrong; PLANAR planes are one-plane tensors each, so the
       // bf16x3 row-packed stages take the merged form too)
       static const bool x3_merge_off = getenv("VSG_X3_NO_MERGED_UPS") != nullptr;   // A/B aid
-      if (opt.merge_ups && (!x3 || (planar_any && us.merged_x3.has_tmap && !x3_merge_off)) && us.merged_tc.has_tmap &&
-          Lout == Lin * us.rate) {
-        // ConvTranspose1d (decoder.py:46) as ONE convolution Cin -> rate*Cout over the input rate: its channels-last
-        // output [nb, Lin, rate*Cout] is, byte for byte, the upsampled [nb, Lin*rate, Cout] tensor
-        EpiTC e;
-        e.bias = us.merged_tc.bias;
-        e.out_act = bUA;
-        if (planar_any) { e.ld = us.rate * ch; e.part_stride = up_part; }
-        if (!one_stream_all) e.out_raw = bU;
-        VSG_TRY(launch_conv_tc(P, W(us.merged_tc, us.merged_x3), xin, nb, Lin, us.merged_in_off0, 1, Lin, 1, 0, Lin, e, opt,
-                               err, st, in_ld, in_part));
-      } else {
-        for (int r = 0; r < us.rate; ++r) {   // one strided launch per polyphase
-          EpiTC e;
-          e.bias = us.phases[r].tc.bias;
-          e.out_act = bUA;
-          e.ld = up_ld; e.part_stride = up_part;
-          if (!one_stream_all) e.out_raw = bU;
-          const int Lq = (Lout - r + us.rate - 1) / us.rate;
-          VSG_TRY(launch_conv_tc(P, W(us.phases[r].tc, us.phases[r].x3), xin, nb, Lin, us.phases[r].in_off0, 1, Lq, us.rate, r,
-                                 Lout, e, opt, err, st, in_ld, in_part));
-        }
-      }
+      const bool merged = opt.merge_ups && (!x3 || (planar_any && us.merged_x3.has_tmap && !x3_merge_off)) &&
+                          us.merged_tc.has_tmap && Lout == Lin * us.rate;
+      VSG_TRY(launch_upsample_tc(P, us, x3, merged, xin, nb, Lin, bUA, one_stream_all ? nullptr : bU, nullptr, up_part, in_ld,
+                                 in_part, opt, err, st));
       // Only leaky_relu(x) is stored for the running stream; the residual x is recovered from it in the consumer's
       // epilogue (a > 0 ? a : a / slope -- as exact as a second, raw copy at the stream's precision), so the upsampler and
       // every non-final conv2 write one tensor instead of two.
@@ -1850,7 +1919,7 @@ extern "C" int vsg_debug_conv1d_bf16(const void* x_bf16, const float* w, const f
                                      const void* add1_bf16, float scale, float* out_f32, void* out_raw_bf16,
                                      void* out_act_bf16, int32_t B, int32_t L, int32_t Cin, int32_t Cout, int32_t k,
                                      int32_t dilation, int32_t flags, int32_t device) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!x_bf16 || !w) return fail(VSG_EINVAL, "null pointer");
   VSG_CUDA_TRY(cudaSetDevice(device));
   cudaDeviceProp prop;
@@ -1904,6 +1973,101 @@ extern "C" int vsg_debug_conv1d_bf16(const void* x_bf16, const float* w, const f
   return rc;
 }
 
+// One launch of conv_tc_kernel with every EpiTC field and every output geometry (tests only; allocates and synchronises).
+// See include/visinger_b200.h.
+namespace {
+struct DebugScope {   // a throw-away pack on `device` (weights, error flag), freed on exit
+  VsgPack P;
+  int* err = nullptr;
+  int open(int device) {
+    VSG_CUDA_TRY(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    VSG_CUDA_TRY(cudaGetDeviceProperties(&prop, device));
+    P.device = device;
+    P.sm_count = prop.multiProcessorCount;
+    VSG_CUDA_TRY(cudaMalloc(&err, sizeof(int)));
+    VSG_CUDA_TRY(cudaMemset(err, 0, sizeof(int)));
+    return VSG_OK;
+  }
+  int finish(int rc) {
+    if (rc != VSG_OK) return rc;
+    cudaError_t ce = cudaDeviceSynchronize();
+    if (ce != cudaSuccess) return fail(VSG_ECUDA, "conv_tc_kernel execution failed: %s", cudaGetErrorString(ce));
+    int h = 0;
+    VSG_CUDA_TRY(cudaMemcpy(&h, err, sizeof(int), cudaMemcpyDeviceToHost));
+    if (h) return fail(VSG_ECUDA, "conv_tc_kernel set its error flag (%d)", h);
+    return VSG_OK;
+  }
+  ~DebugScope() {
+    if (err) cudaFree(err);
+    for (void* q : P.allocs) cudaFree(q);
+  }
+};
+}  // namespace
+
+extern "C" int vsg_debug_conv_tc(const VsgDebugConv* d, int32_t* image_out, int32_t device) {
+  reset_launch_counts();
+  if (!d || !d->x || !d->w) return fail(VSG_EINVAL, "vsg_debug_conv_tc: null descriptor, input or weight");
+  if (d->planes < 1 || d->planes > 3) return fail(VSG_EINVAL, "vsg_debug_conv_tc: planes must be 1, 2 or 3");
+  if (d->mode != EPI_TC_LINEAR && d->mode != EPI_TC_GATE && d->mode != EPI_TC_COUPLE)
+    return fail(VSG_EINVAL, "vsg_debug_conv_tc: mode must be linear (0), gate (1) or couple (2)");
+  if (d->epi_sigs < 0 || d->epi_sigs > 2) return fail(VSG_EINVAL, "vsg_debug_conv_tc: epi_sigs must be 0, 1 or 2");
+  if (d->B <= 0 || d->Lin <= 0 || d->Cin <= 0 || d->Cout <= 0 || d->k <= 0 || d->dil <= 0 || d->Lq <= 0 || d->Lout <= 0 ||
+      d->out_stride <= 0 || d->out_phase < 0 || d->out_phase >= d->out_stride || (d->Lq - 1) * d->out_stride + d->out_phase >= d->Lout)
+    return fail(VSG_EINVAL, "vsg_debug_conv_tc: bad shape or output geometry");
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  std::vector<float> W(d->w, d->w + (size_t)d->Cout * d->Cin * d->k), bz(d->Cout, 0.f);
+  if (d->bias) bz.assign(d->bias, d->bias + d->Cout);
+  ConvWTC wt;
+  VSG_TRY(pack_conv_tc(&sc.P, W, bz, d->Cout, d->Cin, d->k, &wt, d->planes));
+  EpiTC e;
+  e.mode = d->mode; e.mask = d->mask; e.couple_sign = d->couple_sign;
+  e.ld = d->ld; e.part_stride = d->part_stride;
+  e.add0_is_act = d->add0_is_act;
+  e.bias = d->bias ? wt.bias : nullptr;
+  e.bcond = d->bcond; e.bcond_bs = d->bcond_bs;
+  e.add0 = (const __nv_bfloat16*)d->add0; e.add1 = (const __nv_bfloat16*)d->add1;
+  e.scale = d->scale; e.slope = d->slope;
+  e.out_raw = (__nv_bfloat16*)d->out_raw; e.out_act = (__nv_bfloat16*)d->out_act; e.out_f32 = d->out_f32;
+  TCOptions opt;
+  opt.epi_sigs = d->epi_sigs;
+  int img = -1;
+  const int rc = launch_conv_tc(&sc.P, wt, (const __nv_bfloat16*)d->x, d->B, d->Lin, d->in_off0, d->dil, d->Lq, d->out_stride,
+                                d->out_phase, d->Lout, e, opt, sc.err, 0, d->x_ld, d->x_part_stride, &img);
+  if (image_out) *image_out = img;
+  return sc.finish(rc);
+}
+
+// The decoder's upsampler (ConvTranspose1d + bias + leaky_relu) as the generator launches it (tests only; allocates and
+// synchronises).  See include/visinger_b200.h.
+extern "C" int vsg_debug_upsample_tc(const void* x_bf16, const float* w, const float* bias, int32_t Cin, int32_t Cout,
+                                     int32_t rate, int32_t k, int32_t B, int32_t Lin, void* out_act_bf16, void* out_raw_bf16,
+                                     float* out_f32, int32_t flags, int32_t* image_out, int32_t device) {
+  reset_launch_counts();
+  if (!x_bf16 || !w || !bias || !out_act_bf16) return fail(VSG_EINVAL, "vsg_debug_upsample_tc: null input, weight, bias or output");
+  if (Cin <= 0 || Cout <= 0 || B <= 0 || Lin <= 0) return fail(VSG_EINVAL, "vsg_debug_upsample_tc: bad shape");
+  const bool merged = flags & 1, x3 = flags & 2, planar_in = flags & 4, planar_out = flags & 8;
+  if (!x3 && (planar_in || planar_out)) return fail(VSG_EINVAL, "vsg_debug_upsample_tc: planar layouts need two planes");
+  if (merged && x3 && !planar_out) return fail(VSG_EINVAL, "vsg_debug_upsample_tc: the two-plane merged form writes planar planes");
+  const size_t in_part = (size_t)B * Lin * Cin, out_part = (size_t)B * Lin * rate * Cout;
+  if (out_part >= ((size_t)1 << 31)) return fail(VSG_EINVAL, "vsg_debug_upsample_tc: tensor too large");
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  UpStage us;
+  std::vector<float> W(w, w + (size_t)Cin * Cout * k), b(bias, bias + Cout);
+  VSG_TRY(pack_upsampler(&sc.P, W, b, Cin, Cout, rate, k, &us));
+  if (!(merged ? us.merged_tc.has_tmap : us.phases[0].tc.has_tmap))
+    return fail(VSG_EUNSUPPORTED, "vsg_debug_upsample_tc: channel counts must be multiples of 16");
+  TCOptions opt;
+  int img = -1;
+  const int rc = launch_upsample_tc(&sc.P, us, x3, merged, (const __nv_bfloat16*)x_bf16, B, Lin, (__nv_bfloat16*)out_act_bf16,
+                                    (__nv_bfloat16*)out_raw_bf16, out_f32, planar_out ? (int)out_part : 0,
+                                    planar_in ? Cin : 0, planar_in ? (int)in_part : 0, opt, sc.err, 0, &img);
+  if (image_out) *image_out = img;
+  return sc.finish(rc);
+}
+
 // Per-layer parity hook for the fused ResBlock1 pair (tests only; allocates and synchronises).
 //   xa: device bf16 [B, L, C] = leaky_relu(x); w1/w2: HOST fp32 [C][C][k]; b1/b2: HOST fp32 [C]; add0/add1 as above;
 //   v = (conv1d(leaky_relu(conv1d(xa, w1, dilation d1) + b1), w2) + b2 + add0 + add1) * scale.
@@ -1911,7 +2075,7 @@ extern "C" int vsg_debug_pair_bf16(const void* xa_bf16, const float* w1, const f
                                    const void* add0_bf16, const void* add1_bf16, float scale, float* out_f32,
                                    void* out_raw_bf16, void* out_act_bf16, int32_t B, int32_t L, int32_t C, int32_t k,
                                    int32_t d1, int32_t device) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!xa_bf16 || !w1 || !w2 || !b1 || !b2) return fail(VSG_EINVAL, "null pointer");
   VSG_CUDA_TRY(cudaSetDevice(device));
   cudaDeviceProp prop;
@@ -1962,7 +2126,7 @@ extern "C" int vsg_debug_resblock_bf16(const void* xa_bf16, const float* w, cons
                                        const int32_t* dilations, const void* add1_bf16, float scale, float* out_f32,
                                        void* out_raw_bf16, void* out_act_bf16, int32_t B, int32_t L, int32_t C, int32_t k,
                                        int32_t max_mb, int32_t sets, int32_t device) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!xa_bf16 || !w || !b || !dilations || n_pairs < 1 || n_pairs > VSG_MAX_RESBLOCK_DILATIONS) return fail(VSG_EINVAL, "bad argument");
   VSG_CUDA_TRY(cudaSetDevice(device));
   cudaDeviceProp prop;
@@ -2056,7 +2220,7 @@ extern "C" int vsg_debug_resblock_bf16(const void* xa_bf16, const float* w, cons
 // Per-kernel parity hook of the bf16 attention kernel (tests only; allocates and synchronises).  See include/visinger_b200.h.
 extern "C" int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev, void* o_bf16,
                                         int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w, int32_t device) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!qkv_bf16 || !mask || !ek || !ev || !o_bf16) return fail(VSG_EINVAL, "null pointer");
   if (B < 1 || T < 1 || n_heads < 1 || w < 0) return fail(VSG_EINVAL, "bad argument");
   VSG_CUDA_TRY(cudaSetDevice(device));
@@ -2082,7 +2246,7 @@ extern "C" int vsg_debug_attention_bf16(const void* qkv_bf16, const float* mask,
 extern "C" int vsg_debug_attention_split_bf16(const void* qkv_bf16, const float* mask, const float* ek, const float* ev,
                                               void* o_bf16, int32_t B, int32_t T, int32_t n_heads, int32_t dk, int32_t w,
                                               int32_t key_chunk, int32_t device) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!qkv_bf16 || !mask || !ek || !ev || !o_bf16) return fail(VSG_EINVAL, "null pointer");
   if (B < 1 || T < 1 || n_heads < 1 || w < 0 || dk < 1) return fail(VSG_EINVAL, "bad argument");
   if (key_chunk == 0) key_chunk = 128 * tc::kAtMaxTiles;
@@ -2114,7 +2278,7 @@ extern "C" int vsg_debug_attention_split_bf16(const void* qkv_bf16, const float*
 // Per-kernel parity hook of the bf16 encoder's fused LayerNorm -> condition -> mask step (tests only; synchronises).
 extern "C" int vsg_debug_layernorm_bf16(void* x_bf16, const float* gamma, const float* beta, const float* g, int32_t g_t,
                                         const float* mask, float eps, int32_t B, int32_t T, int32_t C, int32_t device) {
-  g_launches = 0;
+  reset_launch_counts();
   if (!x_bf16 || !gamma || !beta || !mask) return fail(VSG_EINVAL, "null pointer");
   if (B < 1 || T < 1) return fail(VSG_EINVAL, "bad argument");
   if (C < 2 || C > 256 || (C & 1)) return fail(VSG_EUNSUPPORTED, "LayerNorm over %d channels (supported: even, <= 256)", C);

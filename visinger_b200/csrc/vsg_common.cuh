@@ -19,6 +19,14 @@ namespace vsg {
 
 extern thread_local char g_err[1024];
 extern thread_local int g_launches;
+// launches of conv_tc_kernel per epilogue image (EPI_SIG_*, conv_tc.cuh) since the last reset: the tests read them to see
+// which images a call ran
+constexpr int kImageSlots = 16;
+extern thread_local int g_image_launches[kImageSlots];
+inline void reset_launch_counts() {
+  g_launches = 0;
+  memset(g_image_launches, 0, sizeof(g_image_launches));
+}
 
 inline int fail(int code, const char* fmt, ...) {
   va_list ap;
