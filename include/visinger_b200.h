@@ -498,6 +498,32 @@ int vsg_debug_pair_bf16(const void* xa_bf16, const float* w1, const float* b1, c
                         void* out_act_bf16, int32_t B, int32_t L, int32_t C, int32_t k, int32_t d1, int32_t device);
 
 /*
+ * The fused ResBlock1 pair kernel in every form the decoder launches it (tests only; allocates and synchronises):
+ *   v = (conv1d(leaky_relu(conv1d(xa, w1, dilation d1) + b1, 0.1), w2) + b2 + residual + add1) * scale
+ * residual = add0 (add0_is_act = 0) or the residual r recovered from add0 = leaky_relu(r, 0.1) (add0_is_act = 1: the
+ * decoder's single activated stream).  xa, add0, add1, out_raw (bf16(v)), out_act (leaky_relu(v)): device bf16 [B, L, C]
+ * channels-last; out_f32: device fp32 [B, L, C]; w1, w2: HOST fp32 [C][C][k]; b1, b2: HOST fp32 [C].  add0, add1 and the
+ * outputs may be NULL.  C in {16, 32}.  *image_out = the EPI_SIG_* epilogue image of conv2 (see vsg_debug_conv_tc): an
+ * fp32 copy runs the generic image, otherwise the image the decoder would launch.
+ */
+typedef struct VsgDebugPair {
+  const void* xa;
+  const float* w1;
+  const float* b1;
+  const float* w2;
+  const float* b2;
+  const void* add0;
+  const void* add1;
+  void* out_raw;
+  void* out_act;
+  float* out_f32;
+  int32_t add0_is_act;
+  float scale;
+  int32_t B, L, C, k, d1;
+} VsgDebugPair;
+int vsg_debug_pair_tc(const VsgDebugPair* d, int32_t* image_out, int32_t device);
+
+/*
  * Per-layer parity hook for the whole-ResBlock1 kernel (tests and tuning only; allocates and synchronises):
  *   for q in 0..n_pairs-1:  x = conv1d(leaky_relu(conv1d(leaky_relu(x), w[2q], dilation d_q) + b[2q]), w[2q+1]) + b[2q+1] + x
  *   out = (x [+ add1]) * scale
@@ -560,6 +586,11 @@ int vsg_debug_plan(int32_t Cin, int32_t Cout, int32_t k, int32_t dilation, int32
  * form, tiles per utterance, tensor-memory columns }.  VSG_EUNSUPPORTED: the shape runs on the per-convolution kernels. */
 int vsg_debug_rp_plan(int32_t C, int32_t k, int32_t n_pairs, const int32_t* dilations, int32_t L, int32_t variant,
                       int32_t* out);
+
+/* Host-only (no GPU): the tile plan of the fused ResBlock1 pair kernel (see vsg_debug_pair_tc) for C channels, k taps,
+ * conv1 dilation d1, L time steps per utterance, n_adds adds and n_outs bf16 outputs.  out[3] = { 128-row blocks per tile,
+ * valid output rows per tile, tiles per utterance }.  VSG_EUNSUPPORTED: the decoder runs such a pair as two convolutions. */
+int vsg_debug_pair_plan(int32_t C, int32_t k, int32_t d1, int32_t L, int32_t n_adds, int32_t n_outs, int32_t* out);
 
 /* Process-wide tuning defaults of the tensor-core path: activation-operand feeding mode, resident weights, and the
  * L2-resident batch tiling of the decoder (target MB of one intermediate tensor per sub-batch, 0 = no tiling, <0 =

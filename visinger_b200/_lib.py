@@ -100,6 +100,14 @@ class VsgDebugConv(ctypes.Structure):
                                                "epi_sigs")])
 
 
+class VsgDebugPair(ctypes.Structure):
+    """Descriptor of vsg_debug_pair_tc (include/visinger_b200.h)."""
+    _fields_ = ([(n, ctypes.c_void_p) for n in ("xa", "w1", "b1", "w2", "b2", "add0", "add1", "out_raw", "out_act",
+                                                "out_f32")] +
+                [("add0_is_act", ctypes.c_int32), ("scale", ctypes.c_float)] +
+                [(n, ctypes.c_int32) for n in ("B", "L", "C", "k", "d1")])
+
+
 # epilogue images of the convolution kernel (csrc/conv_tc.cuh, EPI_SIG_*), as vsg_debug_conv_tc and vsg_last_launch_images
 # number them
 EPI_SIG = dict(GENERIC=0, ACT=1, RES_ACT=2, LINEAR=3, X6=4, SUM0=5, SUM1=6, FINAL=7, POST=8, ACT_X3=9, RES_ACT_X3=10,
@@ -219,6 +227,8 @@ def lib() -> ctypes.CDLL:
                                             ctypes.POINTER(ctypes.c_int32), i32]
         L.vsg_set_tc_options.restype = ctypes.c_int
         L.vsg_set_tc_options.argtypes = [i32, i32, i32, i32]
+        L.vsg_debug_pair_tc.restype = ctypes.c_int
+        L.vsg_debug_pair_tc.argtypes = [ctypes.POINTER(VsgDebugPair), ctypes.POINTER(ctypes.c_int32), i32]
         L.vsg_debug_pair_bf16.restype = ctypes.c_int
         L.vsg_debug_pair_bf16.argtypes = [vp, vp, vp, vp, vp, vp, vp, ctypes.c_float, vp, vp, vp, i32, i32, i32, i32, i32, i32]
         L.vsg_enc_pack_create.restype = ctypes.c_int
@@ -692,6 +702,25 @@ def debug_pair_bf16(xa_bld: torch.Tensor, w1, b1, w2, b2, d1: int, add0=None, ad
                                    dev.index or 0)
     check(rc, "vsg_debug_pair_bf16")
     return out, raw, act
+
+
+def debug_pair_tc(xa, w1, b1, w2, b2, d1: int, *, add0=None, add0_is_act=0, add1=None, scale=1.0, out_raw=None,
+                  out_act=None, out_f32=None) -> int:
+    """The fused ResBlock1 pair through vsg_debug_pair_tc (include/visinger_b200.h).  xa, adds and outputs are
+    caller-allocated CUDA tensors [B, L, C] (outputs written in place); w1 / w2 [C, C, k] and b1 / b2 [C] may live anywhere.
+    Returns the EPI_SIG_* image of conv2's epilogue."""
+    require_cuda(xa, "xa")
+    for t in (xa, add0, add1, out_raw, out_act, out_f32):
+        assert t is None or (t.is_cuda and t.is_contiguous())
+    B, L, C = xa.shape
+    k = w1.shape[2]
+    h = [t.detach().to("cpu", torch.float32).contiguous() for t in (w1, b1, w2, b2)]
+    d = VsgDebugPair(xa.data_ptr(), *[t.data_ptr() for t in h], _ptr(add0), _ptr(add1), _ptr(out_raw), _ptr(out_act),
+                     _ptr(out_f32), add0_is_act, scale, B, L, C, k, d1)
+    img = ctypes.c_int32(-1)
+    torch.cuda.synchronize(xa.device)
+    check(lib().vsg_debug_pair_tc(ctypes.byref(d), ctypes.byref(img), xa.device.index or 0), "vsg_debug_pair_tc")
+    return int(img.value)
 
 
 def debug_resblock_bf16(xa_bld: torch.Tensor, ws, bs, dilations, add1=None, scale: float = 1.0, max_mb: int = 0, sets: int = 0,

@@ -489,6 +489,14 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
 // 128-row blocks per tile of the fused pair: tiles of the same byte size at both channel counts (per-tile costs are what
 // the low-channel stages are bound by)
 static inline int pair_mb(int C) { return C == 16 ? 4 : 2; }
+// TMA store boxes per tile (one box holds <= 256 rows) and valid output rows per tile.  With two boxes the box height must
+// be a multiple of 8 rows so that both start on a swizzle-atom boundary of the staging tile (a few more halo rows are
+// recomputed).
+static inline int pair_eboxes(int C) { return (128 * pair_mb(C) + 255) / 256; }
+static inline int pair_valid_rows(int C, int k) {
+  const int rows = 128 * pair_mb(C) - (k - 1), n = pair_eboxes(C);
+  return n == 1 ? rows : (rows / (8 * n)) * (8 * n);
+}
 
 bool pair_supported(const ConvWTC& w1, const ConvWTC& w2, int d1, int L, int n_adds, int n_outs) {
   const int C = w1.Cin, k = w1.ktaps;
@@ -506,16 +514,13 @@ bool pair_supported(const ConvWTC& w1, const ConvWTC& w2, int d1, int L, int n_a
 
 // x_new = conv2(leaky_relu(conv1(xa) + b1)) + b2 [+ add0 + add1] [* scale]; xa = leaky_relu(x) [B, L, C] bf16.
 int launch_pair_tc(const VsgPack* P, const ConvWTC& w1, const ConvWTC& w2, const __nv_bfloat16* xa, int B, int L, int d1,
-                   const EpiTC& e, const TCOptions& opt, int* error_flag, cudaStream_t st) {
+                   const EpiTC& e, const TCOptions& opt, int* error_flag, cudaStream_t st, int* image_out = nullptr) {
   const int C = w1.Cin, k = w1.ktaps, mb = pair_mb(C);
   const int h2 = (k - 1) / 2, pad1 = (k - 1) * d1 / 2, halo1 = (k - 1) * d1;
   // the input is read with a halo that other CTAs' output tiles cover: an aliased output is a data race
   if ((const void*)xa == (const void*)e.out_act || (const void*)xa == (const void*)e.out_raw)
     return fail(VSG_EINVAL, "fused pair must not run in place (output aliases the activated input)");
-  // valid output rows per tile.  One TMA box holds <= 256 rows; with two boxes the box height must be a multiple of 8
-  // rows so that both start on a swizzle-atom boundary of the staging tile (a few more halo rows are recomputed).
-  const int n_eboxes = (128 * mb + 255) / 256;
-  const int V = n_eboxes == 1 ? 128 * mb - (k - 1) : ((128 * mb - (k - 1)) / (8 * n_eboxes)) * (8 * n_eboxes);
+  const int n_eboxes = pair_eboxes(C), V = pair_valid_rows(C, k);
   const int n_adds = (e.add0 ? 1 : 0) + (e.add1 ? 1 : 0), n_outs = (e.out_raw ? 1 : 0) + (e.out_act ? 1 : 0);
   ConvTC p1, p2;
   memset(&p1, 0, sizeof(p1));
@@ -626,6 +631,7 @@ int launch_pair_tc(const VsgPack* P, const ConvWTC& w1, const ConvWTC& w2, const
   cudaError_t le = cudaLaunchKernelEx(&cfg, pair_kernels[C == 16 ? 0 : 1][pv], tmA, w1.tmap, w2.tmap, tmAdd0, tmAdd1, tmRaw, tmAct, p1, p2);
   if (le != cudaSuccess) return fail(VSG_ECUDA, "launch of pair_tc_kernel failed: %s", cudaGetErrorString(le));
   VSG_LAUNCH_CHECK("pair_tc_kernel");
+  if (image_out) *image_out = pv == 1 ? EPI_SIG_RES_ACT : pv == 2 ? EPI_SIG_LINEAR : EPI_SIG_GENERIC;
   return VSG_OK;
 }
 
@@ -2119,6 +2125,36 @@ extern "C" int vsg_debug_pair_bf16(const void* xa_bf16, const float* w1, const f
   return rc;
 }
 
+// The fused pair as the decoder launches it, add0 activated or raw (tests only; allocates and synchronises).
+// See include/visinger_b200.h.
+extern "C" int vsg_debug_pair_tc(const VsgDebugPair* d, int32_t* image_out, int32_t device) {
+  reset_launch_counts();
+  if (!d || !d->xa || !d->w1 || !d->b1 || !d->w2 || !d->b2) return fail(VSG_EINVAL, "vsg_debug_pair_tc: null descriptor, input, weight or bias");
+  if (d->B <= 0 || d->L <= 0 || d->C <= 0 || d->k <= 0 || d->d1 <= 0) return fail(VSG_EINVAL, "vsg_debug_pair_tc: bad shape");
+  if (d->add0_is_act && !d->add0) return fail(VSG_EINVAL, "vsg_debug_pair_tc: add0_is_act without add0");
+  const int C = d->C, k = d->k;
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  std::vector<float> W1(d->w1, d->w1 + (size_t)C * C * k), W2(d->w2, d->w2 + (size_t)C * C * k), B1(d->b1, d->b1 + C),
+      B2(d->b2, d->b2 + C);
+  ConvWTC wt1, wt2;
+  VSG_TRY(pack_conv_tc(&sc.P, W1, B1, C, C, k, &wt1));
+  VSG_TRY(pack_conv_tc(&sc.P, W2, B2, C, C, k, &wt2));
+  if (!pair_supported(wt1, wt2, d->d1, d->L, (d->add0 ? 1 : 0) + (d->add1 ? 1 : 0), (d->out_raw ? 1 : 0) + (d->out_act ? 1 : 0)))
+    return fail(VSG_EUNSUPPORTED, "vsg_debug_pair_tc: shape not supported by the fused pair");
+  EpiTC e;
+  e.bias = wt2.bias;
+  e.add0 = (const __nv_bfloat16*)d->add0; e.add1 = (const __nv_bfloat16*)d->add1;
+  e.add0_is_act = d->add0_is_act;
+  e.scale = d->scale; e.out_f32 = d->out_f32;
+  e.out_raw = (__nv_bfloat16*)d->out_raw; e.out_act = (__nv_bfloat16*)d->out_act;
+  TCOptions opt;
+  int img = -1;
+  const int rc = launch_pair_tc(&sc.P, wt1, wt2, (const __nv_bfloat16*)d->xa, d->B, d->L, d->d1, e, opt, sc.err, 0, &img);
+  if (image_out) *image_out = img;
+  return sc.finish(rc);
+}
+
 // Per-layer parity hook for the whole-ResBlock1 kernel (tests and tuning only; allocates and synchronises).
 //   xa: device bf16 [B, L, C] = leaky_relu(x); w: HOST fp32 [2 * n_pairs][C][C][k] in the order c1_0, c2_0, c1_1, ...;
 //   b: HOST fp32 [2 * n_pairs][C]; out = (resblock1(x) [+ add1]) * scale.
@@ -2309,6 +2345,20 @@ extern "C" int vsg_debug_plan(int32_t Cin, int32_t Cout, int32_t k, int32_t dila
   TCOptions opt = g_default_opts;
   opt.plan_only = 1;
   return launch_conv_tc(&tmp, wt, &dummy_in, B, L, -((k - 1) * dilation / 2), dilation, L, 1, 0, L, e, opt, nullptr, 0);
+}
+
+// Host-only: the tile plan of the fused ResBlock1 pair (pair_tc.cuh) for one shape; no GPU needed.
+//   out[3]: 128-row blocks per tile, valid output rows per tile, tiles per utterance
+// Returns VSG_EUNSUPPORTED when the pair kernel does not take the shape (the decoder then runs the two convolutions apart).
+extern "C" int vsg_debug_pair_plan(int32_t C, int32_t k, int32_t d1, int32_t L, int32_t n_adds, int32_t n_outs, int32_t* out) {
+  if (!out || C <= 0 || k <= 0 || d1 <= 0 || L <= 0 || n_adds < 0 || n_adds > 2 || n_outs < 0 || n_outs > 2)
+    return fail(VSG_EINVAL, "bad argument");
+  ConvWTC w;                                  // what pack_conv_tc would record for this shape
+  w.Cin = C; w.Cout = C; w.CinT = C; w.CoutT = C; w.ktaps = k; w.has_tmap = true; w.x3 = false; w.planes = 1;
+  if (!pair_supported(w, w, d1, L, n_adds, n_outs)) return fail(VSG_EUNSUPPORTED, "shape not supported by the fused pair");
+  const int V = pair_valid_rows(C, k);
+  out[0] = pair_mb(C); out[1] = V; out[2] = (L + V - 1) / V;
+  return VSG_OK;
 }
 
 // Host-only: the tile plan of the row-packed whole-ResBlock1 kernel (rp_tc.cuh) for one resblock shape; no GPU needed.
