@@ -277,6 +277,34 @@ int vsg_infer_zp(const VsgPack* pack, const float* z_p, const float* mask, const
                  int32_t B, int32_t T, int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * Streaming synthesis: flow and decoder over a window of latent frames.  Only the prior network needs the whole
+ * utterance; everything downstream of z_p is convolutional with a finite receptive field, so a caller can sample z_p once
+ * and then produce the waveform window by window -- to start playback early, or to interleave long requests -- with a
+ * workspace that does not grow with T.  Every window is BIT-IDENTICAL to the same frames of the one-pass call, in all
+ * three precisions: the flow runs over the window plus Cf + Cd frames of context each side and the decoder over the
+ * window plus Cd, the length-dependent kernel choices are those of the whole (B, T) batch, and only the central samples
+ * are stored (DESIGN.md section 4.8).  Concatenated windows equal the one-pass waveform; windows may come in any order.
+ */
+/* Context frames each side that a window needs for exact results: the flow's (reverse) and the decoder's receptive
+ * fields in latent frames, derived from the pack's config (0 for an absent part).  Host only. */
+int vsg_window_context(const VsgPack* pack, int32_t* flow_frames, int32_t* dec_frames);
+/* Workspace of the window calls for windows of up to max_frames output frames of a (B, T) batch; it does not grow with T
+ * (the sub-batch split the whole batch uses may make it smaller).  0 on invalid arguments. */
+size_t vsg_window_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t max_frames, int32_t precision);
+/* Frames [t0, t1) of vsg_infer_zp(z_p [B, C, T], mask [B, 1, T], g) bit for bit.  wav: row b at wav + b * wav_ld receives
+ * the samples [t0 * hop, t1 * hop) of utterance b; z_q_out: NULL or fp32 [B, C, t1 - t0].  z_p and mask are read in place.
+ * VSG_EINVAL: t0 < 0, t1 > T, t0 >= t1, a null pointer, wav_ld < (t1 - t0) * hop; VSG_ENOMEM: a workspace smaller than
+ * vsg_window_workspace_bytes(B, T, t1 - t0); both before any launch.  No allocation, no synchronisation: capturable. */
+int vsg_infer_zp_window(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav,
+                        int64_t wav_ld, float* z_q_out, int32_t B, int32_t T, int32_t t0, int32_t t1, int32_t precision,
+                        void* workspace, size_t workspace_bytes, void* stream);
+/* The decoder alone: samples [t0 * hop, t1 * hop) of vsg_generator_forward(z [B, C, T], g) bit for bit, with the rules of
+ * vsg_infer_zp_window. */
+int vsg_generator_forward_window(const VsgPack* pack, const float* z, const float* g, float* wav, int64_t wav_ld,
+                                 int32_t B, int32_t T, int32_t t0, int32_t t1, int32_t precision,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * The whole model: VISinger.forward(infer=True) from note tokens to waveform in one call
  * (VISinger(ph_dict_size, pitch_size, dur_size, hparams), the fields below; window_size is RelativeEncoder's 4,
  * spk_embed_dim the 256 inputs of spk_embed_proj).  The speaker condition has hot.flow_gin (= hot.dec_gin) channels.

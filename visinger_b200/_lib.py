@@ -287,6 +287,14 @@ def lib() -> ctypes.CDLL:
         L.vsg_normal_noise.argtypes = [vp, vp, i32, i32, i32, vp]
         L.vsg_debug_position_table.restype = ctypes.c_int
         L.vsg_debug_position_table.argtypes = [vp, i32, i32, vp, vp]
+        L.vsg_window_context.restype = ctypes.c_int
+        L.vsg_window_context.argtypes = [vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]
+        L.vsg_window_workspace_bytes.restype = sz
+        L.vsg_window_workspace_bytes.argtypes = [vp, i32, i32, i32, i32]
+        L.vsg_infer_zp_window.restype = ctypes.c_int
+        L.vsg_infer_zp_window.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int64, vp, i32, i32, i32, i32, i32, vp, sz, vp]
+        L.vsg_generator_forward_window.restype = ctypes.c_int
+        L.vsg_generator_forward_window.argtypes = [vp, vp, vp, vp, ctypes.c_int64, i32, i32, i32, i32, i32, vp, sz, vp]
         if L.vsg_abi_version() != 1:
             raise RuntimeError("visinger_b200: ABI version mismatch between _lib.py and the shared library")
         _lib = L
@@ -362,6 +370,15 @@ class Pack:
 
     def workspace_bytes(self, B: int, T: int, precision: int) -> int:
         return int(lib().vsg_workspace_bytes(self._h, B, T, precision))
+
+    def window_context(self):
+        """(flow, decoder) context frames each side of a streaming window (vsg_window_context)."""
+        cf, cd = ctypes.c_int32(), ctypes.c_int32()
+        check(lib().vsg_window_context(self._h, ctypes.byref(cf), ctypes.byref(cd)), "vsg_window_context")
+        return int(cf.value), int(cd.value)
+
+    def window_workspace_bytes(self, B: int, T: int, max_frames: int, precision: int) -> int:
+        return int(lib().vsg_window_workspace_bytes(self._h, B, T, max_frames, precision))
 
     def __del__(self):
         try:

@@ -36,7 +36,7 @@ namespace vsg {
 // the mask rides on the final layout change), false if the caller still has to
 int run_flow(const VsgPack* pack, const float* x, const float* mask, const float* g, float* y, int B, int T, int reverse,
              int precision, Workspace& ws, cudaStream_t st, bool* masked, const float* ps_logs, const float* ps_noise,
-             bool* sampled) {
+             bool* sampled, int x_ld) {
   // ps_logs / ps_noise (with `sampled`): x is mu_p; *sampled = true if the flow's first kernel drew the prior sample itself
   if (sampled) *sampled = false;
   const bool want = masked && *masked;
@@ -48,9 +48,9 @@ int run_flow(const VsgPack* pack, const float* x, const float* mask, const float
     if (masked) *masked = want;
     if (sampled && ps_logs && ps_noise) *sampled = true;
     return flow_forward_tc(pack, x, mask, g, y, B, T, reverse, ws, st, tc1 ? 1 : 3, want ? mask : nullptr,
-                           sampled ? ps_logs : nullptr, sampled ? ps_noise : nullptr);
+                           sampled ? ps_logs : nullptr, sampled ? ps_noise : nullptr, x_ld);
   }
-  return flow_forward_f32(pack, x, mask, g, y, B, T, reverse, ws, st);
+  return flow_forward_f32(pack, x, mask, g, y, B, T, reverse, ws, st, x_ld);
 }
 
 }  // namespace vsg
@@ -268,3 +268,185 @@ int infer_zp_run(const VsgPack* pack, const float* z_p, const float* mask, const
 }
 
 }  // namespace vsg
+
+// ---- streaming windows ------------------------------------------------------------------------------------------------
+// A window's frames [t0, t1) are computed exactly as the one-pass call computes them: the flow runs over
+// [fa, fb) = [t0 - Cf - Cd, t1 + Cf + Cd) and the decoder over [da, db) = [t0 - Cd, t1 + Cd) of the flow's output (both
+// clipped to [0, T), where the window's zero padding is the utterance's own), Cf / Cd being the receptive fields of the
+// flow (reverse) and of the decoder in frames.  Each output is a function of the inputs in its receptive field only, every
+// kernel sums each output in an order that does not depend on where the output sits in a tile (DESIGN.md 4.8), and the
+// kernel choices are those of the whole batch (dec_window_needs_tc), so the central frames come out bit for bit.
+namespace {
+
+long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+int flow_context(const VsgPack* p) {
+  if (!p->has_flow) return 0;
+  const VsgConfig& c = p->cfg;
+  int r = 0, dil = 1;
+  for (int i = 0; i < c.flow_n_layers; ++i) {   // WaveNet in_layers: padding (K * dil - dil) / 2; pre / post are 1x1
+    const int span = (c.flow_kernel_size - 1) * dil, pad = (c.flow_kernel_size * dil - dil) / 2;
+    r += std::max(pad, span - pad);
+    dil *= c.flow_dilation_rate;
+  }
+  return r * c.flow_n_flows;   // each coupling layer widens the field by its WaveNet's reach
+}
+
+// Walk the receptive field of output frame 0 (samples [0, hop)) back through the decoder's layers, noting at every rate
+// the frames its samples lie in: a window's tensor at that rate covers whole frames [da, db) of it.
+int dec_context(const VsgPack* p) {
+  if (!p->has_dec) return 0;
+  const VsgConfig& c = p->cfg;
+  long long R = p->hop, lo = 0, hi = p->hop - 1, left = 0, right = 0;
+  auto note = [&]() { left = std::max(left, -floor_div(lo, R)); right = std::max(right, floor_div(hi, R)); };
+  auto conv = [&](int k, int d) { const int pad = (k * d - d) / 2; lo -= pad; hi += (k - 1) * d - pad; };
+  conv(p->conv_post_k, 1);   // conv_post, padding 3                     decoder.py:31,55-57
+  note();
+  for (int i = c.dec_n_ups - 1; i >= 0; --i) {
+    long long rlo = 0, rhi = 0;   // the NK resblocks of a stage run in parallel on its upsampled input: the widest
+    for (int j = 0; j < c.dec_n_kernels; ++j) {
+      const long long lo0 = lo, hi0 = hi;
+      const int k = c.dec_resblock_kernel_sizes[j];
+      for (int q = c.dec_n_dilations[j] - 1; q >= 0; --q) {
+        if (c.dec_resblock == 1) conv(k, 1);       // ResBlock1 conv2                      decoder.py:91-104
+        conv(k, c.dec_resblock_dilations[j][q]);   // conv1 (ResBlock2: its only conv)     decoder.py:124-133
+      }
+      rlo = std::min(rlo, lo - lo0); rhi = std::max(rhi, hi - hi0);
+      lo = lo0; hi = hi0;
+    }
+    lo += rlo; hi += rhi;
+    note();
+    // ups[i] = ConvTranspose1d(k, stride r, padding (k - r) / 2): y[n] = sum_m x[m] w[n + pad - m r]   decoder.py:24-26
+    const int r = c.dec_upsample_rates[i], k = c.dec_upsample_kernel_sizes[i], pad = (k - r) / 2;
+    lo = -floor_div(-(lo + pad - k + 1), r);
+    hi = floor_div(hi + pad, r);
+    R /= r;
+    note();
+  }
+  conv(7, 1);   // conv_pre, padding 3                                    decoder.py:19
+  note();
+  return (int)std::max(left, right);
+}
+
+struct WinRange { int fa, fb, da, db; };
+
+int window_needs(const VsgPack* p, int B, int T, int precision, int* need, int* align) {
+  *need = 1; *align = 1;
+  if (precision == VSG_PRECISION_FP32) return VSG_OK;   // the FFMA kernels choose nothing by length
+  return dec_window_needs_tc(p, B, T, precision == VSG_PRECISION_BF16X3, need, align);
+}
+
+int window_ranges(const VsgPack* p, int B, int T, int t0, int t1, int precision, bool flow, WinRange* r) {
+  int need, A;
+  VSG_TRY(window_needs(p, B, T, precision, &need, &A));
+  const int Cd = dec_context(p), Cf = flow ? flow_context(p) : 0;
+  int da = std::max(0, t0 - Cd) / A * A, db = std::min(T, (std::min(T, t1 + Cd) + A - 1) / A * A);
+  if (db - da < need) {   // a kernel of the whole batch's choice needs a longer stage: widen, never switch kernels
+    db = std::min(T, da + (need + A - 1) / A * A);
+    if (db - da < need) da = std::max(0, (db - need) / A * A);
+  }
+  r->da = da; r->db = db;
+  r->fa = std::max(0, da - Cf); r->fb = std::min(T, db + Cf);
+  return VSG_OK;
+}
+
+// flow + decoder scratch of windows of up to n frames (0 on invalid arguments); an upper bound of window_ranges' spans
+size_t window_ws(const VsgPack* p, int B, int T, int n, int precision) {
+  if (check_common(p, B, T, precision) != VSG_OK || !p->has_dec || n < 1 || T < 1) return 0;
+  int need, A;
+  if (window_needs(p, B, T, precision, &need, &A) != VSG_OK) return 0;
+  n = std::min(n, T);
+  const int Cd = dec_context(p), Cf = flow_context(p);
+  const int Wd = std::min(T, std::max(n + 2 * Cd + 2 * (A - 1), need + A - 1)), Wf = std::min(T, Wd + 2 * Cf);
+  const size_t dec = precision == VSG_PRECISION_FP32 ? dec_ws_bytes_f32(p, B, Wd)
+                                                     : dec_ws_bytes_tc(p, B, Wd, precision == VSG_PRECISION_BF16X3, T);
+  const size_t z = p->has_flow ? align256((size_t)B * p->cfg.flow_channels * Wf * sizeof(float)) : 0;
+  return z + std::max(flow_ws(p, B, Wf, precision), dec) + 1024;
+}
+
+int check_window(const VsgPack* pack, const void* in, float* wav, int64_t wav_ld, int B, int T, int t0, int t1,
+                 int precision, void* workspace, size_t workspace_bytes) {
+  VSG_TRY(check_common(pack, B, T, precision));
+  if (!pack->has_dec) return fail(VSG_EINVAL, "pack has no decoder");
+  if (t0 < 0 || t1 > T || t0 >= t1) return fail(VSG_EINVAL, "window [%d, %d) is not a non-empty part of [0, %d)", t0, t1, T);
+  if (B == 0) return VSG_OK;
+  if (!in || !wav) return fail(VSG_EINVAL, "null pointer");
+  if (wav_ld < (int64_t)(t1 - t0) * pack->hop)
+    return fail(VSG_EINVAL, "wav_ld %lld is shorter than the window's %lld samples", (long long)wav_ld,
+                (long long)(t1 - t0) * pack->hop);
+  if ((long long)T * pack->hop > 0x7fffffffLL / 4) return fail(VSG_EUNSUPPORTED, "sequence too long (%d frames)", T);
+  if (!workspace) return fail(VSG_ENOMEM, "workspace is NULL");
+  int need, A;
+  VSG_TRY(window_needs(pack, B, T, precision, &need, &A));
+  const size_t want = window_ws(pack, B, T, t1 - t0, precision);
+  if (workspace_bytes < want) return fail(VSG_ENOMEM, "window workspace too small: need %zu bytes", want);
+  return VSG_OK;
+}
+
+}  // namespace
+
+extern "C" int vsg_window_context(const VsgPack* pack, int32_t* flow_frames, int32_t* dec_frames) {
+  if (!pack || !flow_frames || !dec_frames) return fail(VSG_EINVAL, "null pointer");
+  *flow_frames = flow_context(pack);
+  *dec_frames = dec_context(pack);
+  return VSG_OK;
+}
+
+extern "C" size_t vsg_window_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t max_frames,
+                                             int32_t precision) {
+  return window_ws(pack, B, T, max_frames, precision);
+}
+
+extern "C" int vsg_infer_zp_window(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav,
+                                   int64_t wav_ld, float* z_q_out, int32_t B, int32_t T, int32_t t0, int32_t t1,
+                                   int32_t precision, void* workspace, size_t workspace_bytes, void* stream) {
+  reset_launch_counts();
+  if (pack && (!pack->has_flow || !pack->has_dec))
+    return fail(VSG_EINVAL, "vsg_infer_zp_window needs a pack with both flow and decoder");
+  if (pack && pack->cfg.flow_channels != pack->cfg.dec_initial_channel)
+    return fail(VSG_EINVAL, "flow channels (%d) != decoder initial_channel (%d)", pack->cfg.flow_channels,
+                pack->cfg.dec_initial_channel);
+  VSG_TRY(check_window(pack, z_p, wav, wav_ld, B, T, t0, t1, precision, workspace, workspace_bytes));
+  if (B == 0) return VSG_OK;
+  if (!mask) return fail(VSG_EINVAL, "null pointer");
+  WinRange r;
+  VSG_TRY(window_ranges(pack, B, T, t0, t1, precision, true, &r));
+  DeviceGuard dg(pack->device);
+  if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int C = pack->cfg.flow_channels, Tf = r.fb - r.fa;
+  Workspace ws(workspace, workspace_bytes);
+  float* z = ws.take<float>((size_t)B * C * Tf);
+  if (ws.overflow) return fail(VSG_ENOMEM, "workspace too small");
+  const size_t mark = ws.off;
+  // z_q = flow(z_p, mask, g, reverse=True) * mask over [fa, fb), read in place from the caller's [B, C, T] z_p and mask
+  bool masked = true;
+  VSG_TRY(run_flow(pack, z_p + r.fa, mask + r.fa, g, z, B, Tf, 1, precision, ws, st, &masked, nullptr, nullptr, nullptr, T));
+  if (!masked) VSG_TRY(mask_mul(z, mask + r.fa, z, B, C, Tf, st, T));
+  if (z_q_out)
+    VSG_CUDA_TRY(cudaMemcpy2DAsync(z_q_out, (size_t)(t1 - t0) * sizeof(float), z + (t0 - r.fa), (size_t)Tf * sizeof(float),
+                                   (size_t)(t1 - t0) * sizeof(float), (size_t)B * C, cudaMemcpyDeviceToDevice, st));
+  ws.off = mark;
+  // wav = decoder(z_q) over [da, db); its samples of [t0, t1) straight into the caller's rows
+  const DecWin w{T, Tf, (long long)wav_ld, (t0 - r.da) * pack->hop, (t1 - r.da) * pack->hop};
+  const float* zd = z + (r.da - r.fa);
+  if (precision == VSG_PRECISION_FP32) return generator_forward_f32(pack, zd, g, wav, B, r.db - r.da, ws, st, &w);
+  return generator_forward_tc(pack, zd, g, wav, B, r.db - r.da, ws, st, precision == VSG_PRECISION_BF16X3, &w);
+}
+
+extern "C" int vsg_generator_forward_window(const VsgPack* pack, const float* z, const float* g, float* wav, int64_t wav_ld,
+                                            int32_t B, int32_t T, int32_t t0, int32_t t1, int32_t precision,
+                                            void* workspace, size_t workspace_bytes, void* stream) {
+  reset_launch_counts();
+  VSG_TRY(check_window(pack, z, wav, wav_ld, B, T, t0, t1, precision, workspace, workspace_bytes));
+  if (B == 0) return VSG_OK;
+  WinRange r;
+  VSG_TRY(window_ranges(pack, B, T, t0, t1, precision, false, &r));
+  DeviceGuard dg(pack->device);
+  if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  Workspace ws(workspace, workspace_bytes);
+  const DecWin w{T, T, (long long)wav_ld, (t0 - r.da) * pack->hop, (t1 - r.da) * pack->hop};
+  if (precision == VSG_PRECISION_FP32) return generator_forward_f32(pack, z + r.da, g, wav, B, r.db - r.da, ws, st, &w);
+  return generator_forward_tc(pack, z + r.da, g, wav, B, r.db - r.da, ws, st, precision == VSG_PRECISION_BF16X3, &w);
+}

@@ -90,11 +90,14 @@ struct ConvTC {
   float scale;                  // applied after the adds
   float slope;                  // leaky_relu slope for out_act
   int mode;                     // EPI_TC_LINEAR / EPI_TC_GATE / EPI_TC_COUPLE
-  const float* mask;            // [B][Lout] row mask or null (LINEAR: v *= mask; COUPLE: see below)
+  const float* mask;            // [B][mask_ld] row mask or null (LINEAR: v *= mask; COUPLE: see below)
+  int mask_ld;                  // floats between the mask rows of two utterances (Lout, or the whole batch's T for a window)
   int couple_sign;              // COUPLE: -1 reverse  x1 = (x1 - m) * mask,  +1 forward  x1 = m + x1 * mask
   uint32_t e_out_swz_mask;      // swizzle of the output staging rows (GATE halves the row width)
   float* out_f32;               // optional fp32 copy of the raw value [B, Lout, Cout] (debug / parity hook); EPI_TC_TANH: the output
   int tanh_cols;                // EPI_TC_TANH: out_f32[(b * Lq + q) * tanh_cols + i] = tanh(acc[i]), i < tanh_cols (<= 4)
+  long long tanh_ld;            // EPI_TC_TANH, 0: as above; else only samples n = q * tanh_cols + i in [tanh_s0, tanh_s1) are
+  int tanh_s0, tanh_s1;         //   stored, at out_f32[b * tanh_ld + n - tanh_s0] (a streaming window's central samples)
   int mag_ch;                   // EPI_TC_MAG: output channels >= mag_ch are written as 0 (the consumer's zero pad channels)
   int* error_flag;              // set to 1 if a barrier wait times out
 };
@@ -532,7 +535,7 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
           if (lane == 0) mbar_arrive(acc_empty0 + 8u * as);
         }
         float mk = 1.0f;
-        if (maskp) mk = (q < p.Lq) ? __ldg(maskp + (long long)b * p.Lout + q) : 0.f;
+        if (maskp) mk = (q < p.Lq) ? __ldg(maskp + (long long)b * p.mask_ld + q) : 0.f;
         if (bias_hoisted) {
 #pragma unroll
           for (int i = 0; i < CW; ++i) v[i] += bias_r[i];
@@ -640,7 +643,12 @@ __device__ __forceinline__ void conv_tc_epilogue(const CUtensorMap& tmAdd0, cons
             v[c] = och + c < p.mag_ch ? sqrtf(fmaf(v[2 * c], v[2 * c], fmaf(v[2 * c + 1], v[2 * c + 1], 1e-6f))) * mk : 0.f;
         }
         if (MODE == EPI_TC_TANH) {   // one 16-byte store per row; the lanes of a warp cover 512 contiguous bytes
-          if (srow < tile_stride && q < p.Lq) {
+          if (srow < tile_stride && q < p.Lq && p.tanh_ld) {   // window: the central samples only, straight to the caller
+            for (int i = 0; i < p.tanh_cols; ++i) {
+              const int n = q * p.tanh_cols + i;
+              if (n >= p.tanh_s0 && n < p.tanh_s1) p.out_f32[(long long)b * p.tanh_ld + (n - p.tanh_s0)] = tanhf(v[i]);
+            }
+          } else if (srow < tile_stride && q < p.Lq) {
             float* dst = p.out_f32 + ((long long)b * p.Lq + q) * p.tanh_cols;
             if (p.tanh_cols == 4) {
               *reinterpret_cast<float4*>(dst) = make_float4(tanhf(v[0]), tanhf(v[1]), tanhf(v[2]), tanhf(v[3]));
@@ -980,9 +988,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 // planes = 3: [hi | mid | lo], the fp32 value exactly (the flow at the fp32 tolerance).
 // ps_logs != null: x is mu_p and the value laid out is the prior sample z_p = (mu_p + noise * exp(logs_p)) * mask
 // (models/visinger.py:107; the arithmetic of prior_sample_kernel), so the hot path needs no fp32 z_p tensor at all.
+// x_ld > 0: x (and ps_*) are frames [0, T) of rows of x_ld frames -- a streaming window read in place from the whole batch.
 __global__ void transpose_to_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ y, int C, int T,
                                          int planes, const float* __restrict__ ps_logs = nullptr,
-                                         const float* __restrict__ ps_noise = nullptr, const float* __restrict__ ps_mask = nullptr) {
+                                         const float* __restrict__ ps_noise = nullptr, const float* __restrict__ ps_mask = nullptr,
+                                         int x_ld = 0) {
+  const int ld = x_ld > 0 ? x_ld : T;
   __shared__ float tile[32][33];
   const int b = blockIdx.z, c0 = blockIdx.y * 32, t0 = blockIdx.x * 32;
   const int tx = threadIdx.x, ty = threadIdx.y;   // 32 x 8
@@ -990,9 +1001,9 @@ __global__ void transpose_to_bf16_kernel(const float* __restrict__ x, __nv_bfloa
     const int c = c0 + i, t = t0 + tx;
     float v = 0.f;
     if (c < C && t < T) {
-      const long long idx = ((long long)b * C + c) * T + t;
+      const long long idx = ((long long)b * C + c) * ld + t;
       v = x[idx];
-      if (ps_logs) v = (v + ps_noise[idx] * expf(ps_logs[idx])) * ps_mask[(long long)b * T + t];
+      if (ps_logs) v = (v + ps_noise[idx] * expf(ps_logs[idx])) * ps_mask[(long long)b * ld + t];
     }
     tile[i][tx] = v;
   }
@@ -1040,9 +1051,10 @@ __global__ void posterior_sample_from_stats_kernel(const float* __restrict__ sta
 }
 
 // [B, T, planes * C] bf16 -> [B, C, T] fp32 (the planes of a value are summed); flip != 0 reverses the channel order
-// (an odd number of Flips); mask != null: the output is multiplied by mask[b][t] (`z * mask`, models/visinger.py:109-111).
+// (an odd number of Flips); mask != null: the output is multiplied by mask[b][t] (`z * mask`, models/visinger.py:109-111),
+// mask rows mask_ld apart (0: T).
 __global__ void transpose_from_bf16_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ y, int C, int T,
-                                           int flip, int planes, const float* __restrict__ mask = nullptr) {
+                                           int flip, int planes, const float* __restrict__ mask = nullptr, int mask_ld = 0) {
   __shared__ float tile[32][33];
   const int b = blockIdx.z, c0 = blockIdx.y * 32, t0 = blockIdx.x * 32;
   const int tx = threadIdx.x, ty = threadIdx.y;   // 32 x 8
@@ -1057,23 +1069,26 @@ __global__ void transpose_from_bf16_kernel(const __nv_bfloat16* __restrict__ x, 
   for (int i = ty; i < 32; i += 8) {
     const int c = c0 + i, t = t0 + tx;
     if (c < C && t < T)
-      y[((long long)b * C + (flip ? C - 1 - c : c)) * T + t] = mask ? tile[tx][i] * mask[(long long)b * T + t] : tile[tx][i];
+      y[((long long)b * C + (flip ? C - 1 - c : c)) * T + t] =
+          mask ? tile[tx][i] * mask[(long long)b * (mask_ld > 0 ? mask_ld : T) + t] : tile[tx][i];
   }
 }
 
 // conv_post on the channels-last bf16 stream: input is already leaky_relu'd (out_act of the last stage).
 // wav[b, n] = tanh(sum_{j, c} w[c][j] * x[b, n + j - pad, c]).  One thread per sample.
-// split != 0: rows are [hi (C) | lo (C)] and x = hi + lo.
+// split != 0: rows are [hi (C) | lo (C)] and x = hi + lo.  wav_ld > 0: only samples [n0, n1) are computed, into rows of
+// wav wav_ld apart (a streaming window's central samples); else n0 = 0, n1 = L and the rows are L apart.
 __global__ void conv_post_bf16_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ w /*[C][k]*/,
-                                      float* __restrict__ wav, int C, int L, int k, int split) {
+                                      float* __restrict__ wav, int C, int L, int k, int split, int n0 = 0, int n1 = 0,
+                                      long long wav_ld = 0) {
   extern __shared__ float wsm[];   // [k][C]
   for (int i = threadIdx.x; i < C * k; i += blockDim.x) {
     const int c = i / k, j = i - c * k;
     wsm[j * C + c] = w[i];
   }
   __syncthreads();
-  const int n = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
-  if (n >= L) return;
+  const int n = n0 + blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
+  if (n >= (wav_ld ? n1 : L)) return;
   const int pad = (k - 1) / 2, W = split ? 2 * C : C;
   float s = 0.f;
   for (int j = 0; j < k; ++j) {
@@ -1093,7 +1108,7 @@ __global__ void conv_post_bf16_kernel(const __nv_bfloat16* __restrict__ x, const
       for (int i = 0; i < 8; ++i) s = fmaf(wsm[j * C + c8 * 8 + i], f[i], s);
     }
   }
-  wav[(long long)b * L + n] = tanhf(s);
+  wav[wav_ld ? (long long)b * wav_ld + (n - n0) : (long long)b * L + n] = tanhf(s);
 }
 
 // conv_post for the shapes the model actually has (C = 16 channels, k = 7), plain bf16: every thread produces S
@@ -1148,10 +1163,12 @@ __global__ void __launch_bounds__(128) conv_post_bf16_win_kernel(const __nv_bflo
 // samples of one utterance; the 128 * S + K - 1 input rows (C bf16 each) are fetched with fully coalesced 16-byte loads
 // (the window kernel above has every lane 8 rows = 256 B apart: 32 sectors per load instruction, and the L1 pipe, not
 // HBM, set its pace: 93 us for 173 MB) and every thread then slides its window over shared memory.  Rows are padded by
-// 16 bytes per S rows so that the lanes' 16-byte reads fall into distinct banks.
+// 16 bytes per S rows so that the lanes' 16-byte reads fall into distinct banks.  wav_ld > 0: only samples [s0, s1) are
+// stored, into rows of wav wav_ld apart (a streaming window's central samples).
 template <int C, int K, int S>
 __global__ void __launch_bounds__(128) conv_post_bf16_smem_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ w /*[C][K]*/,
-                                                                  float* __restrict__ wav, int L, int tiles_per_b, int total_tiles) {
+                                                                  float* __restrict__ wav, int L, int tiles_per_b, int total_tiles,
+                                                                  int s0 = 0, int s1 = 0, long long wav_ld = 0) {
   static_assert(C == 16 && S == 8, "layout below assumes 32-byte rows and 8 samples per thread");
   constexpr int TS = 128 * S;                    // samples per tile
   constexpr int ROWS = TS + K - 1;
@@ -1195,6 +1212,12 @@ __global__ void __launch_bounds__(128) conv_post_bf16_smem_kernel(const __nv_bfl
       }
     }
     const int n0 = n_tile0 + r0;
+    if (wav_ld) {
+#pragma unroll
+      for (int i = 0; i < S; ++i)
+        if (n0 + i >= s0 && n0 + i < s1) wav[(long long)b * wav_ld + (n0 + i - s0)] = tanhf(acc[i]);
+      continue;
+    }
     float* out = wav + (long long)b * L + n0;
     if (n0 + S <= L && (((long long)b * L + n0) & 3) == 0) {
       reinterpret_cast<float4*>(out)[0] = make_float4(tanhf(acc[0]), tanhf(acc[1]), tanhf(acc[2]), tanhf(acc[3]));

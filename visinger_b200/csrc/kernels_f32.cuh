@@ -44,7 +44,7 @@ struct ConvF32 {
   int rs_split;      // EPI_RES_SKIP: channels [0, rs_split) update the state, the rest go to the skip sum
   int y2_first;      // EPI_RES_SKIP: skip sum is written, not accumulated (first layer)
   int y2_mask;       // EPI_RES_SKIP: multiply the skip sum by the mask (last layer)
-  int couple_sign;   // EPI_COUPLE: +1 forward (x1 = m + x1*mask), -1 reverse (x1 = (x1 - m)*mask)
+  int couple_sign;   // EPI_COUPLE: +1 forward (x1 = m + x1*mask), -1 reverse (x1 = (x1 - m)*mask); x1 from res if set
 };
 
 constexpr int F32_CI_CHUNK = 8;
@@ -174,9 +174,11 @@ __global__ void __launch_bounds__(256) conv_f32_kernel(const ConvF32 p) {
             *yp = o;
           }
         } else {  // EPI_COUPLE
+          // (res != null: the old x1 is read from there -- a flow's first touch of the caller's input -- instead of y)
           const float m = v * mk;
           float* yp = p.y + (long long)b * p.y_bs + (long long)co * p.y_cs + n;
-          *yp = p.couple_sign > 0 ? (m + *yp * mk) : ((*yp - m) * mk);
+          const float x1 = p.res ? p.res[(long long)b * p.res_bs + (long long)co * p.res_cs + n] : *yp;
+          *yp = p.couple_sign > 0 ? (m + x1 * mk) : ((x1 - m) * mk);
         }
       }
     }
@@ -226,12 +228,12 @@ __global__ void posterior_sample_kernel(const float* __restrict__ stats, const f
 
 // ---- y = x * mask (z_q * mask before the decoder, models/visinger.py:109-111) -----------------
 __global__ void mask_mul_kernel(const float* __restrict__ x, const float* __restrict__ mask, float* __restrict__ y,
-                                int C, int T, long long total) {
+                                int C, int T, long long total, int mask_ld) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const long long bt = i / ((long long)C * T);
   const int t = (int)(i % T);
-  y[i] = x[i] * mask[bt * T + t];
+  y[i] = x[i] * mask[bt * mask_ld + t];
 }
 
 // ---- channel flip (only needed when n_flows is odd: the folded flips do not cancel) -----------
@@ -248,14 +250,16 @@ __global__ void flip_channels_kernel(float* __restrict__ x, int C, int T, long l
 }
 
 // ---- conv_post (C -> 1, k taps, no bias) fused with the leading leaky_relu and trailing tanh --
-// decoder.py:55-57.  One thread per output sample; reads are coalesced along time.
+// decoder.py:55-57.  One thread per output sample; reads are coalesced along time.  Samples [n0, n1) of each utterance go
+// to wav rows wav_ld apart (the whole output: 0, L, L; a streaming window: its central samples).
 __global__ void conv_post_f32_kernel(const float* __restrict__ x, const float* __restrict__ w /*[C][k]*/,
-                                     float* __restrict__ wav, int C, int L, int k, float slope) {
+                                     float* __restrict__ wav, int C, int L, int k, float slope, int n0, int n1,
+                                     long long wav_ld) {
   extern __shared__ float wsm[];
   for (int i = threadIdx.x; i < C * k; i += blockDim.x) wsm[i] = w[i];
   __syncthreads();
-  const int n = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
-  if (n >= L) return;
+  const int n = n0 + blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
+  if (n >= n1) return;
   const int pad = (k - 1) / 2;
   const float* xb = x + (long long)b * C * L;
   float s = 0.f;
@@ -266,7 +270,7 @@ __global__ void conv_post_f32_kernel(const float* __restrict__ x, const float* _
       if (pos >= 0 && pos < L) s = fmaf(wsm[c * k + j], lrelu(xr[pos], slope), s);
     }
   }
-  wav[(long long)b * L + n] = tanhf(s);
+  wav[(long long)b * wav_ld + (n - n0)] = tanhf(s);
 }
 
 }  // namespace vsg

@@ -7,7 +7,18 @@ namespace vsg {
 int launch_cond(const float* W, const float* bias, const float* g, float* out, int O, int I, int B, cudaStream_t st);
 int prior_sample(const float* mu, const float* logs, const float* noise, const float* mask, float* z, int B, int C,
                  int T, cudaStream_t st);
-int mask_mul(const float* x, const float* mask, float* y, int B, int C, int T, cudaStream_t st);
+int mask_mul(const float* x, const float* mask, float* y, int B, int C, int T, cudaStream_t st, int mask_ld = 0);
+
+// The decoder over a window of frames of a longer batch (vsg_generator_forward_window / vsg_infer_zp_window): z holds the
+// window's frames in rows of z_ld frames; wav row b (at wav + b * wav_ld) receives the window's samples [s0, s1).
+// T_plan is the whole padded batch's length: every kernel choice that depends on a length is taken from it, so that a
+// window computes each sample with the kernels -- and the rounding -- of the one-pass call.
+struct DecWin {
+  int T_plan;
+  int z_ld;
+  long long wav_ld;
+  int s0, s1;
+};
 
 // output stage (output.cu): peak-normalise -> x 32767 -> int16 (utils/audio/io.py:8-14)
 int wav_to_int16(const float* wav, const int32_t* lengths, int16_t* pcm, float* peak, int B, int L, int norm, cudaStream_t st);
@@ -15,21 +26,28 @@ int wav_to_int16(const float* wav, const int32_t* lengths, int16_t* pcm, float* 
 // fp32 parity mode (run_f32.cu)
 size_t flow_ws_bytes_f32(const VsgPack* P, int B, int T);
 size_t dec_ws_bytes_f32(const VsgPack* P, int B, int T);
+// x_ld > 0: x and mask are T frames of rows x_ld frames long (a window read in place); y is [B, C, T]
 int flow_forward_f32(const VsgPack* P, const float* x, const float* mask, const float* g, float* y, int B, int T,
-                     int reverse, Workspace& ws, cudaStream_t st);
+                     int reverse, Workspace& ws, cudaStream_t st, int x_ld = 0);
 int generator_forward_f32(const VsgPack* P, const float* z, const float* g, float* wav, int B, int T, Workspace& ws,
-                          cudaStream_t st);
+                          cudaStream_t st, const DecWin* win = nullptr);
 
 // bf16 tensor-core mode (run_tc.cu)
 size_t flow_ws_bytes_tc(const VsgPack* P, int B, int T, int planes = 1);
-size_t dec_ws_bytes_tc(const VsgPack* P, int B, int T, bool x3);
+// T_plan > 0: the decoder over T-frame windows of a T_plan-frame batch (sub-batch split taken from T_plan)
+size_t dec_ws_bytes_tc(const VsgPack* P, int B, int T, bool x3, int T_plan = 0);
 int flow_forward_tc(const VsgPack* P, const float* x, const float* mask, const float* g, float* y, int B, int T,
                     int reverse, Workspace& ws, cudaStream_t st, int planes = 1, const float* out_mask = nullptr,   // out_mask: y * mask
-                    const float* ps_logs = nullptr, const float* ps_noise = nullptr);   // x = mu_p: prior sampling at the entry   // planes = 3: fp32 tolerance (bf16x3 mode)
+                    const float* ps_logs = nullptr, const float* ps_noise = nullptr,   // x = mu_p: prior sampling at the entry   // planes = 3: fp32 tolerance (bf16x3 mode)
+                    int x_ld = 0);   // x_ld > 0: x and mask are T frames of rows x_ld frames long (a window read in place)
 // VSG_X3_FLOW_FFMA=1 in the environment: the bf16x3 mode runs the flow on the fp32 CUDA-core kernels (A/B measurements)
 bool x3_flow_on_tensor_cores();
 int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float* wav, int B, int T, Workspace& ws,
-                         cudaStream_t st, bool x3);
+                         cudaStream_t st, bool x3, const DecWin* win = nullptr);
+// What the kernels the one-pass decoder picks for a (B, T) batch ask of a window of it: at least *min_frames frames (the
+// row-packed and fused kernels' shortest stage), starting and ending on multiples of *align frames (the row-packed
+// kernels' time steps per row at each stage's rate).  VSG_EUNSUPPORTED if a chosen conv_post kernel has no window form.
+int dec_window_needs_tc(const VsgPack* P, int B, int T, bool x3, int* min_frames, int* align);
 
 
 // PosteriorEncoder (f32: run_f32.cu, bf16: run_tc.cu)
@@ -65,7 +83,7 @@ int length_regulate(const float* enc, const long long* mel2ph, const float* tabl
 // vsg_flow_forward after validation (api.cu): the precision's flow kernels; see api.cu for masked / ps_* / sampled
 int run_flow(const VsgPack* pack, const float* x, const float* mask, const float* g, float* y, int B, int T, int reverse,
              int precision, Workspace& ws, cudaStream_t st, bool* masked = nullptr, const float* ps_logs = nullptr,
-             const float* ps_noise = nullptr, bool* sampled = nullptr);
+             const float* ps_noise = nullptr, bool* sampled = nullptr, int x_ld = 0);
 
 // The linear spectrogram (spec.cuh).  mask [B, T] = t < lengths[b] (lengths clamped to [0, T]).
 int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st);

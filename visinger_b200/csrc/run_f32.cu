@@ -67,16 +67,22 @@ size_t flow_ws_bytes_f32(const VsgPack* P, int B, int T) {
 
 // ResidualCouplingBlock.forward, modules/visinger/flow.py:33-40, with the Flips folded away.
 int flow_forward_f32(const VsgPack* P, const float* x, const float* mask, const float* g, float* y, int B, int T,
-                     int reverse, Workspace& ws, cudaStream_t st) {
+                     int reverse, Workspace& ws, cudaStream_t st, int x_ld) {
   const VsgConfig& c = P->cfg;
   const int C = c.flow_channels, H = c.flow_hidden, NL = c.flow_n_layers, NF = c.flow_n_flows, half = C / 2;
   const int condO = 2 * H * NL;
+  const int ld = x_ld > 0 ? x_ld : T;
   float* cond = ws.take<float>((size_t)B * NF * condO);
   float* h = ws.take<float>((size_t)B * H * T);
   float* acts = ws.take<float>((size_t)B * H * T);
   float* out = ws.take<float>((size_t)B * H * T);
   if (ws.overflow) return fail(VSG_ENOMEM, "flow workspace too small: need %zu bytes", ws.off);
-  if (y != x) VSG_CUDA_TRY(cudaMemcpyAsync(y, x, (size_t)B * C * T * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  // Each channel half is read from x until a coupling first writes it into y (its epilogue reads the old x1 from x), so
+  // the input is never copied -- nor gathered, when x is a window of a longer batch.  (y may alias x.)
+  const float* src[2] = {x, x + (long long)half * ld};
+  long long src_bs[2] = {(long long)C * ld, (long long)C * ld};
+  int src_cs[2] = {ld, ld};
+  bool in_y[2] = {false, false};
   if (c.flow_gin > 0) {
     if (!g) return fail(VSG_EINVAL, "flow was built with gin_channels=%d but g is NULL", c.flow_gin);
     for (int f = 0; f < NF; ++f)
@@ -88,12 +94,12 @@ int flow_forward_f32(const VsgPack* P, const float* x, const float* mask, const 
     const int f = reverse ? NF - 1 - step : step;
     const int flipped = reverse ? (NF - f) & 1 : f & 1;   // parity of Flips applied so far
     const FlowLayer& fl = P->flow_layers[f];
-    const float* x0 = y + (flipped ? (long long)half * T : 0);   // conditioning half (never modified here)
-    float* x1 = y + (flipped ? 0 : (long long)half * T);         // half that is updated in place
+    const int h0 = flipped ? 1 : 0, h1 = 1 - h0;                  // conditioning half (never modified here), updated half
+    float* x1 = y + (long long)h1 * half * T;
     // h = pre(x0) * mask                                           flow.py:68
     {
-      ConvF32 p = base_conv(fl.pre[flipped], x0, CT, T, T, 0, 1);
-      p.y = h; p.y_bs = HT; p.y_cs = T; p.mask = mask; p.mask_bs = T;
+      ConvF32 p = base_conv(fl.pre[flipped], src[h0], src_bs[h0], src_cs[h0], T, 0, 1);
+      p.y = h; p.y_bs = HT; p.y_cs = T; p.mask = mask; p.mask_bs = ld;
       VSG_TRY(launch_conv_f32(p, B, st));
     }
     // WaveNet                                                       encoder.py:174-195
@@ -116,7 +122,7 @@ int flow_forward_f32(const VsgPack* P, const float* x, const float* mask, const 
         p.y = h; p.y_bs = HT; p.y_cs = T;
         p.y2 = out; p.y2_bs = HT; p.y2_cs = T;
         p.y2_first = (i == 0); p.y2_mask = last;
-        p.mask = mask; p.mask_bs = T;
+        p.mask = mask; p.mask_bs = ld;
         VSG_TRY(launch_conv_f32(p, B, st));
       }
       dil *= c.flow_dilation_rate;
@@ -125,10 +131,18 @@ int flow_forward_f32(const VsgPack* P, const float* x, const float* mask, const 
     {
       ConvF32 p = base_conv(fl.post[flipped], out, HT, T, T, 0, 1);
       p.epi = EPI_COUPLE; p.couple_sign = reverse ? -1 : 1;
-      p.y = x1; p.y_bs = CT; p.y_cs = T; p.mask = mask; p.mask_bs = T;
+      p.y = x1; p.y_bs = CT; p.y_cs = T; p.mask = mask; p.mask_bs = ld;
+      if (!in_y[h1]) { p.res = src[h1]; p.res_bs = src_bs[h1]; p.res_cs = src_cs[h1]; }
       VSG_TRY(launch_conv_f32(p, B, st));
     }
+    src[h1] = x1; src_bs[h1] = CT; src_cs[h1] = T; in_y[h1] = true;
   }
+  for (int hh = 0; hh < 2; ++hh)   // a half no coupling wrote (one flow only) is copied
+    if (!in_y[hh] && src[hh] != y + (long long)hh * half * T)
+      for (int b = 0; b < B; ++b)
+        VSG_CUDA_TRY(cudaMemcpy2DAsync(y + ((long long)b * C + hh * half) * T, (size_t)T * sizeof(float),
+                                       src[hh] + (long long)b * C * ld, (size_t)ld * sizeof(float), (size_t)T * sizeof(float),
+                                       half, cudaMemcpyDeviceToDevice, st));
   if (NF & 1) {   // an odd number of Flips does not cancel
     const long long n = (long long)B * half * T;
     flip_channels_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(y, C, T, n);
@@ -369,7 +383,7 @@ size_t dec_ws_bytes_f32(const VsgPack* P, int B, int T) {
 
 // Generator.forward, modules/visinger/decoder.py:40-59.
 int generator_forward_f32(const VsgPack* P, const float* z, const float* g, float* wav, int B, int T, Workspace& ws,
-                          cudaStream_t st) {
+                          cudaStream_t st, const DecWin* win) {
   const VsgConfig& c = P->cfg;
   const int UIC = c.dec_upsample_initial_channel, NK = c.dec_n_kernels;
   const size_t E = dec_max_elems(P, B, T);
@@ -385,7 +399,8 @@ int generator_forward_f32(const VsgPack* P, const float* z, const float* g, floa
   }
   // x = conv_pre(z) + cond(g)                                        decoder.py:41-43
   {
-    ConvF32 p = base_conv(P->conv_pre, z, (long long)c.dec_initial_channel * T, T, T, -3, 1);
+    const int z_ld = win ? win->z_ld : T;
+    ConvF32 p = base_conv(P->conv_pre, z, (long long)c.dec_initial_channel * z_ld, z_ld, T, -3, 1);
     if (c.dec_gin > 0) { p.bcond = cond; p.bcond_bs = UIC; }
     p.y = bufS; p.y_bs = (long long)UIC * T; p.y_cs = T;
     VSG_TRY(launch_conv_f32(p, B, st));
@@ -438,9 +453,10 @@ int generator_forward_f32(const VsgPack* P, const float* z, const float* g, floa
   }
   // wav = tanh(conv_post(leaky_relu(x)))                               decoder.py:55-57
   {
-    dim3 grid((L + 255) / 256, B);
-    conv_post_f32_kernel<<<grid, 256, (size_t)ch * P->conv_post_k * sizeof(float), st>>>(bufS, P->conv_post_w, wav, ch,
-                                                                                          L, P->conv_post_k, 0.1f);
+    const int n0 = win ? win->s0 : 0, n1 = win ? win->s1 : L;
+    dim3 grid((n1 - n0 + 255) / 256, B);
+    conv_post_f32_kernel<<<grid, 256, (size_t)ch * P->conv_post_k * sizeof(float), st>>>(
+        bufS, P->conv_post_w, wav, ch, L, P->conv_post_k, 0.1f, n0, n1, win ? win->wav_ld : (long long)L);
     VSG_LAUNCH_CHECK("conv_post_f32_kernel");
   }
   return VSG_OK;
@@ -455,10 +471,10 @@ int prior_sample(const float* mu, const float* logs, const float* noise, const f
   return VSG_OK;
 }
 
-int mask_mul(const float* x, const float* mask, float* y, int B, int C, int T, cudaStream_t st) {
+int mask_mul(const float* x, const float* mask, float* y, int B, int C, int T, cudaStream_t st, int mask_ld) {
   const long long n = (long long)B * C * T;
   if (n == 0) return VSG_OK;
-  mask_mul_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, mask, y, C, T, n);
+  mask_mul_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, mask, y, C, T, n, mask_ld > 0 ? mask_ld : T);
   VSG_LAUNCH_CHECK("mask_mul_kernel");
   return VSG_OK;
 }

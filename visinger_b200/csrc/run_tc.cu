@@ -1,4 +1,6 @@
 // bf16 tensor-core mode: weight pre-pack, TMA tensor maps, launch logic and the Generator driver.
+#include <numeric>
+
 #include "vsg_common.cuh"
 #include "run.cuh"
 #include "pack_tc.cuh"
@@ -93,7 +95,8 @@ constexpr size_t kSmemMax = 227 * 1024;
 
 struct EpiTC {
   int mode = EPI_TC_LINEAR;
-  const float* mask = nullptr;      // [B][Lout]
+  const float* mask = nullptr;      // [B][mask_ld]
+  int mask_ld = 0;                  // 0: Lout
   int couple_sign = -1;
   int ld = 0;                       // leading dimension (channels per row) of the add / out tensors; 0 = their own width
   int part_stride = 0;              // channels between the bf16 planes of the add / out tensors; 0 = their own width
@@ -108,6 +111,8 @@ struct EpiTC {
   __nv_bfloat16* out_act = nullptr;
   float* out_f32 = nullptr;
   int tanh_cols = 0;                // EPI_TC_TANH: samples per row written to out_f32
+  long long tanh_ld = 0;            // EPI_TC_TANH, > 0: only samples [tanh_s0, tanh_s1), at out_f32 + b * tanh_ld (conv_tc.cuh)
+  int tanh_s0 = 0, tanh_s1 = 0;
   int mag_ch = 0;                   // EPI_TC_MAG: output channels below this are magnitudes, the rest are written as 0
 };
 
@@ -358,7 +363,7 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
   p.total_tiles = p.m_tiles_per_b * p.n_ntiles * B;
   p.e_swz_mask = cw >= 64 ? 7u : cw >= 32 ? 3u : 1u;
   p.e_out_swz_mask = ow >= 64 ? 7u : ow >= 32 ? 3u : ow >= 16 ? 1u : 0u;
-  p.mode = e.mode; p.mask = e.mask; p.couple_sign = e.couple_sign;
+  p.mode = e.mode; p.mask = e.mask; p.mask_ld = e.mask_ld > 0 ? e.mask_ld : Lout; p.couple_sign = e.couple_sign;
   p.has_add0 = e.add0 != nullptr; p.has_add1 = e.add1 != nullptr;
   p.has_raw = e.out_raw != nullptr; p.has_act = e.out_act != nullptr;
   p.add0_is_act = e.add0_is_act;
@@ -372,6 +377,7 @@ int launch_conv_tc(const VsgPack* P, const ConvWTC& w, const __nv_bfloat16* x, i
   p.scale = e.scale; p.slope = e.slope;
   p.out_f32 = e.out_f32;
   p.tanh_cols = e.tanh_cols;
+  p.tanh_ld = e.tanh_ld; p.tanh_s0 = e.tanh_s0; p.tanh_s1 = e.tanh_s1;
   p.mag_ch = e.mag_ch;
   p.error_flag = error_flag;
 
@@ -1083,7 +1089,8 @@ size_t flow_ws_bytes_tc(const VsgPack* P, int B, int T, int planes) {
 // the fp32 value exactly) and every product runs as six plane products, small ones first (launch_conv_tc): the flow at
 // north_star's fp32 tolerance (z <= 1e-5) on tcgen05 -- the bf16x3 precision mode.
 int flow_forward_tc(const VsgPack* P, const float* x, const float* mask, const float* g, float* y, int B, int T,
-                    int reverse, Workspace& ws, cudaStream_t st, int planes, const float* out_mask, const float* ps_logs, const float* ps_noise) {
+                    int reverse, Workspace& ws, cudaStream_t st, int planes, const float* out_mask, const float* ps_logs, const float* ps_noise,
+                    int x_ld) {
   const VsgConfig& c = P->cfg;
   const int C = c.flow_channels, H = c.flow_hidden, NL = c.flow_n_layers, NF = c.flow_n_flows, half = C / 2;
   const int K = c.flow_kernel_size;
@@ -1120,7 +1127,7 @@ int flow_forward_tc(const VsgPack* P, const float* x, const float* mask, const f
   }
   {
     dim3 grid((T + 31) / 32, (C + 31) / 32, B), block(32, 8);
-    transpose_to_bf16_kernel<<<grid, block, 0, st>>>(x, u, C, T, planes, ps_logs, ps_noise, mask);   // (ps_*: x = mu_p, prior sampling fused)
+    transpose_to_bf16_kernel<<<grid, block, 0, st>>>(x, u, C, T, planes, ps_logs, ps_noise, mask, x_ld);   // (ps_*: x = mu_p, prior sampling fused)
     VSG_LAUNCH_CHECK("transpose_to_bf16_kernel");
   }
   for (int step = 0; step < NF; ++step) {
@@ -1132,7 +1139,7 @@ int flow_forward_tc(const VsgPack* P, const float* x, const float* mask, const f
     {  // h = pre(x0) * mask  (merged: and out = 0)
       const ConvWTC& w = merged ? fl.pre2_tc[flipped][x6 ? 1 : 0] : x6 ? fl.pre_x6[flipped] : fl.pre_tc[flipped];
       EpiTC e;
-      e.bias = w.bias; e.mask = mask; e.out_raw = hs;
+      e.bias = w.bias; e.mask = mask; e.mask_ld = x_ld; e.out_raw = hs;
       if (!merged) { e.ld = hs_ld; e.part_stride = 2 * H; }
       VSG_TRY(launch_conv_tc(P, w, x0, B, T, 0, 1, T, 1, 0, T, e, opt, err, st, planes * C, C));
     }
@@ -1153,19 +1160,19 @@ int flow_forward_tc(const VsgPack* P, const float* x, const float* mask, const f
                               //  on the valid frames and the sum is masked after the last layer anyway, encoder.py:195)
         const ConvWTC& w = fl.rs_tc[x6 ? 1 : 0][i];
         EpiTC e;
-        e.bias = w.bias; e.add0 = hs; e.mask = mask; e.out_raw = hs;
+        e.bias = w.bias; e.add0 = hs; e.mask = mask; e.mask_ld = x_ld; e.out_raw = hs;
         VSG_TRY(launch_conv_tc(P, w, acts, B, T, 0, 1, T, 1, 0, T, e, opt, err, st));
       } else {
         if (!last) {  // h = (h + res(acts)) * mask
           const ConvWTC& w = x6 ? fl.res_x6[i] : fl.res_tc[i];
           EpiTC e;
-          e.bias = w.bias; e.add0 = h; e.mask = mask; e.out_raw = h; e.ld = hs_ld; e.part_stride = 2 * H;
+          e.bias = w.bias; e.add0 = h; e.mask = mask; e.mask_ld = x_ld; e.out_raw = h; e.ld = hs_ld; e.part_stride = 2 * H;
           VSG_TRY(launch_conv_tc(P, w, acts, B, T, 0, 1, T, 1, 0, T, e, opt, err, st));
         }
         {  // out (+)= skip(acts); masked after the last layer
           const ConvWTC& w = x6 ? fl.skip_x6[i] : fl.skip_tc[i];
           EpiTC e;
-          e.bias = w.bias; e.add0 = (i > 0 || merged) ? out : nullptr; e.mask = last ? mask : nullptr; e.out_raw = out;
+          e.bias = w.bias; e.add0 = (i > 0 || merged) ? out : nullptr; e.mask = last ? mask : nullptr; e.mask_ld = x_ld; e.out_raw = out;
           e.ld = hs_ld; e.part_stride = 2 * H;
           VSG_TRY(launch_conv_tc(P, w, acts, B, T, 0, 1, T, 1, 0, T, e, opt, err, st));
         }
@@ -1176,13 +1183,13 @@ int flow_forward_tc(const VsgPack* P, const float* x, const float* mask, const f
       const ConvWTC& w = x6 ? fl.post_x6[flipped] : fl.post_tc[flipped];
       EpiTC e;
       e.mode = EPI_TC_COUPLE; e.couple_sign = reverse ? -1 : 1;
-      e.bias = w.bias; e.mask = mask; e.add0 = x1; e.out_raw = x1; e.ld = planes * C; e.part_stride = C;
+      e.bias = w.bias; e.mask = mask; e.mask_ld = x_ld; e.add0 = x1; e.out_raw = x1; e.ld = planes * C; e.part_stride = C;
       VSG_TRY(launch_conv_tc(P, w, out, B, T, 0, 1, T, 1, 0, T, e, opt, err, st, hs_ld, 2 * H));
     }
   }
   {
     dim3 grid((T + 31) / 32, (C + 31) / 32, B), block(32, 8);
-    transpose_from_bf16_kernel<<<grid, block, 0, st>>>(u, y, C, T, (NF & 1) ? 1 : 0, planes, out_mask);   // (out_mask: y * mask)
+    transpose_from_bf16_kernel<<<grid, block, 0, st>>>(u, y, C, T, (NF & 1) ? 1 : 0, planes, out_mask, x_ld);   // (out_mask: y * mask)
     VSG_LAUNCH_CHECK("transpose_from_bf16_kernel");
   }
   return VSG_OK;
@@ -1550,17 +1557,20 @@ int g_l2_tensor_mb = 0;       // target size of one intermediate tensor of a sub
                               // (11.4 ms -> 16.0 ms per B16xT1000 step at 13 MB), so it is off until the fused kernels land.
 int g_min_tiles = 592;        // keep >= 4 waves of 148 CTAs per launch when sub-batching
 
-SubBatchPlan plan_sub_batches(const VsgPack* P, int B, int T) {
+// T_plan > 0: the split of a T_plan-frame batch (a streaming window runs with the whole batch's split), buffers for T frames
+SubBatchPlan plan_sub_batches(const VsgPack* P, int B, int T, int T_plan = 0) {
   SubBatchPlan pl;
   pl.inter_elems = 0;
   pl.io_elems = (size_t)B * P->cfg.dec_upsample_initial_channel * T;
-  long long L = T;
+  long long L = T, Lp = T_plan > 0 ? T_plan : T;
   for (size_t i = 0; i < P->ups.size(); ++i) {
     const UpStage& us = P->ups[i];
     L *= us.rate;
+    Lp *= us.rate;
     const size_t per_utt = (size_t)us.Cout * (size_t)L;            // elements of one stage tensor of one utterance
-    const long long tiles_per_utt = (L + 127) / 128;
-    long long sub = std::max<long long>(1, ((long long)g_l2_tensor_mb << 20) / (long long)(per_utt * 2));
+    const size_t per_utt_p = (size_t)us.Cout * (size_t)Lp;
+    const long long tiles_per_utt = (Lp + 127) / 128;
+    long long sub = std::max<long long>(1, ((long long)g_l2_tensor_mb << 20) / (long long)(per_utt_p * 2));
     if (sub * tiles_per_utt < g_min_tiles) sub = (g_min_tiles + tiles_per_utt - 1) / tiles_per_utt;
     if (g_l2_tensor_mb <= 0 || sub * 2 > B) sub = B;               // not worth splitting
     static const int only_c = getenv("VSG_L2_ONLY_C") ? atoi(getenv("VSG_L2_ONLY_C")) : 0;   // A/B aid: sub-batch one stage width only
@@ -1636,22 +1646,133 @@ static int chain_streams_for(int device, cudaStream_t caller, ChainStreams** out
   return VSG_OK;
 }
 
-size_t dec_ws_bytes_tc(const VsgPack* P, int B, int T, bool x3) {
-  const SubBatchPlan pl = plan_sub_batches(P, B, T);
+size_t dec_ws_bytes_tc(const VsgPack* P, int B, int T, bool x3, int T_plan) {
+  const SubBatchPlan pl = plan_sub_batches(P, B, T, T_plan);
   const size_t np = x3 ? 2 : 1;
   return align256((size_t)B * T * P->cfg.dec_initial_channel * 2 * np) + align256((size_t)B * P->cfg.dec_upsample_initial_channel * 4) +
          2 * align256(pl.io_elems * 2 * np) + (7 + 4 * (kMaxChains - 1)) * align256(pl.inter_elems * 2 * np) + 512;
+}
+
+// ---- kernel choices of the decoder ---------------------------------------------------------------------------------
+// Several choices depend on a stage's length, and the kernels they pick do not round alike: the row-packed and whole-
+// resblock kernels keep the resblock residual in fp32 (TMEM), the per-convolution path stores it in bf16 between the
+// convolutions; the fused pair rounds its intermediate like the per-convolution path but is only taken on long stages.  So
+// every such choice is made from the WHOLE padded batch's stage length L (and its sub-batch nb): a streaming window
+// (DecWin) runs the kernels the one-pass call runs, and if one of them cannot take the window's length the window is
+// widened (dec_window_needs_tc) -- the kernel is never switched.
+struct StageChoice { bool rb, rp, stage_planar; };
+
+bool dec_one_stream(const TCOptions& opt, bool x3) {
+  // Only leaky_relu(x) is stored for the running stream; split-bf16 recovers the residual from the two planes in fp32
+  // (x = a >= 0 ? a : a / slope: as exact as a raw copy at ~16 mantissa bits) unless VSG_X3_TWO_STREAMS=1
+  static const bool x3_two_streams = getenv("VSG_X3_TWO_STREAMS") != nullptr && getenv("VSG_X3_TWO_STREAMS")[0] == '1';
+  return opt.single_stream && !(x3 && x3_two_streams);
+}
+
+StageChoice stage_choice(const VsgPack* P, int i, int B, int nb, int L, bool x3, const TCOptions& opt) {
+  const VsgConfig& c = P->cfg;
+  const UpStage& us = P->ups[i];
+  const int ch = us.Cout, NK = c.dec_n_kernels;
+  const bool one_stream_all = dec_one_stream(opt, x3);
+  StageChoice sc;
+  // C <= 64 stages: every ResBlock1 is ONE kernel (rb_tc.cuh); the three launches of a stage are chained through the
+  // running sum, so they stay on the caller's stream (their CTAs own all of tensor memory and cannot co-reside anyway)
+  sc.rb = c.dec_resblock == 1 && !x3 && opt.fuse_rb && ch <= 64;
+  for (int j = 0; j < NK && sc.rb; ++j) {
+    RbPlan rp;
+    sc.rb = rb_plan(us.blocks[j], ch, L, opt, &rp) && L >= 256;
+  }
+  static const int rp_max_c_env = getenv("VSG_RP_MAX_C") ? atoi(getenv("VSG_RP_MAX_C")) : -1;   // A/B aid
+  const int rp_max_c = rp_max_c_env >= 0 ? rp_max_c_env : opt.rp_max_c;
+  // (bf16x3: the kernel's split-bf16 instantiation; it reads the single activated stream)
+  // (its planar planes are addressed through the conv kernel's int part_stride: nb * L * ch must fit)
+  sc.rp = c.dec_resblock == 1 && (x3 ? (opt.rp_x3 && one_stream_all && (size_t)nb * L * ch < ((size_t)1 << 31)) : true) &&
+          opt.fuse_rp && ch <= rp_max_c;
+  for (int j = 0; j < NK && sc.rp; ++j) {
+    RpPlan rp;
+    sc.rp = rp_plan(us.blocks[j], ch, L, opt, &rp, x3) && L >= 256;
+  }
+  // bf16x3 per-convolution ResBlock1 stages: every tensor of the stage planar through the conv kernel's ld / part_stride
+  // (the stage output too, unless conv_post reads it): that is what lets them take the merged-polyphase upsampler as
+  // well.  VSG_X3_PLANAR=0 (A/B aid): rows [hi | lo] as before
+  static const bool x3_planar_on = !(getenv("VSG_X3_PLANAR") && getenv("VSG_X3_PLANAR")[0] == '0');
+  sc.stage_planar = x3 && !sc.rp && x3_planar_on && one_stream_all && c.dec_resblock == 1 && !sc.rb && nb == B &&
+                    i + 1 < c.dec_n_ups && (size_t)nb * L * ch < ((size_t)1 << 31);
+  return sc;
+}
+
+// measured on B200 (tools/time_pair.py, B=16): C=32 pair 156-204 us vs 188-241 us un-fused; at C=16 the single epilogue
+// warp set of the one-CTA-per-SM pair kernel is slower (239-275 us) than two co-resident un-fused CTAs (210-235 us), so
+// only C=32 is fused by default (fuse_pairs == 2 forces both).
+bool pair_choice(const VsgPack* P, const ResBlockPack& rb, int q, int ch, int L, bool x3, const TCOptions& opt, bool has_add1,
+                 int n_outs) {
+  return P->cfg.dec_resblock == 1 && !x3 && opt.fuse_pairs && (ch == 32 || ch == 16 || opt.fuse_pairs == 2) &&
+         pair_supported(rb.c1_tc[q], rb.c2_tc[q], rb.dilations[q], L, 1 + (has_add1 ? 1 : 0), n_outs);
+}
+
+// conv_post: 0 tcgen05, rows of 4 samples | 1 register-window kernel | 2 shared-memory-window kernel (A/B aids) |
+// 3 tcgen05 bf16x3, rows of 2 samples | 4 one thread per sample
+int post_choice(const VsgPack* P, int ch, int L, bool x3, const TCOptions& opt) {
+  if (!x3 && ch == 16 && P->conv_post_k == 7) {   // the model's shape
+    if (opt.conv_post == 0 && P->conv_post_S == 4 && L % 4 == 0) return 0;
+    return opt.conv_post == 1 ? 1 : 2;
+  }
+  if (x3 && ch == 16 && P->conv_post_k == 7 && P->conv_post_rp_x3.has_tmap && L % 2 == 0 && opt.conv_post == 0) return 3;
+  return 4;
+}
+
+int dec_window_needs_tc(const VsgPack* P, int B, int T, bool x3, int* min_frames, int* align) {
+  const VsgConfig& c = P->cfg;
+  const TCOptions opt = g_default_opts;
+  const SubBatchPlan pl = plan_sub_batches(P, B, T);
+  const bool one_stream = dec_one_stream(opt, x3);
+  int need = 1, A = 1;
+  long long R = 1;                               // samples per frame at the current stage
+  auto min_len = [&](long long Lmin) { need = std::max(need, (int)((Lmin + R - 1) / R)); };
+  // a kernel with S time steps per row sums each output in an order set by its row phase: windows start and end where
+  // the one-pass call has phase 0, i.e. on multiples of S / gcd(S, R) frames
+  auto row_phase = [&](int S) { const int a = S / (int)std::gcd((long long)S, R); A = A / std::gcd(A, a) * a; };
+  int ch = c.dec_upsample_initial_channel;
+  for (int i = 0; i < c.dec_n_ups; ++i) {
+    const UpStage& us = P->ups[i];
+    R *= us.rate;
+    ch = us.Cout;
+    const int L = (int)(T * R);
+    for (int b0 = 0; b0 < B; b0 += pl.sub[i]) {
+      const int nb = std::min(pl.sub[i], B - b0);
+      const StageChoice sc = stage_choice(P, i, B, nb, L, x3, opt);
+      if (sc.rb) min_len(256);
+      if (sc.rp) { min_len(256); row_phase(64 / ch); }
+      if (sc.rb || sc.rp) continue;
+      for (int j = 0; j < c.dec_n_kernels; ++j) {
+        const ResBlockPack& rb = us.blocks[j];
+        const int nd = (int)rb.dilations.size();
+        for (int q = 0; q < nd; ++q) {
+          const bool last = q == nd - 1;
+          if (pair_choice(P, rb, q, ch, L, x3, opt, last && j > 0, last ? 1 : (one_stream ? 1 : 2))) min_len(128 * pair_mb(ch));
+        }
+      }
+    }
+  }
+  const int post = post_choice(P, ch, (int)(T * R), x3, opt);
+  if (post == 1) return fail(VSG_EUNSUPPORTED, "the register-window conv_post kernel (tuning option) has no window form");
+  if (post == 0) row_phase(4);
+  if (post == 3) row_phase(2);
+  *min_frames = std::min(need, T);
+  *align = A;
+  return VSG_OK;
 }
 
 // Generator.forward (modules/visinger/decoder.py:40-59) on the tensor-core kernels.
 // x3: split-bf16 mode -- every activation tensor carries two bf16 planes [hi | lo] per row and every product is
 // three MMAs (hi*W_hi + hi*W_lo + lo*W_hi): fp32-tolerance results on the tensor cores.
 int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float* wav, int B, int T, Workspace& ws,
-                         cudaStream_t st, bool x3) {
+                         cudaStream_t st, bool x3, const DecWin* win) {
   const VsgConfig& c = P->cfg;
   const int C0 = c.dec_initial_channel, UIC = c.dec_upsample_initial_channel, NK = c.dec_n_kernels;
   if (!P->conv_pre_tc.has_tmap) return fail(VSG_EUNSUPPORTED, "bf16 decoder needs channel counts that are multiples of 16");
-  const SubBatchPlan pl = plan_sub_batches(P, B, T);
+  const int T_plan = win ? win->T_plan : T;     // every length-dependent kernel choice below is made from the whole batch
+  const SubBatchPlan pl = plan_sub_batches(P, B, T, T_plan);
   typedef __nv_bfloat16 bf;
   const size_t np = x3 ? 2 : 1;             // bf16 planes per activation tensor
   auto W = [&](const ConvWTC& plain, const ConvWTC& split) -> const ConvWTC& { return x3 ? split : plain; };
@@ -1686,7 +1807,7 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
   }
   {  // boundary: [B, C, T] fp32 -> [B, T, C] bf16, once
     dim3 grid((T + 31) / 32, (C0 + 31) / 32, B), block(32, 8);
-    transpose_to_bf16_kernel<<<grid, block, 0, st>>>(z, zt, C0, T, x3 ? 2 : 1);
+    transpose_to_bf16_kernel<<<grid, block, 0, st>>>(z, zt, C0, T, x3 ? 2 : 1, nullptr, nullptr, nullptr, win ? win->z_ld : 0);
     VSG_LAUNCH_CHECK("transpose_to_bf16_kernel");
   }
   int cur_io = 0;
@@ -1697,16 +1818,16 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
     e.out_act = io[cur_io];
     VSG_TRY(launch_conv_tc(P, W(P->conv_pre_tc, P->conv_pre_x3), zt, B, T, -3, 1, T, 1, 0, T, e, opt, err, st));
   }
-  // Only leaky_relu(x) is stored for the running stream (see below); split-bf16 recovers the residual from the two
-  // planes in fp32 (x = a >= 0 ? a : a / slope: as exact as a raw copy at ~16 mantissa bits) unless VSG_X3_TWO_STREAMS=1
-  static const bool x3_two_streams = getenv("VSG_X3_TWO_STREAMS") != nullptr && getenv("VSG_X3_TWO_STREAMS")[0] == '1';
-  const bool one_stream_all = opt.single_stream && !(x3 && x3_two_streams);
+  // Only leaky_relu(x) is stored for the running stream (see below and dec_one_stream)
+  const bool one_stream_all = dec_one_stream(opt, x3);
   int L = T, ch = UIC;
+  long long Lp = T_plan;                      // the stage length of the whole batch: the kernel choices' length
   bool prev_planar = false;                   // bf16x3: the stage input is a planar two-plane tensor
   for (int i = 0; i < c.dec_n_ups; ++i) {
     const UpStage& us = P->ups[i];
     const int Lin = L, Cin = ch, Lout = L * us.rate;
     ch = us.Cout; L = Lout;
+    Lp *= us.rate;
     const bf* stage_in = io[cur_io];
     bf* stage_out = io[cur_io ^ 1];
     bool stage_planar_out = false;
@@ -1714,32 +1835,13 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
       const int nb = std::min(pl.sub[i], B - b0);
       const bf* xin = stage_in + (size_t)b0 * Lin * Cin * (prev_planar ? 1 : np);   // (planar: plane 0 of utterance b0)
       bf* xout = stage_out + (size_t)b0 * L * ch * np;
-      // C <= 64 stages: every ResBlock1 is ONE kernel (rb_tc.cuh); the three launches of a stage are chained through the
-      // running sum, so they stay on the caller's stream (their CTAs own all of tensor memory and cannot co-reside anyway)
-      bool rb_stage = c.dec_resblock == 1 && !x3 && opt.fuse_rb && ch <= 64;
-      for (int j = 0; j < NK && rb_stage; ++j) {
-        RbPlan rp;
-        rb_stage = rb_plan(us.blocks[j], ch, L, opt, &rp) && L >= 256;
-      }
-      static const int rp_max_c_env = getenv("VSG_RP_MAX_C") ? atoi(getenv("VSG_RP_MAX_C")) : -1;   // A/B aid
-      const int rp_max_c = rp_max_c_env >= 0 ? rp_max_c_env : opt.rp_max_c;
-      // (bf16x3: the kernel's split-bf16 instantiation; it reads the single activated stream)
-      // (its planar planes are addressed through the conv kernel's int part_stride: nb * L * ch must fit)
-      bool rp_stage = c.dec_resblock == 1 && (x3 ? (opt.rp_x3 && one_stream_all && (size_t)nb * L * ch < ((size_t)1 << 31)) : true) &&
-                      opt.fuse_rp && ch <= rp_max_c;
-      for (int j = 0; j < NK && rp_stage; ++j) {
-        RpPlan rp;
-        rp_stage = rp_plan(us.blocks[j], ch, L, opt, &rp, x3) && L >= 256;
-      }
+      const StageChoice sc = stage_choice(P, i, B, nb, (int)Lp, x3, opt);
+      const bool rb_stage = sc.rb, rp_stage = sc.rp;
       // bf16x3 row-packed stages: the upsampler writes its two planes PLANAR ([2][nb, L, ch]: each plane is then an
-      // ordinary one-plane tensor for the resblock kernel's row-packed tensor map), as is the running resblock sum
+      // ordinary one-plane tensor for the resblock kernel's row-packed tensor map), as is the running resblock sum;
+      // the per-convolution ResBlock1 stages of the bf16x3 mode are planar too (stage_choice)
       const bool planar = x3 && rp_stage;
-      // ... and so do the per-convolution ResBlock1 stages of the bf16x3 mode (every tensor of the stage planar through the
-      // conv kernel's ld / part_stride; the stage output too, unless conv_post reads it): that is what lets them take the
-      // merged-polyphase upsampler as well.  VSG_X3_PLANAR=0 (A/B aid): rows [hi | lo] as before
-      static const bool x3_planar_on = !(getenv("VSG_X3_PLANAR") && getenv("VSG_X3_PLANAR")[0] == '0');
-      const bool stage_planar = x3 && !planar && x3_planar_on && one_stream_all && c.dec_resblock == 1 && !rb_stage && nb == B &&
-                                i + 1 < c.dec_n_ups && (size_t)nb * L * ch < ((size_t)1 << 31);
+      const bool stage_planar = sc.stage_planar;
       const bool planar_any = planar || stage_planar;
       stage_planar_out = stage_planar;
       const int up_ld = planar_any ? ch : 0, up_part = planar_any ? (int)((size_t)nb * L * ch) : 0;
@@ -1800,12 +1902,8 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
             if (j == NK - 1) { e2.scale = 1.0f / (float)NK; e2.out_act = xout; }
             else e2.out_raw = bS;
           }
-          // measured on B200 (tools/time_pair.py, B=16): C=32 pair 156-204 us vs 188-241 us un-fused; at C=16 the single
-          // epilogue warp set of the one-CTA-per-SM pair kernel is slower (239-275 us) than two co-resident un-fused CTAs
-          // (210-235 us), so only C=32 is fused by default (fuse_pairs == 2 forces both).
           const int n_outs_pair = last ? 1 : (one_stream ? 1 : 2);
-          const bool fuse = c.dec_resblock == 1 && !x3 && opt.fuse_pairs && (ch == 32 || ch == 16 || opt.fuse_pairs == 2) &&
-                            pair_supported(rb.c1_tc[q], rb.c2_tc[q], d, L, 1 + (e2.add1 ? 1 : 0), n_outs_pair);
+          const bool fuse = pair_choice(P, rb, q, ch, (int)Lp, x3, opt, e2.add1 != nullptr, n_outs_pair);
           if (fuse) {
             // low-channel stages: both convs of the pair in ONE kernel, the intermediate never leaves the SM
             // The pair kernel reads its input with a halo (rows of the NEIGHBOUR tiles) while other CTAs store their
@@ -1869,15 +1967,18 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
     prev_planar = stage_planar_out;
   }
   {  // wav = tanh(conv_post(leaky_relu(x)))   (decoder.py:55-57); the stage output already holds leaky_relu(x)
-    if (!x3 && ch == 16 && P->conv_post_k == 7) {   // the model's shape: sliding-window kernel
+    // (a window: only its central samples [s0, s1) are computed or stored, straight into the caller's rows)
+    const int post = post_choice(P, ch, (int)Lp, x3, opt);
+    if (win && post == 1) return fail(VSG_EUNSUPPORTED, "the register-window conv_post kernel (tuning option) has no window form");
+    if (post == 0 || post == 1 || post == 2) {   // the model's shape (16 channels, k = 7)
       constexpr int S = 8;
-      const int post_mode = opt.conv_post;        // 0 tensor cores, 1 register-window kernel, 2 shared-memory kernel (A/B)
-      if (post_mode == 0 && P->conv_post_S == 4 && L % 4 == 0) {
+      if (post == 0) {
         // conv_post on the tensor cores: rows of 4 samples x 16 channels, Conv1d(64 -> 16, 3 row taps), tanh epilogue
         EpiTC e;
         e.mode = EPI_TC_TANH; e.out_f32 = wav; e.tanh_cols = 4;
+        if (win) { e.tanh_ld = win->wav_ld; e.tanh_s0 = win->s0; e.tanh_s1 = win->s1; }
         VSG_TRY(launch_conv_tc(P, P->conv_post_rp, io[cur_io], B, L / 4, -1, 1, L / 4, 1, 0, L / 4, e, opt, err, st));
-      } else if (post_mode == 1) {
+      } else if (post == 1) {
         const int gpb = (L + S - 1) / S, total = gpb * B;
         const int blocks = std::min((total + 127) / 128, 8 * P->sm_count);
         conv_post_bf16_win_kernel<16, 7, S><<<blocks, 128, 0, st>>>(io[cur_io], P->conv_post_w, wav, L, gpb, total);
@@ -1885,18 +1986,21 @@ int generator_forward_tc(const VsgPack* P, const float* z, const float* g, float
       } else {
         const int tpb = (L + 128 * S - 1) / (128 * S), total = tpb * B;
         const int blocks = std::min(total, 6 * P->sm_count);
-        conv_post_bf16_smem_kernel<16, 7, S><<<blocks, 128, 0, st>>>(io[cur_io], P->conv_post_w, wav, L, tpb, total);
+        conv_post_bf16_smem_kernel<16, 7, S><<<blocks, 128, 0, st>>>(io[cur_io], P->conv_post_w, wav, L, tpb, total,
+                                                                    win ? win->s0 : 0, win ? win->s1 : 0, win ? win->wav_ld : 0);
         VSG_LAUNCH_CHECK("conv_post_bf16_smem_kernel");
       }
-    } else if (x3 && ch == 16 && P->conv_post_k == 7 && P->conv_post_rp_x3.has_tmap && L % 2 == 0 && opt.conv_post == 0) {
+    } else if (post == 3) {
       // bf16x3: rows of 2 samples x [hi | lo] x 16 channels, Conv1d(64 -> 16, 5 row taps) on [W_hi | W_lo], tanh epilogue
       EpiTC e;
       e.mode = EPI_TC_TANH; e.out_f32 = wav; e.tanh_cols = 2;
+      if (win) { e.tanh_ld = win->wav_ld; e.tanh_s0 = win->s0; e.tanh_s1 = win->s1; }
       VSG_TRY(launch_conv_tc(P, P->conv_post_rp_x3, io[cur_io], B, L / 2, -2, 1, L / 2, 1, 0, L / 2, e, opt, err, st));
     } else {
-      dim3 grid((L + 255) / 256, B);
-      conv_post_bf16_kernel<<<grid, 256, (size_t)ch * P->conv_post_k * sizeof(float), st>>>(io[cur_io], P->conv_post_w, wav,
-                                                                                             ch, L, P->conv_post_k, x3 ? 1 : 0);
+      const int n0 = win ? win->s0 : 0, n1 = win ? win->s1 : L;
+      dim3 grid((n1 - n0 + 255) / 256, B);
+      conv_post_bf16_kernel<<<grid, 256, (size_t)ch * P->conv_post_k * sizeof(float), st>>>(
+          io[cur_io], P->conv_post_w, wav, ch, L, P->conv_post_k, x3 ? 1 : 0, n0, n1, win ? win->wav_ld : 0);
       VSG_LAUNCH_CHECK("conv_post_bf16_kernel");
     }
   }

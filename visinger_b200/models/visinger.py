@@ -137,6 +137,61 @@ class HotPath(PackedModuleMixin, nn.Module):
         self.last_launches = _lib.last_launch_count()
         return wav, z_q
 
+    @torch.no_grad()
+    def stream(self, z_p, mask, g, chunk_frames: int):
+        """`infer_zp`'s waveform in pieces: a generator of wav chunks [B, 1, n * hop], n = chunk_frames (the last chunk
+        may be shorter), one `vsg_infer_zp_window` call each.  The concatenated chunks equal `infer_zp(z_p, mask, g)[0]`
+        bit for bit, in every precision.  One workspace of `vsg_window_workspace_bytes` -- independent of T -- serves the
+        whole stream.  z_p, mask and g must stay unchanged until the stream is exhausted."""
+        _lib.require_cuda(z_p, "z_p")
+        _lib.require_cuda(mask, "mask")
+        B, C, T = z_p.shape
+        if C != self.flow.channels or mask.numel() != B * T:
+            raise RuntimeError(f"expected z_p [B, {self.flow.channels}, T] and mask [B, 1, T]")
+        if chunk_frames < 1:
+            raise RuntimeError("chunk_frames must be >= 1")
+        use_g = self._check_g(g, B)
+        pack = self._pack()
+        prec = _lib.precision_code(self.precision)
+        zc, mc = _lib.as_f32c(z_p), _lib.as_f32c(mask)
+        gc = _lib.as_f32c(g) if use_g else None
+        dev, hop = z_p.device, self.decoder.hop_size
+        n = min(chunk_frames, T)
+        ws = torch.empty(max(pack.window_workspace_bytes(B, T, n, prec), 1), dtype=torch.uint8, device=dev) if T else None
+        for t0 in range(0, T, n):
+            t1 = min(T, t0 + n)
+            wav = torch.empty(B, 1, (t1 - t0) * hop, dtype=torch.float32, device=dev)
+            if B:
+                with torch.cuda.device(dev):
+                    rc = _lib.lib().vsg_infer_zp_window(pack.handle, zc.data_ptr(), mc.data_ptr(),
+                                                        gc.data_ptr() if use_g else None, wav.data_ptr(), (t1 - t0) * hop,
+                                                        None, B, T, t0, t1, prec, ws.data_ptr(), ws.numel(),
+                                                        _lib.stream_ptr(dev))
+                _lib.check(rc, "vsg_infer_zp_window")
+                self.last_launches = _lib.last_launch_count()
+            yield wav
+
+    @torch.no_grad()
+    def decode_window(self, z, g, t0: int, t1: int):
+        """Frames [t0, t1) of `decode(z, g)` (vsg_generator_forward_window): wav [B, 1, (t1 - t0) * hop], bit for bit."""
+        _lib.require_cuda(z, "z")
+        B, _, T = z.shape
+        pack = self._pack()
+        prec = _lib.precision_code(self.precision)
+        zc = _lib.as_f32c(z)
+        use_g = self._check_g(g, B)
+        gc = _lib.as_f32c(g) if use_g else None
+        hop = self.decoder.hop_size
+        wav = torch.empty(B, 1, max(t1 - t0, 0) * hop, dtype=torch.float32, device=z.device)
+        with torch.cuda.device(z.device):
+            ws = _lib.workspace(z.device, pack.window_workspace_bytes(B, T, max(t1 - t0, 1), prec))
+            rc = _lib.lib().vsg_generator_forward_window(pack.handle, zc.data_ptr(), gc.data_ptr() if use_g else None,
+                                                         wav.data_ptr(), max(t1 - t0, 0) * hop, B, T, t0, t1, prec,
+                                                         ws.data_ptr(), ws.numel(), _lib.stream_ptr(z.device))
+        _lib.check(rc, "vsg_generator_forward_window")
+        self.last_launches = _lib.last_launch_count()
+        return wav
+
     def _check_g(self, g, B: int) -> bool:
         """The reference broadcasts g [B, gin, 1] over time (models/visinger.py:84); anything else would be misread
         as B*gin floats through the raw pointer, so it is rejected here.  Returns whether g is used."""
@@ -414,6 +469,23 @@ class VISinger(nn.Module):
             ret["wav_out"] = wav.squeeze(1)
             ret["z_q"] = z_q
             return ret
+
+    def forward_streaming(self, text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed=None, spk_id=None, f0=None,
+                          uv=None, chunk_frames: int = 250, noise=None):
+        """`forward(..., infer=True)`'s waveform as a stream: a generator of fp32 chunks [B, 1, n * hop] of chunk_frames
+        latent frames each (the last may be shorter).  The prior network (global attention) runs once, on the first
+        `next()`; flow and decoder then run window by window (`HotPath.stream`, vsg_infer_zp_window), every chunk bit
+        for bit the same samples as the one-pass waveform, with a workspace that does not grow with the length.
+        The chunks are float.  Peak-normalised int16 (`save_wav` with norm, utils/audio/io.py:8-14) needs the whole
+        utterance's peak; a stream converts each chunk on its own with vsg_wav_to_int16(norm = 0)
+        (`utils.audio.io.wav_to_int16(chunk, norm=False)`)."""
+        if not mel2ph.is_cuda:
+            raise RuntimeError("forward_streaming runs on the native path: inputs must be CUDA tensors")
+        with torch.no_grad():
+            self._hot.precision = self.precision
+            z_p, mask, spk_emb = self.prior(text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed, spk_id, f0, uv, {},
+                                            noise=noise, sample=True)
+        yield from self._hot.stream(z_p, mask, spk_emb, chunk_frames)
 
     def forward_graphed(self, text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed=None, spk_id=None, noise=None):
         """`forward(..., infer=True)` replayed from one CUDA graph per input shape (prior network + prior sampling + flow +
