@@ -597,6 +597,78 @@ int vsg_debug_attention_f32(const float* qkv, const float* mask, const float* ek
 int vsg_debug_layernorm_bf16(void* x_bf16, const float* gamma, const float* beta, const float* g, int32_t g_t,
                              const float* mask, float eps, int32_t B, int32_t T, int32_t C, int32_t device);
 
+/*
+ * Per-launch hooks of the fp32 (FFMA) mode's kernels (tests only; each allocates and synchronises, except the plan).
+ * Argument errors return VSG_EINVAL before the device is touched.
+ *
+ * vsg_debug_conv_f32: one launch of the fp32 convolution kernel with every field the library's drivers set.  Layout
+ * [B, C, T], time contiguous: element (b, c, t) of a tensor lives at b * *_bs + c * *_cs + t.  Output row q < Lq is time
+ * step n = q * out_stride + out_phase (< Lout) and reads input steps q + in_off0 + j * dil (zero outside 0 .. Lin - 1),
+ * through f(v) = leaky_relu(v, slope) if pre_lrelu (slope 0: ReLU), else v:
+ *   v[co] = sum_{ci, j} w[co][ci][j] * f(x[b, ci, q + in_off0 + j * dil]) + bias[co] + bcond[b * bcond_bs + co]
+ *   mk = mask[b * mask_bs + n] (1 without a mask)
+ *   linear (epi 0):   u = (v + res[b, co, n]) * mk;  y[b, co, n] = u (acc_mode 0) | y + u (1) | (y + u) / acc_div (2)
+ *   gate (epi 1):     y[b, c, n] = tanh(v[2c]) * sigmoid(v[2c + 1]) for c < Cout / 2
+ *   res_skip (epi 2): co < rs_split: y[b, co, n] = (y + v) * mk;  otherwise y2[b, co - rs_split, n] = v (y2_first) or
+ *                     y2 + v, times mk if y2_mask
+ *   couple (epi 3):   m = v * mk; x1 = res[b, co, n] if res is given, else y[b, co, n];
+ *                     y[b, co, n] = m + x1 * mk (couple_sign +1) | (x1 - m) * mk (couple_sign -1)
+ *   magnitude (epi 4, VSG_DEBUG_F32_MAG; no bias or bcond): y[b, c, n] = sqrt(v[2c]^2 + v[2c + 1]^2 + 1e-6) * mk
+ * (y + u in acc_mode 1 / 2 and the res_skip / couple forms read the old value at the same element.)  res may equal y.
+ * gate_interleave (gate only): w and bias are the reference module's [tanh half | sigmoid half] order (channel c and c +
+ * Cout / 2 form output c), packed by the library's interleave; bcond is then indexed in the packed order, channel c of
+ * the tanh half at 2c and of the sigmoid half at 2c + 1.  Without it, w and bias are already in the packed order.
+ * x, bcond, res, mask, y, y2: device fp32; w (fp32 [Cout][Cin][k]) and bias (fp32 [Cout] or NULL) live on the host.
+ * tile_out[2] (or NULL) = { warps along the channels, warps along time } of the launched tile configuration.
+ * VSG_EUNSUPPORTED (and no launch) where vsg_debug_conv_f32_plan refuses the shape.
+ */
+#define VSG_DEBUG_F32_MAG 4
+typedef struct VsgDebugConvF32 {
+  const float* x;
+  const float* w;
+  const float* bias;
+  const float* bcond;
+  const float* res;
+  const float* mask;
+  float* y;
+  float* y2;
+  int64_t x_bs, y_bs, res_bs, y2_bs;
+  int32_t x_cs, y_cs, res_cs, y2_cs;
+  int32_t B, Cin, Lin, Cout, k, dil, in_off0;
+  int32_t pre_lrelu;
+  float slope;
+  int32_t bcond_bs, mask_bs;
+  int32_t Lq, out_stride, out_phase, Lout;
+  int32_t epi, acc_mode;
+  float acc_div;
+  int32_t rs_split, y2_first, y2_mask, couple_sign, gate_interleave;
+} VsgDebugConvF32;
+int vsg_debug_conv_f32(const VsgDebugConvF32* d, int32_t* tile_out, int32_t device);
+
+/* Host only (no GPU): the tile plan of the fp32 convolution kernel for Cout output channels and k taps at dilation dil.
+ * out[3] = { warps along the channels, warps along time, dynamic shared memory in bytes }: 2 x 4 warps (1024 time steps
+ * per tile) for Cout <= 16, 4 x 2 (512) for Cout <= 32, else 8 x 1 (256); shared memory 4 * 8 * ((time steps per tile +
+ * (k - 1) * dil) + k * channels per tile).  VSG_EUNSUPPORTED above 200 KB. */
+int vsg_debug_conv_f32_plan(int32_t Cout, int32_t k, int32_t dil, int32_t* out);
+
+/* The fp32 decoder's upsampler as the generator runs it: y = conv_transpose1d(leaky_relu(x, 0.1), w, bias, stride = rate,
+ * padding = (k - rate) / 2) (modules/visinger/decoder.py:45-46) as `rate` polyphase launches of the fp32 convolution.
+ * x: device fp32 [B, Cin, Lin]; y: device fp32 [B, Cout, Lin * rate]; w: HOST fp32 [Cin][Cout][k]; bias: HOST fp32 [Cout].
+ * Needs k >= rate and k - rate even. */
+int vsg_debug_upsample_f32(const float* x, const float* w, const float* bias, int32_t Cin, int32_t Cout, int32_t rate,
+                           int32_t k, int32_t B, int32_t Lin, float* y, int32_t device);
+
+/* The fp32 decoder's conv_post: wav = tanh(conv1d(leaky_relu(x, slope), w, padding = (k - 1) / 2)) (decoder.py:55-57), C
+ * channels to one, no bias.  x: device fp32 [B, C, L]; w: HOST fp32 [C][k].  Samples n0 <= n < n1 of utterance b go to
+ * wav[b * wav_ld + n - n0] (device fp32); nothing else is written.  Needs 0 <= n0 < n1 <= L and wav_ld >= n1 - n0. */
+int vsg_debug_conv_post_f32(const float* x, const float* w, int32_t C, int32_t L, int32_t k, float slope, int32_t B,
+                            int32_t n0, int32_t n1, float* wav, int64_t wav_ld, int32_t device);
+
+/* The speaker-condition GEMV of every mode: out[b][o] = bias[o] + sum_i W[o][i] * g[b][i].  W [O][I], bias [O] (or NULL),
+ * g [B][I], out [B][O]: device fp32. */
+int vsg_debug_cond_f32(const float* W, const float* bias, const float* g, float* out, int32_t O, int32_t I, int32_t B,
+                       int32_t device);
+
 /* Tuning aids for tools/tune_plans.py: force the tile plan (0 / -1 = automatic) and the number of timed repetitions of
  * the following vsg_debug_conv1d_bf16 calls; average kernel milliseconds of the last such call. */
 int vsg_debug_set_plan(int32_t mb, int32_t cw, int32_t two_ctas, int32_t resident, int32_t reps);

@@ -108,6 +108,23 @@ class VsgDebugPair(ctypes.Structure):
                 [(n, ctypes.c_int32) for n in ("B", "L", "C", "k", "d1")])
 
 
+class VsgDebugConvF32(ctypes.Structure):
+    """Descriptor of vsg_debug_conv_f32 (include/visinger_b200.h)."""
+    _fields_ = ([(n, ctypes.c_void_p) for n in ("x", "w", "bias", "bcond", "res", "mask", "y", "y2")] +
+                [(n, ctypes.c_int64) for n in ("x_bs", "y_bs", "res_bs", "y2_bs")] +
+                [(n, ctypes.c_int32) for n in ("x_cs", "y_cs", "res_cs", "y2_cs", "B", "Cin", "Lin", "Cout", "k", "dil",
+                                               "in_off0", "pre_lrelu")] +
+                [("slope", ctypes.c_float)] +
+                [(n, ctypes.c_int32) for n in ("bcond_bs", "mask_bs", "Lq", "out_stride", "out_phase", "Lout", "epi",
+                                               "acc_mode")] +
+                [("acc_div", ctypes.c_float)] +
+                [(n, ctypes.c_int32) for n in ("rs_split", "y2_first", "y2_mask", "couple_sign", "gate_interleave")])
+
+
+# epilogues of vsg_debug_conv_f32 (csrc/kernels_f32.cuh EPI_*, and the magnitude instantiation)
+EPI_F32 = dict(LINEAR=0, GATE=1, RES_SKIP=2, COUPLE=3, MAG=4)
+ACC_SET, ACC_ADD, ACC_ADD_DIV = 0, 1, 2
+
 # epilogue images of the convolution kernel (csrc/conv_tc.cuh, EPI_SIG_*), as vsg_debug_conv_tc and vsg_last_launch_images
 # number them
 EPI_SIG = dict(GENERIC=0, ACT=1, RES_ACT=2, LINEAR=3, X6=4, SUM0=5, SUM1=6, FINAL=7, POST=8, ACT_X3=9, RES_ACT_X3=10,
@@ -225,6 +242,16 @@ def lib() -> ctypes.CDLL:
         L.vsg_debug_upsample_tc.restype = ctypes.c_int
         L.vsg_debug_upsample_tc.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, i32,
                                             ctypes.POINTER(ctypes.c_int32), i32]
+        L.vsg_debug_conv_f32.restype = ctypes.c_int
+        L.vsg_debug_conv_f32.argtypes = [ctypes.POINTER(VsgDebugConvF32), ctypes.POINTER(ctypes.c_int32), i32]
+        L.vsg_debug_conv_f32_plan.restype = ctypes.c_int
+        L.vsg_debug_conv_f32_plan.argtypes = [i32, i32, i32, ctypes.POINTER(ctypes.c_int32)]
+        L.vsg_debug_upsample_f32.restype = ctypes.c_int
+        L.vsg_debug_upsample_f32.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, i32]
+        L.vsg_debug_conv_post_f32.restype = ctypes.c_int
+        L.vsg_debug_conv_post_f32.argtypes = [vp, vp, i32, i32, i32, ctypes.c_float, i32, i32, i32, vp, ctypes.c_int64, i32]
+        L.vsg_debug_cond_f32.restype = ctypes.c_int
+        L.vsg_debug_cond_f32.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32]
         L.vsg_set_tc_options.restype = ctypes.c_int
         L.vsg_set_tc_options.argtypes = [i32, i32, i32, i32]
         L.vsg_debug_pair_tc.restype = ctypes.c_int
@@ -695,6 +722,97 @@ def debug_upsample_tc(x, w, bias, rate: int, flags: int, out_act, out_raw=None, 
                                       _ptr(out_raw), _ptr(out_f32), flags, ctypes.byref(img), x.device.index or 0),
           "vsg_debug_upsample_tc")
     return int(img.value)
+
+
+def debug_conv_f32_plan(Cout: int, k: int, dil: int):
+    """vsg_debug_conv_f32_plan (host only): (warps along channels, warps along time, dynamic shared memory bytes), or None
+    where the kernel refuses the shape (VSG_EUNSUPPORTED)."""
+    out = (ctypes.c_int32 * 3)()
+    rc = lib().vsg_debug_conv_f32_plan(Cout, k, dil, out)
+    if rc == -4:
+        return None
+    check(rc, "vsg_debug_conv_f32_plan")
+    return int(out[0]), int(out[1]), int(out[2])
+
+
+def debug_conv_f32(x, w, bias=None, *, B, Cin, Lin, Lq, Lout=None, x_bs=None, x_cs=None, dil=1, in_off0=None,
+                   pre_lrelu=0, slope=0.1, bcond=None, bcond_bs=0, out_stride=1, out_phase=0, epi=0, y=None, y_bs=None,
+                   y_cs=None, res=None, res_bs=None, res_cs=None, y2=None, y2_bs=None, y2_cs=None, mask=None, mask_bs=None,
+                   acc_mode=ACC_SET, acc_div=1.0, rs_split=0, y2_first=0, y2_mask=0, couple_sign=1, gate_interleave=0,
+                   check_rc=True):
+    """One launch of the fp32 convolution kernel through vsg_debug_conv_f32 (include/visinger_b200.h).  Tensors are flat
+    CUDA fp32 buffers addressed through the given strides (outputs written in place); strides default to a dense
+    [B, C, L] layout.  w [Cout, Cin, k] and bias [Cout] may live anywhere.  in_off0 defaults to -(k - 1) * dil / 2.
+    Returns ((warps along channels, warps along time), rc); raises on an error unless check_rc is False."""
+    for t in (x, bcond, res, mask, y, y2):
+        assert t is None or (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous())
+    Cout, wc, k = w.shape
+    assert wc == Cin
+    Lout = Lq if Lout is None else Lout
+    x_cs = Lin if x_cs is None else x_cs
+    x_bs = Cin * x_cs if x_bs is None else x_bs
+    ych = Cout // 2 if epi in (1, 4) else (rs_split if epi == 2 else Cout)
+    y_cs = Lout if y_cs is None else y_cs
+    y_bs = ych * y_cs if y_bs is None else y_bs
+    res_cs = Lout if res_cs is None else res_cs
+    res_bs = Cout * res_cs if res_bs is None else res_bs
+    y2_cs = Lout if y2_cs is None else y2_cs
+    y2_bs = (Cout - rs_split) * y2_cs if y2_bs is None else y2_bs
+    mask_bs = Lout if mask_bs is None else mask_bs
+    wh = w.detach().to("cpu", torch.float32).contiguous()
+    bh = bias.detach().to("cpu", torch.float32).contiguous() if bias is not None else None
+    d = VsgDebugConvF32(_ptr(x), wh.data_ptr(), _ptr(bh), _ptr(bcond), _ptr(res), _ptr(mask), _ptr(y), _ptr(y2),
+                        x_bs, y_bs, res_bs, y2_bs, x_cs, y_cs, res_cs, y2_cs, B, Cin, Lin, Cout, k, dil,
+                        -((k - 1) * dil // 2) if in_off0 is None else in_off0, pre_lrelu, slope, bcond_bs, mask_bs, Lq,
+                        out_stride, out_phase, Lout, epi, acc_mode, acc_div, rs_split, y2_first, y2_mask, couple_sign,
+                        gate_interleave)
+    tile = (ctypes.c_int32 * 2)()
+    dev = x.device if x is not None else torch.device("cuda", 0)
+    if dev.type == "cuda":
+        torch.cuda.synchronize(dev)
+    rc = lib().vsg_debug_conv_f32(ctypes.byref(d), tile, dev.index or 0)
+    if check_rc:
+        check(rc, "vsg_debug_conv_f32")
+    return (int(tile[0]), int(tile[1])), rc
+
+
+def debug_upsample_f32(x, w, bias, rate: int, y) -> None:
+    """The fp32 decoder's upsampler through vsg_debug_upsample_f32: x CUDA fp32 [B, Cin, Lin], w [Cin, Cout, k] (the
+    ConvTranspose1d weight) and bias [Cout] anywhere, y CUDA fp32 [B, Cout, Lin * rate] written in place."""
+    require_cuda(x, "x")
+    for t in (x, y):
+        assert t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()
+    Cin, Cout, k = w.shape
+    B, _, Lin = x.shape
+    wh = w.detach().to("cpu", torch.float32).contiguous()
+    bh = bias.detach().to("cpu", torch.float32).contiguous()
+    torch.cuda.synchronize(x.device)
+    check(lib().vsg_debug_upsample_f32(x.data_ptr(), wh.data_ptr(), bh.data_ptr(), Cin, Cout, rate, k, B, Lin, y.data_ptr(),
+                                       x.device.index or 0), "vsg_debug_upsample_f32")
+
+
+def debug_conv_post_f32(x, w, slope: float, n0: int, n1: int, wav, wav_ld: int) -> None:
+    """The fp32 conv_post through vsg_debug_conv_post_f32: x CUDA fp32 [B, C, L], w [C, k] anywhere; samples [n0, n1) of
+    utterance b are written to wav (flat CUDA fp32) at b * wav_ld."""
+    require_cuda(x, "x")
+    assert x.dtype == torch.float32 and x.is_contiguous() and wav.is_cuda and wav.is_contiguous()
+    B, C, L = x.shape
+    k = w.shape[-1]
+    wh = w.detach().to("cpu", torch.float32).reshape(C, k).contiguous()
+    torch.cuda.synchronize(x.device)
+    check(lib().vsg_debug_conv_post_f32(x.data_ptr(), wh.data_ptr(), C, L, k, float(slope), B, n0, n1, wav.data_ptr(),
+                                        int(wav_ld), x.device.index or 0), "vsg_debug_conv_post_f32")
+
+
+def debug_cond_f32(W, bias, g, out) -> None:
+    """The condition GEMV through vsg_debug_cond_f32: W [O, I], bias [O] or None, g [B, I], out [B, O], CUDA fp32."""
+    for t in (W, bias, g, out):
+        assert t is None or (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous())
+    O, I = W.shape
+    B = g.shape[0]
+    torch.cuda.synchronize(W.device)
+    check(lib().vsg_debug_cond_f32(W.data_ptr(), _ptr(bias), g.data_ptr(), out.data_ptr(), O, I, B, W.device.index or 0),
+          "vsg_debug_cond_f32")
 
 
 def debug_pair_bf16(xa_bld: torch.Tensor, w1, b1, w2, b2, d1: int, add0=None, add1=None, scale: float = 1.0,

@@ -10,7 +10,7 @@
 //     (decoder.py:45,55,93,97,126);
 //   * epi = the op the reference runs right after the conv: gate (encoder.py:206-213), residual/skip
 //     routing (encoder.py:188-194), coupling (flow.py:78,83), residual add / resblock mean (decoder.py:
-//     48-54,102), tanh (decoder.py:57);
+//     48-54,102);
 //   * MAG (template flag): channel pairs (re, im) -> sqrt(re^2 + im^2 + 1e-6) * mask, the linear spectrogram (spec.cuh).
 #pragma once
 #include <cuda_runtime.h>
@@ -40,7 +40,6 @@ struct ConvF32 {
   float* y2; long long y2_bs; int y2_cs;
   const float* mask; int mask_bs;     // [B, Lout] or null
   int acc_mode; float acc_div;
-  int do_tanh;
   int rs_split;      // EPI_RES_SKIP: channels [0, rs_split) update the state, the rest go to the skip sum
   int y2_first;      // EPI_RES_SKIP: skip sum is written, not accumulated (first layer)
   int y2_mask;       // EPI_RES_SKIP: multiply the skip sum by the mask (last layer)
@@ -161,7 +160,6 @@ __global__ void __launch_bounds__(256) conv_f32_kernel(const ConvF32 p) {
           float* yp = p.y + (long long)b * p.y_bs + (long long)co * p.y_cs + n;
           if (p.acc_mode == ACC_ADD) v = *yp + v;
           else if (p.acc_mode == ACC_ADD_DIV) v = (*yp + v) / p.acc_div;
-          if (p.do_tanh) v = tanhf(v);
           *yp = v;
         } else if (p.epi == EPI_RES_SKIP) {
           if (co < p.rs_split) {

@@ -78,37 +78,8 @@ struct Loader {
   }
 
   template <typename T>
-  int upload(const std::vector<T>& h, T** d) const {
-    void* p = nullptr;
-    VSG_CUDA_TRY(cudaMalloc(&p, h.size() * sizeof(T) + 256));
-    pack->allocs.push_back(p);
-    VSG_CUDA_TRY(cudaMemcpy(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice));
-    *d = (T*)p;
-    return VSG_OK;
-  }
+  int upload(const std::vector<T>& h, T** d) const { return vsg::upload(pack, h, d); }
 };
-
-inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
-
-// Conv1d weight W[co][ci][j] -> fp32 pack [ci][j][CoutP], output channel co stored at perm(co).
-template <typename Perm>
-int pack_conv_f32(const Loader& L, const std::vector<float>& W, const std::vector<float>& b, int Cout, int Cin, int k,
-                  Perm perm, ConvW32* out) {
-  out->Cin = Cin; out->Cout = Cout; out->ktaps = k; out->CoutP = round_up(Cout, 64);
-  std::vector<float> wp((size_t)Cin * k * out->CoutP, 0.f), bp(out->CoutP, 0.f);
-  for (int co = 0; co < Cout; ++co) {
-    const int pc = perm(co);
-    bp[pc] = b[co];
-    for (int ci = 0; ci < Cin; ++ci)
-      for (int j = 0; j < k; ++j) wp[((size_t)ci * k + j) * out->CoutP + pc] = W[((size_t)co * Cin + ci) * k + j];
-  }
-  VSG_TRY(L.upload(wp, &out->w));
-  VSG_TRY(L.upload(bp, &out->bias));
-  return VSG_OK;
-}
-
-struct Identity { int operator()(int c) const { return c; } };
-struct GateInterleave { int H; int operator()(int c) const { return c < H ? 2 * c : 2 * (c - H) + 1; } };
 
 int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
   const VsgConfig& c = P->cfg;
@@ -123,7 +94,7 @@ int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
     // pre: Conv1d(half -> H, 1)       flow.py:60
     VSG_TRY(L.eff_weight(p + "pre", H, half, 1, W));
     VSG_TRY(L.bias(p + "pre", H, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, H, half, 1, Identity{}, &fl.pre[0]));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, H, half, 1, Identity{}, &fl.pre[0]));
     VSG_TRY(pack_conv_tc(P, W, b, H, half, 1, &fl.pre_tc[0]));
     VSG_TRY(pack_conv_tc(P, W, b, H, half, 1, &fl.pre_x6[0], 3));
     auto zero_extend = [&](const std::vector<float>& Wi, const std::vector<float>& bi, int flipped) -> int {
@@ -139,7 +110,7 @@ int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
       std::vector<float> Wf(W.size());
       for (int co = 0; co < H; ++co)
         for (int ci = 0; ci < half; ++ci) Wf[(size_t)co * half + ci] = W[(size_t)co * half + (half - 1 - ci)];
-      VSG_TRY(pack_conv_f32(L, Wf, b, H, half, 1, Identity{}, &fl.pre[1]));
+      VSG_TRY(pack_conv_f32(L.pack, Wf, b, H, half, 1, Identity{}, &fl.pre[1]));
       VSG_TRY(pack_conv_tc(P, Wf, b, H, half, 1, &fl.pre_tc[1]));
       VSG_TRY(pack_conv_tc(P, Wf, b, H, half, 1, &fl.pre_x6[1], 3));
       VSG_TRY(zero_extend(Wf, b, 1));
@@ -147,7 +118,7 @@ int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
     // post: Conv1d(H -> half, 1)      flow.py:62 (mean_only)
     VSG_TRY(L.eff_weight(p + "post", half, H, 1, W));
     VSG_TRY(L.bias(p + "post", half, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, half, H, 1, Identity{}, &fl.post[0]));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, half, H, 1, Identity{}, &fl.post[0]));
     VSG_TRY(pack_conv_tc(P, W, b, half, H, 1, &fl.post_tc[0]));
     VSG_TRY(pack_conv_tc(P, W, b, half, H, 1, &fl.post_x6[0], 3));
     {
@@ -156,7 +127,7 @@ int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
         bf[co] = b[half - 1 - co];
         for (int ci = 0; ci < H; ++ci) Wf[(size_t)co * H + ci] = W[(size_t)(half - 1 - co) * H + ci];
       }
-      VSG_TRY(pack_conv_f32(L, Wf, bf, half, H, 1, Identity{}, &fl.post[1]));
+      VSG_TRY(pack_conv_f32(L.pack, Wf, bf, half, H, 1, Identity{}, &fl.post[1]));
       VSG_TRY(pack_conv_tc(P, Wf, bf, half, H, 1, &fl.post_tc[1]));
       VSG_TRY(pack_conv_tc(P, Wf, bf, half, H, 1, &fl.post_x6[1], 3));
     }
@@ -172,7 +143,7 @@ int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
       const std::string pi = p + "enc.in_layers." + std::to_string(i);
       VSG_TRY(L.eff_weight(pi, 2 * H, H, K, W));
       VSG_TRY(L.bias(pi, 2 * H, b, true));
-      VSG_TRY(pack_conv_f32(L, W, b, 2 * H, H, K, GateInterleave{H}, &fl.in_layers[i]));
+      VSG_TRY(pack_conv_f32(L.pack, W, b, 2 * H, H, K, GateInterleave{H}, &fl.in_layers[i]));
       {   // tensor-core pack: rows permuted so (tanh, sigmoid) halves of a channel sit in adjacent accumulator columns
         GateInterleave gi{H};
         std::vector<float> Wg(W.size()), bg(b.size());
@@ -187,7 +158,7 @@ int pack_flow(const Loader& L, const std::string& pre, VsgPack* P) {
       const std::string pr = p + "enc.res_skip_layers." + std::to_string(i);
       VSG_TRY(L.eff_weight(pr, rs, H, 1, W));
       VSG_TRY(L.bias(pr, rs, b, true));
-      VSG_TRY(pack_conv_f32(L, W, b, rs, H, 1, Identity{}, &fl.res_skip[i]));
+      VSG_TRY(pack_conv_f32(L.pack, W, b, rs, H, 1, Identity{}, &fl.res_skip[i]));
       if (i < NL - 1) {
         VSG_TRY(pack_conv_tc(P, W, b, 2 * H, H, 1, &fl.rs_tc[0][i]));
         VSG_TRY(pack_conv_tc(P, W, b, 2 * H, H, 1, &fl.rs_tc[1][i], 3));
@@ -238,7 +209,7 @@ int pack_enc(const Loader& L, const std::string& p, VsgPack* P) {
   std::vector<float> W, b;
   VSG_TRY(L.eff_weight(p + "pre", H, Cin, 1, W));
   VSG_TRY(L.bias(p + "pre", H, b, true));
-  VSG_TRY(pack_conv_f32(L, W, b, H, Cin, 1, Identity{}, &e.pre));
+  VSG_TRY(pack_conv_f32(L.pack, W, b, H, Cin, 1, Identity{}, &e.pre));
   e.in_pad = round_up(Cin, 64);
   for (int c0 = 0; c0 < e.in_pad; c0 += 1024) {   // tensor-core packs: slabs of <= 1024 (zero-padded) input channels
     const int cs = std::min(1024, e.in_pad - c0);
@@ -257,7 +228,7 @@ int pack_enc(const Loader& L, const std::string& p, VsgPack* P) {
     const std::string pi = p + "enc.in_layers." + std::to_string(i);
     VSG_TRY(L.eff_weight(pi, 2 * H, H, K, W));
     VSG_TRY(L.bias(pi, 2 * H, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, 2 * H, H, K, GateInterleave{H}, &fl.in_layers[i]));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, 2 * H, H, K, GateInterleave{H}, &fl.in_layers[i]));
     {
       GateInterleave gi{H};
       std::vector<float> Wg(W.size()), bg(b.size());
@@ -271,7 +242,7 @@ int pack_enc(const Loader& L, const std::string& p, VsgPack* P) {
     const std::string pr = p + "enc.res_skip_layers." + std::to_string(i);
     VSG_TRY(L.eff_weight(pr, rs, H, 1, W));
     VSG_TRY(L.bias(pr, rs, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, rs, H, 1, Identity{}, &fl.res_skip[i]));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, rs, H, 1, Identity{}, &fl.res_skip[i]));
     if (i < NL - 1) {
       std::vector<float> Wr(W.begin(), W.begin() + (size_t)H * H), br(b.begin(), b.begin() + H);
       std::vector<float> Ws(W.begin() + (size_t)H * H, W.end()), bs(b.begin() + H, b.end());
@@ -298,7 +269,7 @@ int pack_enc(const Loader& L, const std::string& p, VsgPack* P) {
   }
   VSG_TRY(L.eff_weight(p + "proj", 2 * Co, H, 1, W));
   VSG_TRY(L.bias(p + "proj", 2 * Co, b, true));
-  VSG_TRY(pack_conv_f32(L, W, b, 2 * Co, H, 1, Identity{}, &e.proj));
+  VSG_TRY(pack_conv_f32(L.pack, W, b, 2 * Co, H, 1, Identity{}, &e.proj));
   VSG_TRY(pack_conv_tc(P, W, b, 2 * Co, H, 1, &e.proj_tc));
   P->has_enc = true;
   return VSG_OK;
@@ -332,22 +303,22 @@ int pack_relenc(const Loader& L, const std::string& p, VsgPack* P, const char* p
       memcpy(&Wq[(size_t)s * H * H], W.data(), (size_t)H * H * sizeof(float));
       memcpy(&bq[(size_t)s * H], b.data(), (size_t)H * sizeof(float));
     }
-    VSG_TRY(pack_conv_f32(L, Wq, bq, 3 * H, H, 1, Identity{}, &l.qkv));
+    VSG_TRY(pack_conv_f32(L.pack, Wq, bq, 3 * H, H, 1, Identity{}, &l.qkv));
     VSG_TRY(pack_conv_tc(P, Wq, bq, 3 * H, H, 1, &l.qkv_tc));
     VSG_TRY(L.eff_weight(pa + "conv_o", H, H, 1, W));
     VSG_TRY(L.bias(pa + "conv_o", H, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, H, H, 1, Identity{}, &l.o));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, H, H, 1, Identity{}, &l.o));
     VSG_TRY(pack_conv_tc(P, W, b, H, H, 1, &l.o_tc));
     VSG_TRY(vec(pa + "emb_rel_k", (int64_t)nrel * dk, &l.ek));      // heads_share = True: [1][2w+1][dk]
     VSG_TRY(vec(pa + "emb_rel_v", (int64_t)nrel * dk, &l.ev));
     const std::string pf = p + "ffn_layers." + std::to_string(i) + ".";
     VSG_TRY(L.eff_weight(pf + "conv_1", F, H, K, W));
     VSG_TRY(L.bias(pf + "conv_1", F, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, F, H, K, Identity{}, &l.ffn1));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, F, H, K, Identity{}, &l.ffn1));
     VSG_TRY(pack_conv_tc(P, W, b, F, H, K, &l.ffn1_tc));
     VSG_TRY(L.eff_weight(pf + "conv_2", H, F, 1, W));
     VSG_TRY(L.bias(pf + "conv_2", H, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, H, F, 1, Identity{}, &l.ffn2));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, H, F, 1, Identity{}, &l.ffn2));
     VSG_TRY(pack_conv_tc(P, W, b, H, F, 1, &l.ffn2_tc));
     VSG_TRY(vec(p + "norm_layers_1." + std::to_string(i) + ".gamma", H, &l.g1));
     VSG_TRY(vec(p + "norm_layers_1." + std::to_string(i) + ".beta", H, &l.b1));
@@ -357,7 +328,7 @@ int pack_relenc(const Loader& L, const std::string& p, VsgPack* P, const char* p
   if (e.gin > 0) {
     VSG_TRY(L.eff_weight(p + "pre_net", H, e.gin, 1, W));
     VSG_TRY(L.bias(p + "pre_net", H, b, true));
-    VSG_TRY(pack_conv_f32(L, W, b, H, e.gin, 1, Identity{}, &e.pre_net));
+    VSG_TRY(pack_conv_f32(L.pack, W, b, H, e.gin, 1, Identity{}, &e.pre_net));
     VSG_TRY(L.upload(W, &e.pre_w));
     VSG_TRY(L.upload(b, &e.pre_b));
   }
@@ -383,7 +354,7 @@ int pack_decoder(const Loader& L, const std::string& pre, VsgPack* P) {
   // conv_pre: Conv1d(C0 -> UIC, 7, padding 3), no weight norm   decoder.py:19
   VSG_TRY(L.eff_weight(pre + "conv_pre", UIC, C0, 7, W));
   VSG_TRY(L.bias(pre + "conv_pre", UIC, b, true));
-  VSG_TRY(pack_conv_f32(L, W, b, UIC, C0, 7, Identity{}, &P->conv_pre));
+  VSG_TRY(pack_conv_f32(L.pack, W, b, UIC, C0, 7, Identity{}, &P->conv_pre));
   VSG_TRY(pack_conv_tc(P, W, b, UIC, C0, 7, &P->conv_pre_tc));
   VSG_TRY(pack_conv_tc(P, W, b, UIC, C0, 7, &P->conv_pre_x3, 2));
   if (c.dec_gin > 0) {   // cond: Conv1d(gin -> UIC, 1)            decoder.py:37-38
@@ -414,7 +385,7 @@ int pack_decoder(const Loader& L, const std::string& pre, VsgPack* P) {
     std::vector<std::vector<float>> phase_w;
     VSG_TRY(pack_upsampler(P, W, b, st.Cin, st.Cout, st.rate, st.kernel, &st, &phase_w));
     for (int r = 0; r < st.rate; ++r)
-      VSG_TRY(pack_conv_f32(L, phase_w[r], b, st.Cout, st.Cin, (int)(phase_w[r].size() / ((size_t)st.Cout * st.Cin)), Identity{},
+      VSG_TRY(pack_conv_f32(L.pack, phase_w[r], b, st.Cout, st.Cin, (int)(phase_w[r].size() / ((size_t)st.Cout * st.Cin)), Identity{},
                             &st.phases[r].f32));
     // resblocks                                                            decoder.py:28-32
     st.blocks.resize(c.dec_n_kernels);
@@ -434,7 +405,7 @@ int pack_decoder(const Loader& L, const std::string& pre, VsgPack* P) {
         const std::string n1 = pb + (c.dec_resblock == 1 ? "convs1." : "convs.") + std::to_string(q);
         VSG_TRY(L.eff_weight(n1, ch, ch, rb.kernel, W));
         VSG_TRY(L.bias(n1, ch, b, true));
-        VSG_TRY(pack_conv_f32(L, W, b, ch, ch, rb.kernel, Identity{}, &rb.c1[q]));
+        VSG_TRY(pack_conv_f32(L.pack, W, b, ch, ch, rb.kernel, Identity{}, &rb.c1[q]));
         VSG_TRY(pack_conv_tc(P, W, b, ch, ch, rb.kernel, &rb.c1_tc[q]));
         VSG_TRY(pack_conv_tc(P, W, b, ch, ch, rb.kernel, &rb.c1_x3[q], 2));
         if (c.dec_resblock == 1 && rb.dilations[q] == 1) {
@@ -445,7 +416,7 @@ int pack_decoder(const Loader& L, const std::string& pre, VsgPack* P) {
           const std::string n2 = pb + "convs2." + std::to_string(q);
           VSG_TRY(L.eff_weight(n2, ch, ch, rb.kernel, W));
           VSG_TRY(L.bias(n2, ch, b, true));
-          VSG_TRY(pack_conv_f32(L, W, b, ch, ch, rb.kernel, Identity{}, &rb.c2[q]));
+          VSG_TRY(pack_conv_f32(L.pack, W, b, ch, ch, rb.kernel, Identity{}, &rb.c2[q]));
           VSG_TRY(pack_conv_tc(P, W, b, ch, ch, rb.kernel, &rb.c2_tc[q]));
           VSG_TRY(pack_conv_tc(P, W, b, ch, ch, rb.kernel, &rb.c2_x3[q], 2));
           VSG_TRY(pack_conv_rowpacked(P, W, ch, rb.kernel, &rb.c2_rp[q]));

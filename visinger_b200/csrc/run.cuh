@@ -100,6 +100,36 @@ int widen_bf16(const __nv_bfloat16* x, float* y, int B, int C, int ld, int T, cu
 int posterior_core_tc(const VsgPack* P, const __nv_bfloat16* u, const float* mask, const float* g, const float* noise,
                       float* z, float* stats, int B, int T, Workspace& ws, cudaStream_t st);
 
+// The per-launch test hooks' scope: a throw-away pack on `device` (weights, an error flag for the tensor-core kernels),
+// freed on exit; finish() synchronises and reports a failed kernel (named `what`) or a set error flag.
+struct DebugScope {
+  VsgPack P;
+  int* err = nullptr;
+  int open(int device) {
+    VSG_CUDA_TRY(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    VSG_CUDA_TRY(cudaGetDeviceProperties(&prop, device));
+    P.device = device;
+    P.sm_count = prop.multiProcessorCount;
+    VSG_CUDA_TRY(cudaMalloc(&err, sizeof(int)));
+    VSG_CUDA_TRY(cudaMemset(err, 0, sizeof(int)));
+    return VSG_OK;
+  }
+  int finish(int rc, const char* what = "conv_tc_kernel") {
+    if (rc != VSG_OK) return rc;
+    cudaError_t ce = cudaDeviceSynchronize();
+    if (ce != cudaSuccess) return fail(VSG_ECUDA, "%s execution failed: %s", what, cudaGetErrorString(ce));
+    int h = 0;
+    VSG_CUDA_TRY(cudaMemcpy(&h, err, sizeof(int), cudaMemcpyDeviceToHost));
+    if (h) return fail(VSG_ECUDA, "%s set its error flag (%d)", what, h);
+    return VSG_OK;
+  }
+  ~DebugScope() {
+    if (err) cudaFree(err);
+    for (void* q : P.allocs) cudaFree(q);
+  }
+};
+
 // vsg_infer_zp after validation (api.cu): flow reverse from z_p, mask, decoder; shared with vsg_model_forward
 int infer_zp_run(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav, float* z_q_out,
                  int B, int T, int precision, Workspace& ws, cudaStream_t st);

@@ -3,35 +3,47 @@
 #include "kernels_f32.cuh"
 #include "relenc_f32.cuh"
 #include "run.cuh"
+#include "pack_tc.cuh"
 #include "spec.cuh"
 
 namespace vsg {
 
+// The tile configuration of conv_f32_kernel for Cout output channels (8 warps: WARPS_CO x WARPS_Q, each 8 channels x 256
+// rows) and its dynamic shared memory for k taps at dilation dil: a [8][Q_TILE + halo] input window and the [8][k][CO_TILE]
+// weights of one 8-channel chunk.  VSG_EUNSUPPORTED above 200 KB.  The launcher and vsg_debug_conv_f32_plan both use it.
+int conv_f32_plan(int Cout, int ktaps, int dil, int* warps_co, int* warps_q, size_t* smem) {
+  if (ktaps < 1) return fail(VSG_EUNSUPPORTED, "convolution with no taps");
+  const int wc = Cout <= 16 ? 2 : Cout <= 32 ? 4 : 8, wq = 8 / wc;
+  const size_t sm = (size_t)F32_CI_CHUNK * ((256 * wq + (size_t)(ktaps - 1) * dil) + (size_t)ktaps * 8 * wc) * sizeof(float);
+  if (sm > 200 * 1024) return fail(VSG_EUNSUPPORTED, "conv window too large for shared memory (%zu B)", sm);
+  *warps_co = wc; *warps_q = wq; *smem = sm;
+  return VSG_OK;
+}
+
 namespace {
 
-template <bool MAG = false>
-int launch_conv_f32(const ConvF32& p, int B, cudaStream_t st) {
-  if (p.ktaps < 1) return fail(VSG_EUNSUPPORTED, "convolution with no taps");
-  const int halo = (p.ktaps - 1) * p.dil;
-  auto smem_for = [&](int co_tile, int q_tile) {
-    return (size_t)F32_CI_CHUNK * ((q_tile + halo) + p.ktaps * co_tile) * sizeof(float);
-  };
-#define VSG_F32_LAUNCH(WC, WQ)                                                                              \
-  do {                                                                                                      \
-    const size_t sm = smem_for(8 * WC, 256 * WQ);                                                           \
-    if (sm > 200 * 1024) return fail(VSG_EUNSUPPORTED, "conv window too large for shared memory (%zu B)", sm); \
-    if (sm > 48 * 1024)                                                                                     \
-      VSG_CUDA_TRY(cudaFuncSetAttribute(conv_f32_kernel<WC, WQ, MAG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)); \
-    dim3 grid((p.Lq + 256 * WQ - 1) / (256 * WQ), (p.Cout + 8 * WC - 1) / (8 * WC), B);                     \
-    conv_f32_kernel<WC, WQ, MAG><<<grid, 256, sm, st>>>(p);                                                 \
-    VSG_LAUNCH_CHECK("conv_f32_kernel");                                                                    \
-  } while (0)
-  if (p.Lq <= 0) return VSG_OK;
-  if (p.Cout <= 16) VSG_F32_LAUNCH(2, 4);
-  else if (p.Cout <= 32) VSG_F32_LAUNCH(4, 2);
-  else VSG_F32_LAUNCH(8, 1);
-#undef VSG_F32_LAUNCH
+template <int WC, int WQ, bool MAG>
+int launch_conv_f32_tile(const ConvF32& p, int B, size_t sm, cudaStream_t st) {
+  if (sm > 48 * 1024)
+    VSG_CUDA_TRY(cudaFuncSetAttribute(conv_f32_kernel<WC, WQ, MAG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  dim3 grid((p.Lq + 256 * WQ - 1) / (256 * WQ), (p.Cout + 8 * WC - 1) / (8 * WC), B);
+  conv_f32_kernel<WC, WQ, MAG><<<grid, 256, sm, st>>>(p);
+  VSG_LAUNCH_CHECK("conv_f32_kernel");
   return VSG_OK;
+}
+
+// tile_out (optional): the (WARPS_CO, WARPS_Q) configuration launched.
+template <bool MAG = false>
+int launch_conv_f32(const ConvF32& p, int B, cudaStream_t st, int* tile_out = nullptr) {
+  if (p.ktaps < 1) return fail(VSG_EUNSUPPORTED, "convolution with no taps");
+  if (p.Lq <= 0) return VSG_OK;
+  int wc = 0, wq = 0;
+  size_t sm = 0;
+  VSG_TRY(conv_f32_plan(p.Cout, p.ktaps, p.dil, &wc, &wq, &sm));
+  if (tile_out) { tile_out[0] = wc; tile_out[1] = wq; }
+  if (wc == 2) return launch_conv_f32_tile<2, 4, MAG>(p, B, sm, st);
+  if (wc == 4) return launch_conv_f32_tile<4, 2, MAG>(p, B, sm, st);
+  return launch_conv_f32_tile<8, 1, MAG>(p, B, sm, st);
 }
 
 ConvF32 base_conv(const ConvW32& w, const float* x, long long x_bs, int x_cs, int Lin, int in_off0, int dil) {
@@ -381,6 +393,33 @@ size_t dec_ws_bytes_f32(const VsgPack* P, int B, int T) {
          4 * align256(dec_max_elems(P, B, T) * sizeof(float));
 }
 
+// y [B, Cout, Lin * rate] = ConvTranspose1d(leaky_relu(x [B, Cin, Lin], 0.1)) + bias (decoder.py:45-46) as `rate` polyphase
+// convolutions over the input rate, each writing every rate-th output sample.
+int launch_upsample_f32(const UpStage& us, const float* x, int B, int Lin, float* y, cudaStream_t st) {
+  const int Lout = Lin * us.rate;
+  for (int r = 0; r < us.rate; ++r) {
+    ConvF32 p = base_conv(us.phases[r].f32, x, (long long)us.Cin * Lin, Lin, Lin, us.phases[r].in_off0, 1);
+    p.pre_lrelu = 1;
+    p.Lq = (Lout - r + us.rate - 1) / us.rate; p.out_stride = us.rate; p.out_phase = r; p.Lout = Lout;
+    p.y = y; p.y_bs = (long long)us.Cout * Lout; p.y_cs = Lout;
+    VSG_TRY(launch_conv_f32(p, B, st));
+  }
+  return VSG_OK;
+}
+
+// wav = tanh(conv_post(leaky_relu(x [B, C, L], slope)))  (decoder.py:55-57; w [C][k] on the device, no bias): samples
+// [n0, n1) of utterance b go to wav + b * wav_ld.
+int launch_conv_post_f32(const float* x, const float* w, float* wav, int B, int C, int L, int k, float slope, int n0, int n1,
+                         long long wav_ld, cudaStream_t st) {
+  const size_t sm = (size_t)C * k * sizeof(float);
+  if (sm > 48 * 1024) return fail(VSG_EUNSUPPORTED, "conv_post weights exceed 48 KB of shared memory (%zu B)", sm);
+  if (n1 <= n0) return VSG_OK;
+  dim3 grid((n1 - n0 + 255) / 256, B);
+  conv_post_f32_kernel<<<grid, 256, sm, st>>>(x, w, wav, C, L, k, slope, n0, n1, wav_ld);
+  VSG_LAUNCH_CHECK("conv_post_f32_kernel");
+  return VSG_OK;
+}
+
 // Generator.forward, modules/visinger/decoder.py:40-59.
 int generator_forward_f32(const VsgPack* P, const float* z, const float* g, float* wav, int B, int T, Workspace& ws,
                           cudaStream_t st, const DecWin* win) {
@@ -409,14 +448,7 @@ int generator_forward_f32(const VsgPack* P, const float* z, const float* g, floa
   for (int i = 0; i < c.dec_n_ups; ++i) {
     const UpStage& us = P->ups[i];
     const int Lout = L * us.rate;
-    // x = ups[i](leaky_relu(x))  as `rate` polyphase convolutions    decoder.py:45-46
-    for (int r = 0; r < us.rate; ++r) {
-      ConvF32 p = base_conv(us.phases[r].f32, bufS, (long long)ch * L, L, L, us.phases[r].in_off0, 1);
-      p.pre_lrelu = 1;
-      p.Lq = (Lout - r + us.rate - 1) / us.rate; p.out_stride = us.rate; p.out_phase = r; p.Lout = Lout;
-      p.y = bufU; p.y_bs = (long long)us.Cout * Lout; p.y_cs = Lout;
-      VSG_TRY(launch_conv_f32(p, B, st));
-    }
+    VSG_TRY(launch_upsample_f32(us, bufS, B, L, bufU, st));   // x = ups[i](leaky_relu(x))   decoder.py:45-46
     ch = us.Cout; L = Lout;
     const long long bs = (long long)ch * L;
     // xs = sum_j resblock_j(x) ; x = xs / NK                           decoder.py:47-54
@@ -452,14 +484,8 @@ int generator_forward_f32(const VsgPack* P, const float* z, const float* g, floa
     if (NK == 1) { /* xs / 1 == xs */ }
   }
   // wav = tanh(conv_post(leaky_relu(x)))                               decoder.py:55-57
-  {
-    const int n0 = win ? win->s0 : 0, n1 = win ? win->s1 : L;
-    dim3 grid((n1 - n0 + 255) / 256, B);
-    conv_post_f32_kernel<<<grid, 256, (size_t)ch * P->conv_post_k * sizeof(float), st>>>(
-        bufS, P->conv_post_w, wav, ch, L, P->conv_post_k, 0.1f, n0, n1, win ? win->wav_ld : (long long)L);
-    VSG_LAUNCH_CHECK("conv_post_f32_kernel");
-  }
-  return VSG_OK;
+  return launch_conv_post_f32(bufS, P->conv_post_w, wav, B, ch, L, P->conv_post_k, 0.1f, win ? win->s0 : 0,
+                              win ? win->s1 : L, win ? win->wav_ld : (long long)L, st);
 }
 
 int prior_sample(const float* mu, const float* logs, const float* noise, const float* mask, float* z, int B, int C,
@@ -493,4 +519,123 @@ extern "C" int vsg_debug_attention_f32(const float* qkv, const float* mask, cons
   const cudaError_t ce = cudaDeviceSynchronize();
   if (ce != cudaSuccess) return fail(VSG_ECUDA, "relenc_attention_f32_kernel execution failed: %s", cudaGetErrorString(ce));
   return VSG_OK;
+}
+
+// One launch of conv_f32_kernel with every ConvF32 field (tests only; allocates and synchronises).  See include/visinger_b200.h.
+extern "C" int vsg_debug_conv_f32(const VsgDebugConvF32* d, int32_t* tile_out, int32_t device) {
+  using namespace vsg;
+  reset_launch_counts();
+  if (!d || !d->x || !d->w) return fail(VSG_EINVAL, "vsg_debug_conv_f32: null descriptor, input or weight");
+  if (d->epi < EPI_LINEAR || d->epi > VSG_DEBUG_F32_MAG) return fail(VSG_EINVAL, "vsg_debug_conv_f32: epi must be 0 .. 4");
+  if (d->B <= 0 || d->Cin <= 0 || d->Lin <= 0 || d->Cout <= 0 || d->k <= 0 || d->dil <= 0 || d->Lq <= 0 || d->Lout <= 0 ||
+      d->out_stride <= 0 || d->out_phase < 0 || d->out_phase >= d->out_stride ||
+      (long long)(d->Lq - 1) * d->out_stride + d->out_phase >= d->Lout)
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: bad shape or output geometry");
+  const bool pairs = d->epi == EPI_GATE || d->epi == VSG_DEBUG_F32_MAG;
+  if (pairs && d->Cout % 2) return fail(VSG_EINVAL, "vsg_debug_conv_f32: gate and magnitude need an even Cout");
+  if (d->gate_interleave && d->epi != EPI_GATE) return fail(VSG_EINVAL, "vsg_debug_conv_f32: gate_interleave is for the gate");
+  if (d->x_cs < d->Lin || d->x_bs < (long long)d->Cin * d->x_cs)
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: x rows overlap (x_cs < Lin or x_bs < Cin * x_cs)");
+  if (d->mask && d->mask_bs < d->Lout) return fail(VSG_EINVAL, "vsg_debug_conv_f32: mask_bs < Lout");
+  if (d->bcond && d->bcond_bs < d->Cout) return fail(VSG_EINVAL, "vsg_debug_conv_f32: bcond_bs < Cout");
+  if (d->acc_mode < ACC_SET || d->acc_mode > ACC_ADD_DIV || (d->acc_mode != ACC_SET && d->epi != EPI_LINEAR) ||
+      (d->acc_mode == ACC_ADD_DIV && d->acc_div == 0.f))
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: acc_mode must be 0, 1 or 2 (linear only), acc_div nonzero");
+  if (d->res && (d->epi != EPI_LINEAR && d->epi != EPI_COUPLE))
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: res is read by the linear and couple epilogues only");
+  if (d->res && (d->res_cs < d->Lout || d->res_bs < (long long)d->Cout * d->res_cs))
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: res rows overlap (res_cs < Lout or res_bs < Cout * res_cs)");
+  if (d->epi == EPI_COUPLE && d->couple_sign != 1 && d->couple_sign != -1)
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: couple_sign must be +1 or -1");
+  const bool rs = d->epi == EPI_RES_SKIP;
+  if (rs && (d->rs_split < 0 || d->rs_split > d->Cout)) return fail(VSG_EINVAL, "vsg_debug_conv_f32: rs_split outside 0 .. Cout");
+  const int y_ch = rs ? d->rs_split : pairs ? d->Cout / 2 : d->Cout, y2_ch = rs ? d->Cout - d->rs_split : 0;
+  if (y_ch > 0 && (!d->y || d->y_cs < d->Lout || d->y_bs < (long long)y_ch * d->y_cs))
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: y missing or its rows overlap");
+  if (y2_ch > 0 && (!d->y2 || d->y2_cs < d->Lout || d->y2_bs < (long long)y2_ch * d->y2_cs))
+    return fail(VSG_EINVAL, "vsg_debug_conv_f32: y2 missing or its rows overlap");
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  std::vector<float> W(d->w, d->w + (size_t)d->Cout * d->Cin * d->k), bz(d->Cout, 0.f);
+  if (d->bias) bz.assign(d->bias, d->bias + d->Cout);
+  ConvW32 wt;
+  if (d->gate_interleave) VSG_TRY(pack_conv_f32(&sc.P, W, bz, d->Cout, d->Cin, d->k, GateInterleave{d->Cout / 2}, &wt));
+  else VSG_TRY(pack_conv_f32(&sc.P, W, bz, d->Cout, d->Cin, d->k, Identity{}, &wt));
+  ConvF32 p = base_conv(wt, d->x, d->x_bs, d->x_cs, d->Lin, d->in_off0, d->dil);
+  p.pre_lrelu = d->pre_lrelu; p.slope = d->slope;
+  p.bias = d->bias ? wt.bias : nullptr;
+  p.bcond = d->bcond; p.bcond_bs = d->bcond_bs;
+  p.Lq = d->Lq; p.out_stride = d->out_stride; p.out_phase = d->out_phase; p.Lout = d->Lout;
+  p.epi = d->epi == VSG_DEBUG_F32_MAG ? EPI_LINEAR : d->epi;
+  p.y = d->y; p.y_bs = d->y_bs; p.y_cs = d->y_cs;
+  p.res = d->res; p.res_bs = d->res_bs; p.res_cs = d->res_cs;
+  p.y2 = d->y2; p.y2_bs = d->y2_bs; p.y2_cs = d->y2_cs;
+  p.mask = d->mask; p.mask_bs = d->mask_bs;
+  p.acc_mode = d->acc_mode; p.acc_div = d->acc_div;
+  p.rs_split = d->rs_split; p.y2_first = d->y2_first; p.y2_mask = d->y2_mask;
+  p.couple_sign = d->couple_sign;
+  int tile[2] = {0, 0};
+  const int rc = d->epi == VSG_DEBUG_F32_MAG ? launch_conv_f32<true>(p, d->B, 0, tile) : launch_conv_f32(p, d->B, 0, tile);
+  if (tile_out) { tile_out[0] = tile[0]; tile_out[1] = tile[1]; }
+  return sc.finish(rc, "conv_f32_kernel");
+}
+
+// Host only: conv_f32_plan.  See include/visinger_b200.h.
+extern "C" int vsg_debug_conv_f32_plan(int32_t Cout, int32_t k, int32_t dil, int32_t* out) {
+  using namespace vsg;
+  if (!out || Cout <= 0 || k <= 0 || dil <= 0) return fail(VSG_EINVAL, "vsg_debug_conv_f32_plan: bad argument");
+  int wc = 0, wq = 0;
+  size_t sm = 0;
+  VSG_TRY(conv_f32_plan(Cout, k, dil, &wc, &wq, &sm));
+  out[0] = wc; out[1] = wq; out[2] = (int32_t)sm;
+  return VSG_OK;
+}
+
+// The decoder's upsampler as generator_forward_f32 runs it (tests only; allocates and synchronises).
+extern "C" int vsg_debug_upsample_f32(const float* x, const float* w, const float* bias, int32_t Cin, int32_t Cout, int32_t rate,
+                                      int32_t k, int32_t B, int32_t Lin, float* y, int32_t device) {
+  using namespace vsg;
+  reset_launch_counts();
+  if (!x || !w || !bias || !y) return fail(VSG_EINVAL, "vsg_debug_upsample_f32: null input, weight, bias or output");
+  if (Cin <= 0 || Cout <= 0 || B <= 0 || Lin <= 0 || rate <= 0 || k < rate || (k - rate) % 2)
+    return fail(VSG_EINVAL, "vsg_debug_upsample_f32: bad shape (needs k >= rate and k - rate even)");
+  if ((long long)Lin * rate >= (1LL << 31)) return fail(VSG_EINVAL, "vsg_debug_upsample_f32: output too long");
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  UpStage us;
+  std::vector<float> W(w, w + (size_t)Cin * Cout * k), b(bias, bias + Cout);
+  std::vector<std::vector<float>> phase_w;
+  VSG_TRY(pack_upsampler(&sc.P, W, b, Cin, Cout, rate, k, &us, &phase_w));
+  for (int r = 0; r < rate; ++r)
+    VSG_TRY(pack_conv_f32(&sc.P, phase_w[r], b, Cout, Cin, (int)(phase_w[r].size() / ((size_t)Cout * Cin)), Identity{},
+                          &us.phases[r].f32));
+  return sc.finish(launch_upsample_f32(us, x, B, Lin, y, 0), "conv_f32_kernel");
+}
+
+// conv_post_f32_kernel through the generator's launcher (tests only; allocates and synchronises).
+extern "C" int vsg_debug_conv_post_f32(const float* x, const float* w, int32_t C, int32_t L, int32_t k, float slope, int32_t B,
+                                       int32_t n0, int32_t n1, float* wav, int64_t wav_ld, int32_t device) {
+  using namespace vsg;
+  reset_launch_counts();
+  if (!x || !w || !wav) return fail(VSG_EINVAL, "vsg_debug_conv_post_f32: null input, weight or output");
+  if (C <= 0 || L <= 0 || k <= 0 || B <= 0 || n0 < 0 || n1 <= n0 || n1 > L || wav_ld < n1 - n0)
+    return fail(VSG_EINVAL, "vsg_debug_conv_post_f32: bad shape or window (needs 0 <= n0 < n1 <= L, wav_ld >= n1 - n0)");
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  float* dw = nullptr;
+  VSG_TRY(upload(&sc.P, std::vector<float>(w, w + (size_t)C * k), &dw));
+  return sc.finish(launch_conv_post_f32(x, dw, wav, B, C, L, k, slope, n0, n1, wav_ld, 0), "conv_post_f32_kernel");
+}
+
+// launch_cond (cond_gemv_kernel) (tests only; synchronises).
+extern "C" int vsg_debug_cond_f32(const float* W, const float* bias, const float* g, float* out, int32_t O, int32_t I, int32_t B,
+                                  int32_t device) {
+  using namespace vsg;
+  reset_launch_counts();
+  if (!W || !g || !out) return fail(VSG_EINVAL, "vsg_debug_cond_f32: null weight, input or output");
+  if (O <= 0 || I <= 0 || B <= 0 || (long long)O * B * 32 >= (1LL << 31))
+    return fail(VSG_EINVAL, "vsg_debug_cond_f32: bad shape");
+  DebugScope sc;
+  VSG_TRY(sc.open(device));
+  return sc.finish(launch_cond(W, bias, g, out, O, I, B, 0), "cond_gemv_kernel");
 }

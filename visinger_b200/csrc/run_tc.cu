@@ -2085,36 +2085,6 @@ extern "C" int vsg_debug_conv1d_bf16(const void* x_bf16, const float* w, const f
 
 // One launch of conv_tc_kernel with every EpiTC field and every output geometry (tests only; allocates and synchronises).
 // See include/visinger_b200.h.
-namespace {
-struct DebugScope {   // a throw-away pack on `device` (weights, error flag), freed on exit
-  VsgPack P;
-  int* err = nullptr;
-  int open(int device) {
-    VSG_CUDA_TRY(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    VSG_CUDA_TRY(cudaGetDeviceProperties(&prop, device));
-    P.device = device;
-    P.sm_count = prop.multiProcessorCount;
-    VSG_CUDA_TRY(cudaMalloc(&err, sizeof(int)));
-    VSG_CUDA_TRY(cudaMemset(err, 0, sizeof(int)));
-    return VSG_OK;
-  }
-  int finish(int rc) {
-    if (rc != VSG_OK) return rc;
-    cudaError_t ce = cudaDeviceSynchronize();
-    if (ce != cudaSuccess) return fail(VSG_ECUDA, "conv_tc_kernel execution failed: %s", cudaGetErrorString(ce));
-    int h = 0;
-    VSG_CUDA_TRY(cudaMemcpy(&h, err, sizeof(int), cudaMemcpyDeviceToHost));
-    if (h) return fail(VSG_ECUDA, "conv_tc_kernel set its error flag (%d)", h);
-    return VSG_OK;
-  }
-  ~DebugScope() {
-    if (err) cudaFree(err);
-    for (void* q : P.allocs) cudaFree(q);
-  }
-};
-}  // namespace
-
 extern "C" int vsg_debug_conv_tc(const VsgDebugConv* d, int32_t* image_out, int32_t device) {
   reset_launch_counts();
   if (!d || !d->x || !d->w) return fail(VSG_EINVAL, "vsg_debug_conv_tc: null descriptor, input or weight");
