@@ -419,6 +419,37 @@ int vsg_model_convert(const VsgPack* pack, const float* wav, const float* spec, 
                       size_t workspace_bytes, void* stream);
 
 /*
+ * Streaming voice conversion: frames [t0, t1) of vsg_model_convert(wav, spec = NULL, ...) BIT FOR BIT, with a workspace
+ * that does not grow with T.  Voice conversion has no attention: the spectrogram, the posterior's WaveNet, the flow (both
+ * directions) and the decoder all have finite receptive fields, so a window of output frames depends on a bounded
+ * stretch of input audio only.  A recording of any length converts in bounded memory, and audio that is still arriving
+ * converts with a fixed look-ahead.  The decoder runs over [da, db) = the window plus Cd frames each side (widened for
+ * the whole batch's kernel choices as in vsg_infer_zp_window), the flow reverse over [da - Cf, db + Cf), the flow
+ * forward over [da - 2 Cf, db + 2 Cf), the spectrogram and the posterior over [da - 2 Cf - Cp, db + 2 Cf + Cp), all
+ * clipped to [0, T) (DESIGN.md section 4.9).  Windows may come in any order; no state is kept between them.
+ */
+/* Context frames each side of a voice-conversion window: the posterior encoder's, the flow's (each direction) and the
+ * decoder's receptive fields in latent frames.  Host only. */
+int vsg_convert_window_context(const VsgPack* pack, int32_t* post_frames, int32_t* flow_frames, int32_t* dec_frames);
+/* Host only.  The input that window [t0, t1) of a (B, T) batch reads: samples [*s0, *s1) of each utterance's row of wav,
+ * with *s1 widened to cover every frame whose mask the window uses.  The window's result does not depend on samples
+ * outside that span, and is the same for every lengths[b] with lengths[b] * hop >= *s1.  A live caller can emit
+ * frames [t0, t1) as soon as samples [0, *s1) have arrived. */
+int vsg_convert_window_input(const VsgPack* pack, int32_t B, int32_t T, int32_t t0, int32_t t1, int32_t precision,
+                             int64_t* s0, int64_t* s1);
+/* Does not grow with T.  0 on invalid arguments. */
+size_t vsg_convert_window_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t max_frames, int32_t precision);
+/* Frames [t0, t1) of vsg_model_convert(wav, spec = NULL, ...) bit for bit: wav_out row b at wav_out + b * wav_ld receives
+ * samples [t0 * hop, t1 * hop); z_out: NULL or fp32 [B, hidden, t1 - t0] (z_hat).  wav [B, T * hop], lengths, noise
+ * [B, hidden, T] are read in place; seeds / speaker arguments as in vsg_model_convert.  Argument and workspace rules of
+ * vsg_infer_zp_window (VSG_EINVAL / VSG_ENOMEM before any launch); no allocation, no synchronisation, capturable. */
+int vsg_model_convert_window(const VsgPack* pack, const float* wav, const int32_t* lengths,
+                             const int64_t* src_spk_id, const float* src_spk_embed, const int64_t* tgt_spk_id,
+                             const float* tgt_spk_embed, const float* noise, const uint64_t* seeds, float* wav_out,
+                             int64_t wav_ld, float* z_out, int32_t B, int32_t T, int32_t t0, int32_t t1,
+                             int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * Seeded standard-normal noise, out: fp32 [B, C, T].  Element (b, c, t) is Box-Muller on one Philox4x32-10 draw with
  * key (lo32(seeds[b]), hi32(seeds[b])) and counter (t, c, 0, 0): with x0, x1 its first two words,
  *   u1 = (x0 + 1) / 2^32,  u2 = x1 / 2^32,  out = fp32( sqrt(-2 ln u1) * cos(2 pi u2) )   (evaluated in double)

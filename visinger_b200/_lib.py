@@ -322,6 +322,16 @@ def lib() -> ctypes.CDLL:
         L.vsg_infer_zp_window.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int64, vp, i32, i32, i32, i32, i32, vp, sz, vp]
         L.vsg_generator_forward_window.restype = ctypes.c_int
         L.vsg_generator_forward_window.argtypes = [vp, vp, vp, vp, ctypes.c_int64, i32, i32, i32, i32, i32, vp, sz, vp]
+        L.vsg_convert_window_context.restype = ctypes.c_int
+        L.vsg_convert_window_context.argtypes = [vp] + [ctypes.POINTER(ctypes.c_int32)] * 3
+        L.vsg_convert_window_input.restype = ctypes.c_int
+        L.vsg_convert_window_input.argtypes = [vp, i32, i32, i32, i32, i32, ctypes.POINTER(ctypes.c_int64),
+                                               ctypes.POINTER(ctypes.c_int64)]
+        L.vsg_convert_window_workspace_bytes.restype = sz
+        L.vsg_convert_window_workspace_bytes.argtypes = [vp, i32, i32, i32, i32]
+        L.vsg_model_convert_window.restype = ctypes.c_int
+        L.vsg_model_convert_window.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.c_int64, vp, i32, i32, i32,
+                                               i32, i32, vp, sz, vp]
         if L.vsg_abi_version() != 1:
             raise RuntimeError("visinger_b200: ABI version mismatch between _lib.py and the shared library")
         _lib = L
@@ -563,6 +573,23 @@ class ConvertPack(ModelPack):
 
     def convert_workspace_bytes(self, B: int, T: int, precision: int) -> int:
         return int(lib().vsg_convert_workspace_bytes(self._h, B, T, precision))
+
+    def convert_window_context(self):
+        """(posterior, flow, decoder) context frames each side of a voice-conversion window (vsg_convert_window_context)."""
+        cp, cf, cd = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32()
+        check(lib().vsg_convert_window_context(self._h, ctypes.byref(cp), ctypes.byref(cf), ctypes.byref(cd)),
+              "vsg_convert_window_context")
+        return int(cp.value), int(cf.value), int(cd.value)
+
+    def convert_window_input(self, B: int, T: int, t0: int, t1: int, precision: int):
+        """(s0, s1): the samples of each utterance's row that window [t0, t1) reads (vsg_convert_window_input)."""
+        s0, s1 = ctypes.c_int64(), ctypes.c_int64()
+        check(lib().vsg_convert_window_input(self._h, B, T, t0, t1, precision, ctypes.byref(s0), ctypes.byref(s1)),
+              "vsg_convert_window_input")
+        return int(s0.value), int(s1.value)
+
+    def convert_window_workspace_bytes(self, B: int, T: int, max_frames: int, precision: int) -> int:
+        return int(lib().vsg_convert_window_workspace_bytes(self._h, B, T, max_frames, precision))
 
     def spectrogram(self, wav: torch.Tensor, lengths: torch.Tensor, precision: int) -> torch.Tensor:
         """vsg_spectrogram: wav CUDA fp32 [B, T * hop], lengths CUDA int32 [B] (latent frames) -> fp32 [B, bins, T]."""

@@ -15,6 +15,10 @@ int check_common(const VsgPack* pack, int B, int T, int precision) {
   return VSG_OK;
 }
 
+}  // namespace
+
+namespace vsg {
+
 size_t flow_ws(const VsgPack* p, int B, int T, int prec) {
   if (!p->has_flow) return 0;
   if (prec == VSG_PRECISION_BF16) return flow_ws_bytes_tc(p, B, T, 1);
@@ -25,10 +29,6 @@ size_t dec_ws(const VsgPack* p, int B, int T, int prec) {
   if (!p->has_dec) return 0;
   return prec == VSG_PRECISION_FP32 ? dec_ws_bytes_f32(p, B, T) : dec_ws_bytes_tc(p, B, T, prec == VSG_PRECISION_BF16X3);
 }
-
-}  // namespace
-
-namespace vsg {
 
 // fp32: CUDA-core FFMA kernels.  bf16: tcgen05, one bf16 plane.  bf16x3: tcgen05 on three bf16 planes per value (the
 // flow's z <= 1e-5 needs all 24 mantissa bits of its state; the decoder's 1e-4 is met by two planes).
@@ -280,16 +280,25 @@ namespace {
 
 long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 
+}  // namespace
+
+namespace vsg {
+
+int wavenet_context(int kernel, int dilation_rate, int n_layers) {
+  int r = 0, dil = 1;
+  for (int i = 0; i < n_layers; ++i) {   // WaveNet in_layers: padding (K * dil - dil) / 2; pre / post are 1x1
+    const int span = (kernel - 1) * dil, pad = (kernel * dil - dil) / 2;
+    r += std::max(pad, span - pad);
+    dil *= dilation_rate;
+  }
+  return r;
+}
+
 int flow_context(const VsgPack* p) {
   if (!p->has_flow) return 0;
   const VsgConfig& c = p->cfg;
-  int r = 0, dil = 1;
-  for (int i = 0; i < c.flow_n_layers; ++i) {   // WaveNet in_layers: padding (K * dil - dil) / 2; pre / post are 1x1
-    const int span = (c.flow_kernel_size - 1) * dil, pad = (c.flow_kernel_size * dil - dil) / 2;
-    r += std::max(pad, span - pad);
-    dil *= c.flow_dilation_rate;
-  }
-  return r * c.flow_n_flows;   // each coupling layer widens the field by its WaveNet's reach
+  // each coupling layer widens the field by its WaveNet's reach
+  return wavenet_context(c.flow_kernel_size, c.flow_dilation_rate, c.flow_n_layers) * c.flow_n_flows;
 }
 
 // Walk the receptive field of output frame 0 (samples [0, hop)) back through the decoder's layers, noting at every rate
@@ -328,15 +337,13 @@ int dec_context(const VsgPack* p) {
   return (int)std::max(left, right);
 }
 
-struct WinRange { int fa, fb, da, db; };
-
 int window_needs(const VsgPack* p, int B, int T, int precision, int* need, int* align) {
   *need = 1; *align = 1;
   if (precision == VSG_PRECISION_FP32) return VSG_OK;   // the FFMA kernels choose nothing by length
   return dec_window_needs_tc(p, B, T, precision == VSG_PRECISION_BF16X3, need, align);
 }
 
-int window_ranges(const VsgPack* p, int B, int T, int t0, int t1, int precision, bool flow, WinRange* r) {
+int window_ranges(const VsgPack* p, int B, int T, int t0, int t1, int precision, bool flow, WinRange* r, int Cp) {
   int need, A;
   VSG_TRY(window_needs(p, B, T, precision, &need, &A));
   const int Cd = dec_context(p), Cf = flow ? flow_context(p) : 0;
@@ -347,22 +354,57 @@ int window_ranges(const VsgPack* p, int B, int T, int t0, int t1, int precision,
   }
   r->da = da; r->db = db;
   r->fa = std::max(0, da - Cf); r->fb = std::min(T, db + Cf);
+  r->ga = std::max(0, da - 2 * Cf); r->gb = std::min(T, db + 2 * Cf);
+  r->pa = std::max(0, da - 2 * Cf - Cp); r->pb = std::min(T, db + 2 * Cf + Cp);
   return VSG_OK;
 }
 
-// flow + decoder scratch of windows of up to n frames (0 on invalid arguments); an upper bound of window_ranges' spans
-size_t window_ws(const VsgPack* p, int B, int T, int n, int precision) {
+int window_span(const VsgPack* p, int B, int T, int n, int precision) {
   if (check_common(p, B, T, precision) != VSG_OK || !p->has_dec || n < 1 || T < 1) return 0;
   int need, A;
   if (window_needs(p, B, T, precision, &need, &A) != VSG_OK) return 0;
-  n = std::min(n, T);
-  const int Cd = dec_context(p), Cf = flow_context(p);
-  const int Wd = std::min(T, std::max(n + 2 * Cd + 2 * (A - 1), need + A - 1)), Wf = std::min(T, Wd + 2 * Cf);
+  return std::min(T, std::max(std::min(n, T) + 2 * dec_context(p) + 2 * (A - 1), need + A - 1));
+}
+
+size_t window_ws(const VsgPack* p, int B, int T, int n, int precision) {
+  const int Wd = window_span(p, B, T, n, precision);
+  if (!Wd) return 0;
+  const int Cf = flow_context(p), Wf = std::min(T, Wd + 2 * Cf);
   const size_t dec = precision == VSG_PRECISION_FP32 ? dec_ws_bytes_f32(p, B, Wd)
                                                      : dec_ws_bytes_tc(p, B, Wd, precision == VSG_PRECISION_BF16X3, T);
   const size_t z = p->has_flow ? align256((size_t)B * p->cfg.flow_channels * Wf * sizeof(float)) : 0;
   return z + std::max(flow_ws(p, B, Wf, precision), dec) + 1024;
 }
+
+// vsg_infer_zp_window after validation: z_p and mask hold frames [base, base + ld) of the batch in rows of ld frames
+int zp_window_run(const VsgPack* pack, const float* z_p, const float* mask, int base, int ld, const float* g, float* wav,
+                  int64_t wav_ld, float* z_q_out, int B, int T, int t0, int t1, int precision, Workspace& ws,
+                  cudaStream_t st) {
+  WinRange r;
+  VSG_TRY(window_ranges(pack, B, T, t0, t1, precision, true, &r));
+  const int C = pack->cfg.flow_channels, Tf = r.fb - r.fa;
+  float* z = ws.take<float>((size_t)B * C * Tf);
+  if (ws.overflow) return fail(VSG_ENOMEM, "workspace too small");
+  const size_t mark = ws.off;
+  // z_q = flow(z_p, mask, g, reverse=True) * mask over [fa, fb), read in place from the caller's rows
+  bool masked = true;
+  VSG_TRY(run_flow(pack, z_p + (r.fa - base), mask + (r.fa - base), g, z, B, Tf, 1, precision, ws, st, &masked, nullptr,
+                   nullptr, nullptr, ld));
+  if (!masked) VSG_TRY(mask_mul(z, mask + (r.fa - base), z, B, C, Tf, st, ld));
+  if (z_q_out)
+    VSG_CUDA_TRY(cudaMemcpy2DAsync(z_q_out, (size_t)(t1 - t0) * sizeof(float), z + (t0 - r.fa), (size_t)Tf * sizeof(float),
+                                   (size_t)(t1 - t0) * sizeof(float), (size_t)B * C, cudaMemcpyDeviceToDevice, st));
+  ws.off = mark;
+  // wav = decoder(z_q) over [da, db); its samples of [t0, t1) straight into the caller's rows
+  const DecWin w{T, Tf, (long long)wav_ld, (t0 - r.da) * pack->hop, (t1 - r.da) * pack->hop};
+  const float* zd = z + (r.da - r.fa);
+  if (precision == VSG_PRECISION_FP32) return generator_forward_f32(pack, zd, g, wav, B, r.db - r.da, ws, st, &w);
+  return generator_forward_tc(pack, zd, g, wav, B, r.db - r.da, ws, st, precision == VSG_PRECISION_BF16X3, &w);
+}
+
+}  // namespace vsg
+
+namespace {
 
 int check_window(const VsgPack* pack, const void* in, float* wav, int64_t wav_ld, int B, int T, int t0, int t1,
                  int precision, void* workspace, size_t workspace_bytes) {
@@ -409,29 +451,10 @@ extern "C" int vsg_infer_zp_window(const VsgPack* pack, const float* z_p, const 
   VSG_TRY(check_window(pack, z_p, wav, wav_ld, B, T, t0, t1, precision, workspace, workspace_bytes));
   if (B == 0) return VSG_OK;
   if (!mask) return fail(VSG_EINVAL, "null pointer");
-  WinRange r;
-  VSG_TRY(window_ranges(pack, B, T, t0, t1, precision, true, &r));
   DeviceGuard dg(pack->device);
   if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
-  cudaStream_t st = (cudaStream_t)stream;
-  const int C = pack->cfg.flow_channels, Tf = r.fb - r.fa;
   Workspace ws(workspace, workspace_bytes);
-  float* z = ws.take<float>((size_t)B * C * Tf);
-  if (ws.overflow) return fail(VSG_ENOMEM, "workspace too small");
-  const size_t mark = ws.off;
-  // z_q = flow(z_p, mask, g, reverse=True) * mask over [fa, fb), read in place from the caller's [B, C, T] z_p and mask
-  bool masked = true;
-  VSG_TRY(run_flow(pack, z_p + r.fa, mask + r.fa, g, z, B, Tf, 1, precision, ws, st, &masked, nullptr, nullptr, nullptr, T));
-  if (!masked) VSG_TRY(mask_mul(z, mask + r.fa, z, B, C, Tf, st, T));
-  if (z_q_out)
-    VSG_CUDA_TRY(cudaMemcpy2DAsync(z_q_out, (size_t)(t1 - t0) * sizeof(float), z + (t0 - r.fa), (size_t)Tf * sizeof(float),
-                                   (size_t)(t1 - t0) * sizeof(float), (size_t)B * C, cudaMemcpyDeviceToDevice, st));
-  ws.off = mark;
-  // wav = decoder(z_q) over [da, db); its samples of [t0, t1) straight into the caller's rows
-  const DecWin w{T, Tf, (long long)wav_ld, (t0 - r.da) * pack->hop, (t1 - r.da) * pack->hop};
-  const float* zd = z + (r.da - r.fa);
-  if (precision == VSG_PRECISION_FP32) return generator_forward_f32(pack, zd, g, wav, B, r.db - r.da, ws, st, &w);
-  return generator_forward_tc(pack, zd, g, wav, B, r.db - r.da, ws, st, precision == VSG_PRECISION_BF16X3, &w);
+  return zp_window_run(pack, z_p, mask, 0, T, g, wav, wav_ld, z_q_out, B, T, t0, t1, precision, ws, (cudaStream_t)stream);
 }
 
 extern "C" int vsg_generator_forward_window(const VsgPack* pack, const float* z, const float* g, float* wav, int64_t wav_ld,

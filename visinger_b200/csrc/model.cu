@@ -195,14 +195,15 @@ __device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32
   }
 }
 
+// out [B, C, T] holds frames [t_base, t_base + T) of the noise: element (b, c, t) draws counter (t_base + t, c)
 __global__ void normal_noise_kernel(const unsigned long long* __restrict__ seeds, float* __restrict__ out, int C, int T,
-                                    long long n) {
+                                    long long n, int t_base) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const long long CT = (long long)C * T, b = i / CT, r = i - b * CT;
   const uint32_t c = (uint32_t)(r / T), t = (uint32_t)(r - (long long)c * T);
   const unsigned long long s = seeds[b];
-  uint32_t x[4] = {t, c, 0u, 0u};
+  uint32_t x[4] = {(uint32_t)t_base + t, c, 0u, 0u};
   philox4x32_10(x, (uint32_t)s, (uint32_t)(s >> 32));
   const double u1 = ((double)x[0] + 1.0) * 2.3283064365386963e-10, u2 = (double)x[1] * 2.3283064365386963e-10;
   out[i] = (float)(sqrt(-2.0 * log(u1)) * cos(6.283185307179586 * u2));
@@ -222,9 +223,9 @@ int launch_prep(const long long* mel2ph, float* mask, long long n_mask, const fl
   return VSG_OK;
 }
 
-int launch_noise(const uint64_t* seeds, float* out, int B, int C, int T, cudaStream_t st) {
+int launch_noise(const uint64_t* seeds, float* out, int B, int C, int T, cudaStream_t st, int t_base = 0) {
   const long long n = (long long)B * C * T;
-  normal_noise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const unsigned long long*)seeds, out, C, T, n);
+  normal_noise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const unsigned long long*)seeds, out, C, T, n, t_base);
   VSG_LAUNCH_CHECK("normal_noise_kernel");
   return VSG_OK;
 }
@@ -420,6 +421,93 @@ int model_convert(const VsgPack* P, const float* wav, const float* spec, const i
   VSG_TRY(run_flow(m.hot, z, mask, g_src, z_p, B, T, 0, precision, ws, st));
   ws.off = mark0;
   return infer_zp_run(m.hot, z_p, mask, g_tgt, wav_out, z_out, B, T, precision, ws, st);
+}
+
+// ---- voice conversion over a window of frames -----------------------------------------------------------------------
+// Frames [t0, t1) of model_convert(wav): every part is convolutional, so the ranges of window_ranges nest outward from
+// the decoder's -- flow reverse +-Cf, flow forward +-2 Cf, spectrogram and posterior +-(2 Cf + Cp) -- and each part
+// runs over its range with the one pass's kernels (the tcgen05 sums do not depend on tile or row position, the FFMA
+// kernels choose nothing by length, the decoder's choices come from (B, T): DESIGN.md 4.8, 4.9).
+
+int post_context(const ModelPack& m) {
+  const EncPack& en = m.post->enc;
+  return wavenet_context(en.kernel, en.dil_rate, en.n_layers);
+}
+
+size_t convert_window_ws_bytes(const VsgPack* P, int B, int T, int n, int precision) {
+  const ModelPack& m = *P->model;
+  const VsgPack* hot = m.hot;
+  const EncPack& en = m.post->enc;
+  const int Wd = window_span(hot, B, T, n, precision);
+  if (!Wd) return 0;
+  const int Wg = std::min(T, Wd + 4 * flow_context(hot)), Wp = std::min(T, Wg + 2 * post_context(m));
+  const size_t BP = (size_t)B * Wp, BG = (size_t)B * Wg, H = m.cfg.hidden;
+  const bool bf = convert_bf16(precision);
+  const size_t persist = align256(BP * 4) + align256(BG * 4) + 2 * align256((size_t)B * m.gin * 4) + align256(BP * H * 4) +
+                         align256(BG * H * 4);
+  const size_t keep = (bf ? align256(BP * en.in_pad * 2) : align256(BP * m.spec.bins * 4)) + align256(BP * H * 4) +
+                      align256(BP * 2 * en.out_channels * 4);
+  const size_t post = bf ? posterior_ws_bytes_tc(m.post, B, Wp) : posterior_ws_bytes_f32(m.post, B, Wp);
+  const size_t stage1 = keep + std::max(spec_frames_bytes(m.spec, B, Wp, bf) + 256, post);
+  const size_t rest = std::max(flow_ws(hot, B, Wg, precision), window_ws(hot, B, T, n, precision));
+  return persist + std::max(stage1, rest) + 4096;
+}
+
+int model_convert_window(const VsgPack* P, const float* wav, const int32_t* lengths, const int64_t* src_id,
+                         const float* src_embed, const int64_t* tgt_id, const float* tgt_embed, const float* noise,
+                         const uint64_t* seeds, float* wav_out, int64_t wav_ld, float* z_out, int B, int T, int t0, int t1,
+                         int precision, Workspace& ws, cudaStream_t st) {
+  const ModelPack& m = *P->model;
+  const VsgPack* hot = m.hot;
+  const SpecPack& S = m.spec;
+  const EncPack& en = m.post->enc;
+  const int H = m.cfg.hidden, gin = m.gin;
+  WinRange r;
+  VSG_TRY(window_ranges(hot, B, T, t0, t1, precision, true, &r, post_context(m)));
+  const int Wp = r.pb - r.pa, Wg = r.gb - r.ga;
+  const size_t BP = (size_t)B * Wp, BG = (size_t)B * Wg;
+  const bool bf = convert_bf16(precision);
+  // live for the whole call: the masks of the posterior's and the flow's ranges, the conditions, z and z_p
+  float* mask_p = ws.take<float>(BP);
+  float* mask_g = ws.take<float>(BG);
+  float* g_src = ws.take<float>((size_t)B * gin);
+  float* g_tgt = ws.take<float>((size_t)B * gin);
+  float* z = ws.take<float>(BP * H);
+  float* z_p = ws.take<float>(BG * H);
+  const size_t mark0 = ws.off;
+  // live until the posterior has run
+  __nv_bfloat16* u = bf ? ws.take<__nv_bfloat16>(BP * en.in_pad) : nullptr;
+  float* x = bf ? nullptr : ws.take<float>(BP * S.bins);
+  float* nz = ws.take<float>(BP * H);
+  float* stats = ws.take<float>(BP * 2 * en.out_channels);
+  if (ws.overflow) return fail(VSG_ENOMEM, "convert window workspace too small: need %zu bytes", ws.off);
+
+  VSG_TRY(lengths_mask(lengths, mask_p, B, Wp, st, r.pa, T));
+  VSG_TRY(lengths_mask(lengths, mask_g, B, Wg, st, r.ga, T));
+  VSG_TRY(speaker_cond(m, src_id, src_embed, g_src, B, st));
+  VSG_TRY(speaker_cond(m, tgt_id, tgt_embed, g_tgt, B, st));
+  if (noise)   // the posterior's range of the caller's [B, H, T] noise
+    VSG_CUDA_TRY(cudaMemcpy2DAsync(nz, (size_t)Wp * sizeof(float), noise + r.pa, (size_t)T * sizeof(float),
+                                   (size_t)Wp * sizeof(float), (size_t)B * H, cudaMemcpyDeviceToDevice, st));
+  else
+    VSG_TRY(launch_noise(seeds, nz, B, H, Wp, st, r.pa));
+  // z = posterior_encoder(spectrogram(wav), mask, g_src) over [pa, pb), the rows framed from the caller's wav in place
+  if (bf) {
+    VSG_TRY(spectrogram_tc(P, S, en.in_pad, wav, lengths, mask_p, u, B, Wp, ws, st, r.pa, T));
+    VSG_TRY(posterior_core_tc(m.post, u, mask_p, g_src, nz, z, stats, B, Wp, ws, st));
+  } else {
+    const size_t mark = ws.off;
+    VSG_TRY(spectrogram_f32(S, wav, lengths, mask_p, x, B, Wp, ws, st, r.pa, T));
+    ws.off = mark;
+    VSG_TRY(posterior_forward_f32(m.post, x, mask_p, g_src, nz, z, stats, B, Wp, ws, st));
+  }
+  // z_p = flow(z, mask, g_src) over [ga, gb), read in place from the posterior's rows
+  ws.off = mark0;
+  VSG_TRY(run_flow(hot, z + (r.ga - r.pa), mask_p + (r.ga - r.pa), g_src, z_p, B, Wg, 0, precision, ws, st, nullptr,
+                   nullptr, nullptr, nullptr, Wp));
+  // flow reverse under g_tgt and the decoder: the streaming-synthesis window body on z_p's rows
+  ws.off = mark0;
+  return zp_window_run(hot, z_p, mask_g, r.ga, Wg, g_tgt, wav_out, wav_ld, z_out, B, T, t0, t1, precision, ws, st);
 }
 
 // ---- pack creation --------------------------------------------------------------------------------------------------
@@ -747,6 +835,34 @@ int check_convert(const VsgPack* pack, int B, int T, int precision) {
   return VSG_OK;
 }
 
+// the speaker and noise arguments of vsg_model_convert / vsg_model_convert_window (host ids range-checked)
+int check_convert_inputs(const VsgModelConfig& c, int B, const int64_t* src_spk_id, const float* src_spk_embed,
+                         const int64_t* tgt_spk_id, const float* tgt_spk_embed, const float* noise, const uint64_t* seeds) {
+  if (c.use_spk_id != (src_spk_id != nullptr) || c.use_spk_id != (tgt_spk_id != nullptr))
+    return fail(VSG_EINVAL, c.use_spk_id ? "src_spk_id and tgt_spk_id are required (use_spk_id)"
+                                         : "speaker ids given but the model has no use_spk_id");
+  if (c.use_spk_embed != (src_spk_embed != nullptr) || c.use_spk_embed != (tgt_spk_embed != nullptr))
+    return fail(VSG_EINVAL, c.use_spk_embed ? "src_spk_embed and tgt_spk_embed are required (use_spk_embed)"
+                                            : "speaker embeddings given but the model has no use_spk_embed");
+  if (!noise && !seeds) return fail(VSG_EINVAL, "noise and seeds are both NULL: one of them is required");
+  for (const int64_t* ids : {src_spk_id, tgt_spk_id})
+    if (ids)
+      for (int b = 0; b < B; ++b)
+        if (ids[b] < 0 || ids[b] >= c.num_spk)
+          return fail(VSG_EINVAL, "%s_spk_id[%d] = %lld is outside [0, %d)", ids == src_spk_id ? "src" : "tgt", b,
+                      (long long)ids[b], c.num_spk);
+  return VSG_OK;
+}
+
+// a window [t0, t1) of a (B, T) batch: where the window call's arguments differ from the one-pass call's
+int check_convert_window(const VsgPack* pack, int B, int T, int t0, int t1, int precision) {
+  VSG_TRY(check_convert(pack, B, T, precision));
+  if (t0 < 0 || t1 > T || t0 >= t1) return fail(VSG_EINVAL, "window [%d, %d) is not a non-empty part of [0, %d)", t0, t1, T);
+  WinRange r;   // (a kernel the whole batch chooses with no window form: VSG_EUNSUPPORTED)
+  if (B > 0) VSG_TRY(window_ranges(pack->model->hot, B, T, t0, t1, precision, true, &r, post_context(*pack->model)));
+  return VSG_OK;
+}
+
 }  // namespace
 
 extern "C" int vsg_spectrogram(const VsgPack* pack, const float* wav, const int32_t* lengths, float* spec, int32_t B,
@@ -789,19 +905,7 @@ extern "C" int vsg_model_convert(const VsgPack* pack, const float* wav, const fl
   if ((wav == nullptr) == (spec == nullptr)) return fail(VSG_EINVAL, "give exactly one of wav and spec");
   if (spec && spec_out) return fail(VSG_EINVAL, "spec_out receives the spectrogram of wav: it must be NULL when spec is given");
   if (!lengths || !wav_out) return fail(VSG_EINVAL, "null pointer: lengths and wav_out are required");
-  if (c.use_spk_id != (src_spk_id != nullptr) || c.use_spk_id != (tgt_spk_id != nullptr))
-    return fail(VSG_EINVAL, c.use_spk_id ? "src_spk_id and tgt_spk_id are required (use_spk_id)"
-                                         : "speaker ids given but the model has no use_spk_id");
-  if (c.use_spk_embed != (src_spk_embed != nullptr) || c.use_spk_embed != (tgt_spk_embed != nullptr))
-    return fail(VSG_EINVAL, c.use_spk_embed ? "src_spk_embed and tgt_spk_embed are required (use_spk_embed)"
-                                            : "speaker embeddings given but the model has no use_spk_embed");
-  if (!noise && !seeds) return fail(VSG_EINVAL, "noise and seeds are both NULL: one of them is required");
-  for (const int64_t* ids : {src_spk_id, tgt_spk_id})
-    if (ids)
-      for (int b = 0; b < B; ++b)
-        if (ids[b] < 0 || ids[b] >= c.num_spk)
-          return fail(VSG_EINVAL, "%s_spk_id[%d] = %lld is outside [0, %d)", ids == src_spk_id ? "src" : "tgt", b,
-                      (long long)ids[b], c.num_spk);
+  VSG_TRY(check_convert_inputs(c, B, src_spk_id, src_spk_embed, tgt_spk_id, tgt_spk_embed, noise, seeds));
   const size_t need = convert_ws_bytes(pack, B, T, precision);
   if (!workspace || workspace_bytes < need)
     return fail(VSG_ENOMEM, "workspace of %zu bytes is too small: need %zu", workspace ? workspace_bytes : (size_t)0, need);
@@ -810,4 +914,63 @@ extern "C" int vsg_model_convert(const VsgPack* pack, const float* wav, const fl
   Workspace ws(workspace, workspace_bytes);
   return model_convert(pack, wav, spec, lengths, src_spk_id, src_spk_embed, tgt_spk_id, tgt_spk_embed, noise, seeds,
                        wav_out, spec_out, z_out, B, T, precision, ws, (cudaStream_t)stream);
+}
+
+extern "C" int vsg_convert_window_context(const VsgPack* pack, int32_t* post_frames, int32_t* flow_frames,
+                                          int32_t* dec_frames) {
+  if (!pack || !pack->model || !pack->model->post)
+    return fail(VSG_EINVAL, "pack has no posterior encoder or spectrogram (create it with vsg_convert_pack_create)");
+  if (!post_frames || !flow_frames || !dec_frames) return fail(VSG_EINVAL, "null pointer");
+  *post_frames = post_context(*pack->model);
+  *flow_frames = flow_context(pack->model->hot);
+  *dec_frames = dec_context(pack->model->hot);
+  return VSG_OK;
+}
+
+extern "C" int vsg_convert_window_input(const VsgPack* pack, int32_t B, int32_t T, int32_t t0, int32_t t1,
+                                        int32_t precision, int64_t* s0, int64_t* s1) {
+  VSG_TRY(check_convert_window(pack, B, T, t0, t1, precision));
+  if (!s0 || !s1) return fail(VSG_EINVAL, "null pointer");
+  WinRange r;
+  VSG_TRY(window_ranges(pack->model->hot, std::max(B, 1), T, t0, t1, precision, true, &r, post_context(*pack->model)));
+  // spectrogram frames [pa, pb) read rows pa .. pb + taps - 2, row q holding samples [q * hop + off, (q + 1) * hop + off);
+  // the mask of frames up to pb - 1 is set by samples below pb * hop
+  const SpecPack& S = pack->model->spec;
+  const long long hop = S.hop;
+  *s0 = std::max(0LL, r.pa * hop + S.off);
+  *s1 = std::min((long long)T * hop, std::max(r.pb * hop, (r.pb + S.taps - 1) * hop + S.off));
+  return VSG_OK;
+}
+
+extern "C" size_t vsg_convert_window_workspace_bytes(const VsgPack* pack, int32_t B, int32_t T, int32_t max_frames,
+                                                     int32_t precision) {
+  if (!pack || !pack->model || !pack->model->post || B < 0 || T < 0 || B > 65535) return 0;
+  if (precision != VSG_PRECISION_FP32 && precision != VSG_PRECISION_BF16 && precision != VSG_PRECISION_BF16X3) return 0;
+  return convert_window_ws_bytes(pack, B, T, max_frames, precision);
+}
+
+extern "C" int vsg_model_convert_window(const VsgPack* pack, const float* wav, const int32_t* lengths,
+                                        const int64_t* src_spk_id, const float* src_spk_embed, const int64_t* tgt_spk_id,
+                                        const float* tgt_spk_embed, const float* noise, const uint64_t* seeds,
+                                        float* wav_out, int64_t wav_ld, float* z_out, int32_t B, int32_t T, int32_t t0,
+                                        int32_t t1, int32_t precision, void* workspace, size_t workspace_bytes,
+                                        void* stream) {
+  reset_launch_counts();
+  VSG_TRY(check_convert_window(pack, B, T, t0, t1, precision));
+  if (B == 0) return VSG_OK;
+  if (!wav || !lengths || !wav_out) return fail(VSG_EINVAL, "null pointer: wav, lengths and wav_out are required");
+  const int hop = pack->model->spec.hop;
+  if (wav_ld < (int64_t)(t1 - t0) * hop)
+    return fail(VSG_EINVAL, "wav_ld %lld is shorter than the window's %lld samples", (long long)wav_ld,
+                (long long)(t1 - t0) * hop);
+  VSG_TRY(check_convert_inputs(pack->model->cfg, B, src_spk_id, src_spk_embed, tgt_spk_id, tgt_spk_embed, noise, seeds));
+  const size_t need = convert_window_ws_bytes(pack, B, T, t1 - t0, precision);
+  if (!workspace || workspace_bytes < need)
+    return fail(VSG_ENOMEM, "window workspace of %zu bytes is too small: need %zu", workspace ? workspace_bytes : (size_t)0,
+                need);
+  DeviceGuard dg(pack->device);
+  if (!dg.ok) return fail(VSG_ECUDA, "cannot select device %d", pack->device);
+  Workspace ws(workspace, workspace_bytes);
+  return model_convert_window(pack, wav, lengths, src_spk_id, src_spk_embed, tgt_spk_id, tgt_spk_embed, noise, seeds,
+                              wav_out, wav_ld, z_out, B, T, t0, t1, precision, ws, (cudaStream_t)stream);
 }

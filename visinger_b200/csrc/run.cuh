@@ -86,14 +86,16 @@ int run_flow(const VsgPack* pack, const float* x, const float* mask, const float
              const float* ps_noise = nullptr, bool* sampled = nullptr, int x_ld = 0);
 
 // The linear spectrogram (spec.cuh).  mask [B, T] = t < lengths[b] (lengths clamped to [0, T]).
-int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st);
+// t0, T_len (a window): frames [t0, t0 + T) of a T_len-frame batch; T_len = 0 stands for T.
+int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st, int t0 = 0, int T_len = 0);
 size_t spec_frames_bytes(const SpecPack& S, int B, int T, bool tc);
 // fp32: spec [B, bins, T] on the FFMA kernel (run_f32.cu)
 int spectrogram_f32(const SpecPack& S, const float* wav, const int32_t* lengths, const float* mask, float* spec, int B,
-                    int T, Workspace& ws, cudaStream_t st);
+                    int T, Workspace& ws, cudaStream_t st, int t0 = 0, int T_len = 0);
 // bf16: u [B, T, in_pad] channels-last bf16 (the posterior's `pre` input, pad channels 0) on tcgen05 (run_tc.cu)
 int spectrogram_tc(const VsgPack* P, const SpecPack& S, int in_pad, const float* wav, const int32_t* lengths,
-                   const float* mask, __nv_bfloat16* u, int B, int T, Workspace& ws, cudaStream_t st);
+                   const float* mask, __nv_bfloat16* u, int B, int T, Workspace& ws, cudaStream_t st, int t0 = 0,
+                   int T_len = 0);
 // [B, T, ld] bf16 -> [B, C, T] fp32
 int widen_bf16(const __nv_bfloat16* x, float* y, int B, int C, int ld, int T, cudaStream_t st);
 // the bf16 posterior from its channels-last input u [B, T, in_pad] (posterior_forward_tc after its transpose)
@@ -133,5 +135,28 @@ struct DebugScope {
 // vsg_infer_zp after validation (api.cu): flow reverse from z_p, mask, decoder; shared with vsg_model_forward
 int infer_zp_run(const VsgPack* pack, const float* z_p, const float* mask, const float* g, float* wav, float* z_q_out,
                  int B, int T, int precision, Workspace& ws, cudaStream_t st);
+
+// ---- streaming windows (api.cu) ----
+// Workspace of run_flow over T frames in `prec` (0 without a flow).
+size_t flow_ws(const VsgPack* p, int B, int T, int prec);
+// Receptive fields in latent frames each side (vsg_window_context): a WaveNet's (its in_layers' reach; pre / post 1x1),
+// the flow's (one direction) and the decoder's.
+int wavenet_context(int kernel, int dilation_rate, int n_layers);
+int flow_context(const VsgPack* p);
+int dec_context(const VsgPack* p);
+// The ranges a window [t0, t1) of a (B, T) batch runs each part over, nested outward and clipped to [0, T): decoder
+// [da, db) (widened and aligned for the whole batch's kernel choices), flow reverse [fa, fb) = +-Cf, flow forward
+// [ga, gb) = +-2 Cf, spectrogram and posterior [pa, pb) = +-(2 Cf + Cp).
+struct WinRange { int fa, fb, da, db, ga, gb, pa, pb; };
+int window_ranges(const VsgPack* p, int B, int T, int t0, int t1, int precision, bool flow, WinRange* r, int Cp = 0);
+// Upper bound of db - da over windows of up to n frames (0 on invalid arguments).
+int window_span(const VsgPack* p, int B, int T, int n, int precision);
+// Flow reverse + decoder scratch of windows of up to n frames (vsg_window_workspace_bytes; 0 on invalid arguments).
+size_t window_ws(const VsgPack* p, int B, int T, int n, int precision);
+// Frames [t0, t1) of vsg_infer_zp (vsg_infer_zp_window after validation): z_p and mask hold frames [base, base + ld) of
+// the batch in rows of ld frames (the caller's [B, C, T] buffers: base 0, ld T).  Kernel choices come from (B, T).
+int zp_window_run(const VsgPack* pack, const float* z_p, const float* mask, int base, int ld, const float* g, float* wav,
+                  int64_t wav_ld, float* z_q_out, int B, int T, int t0, int t1, int precision, Workspace& ws,
+                  cudaStream_t st);
 
 }  // namespace vsg

@@ -223,9 +223,9 @@ int posterior_forward_f32(const VsgPack* P, const float* x, const float* mask, c
   return VSG_OK;
 }
 
-int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st) {
+int lengths_mask(const int32_t* lengths, float* mask, int B, int T, cudaStream_t st, int t0, int T_len) {
   const long long n = (long long)B * T;
-  lengths_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(lengths, mask, T, n);
+  lengths_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(lengths, mask, T, t0, T_len ? T_len : T, n);
   VSG_LAUNCH_CHECK("lengths_mask_kernel");
   return VSG_OK;
 }
@@ -238,13 +238,14 @@ size_t spec_frames_bytes(const SpecPack& S, int B, int T, bool tc) {
 
 // spec [B, bins, T] = |STFT| * mask: the framed rows, then Conv1d(hop -> 2 bins, taps) with the magnitude epilogue.
 int spectrogram_f32(const SpecPack& S, const float* wav, const int32_t* lengths, const float* mask, float* spec, int B,
-                    int T, Workspace& ws, cudaStream_t st) {
+                    int T, Workspace& ws, cudaStream_t st, int t0, int T_len) {
   const int R = T + S.taps - 1;
+  if (!T_len) T_len = T;
   float* rows = ws.take<float>((size_t)B * S.hop * R);
   if (ws.overflow) return fail(VSG_ENOMEM, "spectrogram workspace too small: need %zu bytes", ws.off);
   const long long n = (long long)B * S.hop * R;
-  spec_frames_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(wav, lengths, rows, T, R, S.hop, S.hop, S.off,
-                                                                           S.taps, n);
+  spec_frames_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(wav, lengths, rows, T_len, R, S.hop, S.hop, S.off,
+                                                                           S.taps, n, t0, (long long)T_len * S.hop);
   VSG_LAUNCH_CHECK("spec_frames_kernel");
   ConvF32 p = base_conv(S.f32, rows, (long long)S.hop * R, R, R, 0, 1);
   p.Lq = T; p.Lout = T;

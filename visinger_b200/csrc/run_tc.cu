@@ -1291,17 +1291,18 @@ int posterior_core_tc(const VsgPack* P, const __nv_bfloat16* u, const float* mas
 // u [B, T, in_pad] = |STFT| * mask in bf16: the framed rows, then Conv1d(hopP -> 2 in_pad, taps) on tcgen05 with the
 // magnitude epilogue (conv_tc.cuh, EPI_TC_MAG), which also zeroes the pad channels.
 int spectrogram_tc(const VsgPack* P, const SpecPack& S, int in_pad, const float* wav, const int32_t* lengths,
-                   const float* mask, __nv_bfloat16* u, int B, int T, Workspace& ws, cudaStream_t st) {
+                   const float* mask, __nv_bfloat16* u, int B, int T, Workspace& ws, cudaStream_t st, int t0, int T_len) {
   if (!S.tc.has_tmap || S.tc.Cout != 2 * in_pad) return fail(VSG_EUNSUPPORTED, "no tensor-core spectrogram pack");
   const int R = T + S.taps - 1;
+  if (!T_len) T_len = T;
   const size_t mark = ws.off;
   __nv_bfloat16* rows = ws.take<__nv_bfloat16>((size_t)B * R * S.hopP);
   int* err = ws.take<int>(1);
   if (ws.overflow) return fail(VSG_ENOMEM, "spectrogram workspace too small: need %zu bytes", ws.off);
   VSG_CUDA_TRY(cudaMemsetAsync(err, 0, sizeof(int), st));
   const long long n = (long long)B * R * S.hopP;
-  spec_frames_kernel<true><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(wav, lengths, rows, T, R, S.hop, S.hopP, S.off,
-                                                                          S.taps, n);
+  spec_frames_kernel<true><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(wav, lengths, rows, T_len, R, S.hop, S.hopP, S.off,
+                                                                          S.taps, n, t0, (long long)T_len * S.hop);
   VSG_LAUNCH_CHECK("spec_frames_kernel");
   EpiTC e;
   e.mode = EPI_TC_MAG; e.mask = mask; e.out_raw = u; e.mag_ch = S.bins;

@@ -12,13 +12,14 @@
 namespace vsg {
 namespace {   // included by run_f32.cu and run_tc.cu: one private copy each
 
-// mask[b, t] = t < clamp(lengths[b], 0, T)
-__global__ void lengths_mask_kernel(const int32_t* __restrict__ lengths, float* __restrict__ mask, int T, long long n) {
+// mask[b, t] = t0 + t < clamp(lengths[b], 0, T_len), t < T: frames [t0, t0 + T) of a T_len-frame batch
+__global__ void lengths_mask_kernel(const int32_t* __restrict__ lengths, float* __restrict__ mask, int T, int t0, int T_len,
+                                    long long n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const long long b = i / T;
   const int t = (int)(i - b * T);
-  mask[i] = t < min(max(lengths[b], 0), T) ? 1.f : 0.f;
+  mask[i] = t0 + t < min(max(lengths[b], 0), T_len) ? 1.f : 0.f;
 }
 
 // Sample index s of an utterance of L samples, reflected about its own ends as torch's 'reflect' padding does (no edge
@@ -31,12 +32,13 @@ __device__ __forceinline__ long long reflect_index(long long s, long long L) {
   return m < L ? m : per - m;
 }
 
-// Framed rows of every utterance: row r, channel j = wav[b, reflect(r*hop + off + j)] for j < hop and the rows that a
-// valid frame reads (r < len + ktaps - 1, len = clamp(lengths[b], 0, T) frames of len * hop samples); 0 elsewhere.
-// CL: bf16 [B, R, hopP] channels-last (tcgen05 operand), else fp32 [B, hopP, R] (FFMA operand).  wav: [B, T * hop].
+// Framed rows r0 .. r0 + R - 1 of every utterance: row r, channel j = wav[b, reflect(r*hop + off + j)] for j < hop and the
+// rows that a valid frame f >= r0 reads (r < len + ktaps - 1 and r0 < len, len = clamp(lengths[b], 0, T) frames of
+// len * hop samples); 0 elsewhere.  CL: bf16 [B, R, hopP] channels-last (tcgen05 operand), else fp32 [B, hopP, R] (FFMA
+// operand).  wav: [B, T * hop], rows wav_ld samples apart; a window (r0 > 0) reads it in place.
 template <bool CL>
 __global__ void spec_frames_kernel(const float* __restrict__ wav, const int32_t* __restrict__ lengths, void* __restrict__ out,
-                                   int T, int R, int hop, int hopP, int off, int ktaps, long long n) {
+                                   int T, int R, int hop, int hopP, int off, int ktaps, long long n, int r0, long long wav_ld) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   int r, j;
@@ -54,9 +56,9 @@ __global__ void spec_frames_kernel(const float* __restrict__ wav, const int32_t*
   }
   const int len = min(max(lengths[b], 0), T);
   float v = 0.f;
-  if (j < hop && r < len + ktaps - 1) {
+  if (j < hop && r0 + r < len + ktaps - 1 && r0 < len) {
     const long long L = (long long)len * hop;
-    v = wav[b * T * (long long)hop + reflect_index((long long)r * hop + off + j, L)];
+    v = wav[b * wav_ld + reflect_index((long long)(r0 + r) * hop + off + j, L)];
   }
   if (CL) reinterpret_cast<__nv_bfloat16*>(out)[i] = __float2bfloat16(v);
   else reinterpret_cast<float*>(out)[i] = v;

@@ -581,6 +581,63 @@ class VISinger(nn.Module):
         model's configuration requires (ids are read on the host).  The posterior noise is `noise` [B, H, T], else drawn
         on the device from `seeds` (int64 [B]), else from seeds taken from torch's default CPU generator.
         Returns {"wav_out": [B, T * hop], "z": z_hat [B, H, T], "spec": the spectrogram the posterior read}."""
+        pack, a, hosts, B, T = self._convert_inputs(wav, spec, lengths, spk_id, spk_embed, tgt_spk_id, tgt_spk_embed, noise,
+                                                    seeds)
+        dev, H = pack.device, self.hidden_size
+        prec = _lib.precision_code(self.precision)
+        wav_out = torch.empty(B, T * pack.hop, dtype=torch.float32, device=dev)
+        z = torch.empty(B, H, T, dtype=torch.float32, device=dev)
+        spec_out = torch.empty(B, pack.bins, T, dtype=torch.float32, device=dev) if wav is not None else None
+        ptr = lambda k: a[k].data_ptr() if k in a else None   # noqa: E731
+        hptr = lambda k: hosts[k].data_ptr() if k in hosts else None   # noqa: E731
+        with torch.cuda.device(dev):
+            ws = _lib.workspace(dev, pack.convert_workspace_bytes(B, T, prec))
+            rc = _lib.lib().vsg_model_convert(
+                pack.handle, ptr("wav"), ptr("spec"), ptr("lengths"), hptr("spk_id"), ptr("spk_embed"), hptr("tgt_spk_id"),
+                ptr("tgt_spk_embed"), ptr("noise"), ptr("seeds"), wav_out.data_ptr(),
+                spec_out.data_ptr() if spec_out is not None else None, z.data_ptr(), B, T, prec, ws.data_ptr(), ws.numel(),
+                _lib.stream_ptr(dev))
+        _lib.check(rc, "vsg_model_convert")
+        self.last_launches = _lib.last_launch_count()
+        return {"wav_out": wav_out, "z": z, "spec": spec_out if spec_out is not None else spec}
+
+    @torch.no_grad()
+    def voice_conversion_streaming(self, wav, lengths, spk_id=None, spk_embed=None, tgt_spk_id=None, tgt_spk_embed=None,
+                                   noise=None, seeds=None, chunk_frames: int = 250):
+        """`voice_conversion(wav, ...)["wav_out"]` as a stream: a generator of fp32 chunks [B, n * hop] of chunk_frames
+        latent frames each (the last may be shorter), one vsg_model_convert_window call each.  The concatenated chunks
+        equal the one-pass waveform bit for bit, in every precision, and one workspace of
+        `convert_window_workspace_bytes` -- independent of the length -- serves the whole stream.  Inputs are validated as
+        `voice_conversion` validates them; without `noise` and `seeds`, seeds are drawn once up front, so every window
+        draws the one pass's noise.  `wav`, `lengths` and `noise` are read in place: they must stay unchanged until the
+        generator is exhausted."""
+        if chunk_frames < 1:
+            raise RuntimeError("chunk_frames must be >= 1")
+        pack, a, hosts, B, T = self._convert_inputs(wav, None, lengths, spk_id, spk_embed, tgt_spk_id, tgt_spk_embed, noise,
+                                                    seeds)
+        dev, hop = pack.device, pack.hop
+        prec = _lib.precision_code(self.precision)
+        n = min(chunk_frames, T)
+        ptr = lambda k: a[k].data_ptr() if k in a else None   # noqa: E731
+        hptr = lambda k: hosts[k].data_ptr() if k in hosts else None   # noqa: E731
+        ws = torch.empty(max(pack.convert_window_workspace_bytes(B, T, n, prec), 1), dtype=torch.uint8, device=dev) \
+            if T else None
+        for t0 in range(0, T, n):
+            t1 = min(T, t0 + n)
+            out = torch.empty(B, (t1 - t0) * hop, dtype=torch.float32, device=dev)
+            if B:
+                with torch.cuda.device(dev):
+                    rc = _lib.lib().vsg_model_convert_window(
+                        pack.handle, ptr("wav"), ptr("lengths"), hptr("spk_id"), ptr("spk_embed"), hptr("tgt_spk_id"),
+                        ptr("tgt_spk_embed"), ptr("noise"), ptr("seeds"), out.data_ptr(), (t1 - t0) * hop, None, B, T, t0,
+                        t1, prec, ws.data_ptr(), ws.numel(), _lib.stream_ptr(dev))
+                _lib.check(rc, "vsg_model_convert_window")
+                self.last_launches = _lib.last_launch_count()
+            yield out
+
+    def _convert_inputs(self, wav, spec, lengths, spk_id, spk_embed, tgt_spk_id, tgt_spk_embed, noise, seeds):
+        """The checks and conversions of voice_conversion's arguments: (pack, device arguments by name, host speaker ids by
+        name, B, T).  Draws seeds from torch's default CPU generator when neither noise nor seeds is given."""
         hp = self.hparams
         if (wav is None) == (spec is None):
             raise RuntimeError("give exactly one of wav and spec")
@@ -628,22 +685,7 @@ class VISinger(nn.Module):
             ins["seeds"] = torch.randint(0, 2 ** 62, (B,), dtype=torch.int64).to(dev)
         a = {k: v.to(torch.int32).contiguous() if k == "lengths" else v.to(torch.int64).contiguous() if k == "seeds"
              else _lib.as_f32c(v) for k, v in ins.items()}
-        prec = _lib.precision_code(self.precision)
-        wav_out = torch.empty(B, T * pack.hop, dtype=torch.float32, device=dev)
-        z = torch.empty(B, H, T, dtype=torch.float32, device=dev)
-        spec_out = torch.empty(B, pack.bins, T, dtype=torch.float32, device=dev) if wav is not None else None
-        ptr = lambda k: a[k].data_ptr() if k in a else None   # noqa: E731
-        hptr = lambda k: hosts[k].data_ptr() if k in hosts else None   # noqa: E731
-        with torch.cuda.device(dev):
-            ws = _lib.workspace(dev, pack.convert_workspace_bytes(B, T, prec))
-            rc = _lib.lib().vsg_model_convert(
-                pack.handle, ptr("wav"), ptr("spec"), ptr("lengths"), hptr("spk_id"), ptr("spk_embed"), hptr("tgt_spk_id"),
-                ptr("tgt_spk_embed"), ptr("noise"), ptr("seeds"), wav_out.data_ptr(),
-                spec_out.data_ptr() if spec_out is not None else None, z.data_ptr(), B, T, prec, ws.data_ptr(), ws.numel(),
-                _lib.stream_ptr(dev))
-        _lib.check(rc, "vsg_model_convert")
-        self.last_launches = _lib.last_launch_count()
-        return {"wav_out": wav_out, "z": z, "spec": spec_out if spec_out is not None else spec}
+        return pack, a, hosts, B, T
 
     @torch.no_grad()
     def forward_native(self, text_tokens, pitch_tokens, dur_tokens, mel2ph, spk_embed=None, spk_id=None, f0=None, uv=None,
